@@ -313,8 +313,25 @@ def run_reference(args):
 
 
 # ----------------------------------------------------------------------------------------------
-def measure(args, precision, ctx):
-    """Time the head at one precision.  Returns the per-precision part of the JSON line."""
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """One float32 / float64 DIR/<name>.npy per array (what a caller of the timed path receives), at most
+    DUMP_LIMIT_BYTES in all."""
+    arrays = {name: t.detach().cpu().numpy() for name, t in arrays.items()}
+    arrays = {name: a if a.dtype in (np.float32, np.float64) else a.astype(np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure(args, precision, ctx, dump_dir=None):
+    """Time the head at one precision.  Returns the per-precision part of the JSON line.  ``dump_dir``: write the
+    outputs of the last timed step there (rank 0; with N > 1 the 2D joints are rank 0's shard)."""
     import torch.distributed as dist
     import fast_3d_human_pose_estimation_b200 as pkg
     from fast_3d_human_pose_estimation_b200 import synth, dist as cdist, _lib
@@ -334,11 +351,11 @@ def measure(args, precision, ctx):
     def step(f, p):
         if gb is None:
             (kl, kr), xyz = model.head(f, p)
-            return xyz, pkg.mpjpe_sums([kl, kr], xyz, g3, g2l, g2r, vis)
+            return kl, kr, xyz, pkg.mpjpe_sums([kl, kr], xyz, g3, g2l, g2r, vis)
         (kl, kr), xyz = model.head(f, p, out_xyz=gb.xyz_slot)
         pkg.mpjpe_sums([kl, kr], xyz, g3, g2l, g2r, vis, out=gb.sums_slot)
         gb.all_gather()
-        return gb
+        return kl, kr, gb
 
     def barrier():
         if world > 1:
@@ -380,8 +397,11 @@ def measure(args, precision, ctx):
         torch.cuda.synchronize()
         xyz, sums = gb.unpack_host()
         xyz, sums = xyz.clone(), sums.clone()
+        kl, kr = out[:2]
     else:
-        xyz, sums = out
+        kl, kr, xyz, sums = out
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, {"kp_l": kl, "kp_r": kr, "xyz": xyz, "mpjpe_sums": sums})
     e2d, e3d = cdist.mpjpe_from_sums(sums)
 
     # ---- N > 1, outside every timed region: the gathered result of the sharded run against an UNSHARDED recompute —
@@ -1130,7 +1150,7 @@ def run_ours(args):
     ctx["flush"] = torch.empty(256 << 20, dtype=torch.uint8, device=dev)   # > 126 MB L2
 
     ctx["numa_cpus"] = numa_cpus
-    main_res = measure(args, args.precision, ctx)
+    main_res = measure(args, args.precision, ctx, dump_dir=args.dump_outputs)
     other = None
     if args.precision != "bf16" and not args.single_precision:
         other = measure(args, "bf16", ctx)      # the tensor-core configuration, reported alongside
@@ -1246,7 +1266,14 @@ def main():
     ap.add_argument("--no-config5", action="store_true", help="skip the 1024-pair sharded full-pipeline run")
     ap.add_argument("--single-precision", action="store_true",
                     help="fp32 run only: skip the bf16 tensor-core measurement reported alongside")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (2D joints per view, 3D joints, MPJPE sums) as DIR/<name>.npy; "
+                         "the inputs are seeded, so runs with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs dumps the timed GPU path: it needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

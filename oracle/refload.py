@@ -5,7 +5,8 @@ Where it is found, in this order:
   2. ``/root/reference`` — the read-only mount of the build container;
   3. ``baseline/_ref/`` — a verbatim, git-ignored copy of the reference's Python files that
      ``__graft_entry__.build()`` makes while (2) exists, so that the reference can ride to the
-     GPU box next to the built ``.so`` (nothing under it is tracked or edited).
+     GPU box next to the built ``.so`` (nothing under it is tracked or edited);
+  4. ``oracle/_ref/`` — a git-ignored copy of the reference project placed there by hand.
 ``tests/golden/make_golden.py`` / ``make_driver_golden.py``, ``tests/test_reference_drivers.py``,
 ``tests/test_oracle_golden.py`` and ``bench.py --impl reference`` use this; the product package
 never does.
@@ -22,11 +23,12 @@ import types
 
 _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASELINE_REF = os.path.join(_REPO, "baseline", "_ref")
+ORACLE_REF = os.path.join(_REPO, "oracle", "_ref")          # a git-ignored copy of the reference checkout, if one is placed there
 
 
 def _candidates():
     env = os.environ.get("CDR_REFERENCE_ROOT")
-    return ([env] if env else []) + ["/root/reference", BASELINE_REF]
+    return ([env] if env else []) + ["/root/reference", BASELINE_REF, ORACLE_REF]
 
 
 def root():

@@ -1,8 +1,12 @@
-"""CPU: host-side pieces of bench.py that must not break the one JSON line (no GPU needed)."""
+"""Host-side pieces of bench.py that must not break the one JSON line (CPU), and what --dump-outputs writes (GPU)."""
 import importlib.util
 import json
 import os
+import subprocess
+import sys
 import time
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -56,6 +60,61 @@ def test_both_arms_share_one_config():
     c = b.bench_config(64, 1)
     assert c == b.bench_config(64, 1) and c["workload"].startswith("CDRNet head") and "BASELINE configs[1]" in c["workload"]
     assert b.bench_config(64, 8)["parallelism"] == "dp8" and json.dumps(c)
+
+
+def test_dump_outputs_writes_float_npy(tmp_path):
+    """--dump-outputs: one DIR/<name>.npy per output, float32 / float64 kept, anything else widened to float64."""
+    import numpy as np
+    import torch
+    b = _bench()
+    xyz = torch.arange(12, dtype=torch.float32).reshape(1, 4, 3)
+    b.dump_outputs(str(tmp_path / "d"), {"xyz": xyz, "sums": torch.ones(4, dtype=torch.float64),
+                                         "u8": torch.full((2, 2), 7, dtype=torch.uint8)})
+    assert sorted(os.listdir(tmp_path / "d")) == ["sums.npy", "u8.npy", "xyz.npy"]
+    a = np.load(tmp_path / "d" / "xyz.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, xyz.numpy())
+    assert np.load(tmp_path / "d" / "sums.npy").dtype == np.float64
+    u8 = np.load(tmp_path / "d" / "u8.npy")
+    assert u8.dtype == np.float64 and (u8 == 7).all()
+    # more than the limit in all: refused before anything is written
+    big = torch.zeros(b.DUMP_LIMIT_BYTES // 8 + 1, dtype=torch.float64)
+    with pytest.raises(ValueError, match="limit"):
+        b.dump_outputs(str(tmp_path / "big"), {"big": big})
+    assert not (tmp_path / "big").exists()
+    # only the GPU arm is timed with outputs to dump
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs",
+                        str(tmp_path / "r")], capture_output=True, text=True)
+    assert r.returncode != 0 and "--impl ours" in r.stderr and not (tmp_path / "r").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_last_timed_step(cuda_pkg, tmp_path):
+    """bench.py --steps 1 --dump-outputs: the dumped arrays are what CDRNet.head + mpjpe_sums return on the bench's
+    seeded inputs (the same model, weights and batch rebuilt here), bit for bit."""
+    import numpy as np
+    import torch
+    from fast_3d_human_pose_estimation_b200 import synth
+    d = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "1",
+                        "--dump-outputs", str(d), "--single-precision", "--no-cpu-baseline", "--no-stream-microbench",
+                        "--no-full-pipeline", "--no-sustained", "--no-config5"], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 1
+    b = 64
+    m = cuda_pkg.CDRNet(synth.make_cfg(18, 19), precision="fp32")
+    m.load_state_dict(synth.make_head_state_dict(seed=0, calibrated=True), strict=False)
+    m = m.cuda().eval()
+    feats = [f.cuda() for f in synth.make_features(b, seed=1)]
+    cams = synth.make_cameras(b, seed=2)
+    gt = synth.make_gt(cams, seed=3)
+    Ps = [torch.from_numpy(cams["P_l"]).cuda(), torch.from_numpy(cams["P_r"]).cuda()]
+    (kl, kr), xyz = m.head(feats, Ps)
+    g = [torch.from_numpy(gt[k]).cuda() for k in ("gt3d", "gt2d_l", "gt2d_r", "vis")]
+    sums = cuda_pkg.mpjpe_sums([kl, kr], xyz, *g)
+    got = {n: np.load(d / (n + ".npy")) for n in ("kp_l", "kp_r", "xyz", "mpjpe_sums")}
+    assert got["xyz"].dtype == np.float32 and got["mpjpe_sums"].dtype == np.float64
+    for n, want in (("kp_l", kl), ("kp_r", kr), ("xyz", xyz), ("mpjpe_sums", sums)):
+        assert np.array_equal(got[n], want.cpu().numpy()), n
 
 
 def test_peaks_and_constants():

@@ -1,5 +1,8 @@
 """SURVEY §8f rank 3, first slice: forward + backward of soft-argmax, DLT and FTL on libcdrhead.so against
 torch autograd through the fp64 oracle (oracle/cdr_oracle.py restates models/cdrnet.py:45-56,120-179)."""
+import json
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -298,13 +301,14 @@ def test_training_step_vs_the_reference_model(cuda_pkg):
     reference CDRNet + its MPJPELoss in train mode on this GPU (fp32, TF32 off) against CDRNet(trainable=True) +
     this package's MPJPELoss: the head's BatchNorm / ReLU, pinv, FTL, soft-argmax, DLT and the loss run forward and
     backward on libcdrhead, the convolutions on cuDNN in both.  Loss, the script's grad_norm, the gradient direction of
-    parameters all over the network and the BatchNorm running statistics after the step."""
+    parameters all over the network and the BatchNorm running statistics after the step.  Where the reference's
+    sources are absent: loss and grad_norm against the reference's recorded ones (tests/golden/reference_recorded.json)."""
     from oracle import refload
-    if not refload.available():
-        pytest.skip("reference sources not present")
-    ref = refload.load()
-    import importlib
-    ref_loss = importlib.import_module("models.loss")
+    live = refload.available()
+    if live:
+        ref = refload.load()
+        import importlib
+        ref_loss = importlib.import_module("models.loss")
     tf32 = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
     torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
     try:
@@ -313,9 +317,11 @@ def test_training_step_vs_the_reference_model(cuda_pkg):
         ours = cuda_pkg.CDRNet(cfg, trainable=True)
         with torch.no_grad():
             ours.decoder.final_layer.weight.mul_(10.0)     # train-mode BN keeps activations O(1): peaky heat-maps need gain
-        theirs = ref.CDRNet(cfg)
-        theirs.load_state_dict(ours.state_dict())
-        ours, theirs = ours.cuda().train(), theirs.cuda().train()
+        ours = ours.cuda().train()
+        if live:
+            theirs = ref.CDRNet(cfg)
+            theirs.load_state_dict(ours.state_dict())
+            theirs = theirs.cuda().train()
         imgs = [x.cuda() for x in synth.make_images(b, seed=1)]
         cams = synth.make_cameras(b, seed=2)
         gt = synth.make_gt(cams, seed=3)
@@ -332,6 +338,15 @@ def test_training_step_vs_the_reference_model(cuda_pkg):
             loss.backward()                                                       # :127
             grads = {n: p.grad.detach().clone() for n, p in model.named_parameters() if p.grad is not None}
             return float(loss), float(torch.norm(torch.cat([g.flatten() for g in grads.values()]))), grads, pred_3ds   # :129-130
+        if not live:
+            rec = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "reference_recorded.json")))
+            l_t, gn_t = rec["training_step"]["loss"], rec["training_step"]["grad_norm"]
+            l_o, gn_o, g_o, xyz = step(ours, cuda_pkg.MPJPELoss(True))
+            print(f"\ntraining step: loss {l_o:.6f} vs reference (recorded) {l_t}; grad_norm {gn_o:.6e} vs {gn_t:.6e}")
+            assert abs(l_o - l_t) <= 1e-4 * abs(l_t)
+            assert abs(gn_o - gn_t) <= 2e-2 * gn_t
+            assert bool(torch.isfinite(xyz).all()) and all(bool(torch.isfinite(g).all()) for g in g_o.values())
+            return
         l_t, gn_t, g_t, _ = step(theirs, ref_loss.MPJPELoss(True))
         l_o, gn_o, g_o, xyz = step(ours, cuda_pkg.MPJPELoss(True))
         print(f"\ntraining step: loss {l_o:.6f} vs reference {l_t:.6f}; grad_norm {gn_o:.6e} vs {gn_t:.6e}")

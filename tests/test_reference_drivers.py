@@ -169,3 +169,86 @@ def test_baseline_driver_with_dropin(cuda_pkg, drivers, dgolden, tmp_path, monke
     g2r = synth._project(pose, meta["cam_right"]["intrinsics"], meta["cam_right"]["rotation"], meta["cam_right"]["translation"])
     want_err = ref.calc_mpjpe([ours["u8_l"], ours["u8_r"]], want3, pose, g2l, g2r, vis)
     assert abs(ours["err"][1] - want_err[1]) <= TOL_MPJPE_MM and abs(ours["err"][0] - want_err[0]) <= TOL_2D_PX
+
+
+# The same comparisons with the reference's stored outputs where its sources are absent: the drivers' glue
+# (ToTensor + Normalize, P = K [R|t], visibility mask, MPJPE) is this library's own (mads.py, geometry.py) and the
+# fp64 oracle's, and the checkpoint is the same seeded init the golden was made with (synth.make_cfg holds the
+# two values of configs/mads_3d.yaml / mads_2d.yaml the models read).
+
+@pytest.fixture
+def no_tf32(monkeypatch):
+    monkeypatch.setattr(torch.backends.cudnn, "allow_tf32", False)
+    monkeypatch.setattr(torch.backends.cuda.matmul, "allow_tf32", False)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("enc", ["torch", "fp32"])
+def test_cdrnet_estimate_matches_driver_golden(cuda_pkg, dgolden, no_tf32, enc):
+    """CDRNetInferencer.estimate's arithmetic (inference.py:70-101) through mads.evaluate_sequence on the driver's
+    frame: 2D / 3D / MPJPE inside the flat tolerances of the reference's own CPU output."""
+    from fast_3d_human_pose_estimation_b200 import mads, synth
+    cfg = synth.make_cfg(101, 19)
+    m = cuda_pkg.CDRNet(cfg, encoder_precision=enc)
+    m.load_state_dict(RD.seeded_state_dict(cuda_pkg.CDRNet, cfg))
+    m = m.cuda().eval()
+    cuda_pkg._lib.lib().cdr_launch_count_reset()
+    got = mads.evaluate_sequence(m, [RD.driver_case()], batch=1)
+    assert cuda_pkg._lib.lib().cdr_launch_count() > 0
+    g = dgolden
+    d2 = max(np.abs(got["pred_2d"][0, 0] - g["cdrnet.kp_l"]).max(), np.abs(got["pred_2d"][1, 0] - g["cdrnet.kp_r"]).max())
+    d3 = np.abs(got["pred_3d"][0] - g["cdrnet.xyz"]).max()
+    print(f"\nCDRNet [encoder {enc}] vs reference driver golden: d2D={d2:.2e}px d3D={d3:.2e}mm "
+          f"MPJPE ({got['mpjpe_2d']:.6f}, {got['mpjpe_3d']:.6f}) vs {g['cdrnet.err']}")
+    assert got["pred_2d"].dtype == np.float32 and got["pred_3d"].shape == (1, 19, 3)
+    assert d2 <= TOL_2D_PX and d3 <= TOL_3D_MM
+    assert abs(got["mpjpe_3d"] - g["cdrnet.err"][1]) <= TOL_MPJPE_MM
+    assert abs(got["mpjpe_2d"] - g["cdrnet.err"][0]) <= TOL_2D_PX
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("enc", ["torch", "fp32"])
+def test_baseline_estimate_matches_driver_golden(cuda_pkg, dgolden, no_tf32, enc):
+    """BaseLine.inference / estimate's arithmetic (baseline.py:45-103) on this library: PoseResNet -> arg-max x4 ->
+    uint8 -> triangulation -> MPJPE, against the reference's stored key points under the same tie rule as
+    test_baseline_driver_with_dropin, and against the fp64 oracle's triangulation / MPJPE on our key points."""
+    from fast_3d_human_pose_estimation_b200 import synth
+    from fast_3d_human_pose_estimation_b200.encoder import IMAGENET_MEAN, IMAGENET_STD
+    from oracle import cdr_oracle as O
+    cfg = synth.make_cfg(101, 19)
+    m = cuda_pkg.PoseResNet(cfg, encoder_precision=enc)
+    m.load_state_dict(RD.seeded_state_dict(cuda_pkg.PoseResNet, cfg))
+    m = m.cuda().eval()
+    img_l, img_r, meta = RD.driver_case()
+    mean = torch.tensor(IMAGENET_MEAN).view(1, 3, 1, 1)
+    std = torch.tensor(IMAGENET_STD).view(1, 3, 1, 1)
+    x = torch.cat([torch.from_numpy(i[None]).permute(0, 3, 1, 2).float().div(255).sub(mean).div(std)
+                   for i in (img_l, img_r)]).cuda()                          # the driver's ToTensor + Normalize
+    with torch.no_grad():
+        u8 = cuda_pkg.baseline_keypoints(m(x)).cpu().numpy()
+    PL, PR = (O.get_projection_matrix(meta[c]["intrinsics"], meta[c]["rotation"], meta[c]["translation"])
+              for c in ("cam_left", "cam_right"))
+    xyz = cuda_pkg.triangulation(PL, PR, u8[0], u8[1])
+    # the targets as the driver builds them (the same lines as test_baseline_driver_with_dropin)
+    pose = np.array(meta["pose_3d"]); mask = np.isnan(pose); pose[mask] = 0
+    vis = np.ones_like(pose); vis[mask] = 0
+    vis = np.logical_and.reduce(vis, axis=1, keepdims=True)
+    g2l = synth._project(pose, meta["cam_left"]["intrinsics"], meta["cam_left"]["rotation"], meta["cam_left"]["translation"])
+    g2r = synth._project(pose, meta["cam_right"]["intrinsics"], meta["cam_right"]["rotation"], meta["cam_right"]["translation"])
+    err = cuda_pkg.calc_mpjpe([u8[0], u8[1]], xyz, pose, g2l, g2r, vis)
+    g = dgolden
+    assert u8.dtype == np.uint8 and u8.shape == (2, 19, 2)
+    decisive = g["baseline.top2_gap"] > 1e-4 * g["baseline.heat_absmax"]          # (view, joint)
+    same = np.stack([(u8[0] == g["baseline.u8_l"]).all(-1), (u8[1] == g["baseline.u8_r"]).all(-1)])
+    print(f"\nPoseResNet [encoder {enc}] vs reference driver golden: key points identical {int(same.sum())}/38 "
+          f"(decisive {int(decisive.sum())}), err {err} vs {g['baseline.err']}")
+    assert same[decisive].all()
+    both = same.all(0)
+    assert both.sum() >= 5
+    np.testing.assert_allclose(xyz[both], g["baseline.xyz"][both], rtol=0, atol=TOL_3D_MM)
+    want3 = O.triangulation(PL, PR, u8[0], u8[1])
+    np.testing.assert_allclose(xyz, want3, rtol=0, atol=TOL_3D_MM)
+    want_err = O.calc_mpjpe([u8[0], u8[1]], want3, pose, g2l, g2r, vis)
+    assert abs(err[1] - want_err[1]) <= TOL_MPJPE_MM and abs(err[0] - want_err[0]) <= TOL_2D_PX
+    if same.all():                      # every key point the reference's: its stored estimate() errors too
+        assert abs(err[1] - g["baseline.err"][1]) <= TOL_MPJPE_MM and abs(err[0] - g["baseline.err"][0]) <= TOL_2D_PX
