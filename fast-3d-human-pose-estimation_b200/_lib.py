@@ -119,6 +119,9 @@ _SIGNATURES = {
     "cdr_mpjpe_reduce": (C.c_int, [_vp, C.c_longlong, C.c_int, _vp, _vp, _vp]),
     "cdr_softargmax_backward": (C.c_int, [_vp, _vp, C.c_longlong, C.c_int, C.c_int, C.c_float, _vp, _vp]),
     "cdr_dlt_backward": (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp, _vp, _vp]),
+    "cdr_deconv_train_workspace_bytes": (C.c_int, [C.c_int] * 5 + [C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
+    "cdr_deconv_train_forward": (C.c_int, [_vp, _vp] + [C.c_int] * 5 + [_vp, _vp, C.c_size_t, _vp, C.c_size_t, _vp]),
+    "cdr_deconv_train_backward": (C.c_int, [_vp, _vp, _vp] + [C.c_int] * 5 + [_vp, _vp, _vp, C.c_size_t, _vp]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

@@ -11,9 +11,15 @@ script can swap them in one call at a time:
     z   = ftl(feat, mats)                             # == CanonicalFusion.ftl(feat, mats)
 
 Projection matrices carry no gradient (they are data in the reference).  CUDA fp32 only; no fallback.
-The convolutions / train-mode BatchNorm of a training step stay torch modules — out of this slice.
+
+The decoder's transposed convolutions have one too, forward and backward on the f16x2 tensor-core GEMM at fp32
+accuracy (independent of torch's TF32 flags):
+
+    y = conv_transpose2d(x, weight)                   # == F.conv_transpose2d(x, weight, stride=2, padding=1)
 """
 from __future__ import annotations
+
+import ctypes as C
 
 import torch
 
@@ -126,3 +132,72 @@ def dlt(P_l, P_r, kp_l, kp_r):
 def ftl(x, mats):
     """CanonicalFusion.ftl on NCHW: x (B, K*blk, H, W), mats (B, R, K) -> (B, R*blk, H, W)."""
     return _FTL.apply(x, mats)
+
+
+def _deconv_args(x, weight):
+    """Checks of conv_transpose2d's inputs, all before any CUDA call: ValueError, there is no fallback."""
+    if not (isinstance(x, torch.Tensor) and isinstance(weight, torch.Tensor)):
+        raise ValueError("conv_transpose2d: x and weight must be tensors")
+    if x.dim() != 4 or weight.dim() != 4 or tuple(weight.shape[2:]) != (4, 4) or weight.shape[0] != x.shape[1]:
+        raise ValueError(f"conv_transpose2d: x (N, Cin, H, W) and weight (Cin, Cout, 4, 4) expected, got "
+                         f"{tuple(x.shape)} and {tuple(weight.shape)}")
+    n, cin, h, w = x.shape
+    cout = weight.shape[1]
+    if n < 1 or cin % 64 or cout % 64 or h != w or h not in (8, 16, 32):
+        raise ValueError(f"conv_transpose2d: unsupported shape x {tuple(x.shape)}, weight {tuple(weight.shape)} "
+                         "(Cin and Cout multiples of 64, H == W in {8, 16, 32})")
+    if x.dtype != torch.float32 or weight.dtype != torch.float32:
+        raise ValueError(f"conv_transpose2d: float32 expected, got {x.dtype} and {weight.dtype}")
+    if not (x.is_cuda and weight.is_cuda) or x.device != weight.device:
+        raise ValueError("conv_transpose2d: x and weight must be CUDA tensors on one device (there is no CPU fallback)")
+    return x.contiguous(), weight.contiguous()
+
+
+class _ConvTranspose2d(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, weight):
+        x, weight = _deconv_args(x, weight)
+        n, cin, h, w = x.shape
+        cout = weight.shape[1]
+        L = _lib.lib()
+        saved_b, ws_b = C.c_size_t(), C.c_size_t()
+        _lib.check(L.cdr_deconv_train_workspace_bytes(n, cin, cout, h, w, C.byref(saved_b), C.byref(ws_b)))
+        dev = x.device
+        y = torch.empty((n, cout, 2 * h, 2 * w), dtype=torch.float32, device=dev)
+        saved = torch.empty(saved_b.value, dtype=torch.uint8, device=dev)     # x as fp16 planes, for the weight gradient
+        ws = torch.empty(ws_b.value, dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(L.cdr_deconv_train_forward(_lib.ptr(x), _lib.ptr(weight), n, cin, cout, h, w, _lib.ptr(y),
+                                                  _lib.ptr(saved), saved_b.value, _lib.ptr(ws), ws_b.value,
+                                                  _lib.current_stream_ptr(dev)))
+        ctx.save_for_backward(saved, weight)
+        ctx.dims = (n, cin, cout, h, w)
+        ctx.ws_bytes = ws_b.value
+        return y
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_y):
+        saved, weight = ctx.saved_tensors
+        n, cin, cout, h, w = ctx.dims
+        need_x, need_w = ctx.needs_input_grad[:2]
+        if not (need_x or need_w):
+            return None, None
+        dy = _chk(grad_y, "conv_transpose2d: grad")
+        dev = dy.device
+        dx = torch.empty((n, cin, h, w), dtype=torch.float32, device=dev) if need_x else None
+        dw = torch.empty((cin, cout, 4, 4), dtype=torch.float32, device=dev) if need_w else None
+        ws = torch.empty(ctx.ws_bytes, dtype=torch.uint8, device=dev)
+        L = _lib.lib()
+        with torch.cuda.device(dev):
+            _lib.check(L.cdr_deconv_train_backward(_lib.ptr(saved), _lib.ptr(weight), _lib.ptr(dy), n, cin, cout, h, w,
+                                                   _lib.ptr(dx), _lib.ptr(dw), _lib.ptr(ws), ctx.ws_bytes,
+                                                   _lib.current_stream_ptr(dev)))
+        return dx, dw
+
+
+def conv_transpose2d(x, weight):
+    """F.conv_transpose2d(x, weight, stride=2, padding=1) for 4x4 kernels without bias, forward and backward on
+    libcdrhead at fp32 accuracy.  x (N, Cin, H, W), weight (Cin, Cout, 4, 4): CUDA float32, Cin and Cout multiples
+    of 64, H == W in {8, 16, 32}; anything else raises ValueError."""
+    return _ConvTranspose2d.apply(x, weight)

@@ -656,3 +656,51 @@ extern "C" int cdr_joint_loss_backward(int kind, const float* pred, const float*
   return launch_joint_loss_backward(kind, pred, target, weight, rows, d, threshold, grad_loss, grad_pred,
                                     (cudaStream_t)stream);
 }
+
+// ------------------------------------------------------------------------------------------
+// Training the decoder's transposed convolutions (gemm_tc.cu: tc_deconv_train_*)
+static int deconv_train_shape(const char* fn, int n, int cin, int cout, int h, int w) {
+  CDR_CHECK_ARG(n > 0 && cin > 0 && cout > 0 && h > 0 && w > 0, "%s: bad shape n=%d cin=%d cout=%d h=%d w=%d", fn, n, cin,
+                cout, h, w);
+  if (cin % 64 != 0 || cout % 64 != 0 || h != w || (w != 8 && w != 16 && w != 32)) {
+    set_error("%s: unsupported shape cin=%d cout=%d h=%d w=%d (channels multiples of 64, h == w in {8, 16, 32})", fn,
+              cin, cout, h, w);
+    return CDR_ERR_UNSUPPORTED;
+  }
+  return CDR_OK;
+}
+static bool al16(const void* p) { return ((uintptr_t)p & 15) == 0; }
+extern "C" int cdr_deconv_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes,
+                                                size_t* workspace_bytes) {
+  CDR_CHECK_ARG(saved_bytes && workspace_bytes, "cdr_deconv_train_workspace_bytes: null pointer");
+  if (int rc = deconv_train_shape("cdr_deconv_train_workspace_bytes", n, cin, cout, h, w)) return rc;
+  *saved_bytes = deconv_train_saved_bytes(n, cin, cout, h, w);
+  *workspace_bytes = deconv_train_workspace_bytes(n, cin, cout, h, w);
+  return CDR_OK;
+}
+extern "C" int cdr_deconv_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w,
+                                        float* y, void* saved, size_t saved_bytes, void* workspace,
+                                        size_t workspace_bytes, void* stream) {
+  CDR_CHECK_ARG(x && weight && y && saved && workspace, "cdr_deconv_train_forward: null pointer");
+  if (int rc = deconv_train_shape("cdr_deconv_train_forward", n, cin, cout, h, w)) return rc;
+  CDR_CHECK_ARG(al16(x) && al16(weight) && al16(y) && ((uintptr_t)saved & 255) == 0 && ((uintptr_t)workspace & 255) == 0,
+                "cdr_deconv_train_forward: tensors must be 16-byte, saved / workspace 256-byte aligned");
+  if (saved_bytes < deconv_train_saved_bytes(n, cin, cout, h, w)) {
+    set_error("cdr_deconv_train_forward: saved %zu < required %zu bytes", saved_bytes,
+              deconv_train_saved_bytes(n, cin, cout, h, w));
+    return CDR_ERR_WORKSPACE;
+  }
+  return tc_deconv_train_forward(x, weight, n, cin, cout, h, w, y, saved, workspace, workspace_bytes,
+                                 (cudaStream_t)stream);
+}
+extern "C" int cdr_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin,
+                                         int cout, int h, int w, float* dx, float* dweight, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
+  CDR_CHECK_ARG(saved && weight && dy && workspace, "cdr_deconv_train_backward: null pointer");
+  if (int rc = deconv_train_shape("cdr_deconv_train_backward", n, cin, cout, h, w)) return rc;
+  CDR_CHECK_ARG(al16(weight) && al16(dy) && al16(dx) && al16(dweight) && ((uintptr_t)saved & 255) == 0 &&
+                    ((uintptr_t)workspace & 255) == 0,
+                "cdr_deconv_train_backward: tensors must be 16-byte, saved / workspace 256-byte aligned");
+  return tc_deconv_train_backward(saved, weight, dy, n, cin, cout, h, w, dx, dweight, workspace, workspace_bytes,
+                                  (cudaStream_t)stream);
+}

@@ -118,7 +118,8 @@ constexpr int kStageBufBytes = 32 * 128;         // TMA-store staging per epilog
 //                ITS producer with atomicMax), so nothing can overflow fp16 and one layer of bound
 //                looseness (~2^7) is far inside the format's 2^27 full-precision window.
 enum TcKind { kKindBF16 = 0, kKindTF32X3 = 1, kKindF16X2 = 2 };
-enum TapMode { kTapNone = 0, kTapDeconv = 1, kTapConv3 = 2 };
+// kTapConv4s2: 4x4 stride-2 pad-1 conv (16 taps), the data gradient of a k4 s2 p1 transposed conv (deconv_train_backward)
+enum TapMode { kTapNone = 0, kTapDeconv = 1, kTapConv3 = 2, kTapConv4s2 = 3 };
 template <int KIND> struct KindTraits;
 template <> struct KindTraits<kKindBF16>   { static constexpr int kElem = 2, kBK = 64, kPlanes = 1, kFmt = kFmtBF16; };
 template <> struct KindTraits<kKindTF32X3> { static constexpr int kElem = 4, kBK = 32, kPlanes = 2, kFmt = kFmtTF32P; };
@@ -162,7 +163,8 @@ struct TcGemmParams {
   int cin;                // K per tap
   int ntaps;              // 1 or 4
   int a4d;                // 1: A through the 4-D NHWC map (shifted / strided taps), 0: 2-D (rows, channels)
-  int tap_mode;           // kTapNone: 1 tap; kTapDeconv: 4 taps of output phase g; kTapConv3: 9 taps (3x3, pad 1)
+  int tap_mode;           // kTapNone: 1 tap; kTapDeconv: 4 taps of output phase g; kTapConv3: 9 taps (3x3, pad 1);
+                          // kTapConv4s2: 16 taps (4x4, stride 2, pad 1)
   int stride;             // 4-D A: input pixel = stride * output pixel + tap shift (map carries the element stride)
   int has_res;            // residual tensor (rows like C, same format) added before the ReLU: its 128 x 128 tile travels
                           // through the operand ring as one extra stage per tile (BN = 128; bf16, or f16x2 hi/lo planes)
@@ -192,6 +194,7 @@ struct TcGemmParams {
   int c_pitch, c_fill;
   int relu;
   int out_mode;           // kOutRows / kOutDeconv or kOutPlanar (fp32)
+  int planar_deconv;      // kOutPlanar of a kTapDeconv launch: output phase g scattered to (2y + g/2, 2x + g%2) of a 2H x 2W map
   int split_store;        // kOutRows + kFmtF16P: planes leave as two 16-row boxes through the two halves of the staging buffer
   int num_tiles;
 };
@@ -266,6 +269,14 @@ __device__ __forceinline__ void store_slab(const TcGemmParams& p, const float (&
   if (!row_ok) return;
   if (p.out_mode == kOutPlanar) {
     float* __restrict__ C = reinterpret_cast<float*>(p.C);
+    if (p.planar_deconv) {
+      const int y = pix / p.W, x = pix - y * p.W;
+      const size_t o = (size_t)(2 * y + (g >> 1)) * (2 * p.W) + 2 * x + (g & 1);
+#pragma unroll
+      for (int j = 0; j < 32; ++j)
+        if (n0c + j < p.n) C[((size_t)img * p.n + n0c + j) * (4 * HW) + o] = v[j];
+      return;
+    }
 #pragma unroll
     for (int j = 0; j < 32; ++j)
       if (n0c + j < p.n) C[((size_t)img * p.n + n0c + j) * HW + pix] = v[j];
@@ -402,7 +413,16 @@ constexpr int kSplitChunk = CDR_SPLIT_CHUNK;
 // TMA loads count their bytes on it (cp.async.bulk.tensor.cta_group::2); stage release, chunk / tile completion are
 // multicast commits to both CTAs' barriers; "accumulator drained" arrivals of the peer's epilogue warps go to the
 // leader's barriers through the cluster window (mapa + mbarrier.arrive.shared::cluster).
-template <int BN, int KIND, int OFMT, int CL>
+//
+// kMN (f16x2, BN = 128, CL = 0): the weight gradient of a k4 s2 p1 transposed conv (deconv_train_backward).  One tile =
+// 128 input channels ci (M) x 128 output channels co (N) of one tap (ky, kx) and one K slice; K = the pixels of x.
+// Both operands are read straight from the pixel-major fp16 planes, so they are MN-major (channels contiguous): A = x,
+// two 64-channel x 64-pixel boxes; B = dy, the same 64 pixels in the same (img, y, x) order through the stride-2 box
+// shifted by (kx - 1, ky - 1).  The UMMA descriptors carry the MN-major SWIZZLE_128B layout (LBO = the 8 KB between
+// the two 64-channel halves, SBO = 1024 B between 8-pixel groups) and the instruction descriptor the transpose bits.
+// The epilogue stores the raw fp32 tile (still times s_x * s_dy) into the slice's partial; wgrad_reduce_kernel sums
+// the slices in a fixed order.
+template <int BN, int KIND, int OFMT, int CL, bool kMN = false>
 __global__ void __launch_bounds__(TcCfg<BN, KIND, OFMT, CL>::kThreads, 1)
 tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_a_lo,
                    const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_b_lo,
@@ -418,6 +438,7 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
   constexpr bool kSplit = KIND != kKindBF16;
   constexpr bool kPair2 = CL == 2;
   static_assert(!kPair2 || KIND != kKindTF32X3, "cta_group::2 is wired for the kind::f16 operand kinds");
+  static_assert(!kMN || (KIND == kKindF16X2 && BN == 128 && CL == 0), "MN-major operands: f16x2, BN = 128, one CTA per tile");
 #ifdef CDR_EXP_NO_LO
   constexpr bool kLoadLo = false;   // timing experiment: hi planes only
 #else
@@ -537,12 +558,34 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
             dy = py - (tap >> 1); dx = px - (tap & 1);
           } else if (p.tap_mode == kTapConv3) {
             dy = tap / 3 - 1; dx = tap - (tap / 3) * 3 - 1;
+          } else if (p.tap_mode == kTapConv4s2) {
+            dy = (tap >> 2) - 1; dx = (tap & 3) - 1;
           }
           const int ys = p.stride * y0 + dy;
           const int arow = g * p.a_group_rows + m0;
           const int bk = tap * p.cin + k0;
           const int brow = g * p.b_group_rows + n_tile * BN + (kPair2 ? (int)cta_rank * (BN / 2) : 0);   // CL = 2: my half of B
-          if constexpr (kPair2) {
+          if constexpr (kMN) {
+            // wgrad: g = slice * 16 + (ky * 4 + kx); 64 pixels of x from k0 of the slice (p.cin pixels per slice; a block
+            // is whole rows of one image since W | 64 | H*W) and the dy pixels (2y - 1 + ky, 2x - 1 + kx) they pair with
+            const int wt = g & 15, pix0 = (g >> 4) * p.cin + k0;
+            const int wimg = pix0 / HW, wy = (pix0 - wimg * HW) / p.W;
+            const int co0 = n_tile * BN;
+            if (ptx::elect_one()) {
+              ptx::mbar_arrive_expect_tx(&full[s], Cfg::kStageBytes);
+#pragma unroll
+              for (int pl = 0; pl < 2; ++pl) {
+                const CUtensorMap* ma = pl ? &tmap_a_lo : &tmap_a;
+                const CUtensorMap* mb = pl ? &tmap_b_lo : &tmap_b;
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                  ptx::tma_load_2d(stage_a(s, pl) + h * (kABytes / 2), ma, &full[s], m0 + 64 * h, pix0);
+                  ptx::tma_load_4d(stage_b(s, pl) + h * (Cfg::kBBytes / 2), mb, &full[s], co0 + 64 * h, (wt & 3) - 1,
+                                   2 * wy + (wt >> 2) - 1, wimg);
+                }
+              }
+            }
+          } else if constexpr (kPair2) {
             // both CTAs count their bytes on the LEADER's barrier of this stage; the leader expects the sum
             const uint32_t full_leader = ptx::mapa_u32(ptx::smem_u32(&full[s]), 0);
             if (ptx::elect_one()) {
@@ -627,8 +670,9 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
       // instruction descriptor: D=f32, A/B format (kind::f16: 0 = f16, 1 = bf16; kind::tf32: 2), both K-major,
       // N=BN, M=128
       constexpr uint32_t fmt = KIND == kKindTF32X3 ? 2u : KIND == kKindBF16 ? 1u : 0u;
+      // (kMN: bits 15 / 16 = A / B MN-major)
       constexpr uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(BN >> 3) << 17) |
-                                 ((uint32_t)((kPair2 ? 2 * kTcBM : kTcBM) >> 4) << 24);
+                                 ((uint32_t)((kPair2 ? 2 * kTcBM : kTcBM) >> 4) << 24) | (kMN ? (3u << 15) : 0u);
       auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t acc_flag) {
         if constexpr (KIND == kKindTF32X3) ptx::umma_tf32(d, a, b, idesc, acc_flag);
         else if constexpr (kPair2) ptx::umma_f16_2sm(d, a, b, idesc, acc_flag);
@@ -639,9 +683,13 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
         if constexpr (kPair2) ptx::umma_commit_2sm_mc(bar, 3);
         else ptx::umma_commit(bar);
       };
-      // smem matrix descriptor (K-major, SWIZZLE_128B): LBO=1, SBO=1024 B, version=1, layout=2
-      constexpr uint64_t desc_hi = ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) |
+      // smem matrix descriptor (K-major, SWIZZLE_128B): LBO=1, SBO=1024 B, version=1, layout=2.  kMN (MN-major,
+      // SWIZZLE_128B): LBO = 8 KB from the first 64 channels to the next 64, SBO = 1024 B from one 8-pixel group to the next
+      constexpr uint64_t desc_hi = ((uint64_t)(kMN ? (kABytes / 2) >> 4 : 1) << 16) | ((uint64_t)(1024 >> 4) << 32) |
                                    ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
+      static_assert(!kMN || Cfg::kBBytes == kABytes, "kMN: A and B halves are both 8 KB apart");
+      // K step of 16: 32 bytes inside the swizzle row (K-major), 16 pixel rows of 128 bytes (MN-major); descriptor units of 16 B
+      constexpr uint64_t kStep = kMN ? 128 : 2;
       auto desc = [&](const uint8_t* ptr) { return desc_hi | (uint64_t)((ptx::smem_u32(ptr) >> 4) & 0x3FFF); };
       auto release_stage = [&](int s) {
         if constexpr (CL == 1) ptx::umma_commit_mc(&empty[s], 3);   // the peer multicasts into this stage too
@@ -684,8 +732,8 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
               const uint32_t first = kb != 0, first_main = kb > kb0;
               if (ptx::elect_one()) {
 #pragma unroll
-                for (int k = 0; k < 4; ++k) {        // K step = 8 tf32 / 16 f16 = 32 bytes
-                  const uint64_t o = (uint64_t)(2 * k);
+                for (int k = 0; k < 4; ++k) {        // K step = 8 tf32 / 16 f16 = 32 bytes (kMN: 2 KB)
+                  const uint64_t o = kStep * (uint64_t)k;
 #ifndef CDR_EXP_NO_CORR   /* timing experiment only: results are wrong without the correction terms */
                   mma(d_corr, dal + o, db + o, k ? 1u : first);            // lo*hi  } whole-tile chain: these
                   mma(d_corr, da + o, dbl + o, 1u);                        // hi*lo  } terms are 2^-11 of the main one
@@ -925,6 +973,17 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
         ptx::tc_fence_before();
         __syncwarp();
         if (lane == 0) arrive_issuer(&tmem_empty[acc]);
+        if constexpr (kMN) {
+          // the slice's raw partial: row ci of (slice, tap) = g, columns co (pitch c_pitch, first c_fill written)
+          if (row_ok) {
+            float* __restrict__ dst = reinterpret_cast<float*>(p.C) + ((size_t)g * p.M + m) * p.c_pitch + n0;
+#pragma unroll
+            for (int c = 0; c < kCols; c += 4)
+              if (n0 + c < p.c_fill)
+                *reinterpret_cast<float4*>(dst + c) = make_float4(sum[c], sum[c + 1], sum[c + 2], sum[c + 3]);
+          }
+          continue;
+        }
         int res_stage = -1;
         if constexpr (kResOK && KIND == kKindF16X2) {
           if (p.has_res) {
@@ -1058,6 +1117,8 @@ struct TcLaunch {
   const float* amax_in;          // overrides in_slot.amax (input stored in another format)
   // encoder convs: H, W above are the OUTPUT pixel grid; the input grid is (stride*H, stride*W)
   int conv3;                     // 3x3, pad 1 (9 taps)
+  int conv4s2;                   // 4x4, stride 2 (set stride = 2), pad 1 (16 taps)
+  int planar_deconv;             // kOutPlanar + deconv: fp32 NCHW output of the 2H x 2W map (phase scatter)
   int stride;                    // 0/1 or 2
   const void* res;               // residual rows (n channels, pitch res_pitch; bf16, or the hi plane of kFmtF16P) added
   const void* res_lo;            // before the ReLU; kFmtF16P: the lo plane and the residual tensor's scale slot
@@ -1142,9 +1203,12 @@ static int launch_tc_t(const TcLaunch& l, cudaStream_t st) {
   p.M = l.n_img * HW;
   p.n_img = l.n_img; p.H = l.H; p.W = l.W; p.cin = l.cin;
   const int stride = l.stride > 1 ? l.stride : 1;
-  const bool a4d = l.deconv || l.conv3 || stride > 1;
-  p.tap_mode = l.deconv ? kTapDeconv : l.conv3 ? kTapConv3 : kTapNone;
-  p.ntaps = l.deconv ? 4 : l.conv3 ? 9 : 1;
+  const bool a4d = l.deconv || l.conv3 || l.conv4s2 || stride > 1;
+  p.tap_mode = l.deconv ? kTapDeconv : l.conv3 ? kTapConv3 : l.conv4s2 ? kTapConv4s2 : kTapNone;
+  p.ntaps = l.deconv ? 4 : l.conv3 ? 9 : l.conv4s2 ? 16 : 1;
+  CDR_CHECK_ARG(!l.conv4s2 || stride == 2, "tap_gemm_tc: the 4x4 tap mode is the stride-2 conv");
+  p.planar_deconv = l.planar_deconv;
+  CDR_CHECK_ARG(!l.planar_deconv || (l.deconv && l.out_mode == kOutPlanar), "tap_gemm_tc: phase scatter needs a planar deconv");
   p.a4d = a4d;
   p.stride = stride;
   p.has_res = l.res != nullptr;
@@ -1593,8 +1657,14 @@ __device__ __forceinline__ float conv_taps_weight(const CdrConvBn& s, int cout, 
   const int tap = kk / cin, ci = kk - tap * cin;
   return (float)((double)s.weight[((size_t)n * cin + ci) * taps + tap] * tc_bn_scale(s, n));
 }
+// the data-gradient operand of a transposed conv (Cin,Cout,4,4) at packed position (ci, tap*Cout + co), tap = ky*4 + kx
+__device__ __forceinline__ float deconv_dgrad_weight(const CdrConvBn& s, int cin, int cout, int ci, int kk) {
+  if (ci >= cin) return 0.f;
+  const int tap = kk / cout, co = kk - tap * cout;
+  return s.weight[((size_t)ci * cout + co) * 16 + tap];
+}
 // kDeconv: 0 = 1x1 conv, 1 = transposed conv (4 phases), >= 2: conv with kDeconv taps in encoder order (use 9; the 1x1
-// convs of the encoder go through mode 0)
+// convs of the encoder go through mode 0), -1: deconv_dgrad_weight (`cout` = Cin rows, `cin` = Cout per tap)
 template <int kDeconv, bool kWrite>
 __global__ void __launch_bounds__(256)
 pack_rows_f16_kernel(CdrConvBn s, int cout, int cin, int k_pitch, int n_pad, __half* __restrict__ w_hi,
@@ -1605,6 +1675,7 @@ pack_rows_f16_kernel(CdrConvBn s, int cout, int cin, int k_pitch, int n_pad, __h
   const int n = row % n_pad, phase = row / n_pad;
   auto val = [&](int kk) -> float {
     if constexpr (kDeconv >= 2) return conv_taps_weight(s, cout, cin, kDeconv, n, kk);
+    if constexpr (kDeconv < 0) return deconv_dgrad_weight(s, cout, cin, n, kk);
     return kDeconv ? deconv_weight(s, cin, cout, phase, n, kk) : conv1x1_weight(s, cout, cin, n, kk);
   };
   float mx = 0.f, l1 = 0.f;
@@ -2642,6 +2713,215 @@ int tc_encoder_forward(const void* enc, const void* x, int n, int h, int w, void
 
 int tc_set_debug(unsigned int* d) {
   CDR_CUDA(cudaMemcpyToSymbol(ptx::g_cdr_debug, &d, sizeof(d)));
+  return CDR_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// Training a ConvTranspose2d(k4, s2, p1, bias=False) at fp32 accuracy: forward, data and weight gradient on the f16x2
+// tap-GEMM (scaled fp16 hi/lo operands, 3 kind::f16 MMAs per product, main term drained every kSplitChunk K blocks).
+//   forward  y  = kTapDeconv (4 phases x 4 taps) over the x planes, weights packed unfolded per call, phase-scattered
+//               straight into NCHW fp32 (kOutPlanar + planar_deconv)
+//   dgrad    dx = kTapConv4s2 (16 taps, stride-2 box over the dy planes), B = [ci][tap*Cout + co], NCHW fp32 out
+//   wgrad    dW = the kMN kernel: per tap a GEMM over the pixels, K split into slices -> fp32 partials ->
+//               wgrad_reduce_kernel (fixed slice order: bitwise deterministic, no atomics)
+// x and dy are encoded with ONE power-of-two scale per tensor (exact amax first): wgrad reduces over pixels, so per-pixel
+// scales would not factor out of its sums.  The x planes and their {amax, scale} slot are what the forward saves.
+struct DtShape {
+  int n, cin, cout, h, w;
+  size_t x_rows() const { return (size_t)n * h * w; }
+  size_t dy_rows() const { return (size_t)n * 4 * h * w; }
+  int npo() const { return round_up(cout, 128); }     // forward: packed output channels per phase
+  int npi() const { return round_up(cin, 128); }      // dgrad: packed output channels
+  // wgrad K slices: powers of two while the tiles do not fill two waves of 148 SMs and a slice keeps >= 16 K blocks.  A
+  // function of the shape only, so the summation order (and the result, bit for bit) does not depend on the device.
+  int slices() const {
+    const long long kb = (long long)n * h * w / 64;
+    const int tiles = (cin / 64 + 1) / 2 * ((cout / 64 + 1) / 2) * 16;
+    int s = 1;
+    while ((long long)tiles * s < 2 * 148 && kb % (2 * s) == 0 && kb / (2 * s) >= 16) s *= 2;
+    return s;
+  }
+};
+struct DtWs {
+  TcLayer L;                 // forward: [4 phases][npo][4*cin]; backward: dgrad [npi][16*cout]
+  void* dy_planes = nullptr; // backward: dy as an fp16 planes buffer [hi | lo | {amax, scale}]
+  float* part = nullptr;     // backward: wgrad partials [slice][tap][cin][npo]
+  size_t bytes = 0;
+};
+static DtWs plan_deconv_train(void* base, const DtShape& d, bool backward) {
+  DtWs ws;
+  Bump1K b(base);
+  if (!backward) {
+    plan_layer(ws.L, b, kKindF16X2, 4 * d.npo(), 4 * d.cin, 4 * d.cin, 128, d.npo(), d.npo(), false);
+  } else {
+    plan_layer(ws.L, b, kKindF16X2, d.npi(), 16 * d.cout, 16 * d.cout, 128, d.npi(), d.npi(), false);
+    ws.dy_planes = b.take(2 * planes_stride_bytes(d.dy_rows(), d.cout) + 1024);
+    ws.part = (float*)b.take((size_t)d.slices() * 16 * d.cin * d.npo() * sizeof(float));
+  }
+  ws.bytes = b.off;
+  return ws;
+}
+size_t deconv_train_saved_bytes(int n, int cin, int cout, int h, int w) {
+  const DtShape d{n, cin, cout, h, w};
+  return 2 * planes_stride_bytes(d.x_rows(), cin) + 1024;
+}
+size_t deconv_train_workspace_bytes(int n, int cin, int cout, int h, int w) {
+  const DtShape d{n, cin, cout, h, w};
+  const size_t f = plan_deconv_train(nullptr, d, false).bytes, bw = plan_deconv_train(nullptr, d, true).bytes;
+  return f > bw ? f : bw;
+}
+
+// NCHW fp32 -> fp16 planes with one tensor scale (exact amax pass first)
+static int to_planes_tensor_scale(const float* in, int n, int c, int hw, const Act& a, ScaleSlot sl, cudaStream_t st) {
+  CDR_CUDA(cudaMemsetAsync(sl.amax, 0, sizeof(float), st));
+  if (int rc = launch_amax_f32(in, nullptr, (long long)n * c * hw, sl.amax, st)) return rc;
+  return launch_nchw_to_rows_f16p(in, nullptr, n, c, hw, a.p[0], a.p[1], c, sl.amax, sl.scale, st);
+}
+
+int tc_deconv_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, float* y,
+                            void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  const DtShape d{n, cin, cout, h, w};
+  DtWs ws = plan_deconv_train(workspace, d, false);
+  if (workspace_bytes < ws.bytes) {
+    set_error("cdr_deconv_train_forward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
+    return CDR_ERR_WORKSPACE;
+  }
+  set_stage("deconv_train_fwd");
+  ScaleSlot sx;
+  const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
+  if (int rc = to_planes_tensor_scale(x, n, cin, h * w, xa, sx, st)) return rc;
+  CdrConvBn cb{};
+  cb.weight = weight;
+  TcLayer& L = ws.L;
+  pack_rows_f16_kernel<1, true><<<L.rows, 256, 0, st>>>(cb, cout, cin, L.k_pitch, L.n_pad, (__half*)L.w[0],
+                                                        (__half*)L.w[1], L.wsi, L.bias, nullptr);
+  CDR_LAUNCH_OK("pack_rows_f16_kernel");
+  if (int rc = layer_maps(L)) return rc;
+  TcLaunch l{};
+  l.A = xa; l.a_pitch = cin;
+  l.n_img = n; l.H = h; l.W = w; l.cin = cin; l.deconv = 1; l.groups = 4;
+  l.a_rows_total = (long long)d.x_rows();
+  l.layer = &L; l.b_group_rows = L.n_pad; l.n = cout; l.bias_group_stride = 0;
+  l.C.p[0] = y; l.relu = 0; l.out_mode = kOutPlanar; l.planar_deconv = 1;
+  l.in_slot = sx;
+  const int rc = launch_tc(l, st);
+  set_stage(nullptr);
+  return rc;
+}
+
+// dW[ci][co][tap] = (sum over slices, in order, of part[slice][tap][ci][co]) / (s_x * s_dy)
+__global__ void __launch_bounds__(256)
+wgrad_reduce_kernel(const float* __restrict__ part, int slices, int cin, int cout, int ldc, const float* __restrict__ sx,
+                    const float* __restrict__ sdy, float* __restrict__ dw) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= (long long)cin * cout * 16) return;
+  const int t = (int)(idx & 15);
+  const long long r = idx >> 4;
+  const int co = (int)(r % cout), ci = (int)(r / cout);
+  const float ix = 1.f / __ldcg(sx), id = 1.f / __ldcg(sdy);      // powers of two: exact
+  float s = 0.f;
+  for (int sl = 0; sl < slices; ++sl) s += __ldcg(part + (((size_t)sl * 16 + t) * cin + ci) * ldc + co);
+  dw[idx] = s * ix * id;
+}
+
+static int launch_wgrad(const DtShape& d, const Act& xa, ScaleSlot sx, const Act& dya, float* part, cudaStream_t st) {
+  using Cfg = TcCfg<128, kKindF16X2, kFmtF16P, 0>;
+  auto kern = tap_gemm_tc_kernel<128, kKindF16X2, kFmtF16P, 0, true>;
+  static DeviceOnce attr_set;
+  if (attr_set.need()) {
+    CDR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
+    attr_set.done();
+  }
+  const int hw = d.h * d.w, slices = d.slices();
+  const long long kb = (long long)d.n * hw / 64;
+  TcGemmParams p{};
+  p.M = d.cin;
+  p.n_img = d.n; p.H = d.h; p.W = d.w;
+  p.cin = (int)(kb / slices) * 64;           // pixels per K slice
+  p.ntaps = 1; p.tap_mode = kTapNone; p.stride = 1;
+  p.groups = 16 * slices;
+  p.n_tiles = d.npo() / 128;
+  p.n = d.cout;
+  p.C = part; p.c_pitch = d.npo(); p.c_fill = d.cout;
+  p.out_mode = kOutPlanar;
+  p.scale_in = sx.scale;
+  p.num_tiles = (d.npi() / 128) * p.groups * p.n_tiles;
+  CUtensorMap ma[2], mb[2];
+  for (int pl = 0; pl < 2; ++pl) {
+    {   // x planes: (pixels, cin) rows, boxes of 64 channels x 64 pixels
+      const uint64_t dims[2] = {(uint64_t)d.cin, (uint64_t)d.x_rows()};
+      const uint64_t strides[1] = {(uint64_t)d.cin};
+      const uint32_t box[2] = {64, 64};
+      if (int rc = make_tmap(&ma[pl], xa.p[pl], kFmtF16P, 2, dims, strides, box)) return rc;
+    }
+    {   // dy planes (n, 2h, 2w, cout) seen with element stride 2: 64 channels x (w x 64/w) pixels x 1 image
+      const uint64_t iw = 2 * (uint64_t)d.w, ih = 2 * (uint64_t)d.h;
+      const uint64_t dims[4] = {(uint64_t)d.cout, iw, ih, (uint64_t)d.n};
+      const uint64_t strides[3] = {(uint64_t)d.cout, (uint64_t)d.cout * iw, (uint64_t)d.cout * iw * ih};
+      const uint32_t box[4] = {64, (uint32_t)(2 * d.w), (uint32_t)(2 * (64 / d.w)), 1};
+      const uint32_t estr[4] = {1, 2, 2, 1};
+      if (int rc = make_tmap(&mb[pl], dya.p[pl], kFmtF16P, 4, dims, strides, box, estr)) return rc;
+    }
+  }
+  const int grid = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
+  cudaLaunchConfig_t cfg{};
+  cudaLaunchAttribute attr[1];
+  int n_attr = 0;
+  if (tc_use_pdl()) {
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    n_attr = 1;
+  }
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(Cfg::kThreads);
+  cfg.dynamicSmemBytes = Cfg::kSmemBytes;
+  cfg.stream = st;
+  cfg.attrs = attr;
+  cfg.numAttrs = n_attr;
+  CDR_CUDA(cudaLaunchKernelEx(&cfg, kern, ma[0], ma[1], mb[0], mb[1], ma[0], ma[0], ma[0], ma[0], p));
+  CDR_LAUNCH_OK("tap_gemm_tc_kernel");
+  return CDR_OK;
+}
+
+int tc_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                             int w, float* dx, float* dw, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  const DtShape d{n, cin, cout, h, w};
+  DtWs ws = plan_deconv_train(workspace, d, true);
+  if (workspace_bytes < ws.bytes) {
+    set_error("cdr_deconv_train_backward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
+    return CDR_ERR_WORKSPACE;
+  }
+  if (!dx && !dw) return CDR_OK;
+  set_stage("deconv_train_bwd");
+  ScaleSlot sd, sx;
+  const Act dya = planes_act(ws.dy_planes, d.dy_rows(), cout, &sd);     // one copy feeds both GEMMs
+  const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
+  if (int rc = to_planes_tensor_scale(dy, n, cout, 4 * h * w, dya, sd, st)) return rc;
+  if (dx) {
+    CdrConvBn cb{};
+    cb.weight = weight;
+    TcLayer& L = ws.L;
+    pack_rows_f16_kernel<-1, true><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
+                                                           (__half*)L.w[1], L.wsi, L.bias, nullptr);
+    CDR_LAUNCH_OK("pack_rows_f16_kernel");
+    if (int rc = layer_maps(L)) return rc;
+    TcLaunch l{};
+    l.A = dya; l.a_pitch = cout;
+    l.n_img = n; l.H = h; l.W = w; l.cin = cout; l.conv4s2 = 1; l.stride = 2; l.groups = 1;
+    l.a_rows_total = (long long)d.dy_rows();
+    l.layer = &L; l.b_group_rows = 0; l.n = cin; l.bias_group_stride = 0;
+    l.C.p[0] = dx; l.relu = 0; l.out_mode = kOutPlanar;
+    l.in_slot = sd;
+    if (int rc = launch_tc(l, st)) return rc;
+  }
+  if (dw) {
+    if (int rc = launch_wgrad(d, xa, sx, dya, ws.part, st)) return rc;
+    const long long total = (long long)cin * cout * 16;
+    wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, d.slices(), cin, cout, d.npo(),
+                                                                                   sx.scale, sd.scale, dw);
+    CDR_LAUNCH_OK("wgrad_reduce_kernel");
+  }
+  set_stage(nullptr);
   return CDR_OK;
 }
 

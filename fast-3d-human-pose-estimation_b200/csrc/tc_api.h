@@ -40,4 +40,12 @@ int tc_encoder_out_shape(const void* enc, int h, int w, int* oh, int* ow, int* o
 int tc_encoder_forward(const void* enc, const void* x, int n, int h, int w, void* out_rows, void* workspace,
                        size_t workspace_bytes, cudaStream_t st);
 
+// Training a ConvTranspose2d(k4, s2, p1, bias=False) at fp32 accuracy (f16x2) — gemm_tc.cu
+size_t deconv_train_saved_bytes(int n, int cin, int cout, int h, int w);
+size_t deconv_train_workspace_bytes(int n, int cin, int cout, int h, int w);
+int tc_deconv_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, float* y,
+                            void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st);
+int tc_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                             int w, float* dx, float* dw, void* workspace, size_t workspace_bytes, cudaStream_t st);
+
 }  // namespace cdr

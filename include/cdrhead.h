@@ -332,6 +332,21 @@ int cdr_joint_loss_forward(int kind, const float* pred, const float* target, con
 int cdr_joint_loss_backward(int kind, const float* pred, const float* target, const float* weight, long long rows, int d,
                             double threshold, const float* grad_loss, float* grad_pred, void* stream);
 
+/* ---- Training the decoder's transposed convolutions: ConvTranspose2d(Cin, Cout, 4, stride 2, padding 1, bias=False) at
+ * fp32 accuracy on the tensor cores (scaled fp16 hi/lo operands, 3 kind::f16 MMAs per product), forward and backward.
+ * x (n, Cin, h, w), weight (Cin, Cout, 4, 4), y / dy (n, Cout, 2h, 2w), all fp32 NCHW, 16-byte aligned.
+ * Supported: Cin and Cout multiples of 64, h == w in {8, 16, 32}, n >= 1 (CDR_ERR_UNSUPPORTED otherwise).
+ * The forward leaves x, re-encoded for the weight gradient, in `saved` (saved_bytes, 256-byte aligned; as large as
+ * an fp16 copy of x plus 1 KB); the backward reads it back.  One workspace (workspace_bytes, 256-byte aligned) serves
+ * both calls.  The backward writes dx (n, Cin, h, w) and / or dweight (Cin, Cout, 4, 4); a NULL pointer skips that
+ * GEMM.  dweight is bitwise deterministic (fixed-order reduction of its K slices, no atomics). */
+int cdr_deconv_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes,
+                                     size_t* workspace_bytes);
+int cdr_deconv_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, float* y,
+                             void* saved, size_t saved_bytes, void* workspace, size_t workspace_bytes, void* stream);
+int cdr_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                              int w, float* dx, float* dweight, void* workspace, size_t workspace_bytes, void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
