@@ -104,6 +104,19 @@ __device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
   lo = x - hi;
 }
 
+// ---- power-of-two scale of the scaled fp16 hi/lo planes (gemm_tc.cu: kFmtF16P): s = 2^(13 - ilogb(amax)) puts the
+// largest |x| in [2^13, 2^14), 4x below fp16 max.  The exponent is capped at 127 so that s stays a finite float for
+// amax < 2^-114 (uncapped, s = +Inf and the encode x * s turns every element into +-Inf or NaN); 1/s = 2^-127 is then an
+// exact subnormal, as the library never flushes denormals.  A zero, infinite or NaN amax gives s = 1.  For amax in
+// [2^-114, FLT_MAX] this is exactly 2^(13 - ilogb(amax)).
+constexpr int kF16TargetExp = 13;
+__device__ __forceinline__ int f16_pow2_exp(float amax) {
+  if (!(amax > 0.f && amax <= 3.40282347e38f)) return 0;
+  const int e = kF16TargetExp - ilogbf(amax);
+  return e < 127 ? e : 127;
+}
+__device__ __forceinline__ float f16_pow2_scale(float amax) { return ldexpf(1.f, f16_pow2_exp(amax)); }
+
 // ---- fixed geometry of the head (models/cdrnet.py:89-91, models/decoder.py:8-13) ----
 constexpr int kFeatC = 2048;   // encoder channels = fusion_in_dim
 constexpr int kFeatHW = 64;    // 8x8 latent

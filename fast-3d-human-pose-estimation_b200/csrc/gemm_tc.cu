@@ -47,7 +47,6 @@ enum ActFmt { kFmtBF16 = 0, kFmtTF32P = 1, kFmtF16P = 2 };
 __host__ __device__ constexpr int fmt_elem(int fmt) { return fmt == kFmtTF32P ? 4 : 2; }
 __host__ __device__ constexpr int fmt_planes(int fmt) { return fmt == kFmtBF16 ? 1 : 2; }
 constexpr float kLoScale = 2048.f;            // 2^11: the lo plane of kFmtF16P is stored times this
-constexpr int kF16TargetExp = 13;             // scaled maxima land in [2^13, 2^14): 4x below fp16 max
 
 // ------------------------------------------------------------------------------------------
 // tensor maps
@@ -780,7 +779,7 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
         float bound = __ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1);
         if constexpr (kResOK)
           if (p.has_res && p.res_amax) bound += __ldcg(p.res_amax);       // |conv + residual| <= bound(conv) + max |residual|
-        if (bound > 0.f && bound < 3.0e38f) es.s_out = ldexpf(1.f, kF16TargetExp - ilogbf(bound));
+        es.s_out = f16_pow2_scale(bound);
         if (blockIdx.x == 0 && threadIdx.x == 64) *p.scale_out = es.s_out;
       }
     }
@@ -1700,7 +1699,7 @@ pack_rows_f16_kernel(CdrConvBn s, int cout, int cin, int k_pitch, int n_pad, __h
     mx = fmaxf(mx, red_max[i]);
     l1 += red_sum[i];
   }
-  const int t = mx > 0.f ? kF16TargetExp - ilogbf(mx) : 0;
+  const int t = f16_pow2_exp(mx);
   if (threadIdx.x == 0) {
     const float b = n < cout ? tc_folded_bias(s, n) : 0.f;
     if (kWrite) {
@@ -2082,7 +2081,7 @@ __global__ void bf16_rows_to_f16p_kernel(const __nv_bfloat16* __restrict__ in, _
                                          __half* __restrict__ lo, long long n, const float* __restrict__ amax,
                                          float* __restrict__ scale_out) {
   const float a = __ldg(amax);
-  const float s = (a > 0.f && a < 3.0e38f) ? ldexpf(1.f, kF16TargetExp - ilogbf(a)) : 1.f;
+  const float s = f16_pow2_scale(a);
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0) *scale_out = s;
   if (i >= n) return;

@@ -46,7 +46,7 @@ nchw_to_rows16_kernel(const float* __restrict__ in, const float* __restrict__ in
   float s = 1.f;
   if constexpr (kF16P) {
     const float a = __ldg(amax);
-    if (a > 0.f && a < 3.0e38f) s = ldexpf(1.f, 13 - ilogbf(a));
+    s = f16_pow2_scale(a);
     if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && threadIdx.x == 0) *scale_out = s;
   }
   const int c0 = blockIdx.x * 64, p0 = blockIdx.y * 64, img = blockIdx.z;
@@ -171,7 +171,7 @@ int launch_amax_f32(const float* in, const float* in2, long long n, float* amax,
   return CDR_OK;
 }
 
-// scaled fp16 hi/lo planes (gemm_tc.cu: kFmtF16P): X = x * s with s = 2^(13 - ilogb(amax)),
+// scaled fp16 hi/lo planes (gemm_tc.cu: kFmtF16P): X = x * s with s = 2^(13 - ilogb(amax)) (common.cuh: f16_pow2_scale),
 // hi = rn_f16(X), lo = rn_f16((X - hi) * 2^11); block (0,0,0) publishes s.
 __global__ void __launch_bounds__(256)
 nchw_to_rows_f16p_kernel(const float* __restrict__ in, const float* __restrict__ in2, int n_first, int C, int HW,
@@ -179,7 +179,7 @@ nchw_to_rows_f16p_kernel(const float* __restrict__ in, const float* __restrict__
                          const float* __restrict__ amax, float* __restrict__ scale_out) {
   __shared__ float tile[32][65];
   const float a = __ldg(amax);
-  const float s = (a > 0.f && a < 3.0e38f) ? ldexpf(1.f, 13 - ilogbf(a)) : 1.f;
+  const float s = f16_pow2_scale(a);
   if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && threadIdx.x == 0) *scale_out = s;
   const int c0 = blockIdx.x * 32, p0 = blockIdx.y * 64, img = blockIdx.z;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
@@ -282,7 +282,7 @@ nchw_to_rows_f16p_rowscale_kernel(const float* __restrict__ in, const float* __r
       mx = v > mx ? v : mx;
     }
     const float a = __uint_as_float(mx);
-    const float s = (a > 0.f && a < 3.0e38f) ? ldexpf(1.f, 13 - ilogbf(a)) : 1.f;
+    const float s = f16_pow2_scale(a);
     sscale[threadIdx.x] = s;
     if (quarter == 0) {
       row_scale[(size_t)img * HW + threadIdx.x] = s;
@@ -595,7 +595,7 @@ ftl_f16p_vec_kernel(const FtlViews<__half> fv, int in_pitch, int blk, long long 
   const bool v1 = blockIdx.y != 0;
   const float inv_s = 1.f / __ldg(scale_in);          // powers of two: exact
   const float bound = __ldg(amax_in) * __ldg(l1max);
-  const float s_out = (bound > 0.f && bound < 3.0e38f) ? ldexpf(1.f, 13 - ilogbf(bound)) : 1.f;
+  const float s_out = f16_pow2_scale(bound);
   if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) *scale_out = s_out;
   float amax = 0.f;
   if (idx < total4) {

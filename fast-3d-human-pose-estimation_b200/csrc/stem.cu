@@ -367,7 +367,7 @@ maxpool3s2_f16p_kernel(const float* __restrict__ in, int Hi, int Wi, int C8, lon
                        __half* __restrict__ lo, float* __restrict__ slot) {
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const float a = __ldg(slot);
-  const float s = (a > 0.f && a < 3.0e38f) ? ldexpf(1.f, 13 - ilogbf(a)) : 1.f;
+  const float s = f16_pow2_scale(a);
   if (idx == 0) slot[1] = s;
   if (idx >= total) return;
   const int c8 = (int)(idx % C8);
@@ -440,7 +440,7 @@ __global__ void pack_stem_f16x2_kernel(CdrConvBn s, __half* __restrict__ w_hi, _
   __syncthreads();
   mx = 0.f;
   for (int i = 0; i < (int)(blockDim.x >> 5); ++i) mx = fmaxf(mx, red[i]);
-  const int t = mx > 0.f ? 13 - ilogbf(mx) : 0;
+  const int t = f16_pow2_exp(mx);
   if (threadIdx.x == 0) {
     wsi[n] = ldexpf(1.f, -t);
     bias[n] = (float)((double)s.bn_bias[n] - (double)s.bn_mean[n] * sc);

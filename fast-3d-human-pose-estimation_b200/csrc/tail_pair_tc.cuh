@@ -325,7 +325,7 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
     if constexpr (kSplit) {
       a_inv = 1.f / __ldcg(p.scale_in);
       const float bound = __ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1);
-      if (bound > 0.f && bound < 3.0e38f) s_out = ldexpf(1.f, kF16TargetExp - ilogbf(bound));
+      s_out = f16_pow2_scale(bound);
     }
     auto wait_a2_free = [&]() {              // own a2_empty[]: released for both CTAs by multicast commits (tail_tc.cuh)
       if constexpr (!kSplit) ptx::mbar_wait(&a2_empty[0], (tl & 1) ^ 1u);
@@ -448,7 +448,7 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
     float fin_scale = 1.f;
     if constexpr (kSplit) {
       const float bound = __ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1);
-      if (bound > 0.f && bound < 3.0e38f) fin_scale = ldexpf(1.f, -(kF16TargetExp - ilogbf(bound)));
+      fin_scale = ldexpf(1.f, -f16_pow2_exp(bound));
     }
     const float kLog2e = 1.4426950408889634f;
     for (int pu = pu0; pu < num_pu; pu += pu_step) {

@@ -390,7 +390,7 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     if constexpr (kSplit) {
       a_inv = 1.f / __ldcg(p.scale_in);
       const float bound = __ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1);
-      if (bound > 0.f && bound < 3.0e38f) s_out = ldexpf(1.f, kF16TargetExp - ilogbf(bound));
+      s_out = f16_pow2_scale(bound);
     }
     // A2 is free for this warp's round of tile tl once the heat MMAs of the round BEFORE it have completed:
     //   bf16 (one round per tile)   : round of tile tl-1                     -> a2_empty[0], phase tl-1
@@ -523,7 +523,7 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     float fin_scale = 1.f;                         // 1 / s(deconv3 activation)
     if constexpr (kSplit) {
       const float bound = __ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1);
-      if (bound > 0.f && bound < 3.0e38f) fin_scale = ldexpf(1.f, -(kF16TargetExp - ilogbf(bound)));
+      fin_scale = ldexpf(1.f, -f16_pow2_exp(bound));
     }
     const float kLog2e = 1.4426950408889634f;
     for (int unit = blockIdx.x; unit < p.num_units; unit += gridDim.x) {

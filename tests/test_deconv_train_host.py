@@ -1,7 +1,10 @@
 """CPU: the index algebra the transposed-convolution training kernels implement (gemm_tc.cu: kTapConv4s2 and the
 MN-major weight-gradient tiles), in fp64 against torch autograd, and the argument checks of conv_transpose2d and of
-the cdr_deconv_train_* entry points, none of which may touch CUDA."""
+the cdr_deconv_train_* entry points, none of which may touch CUDA.  Also the pieces of test_gpu_deconv_train_domain.py
+that need no GPU: its shape table against the wgrad slice plan, and the strictness of its per-element gate."""
 import ctypes as C
+import importlib.util
+import os
 
 import pytest
 import torch
@@ -59,6 +62,67 @@ def test_wgrad_is_16_per_tap_pixel_reductions(problem):
         slices = [xr[k:k + 8].T @ d[k:k + 8] for k in range(0, xr.shape[0], 8)]
         got[:, :, tap // 4, tap % 4] = sum(slices)
     assert torch.allclose(got, dw, rtol=1e-12, atol=1e-12)
+
+
+def _domain():
+    """tests/test_gpu_deconv_train_domain.py (its shape table, slice mirror and gate), imported without a GPU."""
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "test_gpu_deconv_train_domain.py")
+    spec = importlib.util.spec_from_file_location("_deconv_train_domain", path)
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+def test_shape_table_covers_the_plan():
+    """The GPU table reaches every wgrad slice count the plan produces, padded and unpadded channel tiles on both
+    sides, partial kSplitChunk chunks of the forward (4*Cin/64 K blocks) and a slice that ends mid-image."""
+    D = _domain()
+    assert {s for *_, s in D.TABLE} == {1, 2, 4, 8, 16, 32}
+    assert all(D.slices(n, cin, cout, h) == s for n, cin, cout, h, s in D.TABLE)
+    assert {cin % 128 for _, cin, _, _, _ in D.TABLE} == {0, 64}
+    assert {cout % 128 for _, _, cout, _, _ in D.TABLE} == {0, 64}
+    assert any((4 * cin // 64) % 8 for _, cin, _, _, _ in D.TABLE)
+    assert any((n * h * h) % (64 * s) == 0 and (n * h * h // s) % (h * h) for n, _, _, h, s in D.TABLE)
+    # the mirror never grows past 32: the tile count of the smallest layer times 32 already fills two waves
+    assert max(D.slices(n, 64, 64, h) for n in (1, 64, 1024, 4096) for h in (8, 16, 32)) == 32
+
+
+def test_slice_mirror_fits_the_reported_workspace(pkg):
+    """The backward workspace holds the wgrad partials, [slices][16 taps][Cin][round_up(Cout, 128)] fp32: a mirror
+    that counted more slices than the library would not fit in what cdr_deconv_train_workspace_bytes reports."""
+    D = _domain()
+    L = pkg._lib.lib()
+    s, w = C.c_size_t(), C.c_size_t()
+    for n, cin, cout, h, sl in D.TABLE:
+        assert L.cdr_deconv_train_workspace_bytes(n, cin, cout, h, h, C.byref(s), C.byref(w)) == 0
+        assert w.value >= sl * 16 * cin * (cout + 127) // 128 * 128 * 4
+
+
+def _f16_planes(t, keep_lo):
+    """fp64 emulation of the scaled fp16 planes of a tensor (layout.cu: nchw_to_rows_f16p): s = 2^min(13 - ilogb(amax),
+    127), hi = rn_f16(x s), lo = rn_f16((x s - hi) 2^11); decoded as (hi + lo 2^-11) / s, or hi / s alone."""
+    _, e = torch.frexp(t.abs().max())
+    s = 2.0 ** min(13 - (int(e) - 1), 127)
+    X = t * s
+    hi = X.half().double()
+    if not keep_lo:
+        return hi / s
+    return (hi + ((X - hi) * 2048).half().double() / 2048) / s
+
+
+def test_per_element_gate_catches_a_lost_lo_plane():
+    """With x through both planes the forward passes the per-element gate; with the hi plane alone (~2^-12 m) it
+    fails.  So the gate's constant is tight enough to see the lo plane, and c <= 2^-14."""
+    D = _domain()
+    assert D.GATE_C <= 2.0 ** -14
+    g = torch.Generator().manual_seed(0)
+    x = torch.randn((1, 4, 8, 8), generator=g).double()          # fp32 values, held in fp64
+    w = torch.randn((4, 3, 4, 4), generator=g).float().double()
+    ref = F.conv_transpose2d(x, w, stride=2, padding=1)
+    mag = F.conv_transpose2d(x.abs(), w.abs(), stride=2, padding=1)
+    D.gate("y", F.conv_transpose2d(_f16_planes(x, True), w, stride=2, padding=1), ref, mag)
+    with pytest.raises(AssertionError, match="per-element gate"):
+        D.gate("y", F.conv_transpose2d(_f16_planes(x, False), w, stride=2, padding=1), ref, mag, max_gate=False)
 
 
 def test_conv_transpose2d_rejects_without_cuda(pkg, monkeypatch):
