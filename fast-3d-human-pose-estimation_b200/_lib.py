@@ -17,9 +17,8 @@ CDR_PREC_FP32 = 0
 CDR_PREC_BF16 = 1
 CDR_PREC_TF32X3 = 2
 CDR_PREC_F16X2 = 3
-# "fp32" / "f16x2": fp32-accurate results on the tcgen05 tensor cores — the default.  Decoder and conv_layer1 on
-#              scaled fp16 two-term operands (3 kind::f16 MMAs per product), the rest of the fusion block on
-#              3xTF32 (CDR_PREC_F16X2 selects this hybrid pack, gemm_tc.cu: kModeHybrid)
+# "fp32" / "f16x2": fp32-accurate results on the tcgen05 tensor cores — the default.  Fusion block and decoder on
+#              scaled fp16 two-term operands (3 kind::f16 MMAs per product; gemm_tc.cu: kModeF16X2)
 # "tf32x3"   : 3xTF32 split (kind::tf32) everywhere
 # "fp32_ffma": the same arithmetic on CUDA cores (FFMA), kept as the in-library cross-check
 # "bf16"     : bf16 operands on the tensor cores

@@ -28,6 +28,7 @@
 #include <cuda_fp16.h>
 #include <stdlib.h>
 #include <type_traits>
+#include <utility>
 
 #include "jacobi.cuh"
 #include "ptx.cuh"
@@ -194,7 +195,6 @@ struct TcGemmParams {
   int relu;
   int out_mode;           // kOutRows / kOutDeconv or kOutPlanar (fp32)
   int planar_deconv;      // kOutPlanar of a kTapDeconv launch: output phase g scattered to (2y + g/2, 2x + g%2) of a 2H x 2W map
-  int split_store;        // kOutRows + kFmtF16P: planes leave as two 16-row boxes through the two halves of the staging buffer
   int num_tiles;
 };
 
@@ -333,42 +333,10 @@ __device__ __forceinline__ void tma_store_block(const TcGemmParams& p, const voi
                       words[4 * j + 3]);
   ptx::fence_proxy_async();
   __syncwarp();
-#ifndef CDR_EXP_NO_TMASTORE   /* timing experiment only: all epilogue math and staging, no store */
   if (lane == 0) {
     if (p.out_mode == kOutDeconv) ptx::tma_store_5d(tmap, stage, c0, sc.px, sc.x0, sc.py, sc.r0);
     else ptx::tma_store_3d(tmap, stage, c0, sc.m, sc.g);
     ptx::bulk_commit();
-  }
-#endif
-}
-
-// The same for the scaled fp16 hi/lo outputs of row-major layers (kOutRows, OFMT = kFmtF16P), where a warp stores TWO planes
-// through its one 4 KB staging buffer: stored as above, the lo plane had to wait for the TMA engine to finish READING the hi
-// plane's block out of the buffer (ncu source page of out_layer: 13 % of all stall samples on that wait, every tile).  Here
-// the buffer is two 2 KB halves and every plane leaves as two 16-row boxes (hi rows 0-15 -> half 0, hi rows 16-31 -> half 1,
-// lo rows 0-15 -> half 0, ...): a half is rewritten two stores after it was handed to the TMA engine, so
-// cp.async.bulk.wait_group.read 1 is almost always already satisfied.  The output tensor maps carry a 16-row box.
-__device__ __forceinline__ void tma_store_rows_split(const void* tmap, uint8_t* stage, int lane, const uint32_t (&words)[32],
-                                                     int c0, const StoreCoord& sc) {
-#pragma unroll
-  for (int h = 0; h < 2; ++h) {
-    if (lane == 0) ptx::bulk_wait_read<1>();          // the store that last used THIS half has read it
-    __syncwarp();
-    if ((lane >> 4) == h) {
-      const uint32_t base = ptx::smem_u32(stage) + (uint32_t)h * 2048u + (uint32_t)(lane & 15) * 128u;
-#pragma unroll
-      for (int j = 0; j < 8; ++j)
-        ptx::st_shared_v4(base + (uint32_t)((j ^ (lane & 7)) << 4), words[4 * j], words[4 * j + 1], words[4 * j + 2],
-                          words[4 * j + 3]);
-    }
-    ptx::fence_proxy_async();
-    __syncwarp();
-#ifndef CDR_EXP_NO_TMASTORE
-    if (lane == 0) {
-      ptx::tma_store_3d(tmap, stage + h * 2048, c0, sc.m + 16 * h, sc.g);
-      ptx::bulk_commit();
-    }
-#endif
   }
 }
 
@@ -380,10 +348,7 @@ __device__ __forceinline__ void tma_store_rows_split(const void* tmap, uint8_t* 
 // the reference's own fp32 sits at 5.8e-4 px); chains of 4 gave 1.7e-6 / 1.8e-4 px.  8 halves the number of chunk
 // hand-backs between the MMA issuer and the epilogue warps — what made cta_group::2 pairs lose on the 16-K-block layers
 // (every hand-back crosses the cluster): f16x2 deconv2 / deconv3 on pairs 154 / 600 us with chunks of 4, 132 / 527 with 8.
-#ifndef CDR_SPLIT_CHUNK
-#define CDR_SPLIT_CHUNK 8
-#endif
-constexpr int kSplitChunk = CDR_SPLIT_CHUNK;
+constexpr int kSplitChunk = 8;
 
 // CL = 1: CTA pairs (thread-block clusters of 2).  The two CTAs of a pair work on the two N tiles of the SAME
 // 128-pixel block and output phase, so they need the same A tile: each loads half of it (64 pixels) and
@@ -430,19 +395,13 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
                    const TcGemmParams p) {
   using Cfg = TcCfg<BN, KIND, OFMT, CL>;
   // layers that may carry a residual: the bf16 and the f16x2 -> fp16-plane kernels with BN = 128, one CTA per tile
-  // (CL = 1: the multicast pair shares the A tile, every CTA loads ITS N tile's residual into its own copy of the stage)
-  constexpr bool kResOK = BN == 128 && CL != 2 && ((KIND == kKindBF16 && OFMT == kFmtBF16) || (KIND == kKindF16X2 && OFMT == kFmtF16P));
+  constexpr bool kResOK = CL == 0 && BN == 128 && ((KIND == kKindBF16 && OFMT == kFmtBF16) || (KIND == kKindF16X2 && OFMT == kFmtF16P));
   constexpr int S = Cfg::kStages;
   constexpr int kTcBK = Cfg::kBK;
   constexpr bool kSplit = KIND != kKindBF16;
   constexpr bool kPair2 = CL == 2;
   static_assert(!kPair2 || KIND != kKindTF32X3, "cta_group::2 is wired for the kind::f16 operand kinds");
   static_assert(!kMN || (KIND == kKindF16X2 && BN == 128 && CL == 0), "MN-major operands: f16x2, BN = 128, one CTA per tile");
-#ifdef CDR_EXP_NO_LO
-  constexpr bool kLoadLo = false;   // timing experiment: hi planes only
-#else
-  constexpr bool kLoadLo = kSplit;
-#endif
   constexpr int kEpiWarps = Cfg::kEpiWarps;
   constexpr int kCols = Cfg::kColsPerWarp;       // columns of the tile owned by one epilogue warp
   extern __shared__ uint8_t smem_raw[];
@@ -516,12 +475,6 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     if (kPair2 && cta_rank != 0) ptx::mbar_arrive_cluster(ptx::mapa_u32(ptx::smem_u32(bar), 0));
     else ptx::mbar_arrive(bar);
   };
-  // a residual stage is free again: CL = 1 stages are refilled by BOTH CTAs of the pair (each multicasts half of the next A
-  // tile into both), so empty[s] counts two arrivals — this CTA's epilogue and the peer's, each arriving on both barriers
-  auto release_res_stage = [&](int s) {
-    ptx::mbar_arrive(&empty[s]);
-    if constexpr (CL == 1) ptx::mbar_arrive_cluster(ptx::mapa_u32(ptx::smem_u32(&empty[s]), cta_rank ^ 1u));
-  };
   // ... and do not touch anything the previous kernel wrote (activations, scale slots) before it is complete
   ptx::grid_dep_wait();
   const uint32_t tmem_base = *tmem_base_slot;
@@ -591,13 +544,13 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
               if (cta_rank == 0) ptx::mbar_arrive_expect_tx(&full[s], 2 * Cfg::kStageBytes);
               if (p.a4d) {
                 ptx::tma_load_4d_2sm(stage_a(s, 0), &tmap_a, full_leader, k0, dx, ys, img0);
-                if (kLoadLo) ptx::tma_load_4d_2sm(stage_a(s, 1), &tmap_a_lo, full_leader, k0, dx, ys, img0);
+                if (kSplit) ptx::tma_load_4d_2sm(stage_a(s, 1), &tmap_a_lo, full_leader, k0, dx, ys, img0);
               } else {
                 ptx::tma_load_2d_2sm(stage_a(s, 0), &tmap_a, full_leader, k0, arow);
-                if (kLoadLo) ptx::tma_load_2d_2sm(stage_a(s, 1), &tmap_a_lo, full_leader, k0, arow);
+                if (kSplit) ptx::tma_load_2d_2sm(stage_a(s, 1), &tmap_a_lo, full_leader, k0, arow);
               }
               ptx::tma_load_2d_2sm(stage_b(s, 0), &tmap_b, full_leader, bk, brow);
-              if (kLoadLo) ptx::tma_load_2d_2sm(stage_b(s, 1), &tmap_b_lo, full_leader, bk, brow);
+              if (kSplit) ptx::tma_load_2d_2sm(stage_b(s, 1), &tmap_b_lo, full_leader, bk, brow);
             }
           } else {
             // CL = 1: my half of the A tile (64 pixels = 8 KB per plane), delivered to both CTAs of the pair
@@ -606,28 +559,24 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
             const uint32_t off = CL == 1 ? cta_rank * (uint32_t)(kABytes / 2) : 0u;
             const int arow_h = arow + (CL == 1 ? (int)cta_rank * (kTcBM / 2) : 0);
             if (ptx::elect_one()) {
-#ifdef CDR_EXP_NO_LO
-              ptx::mbar_arrive_expect_tx(&full[s], Cfg::kStageBytes / (kSplit ? 2 : 1));
-#else
               ptx::mbar_arrive_expect_tx(&full[s], Cfg::kStageBytes);
-#endif
               if (p.a4d) {
                 if constexpr (CL == 1) {
                   ptx::tma_load_4d_mc(stage_a(s, 0) + off, &tmap_a, &full[s], k0, dx, yh, ih, 3);
-                  if (kLoadLo) ptx::tma_load_4d_mc(stage_a(s, 1) + off, &tmap_a_lo, &full[s], k0, dx, yh, ih, 3);
+                  if (kSplit) ptx::tma_load_4d_mc(stage_a(s, 1) + off, &tmap_a_lo, &full[s], k0, dx, yh, ih, 3);
                 } else {
                   ptx::tma_load_4d(stage_a(s, 0), &tmap_a, &full[s], k0, dx, ys, img0);
-                  if (kLoadLo) ptx::tma_load_4d(stage_a(s, 1), &tmap_a_lo, &full[s], k0, dx, ys, img0);
+                  if (kSplit) ptx::tma_load_4d(stage_a(s, 1), &tmap_a_lo, &full[s], k0, dx, ys, img0);
                 }
               } else if constexpr (CL == 1) {
                 ptx::tma_load_2d_mc(stage_a(s, 0) + off, &tmap_a, &full[s], k0, arow_h, 3);
-                if (kLoadLo) ptx::tma_load_2d_mc(stage_a(s, 1) + off, &tmap_a_lo, &full[s], k0, arow_h, 3);
+                if (kSplit) ptx::tma_load_2d_mc(stage_a(s, 1) + off, &tmap_a_lo, &full[s], k0, arow_h, 3);
               } else {
                 ptx::tma_load_2d(stage_a(s, 0), &tmap_a, &full[s], k0, arow);
-                if (kLoadLo) ptx::tma_load_2d(stage_a(s, 1), &tmap_a_lo, &full[s], k0, arow);
+                if (kSplit) ptx::tma_load_2d(stage_a(s, 1), &tmap_a_lo, &full[s], k0, arow);
               }
               ptx::tma_load_2d(stage_b(s, 0), &tmap_b, &full[s], bk, brow);
-              if (kLoadLo) ptx::tma_load_2d(stage_b(s, 1), &tmap_b_lo, &full[s], bk, brow);
+              if (kSplit) ptx::tma_load_2d(stage_b(s, 1), &tmap_b_lo, &full[s], bk, brow);
             }
           }
           __syncwarp();
@@ -733,10 +682,8 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {        // K step = 8 tf32 / 16 f16 = 32 bytes (kMN: 2 KB)
                   const uint64_t o = kStep * (uint64_t)k;
-#ifndef CDR_EXP_NO_CORR   /* timing experiment only: results are wrong without the correction terms */
                   mma(d_corr, dal + o, db + o, k ? 1u : first);            // lo*hi  } whole-tile chain: these
                   mma(d_corr, da + o, dbl + o, 1u);                        // hi*lo  } terms are 2^-11 of the main one
-#endif
                   mma(d_main, da + o, db + o, k ? 1u : first_main);        // hi*hi, short chain
                 }
                 release_stage(s);
@@ -825,9 +772,6 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
       bool res_in_smem = false;
       auto emit = [&](const float (&a32)[32], int c, auto half_c, uint32_t (&wh)[32], uint32_t (&wl)[32]) {
         constexpr int half = decltype(half_c)::value;     // which 32-column half of a 64-column store block
-#ifdef CDR_EXP_NO_STORE   /* timing experiment only: the epilogue drains TMEM but neither converts nor stores */
-        if (a32[0] != 12345.678f) return;
-#endif
         // c = column inside the warp's range; TMA path gathers two slabs (64 columns) per store
         if (!use_tma) {
           store_slab<KIND, OFMT>(p, a32, n0 + c, g, row_ok, orow, img, pix, HW, bias, wsi, es);
@@ -873,14 +817,9 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
           if (half == 1) {
             const int c0 = n0 + c - 32;            // first channel of the 64-column block
             if (c0 < p.c_fill) {
-              if (OFMT == kFmtF16P && p.split_store) {
-                tma_store_rows_split(&tmap_c, stage, lane, wh, c0, sc);
-                tma_store_rows_split(&tmap_c_lo, stage, lane, wl, c0, sc);
-              } else {
-                tma_store_block<Cfg::kStageBufs - 1>(p, &tmap_c, stage + sbuf * kStageBufBytes, lane, wh, c0, sc);
-                if constexpr (Cfg::kStageBufs > 1) sbuf ^= 1;
-                if constexpr (OFMT == kFmtF16P) tma_store_block<0>(p, &tmap_c_lo, stage, lane, wl, c0, sc);
-              }
+              tma_store_block<Cfg::kStageBufs - 1>(p, &tmap_c, stage + sbuf * kStageBufBytes, lane, wh, c0, sc);
+              if constexpr (Cfg::kStageBufs > 1) sbuf ^= 1;
+              if constexpr (OFMT == kFmtF16P) tma_store_block<0>(p, &tmap_c_lo, stage, lane, wl, c0, sc);
             }
           }
         }
@@ -920,7 +859,7 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
               __syncwarp();
               if (lane == 0 && atomicAdd(&res_cnt[s], 1u) == (uint32_t)(kEpiWarps - 1)) {
                 res_cnt[s] = 0;
-                release_res_stage(s);              // last of the 8 warps hands the stage back to the producer(s)
+                ptx::mbar_arrive(&empty[s]);       // last of the 8 warps hands the stage back to the producer
               }
               ++it_e;
             }
@@ -1015,7 +954,7 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
             __syncwarp();
             if (lane == 0 && atomicAdd(&res_cnt[res_stage], 1u) == (uint32_t)(kEpiWarps - 1)) {
               res_cnt[res_stage] = 0;
-              release_res_stage(res_stage);            // last of the 8 warps hands the stage back to the producer(s)
+              ptx::mbar_arrive(&empty[res_stage]);     // last of the 8 warps hands the stage back to the producer
             }
           }
         }
@@ -1058,17 +997,10 @@ struct TcLayer {            // one packed conv: K-major B operand (1 plane bf16 
   int rows = 0, k = 0, k_pitch = 0, bn = 0, n_pad = 0;
 };
 // Pack modes (TcWeights.kind): 0 = every layer bf16, 1 = every layer 3xTF32,
-// 2 = "hybrid" fp32: fusion block 3xTF32 (its activations carry P's 1e5 dynamic range between
-//     the two FTLs, and it is 5 % of the FLOPs), decoder f16x2.
-enum TcMode { kModeBF16 = 0, kModeTF32X3 = 1, kModeHybrid = 2 };
-// hybrid (the library's "fp32" precision): the whole fusion block runs on scaled fp16 hi/lo planes like the decoder
-// (half the MMA time of 3xTF32); CDR_FUSION_F16=0 at pack time keeps conv_layer2 / out_layer on 3xTF32 (A/B, cross-check)
-static bool tc_fusion_f16() {
-  const char* e = getenv("CDR_FUSION_F16");
-  return !(e && e[0] == '0');
-}
-static inline int mode_fusion_kind(int mode) { return mode == kModeBF16 ? kKindBF16 : kKindTF32X3; }
-static inline int mode_decoder_kind(int mode) {
+// 2 = every layer f16x2 (the library's "fp32" precision): the fusion block and the decoder run on scaled fp16 hi/lo
+//     planes (half the MMA time of 3xTF32).
+enum TcMode { kModeBF16 = 0, kModeTF32X3 = 1, kModeF16X2 = 2 };
+static inline int mode_kind(int mode) {
   return mode == kModeBF16 ? kKindBF16 : mode == kModeTF32X3 ? kKindTF32X3 : kKindF16X2;
 }
 static inline int kind_fmt(int kind) {
@@ -1076,7 +1008,6 @@ static inline int kind_fmt(int kind) {
 }
 struct TcPack {
   int mode = kModeBF16;
-  int fusion_kind = kKindBF16;     // kind of conv_layer2 / out_layer (and of every fusion activation but x0)
   TcLayer cf1, cf2a, cf2b, out, dc[3], fin;
 };
 struct Act {                // an activation buffer: 1 plane (bf16) or hi/lo planes
@@ -1113,7 +1044,6 @@ struct TcLaunch {
   int c_pitch, c_fill, relu, out_mode;
   ScaleSlot in_slot, out_slot;   // kFmtF16P tensors
   const float* in_row_scale;     // overrides in_slot.scale: one scale per A row (2-D A)
-  const float* amax_in;          // overrides in_slot.amax (input stored in another format)
   // encoder convs: H, W above are the OUTPUT pixel grid; the input grid is (stride*H, stride*W)
   int conv3;                     // 3x3, pad 1 (9 taps)
   int conv4s2;                   // 4x4, stride 2 (set stride = 2), pad 1 (16 taps)
@@ -1126,55 +1056,47 @@ struct TcLaunch {
   int pair2;                     // run as cta_group::2 CTA pairs (kernel parameter CL = 2) if the geometry allows
 };
 
-// Programmatic dependent launch of consecutive tap-GEMMs (CDR_PDL=0 turns it off for A/B timing).  Measured on
-// B200: encoder 4.58 -> 4.39 ms, bf16 head 94.9 k -> 97.7 k pairs/s.
-static bool tc_use_pdl() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("CDR_PDL");
-    v = (e && e[0] == '0') ? 0 : 1;
+// The tap-GEMM, decoder-tail and merge kernels are launched with programmatic dependent launch (PDL): the next kernel's
+// CTAs take over SMs as ours retire.  Measured on B200: encoder 4.58 -> 4.39 ms, bf16 head 94.9 k -> 97.7 k pairs/s.  `pair`: thread-block clusters
+// of 2 CTAs (multicast pairs, cta_group::2 pairs).
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t smem, bool pair, cudaStream_t st,
+                              Args&&... args) {
+  cudaLaunchAttribute attr[2];
+  int n_attr = 0;
+  if (pair) {
+    attr[n_attr].id = cudaLaunchAttributeClusterDimension;
+    attr[n_attr].val.clusterDim.x = 2;
+    attr[n_attr].val.clusterDim.y = 1;
+    attr[n_attr].val.clusterDim.z = 1;
+    ++n_attr;
   }
-  return v == 1;
+  attr[n_attr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[n_attr].val.programmaticStreamSerializationAllowed = 1;
+  ++n_attr;
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(block);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cfg.attrs = attr;
+  cfg.numAttrs = n_attr;
+  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
-// fp16-plane row outputs as two 16-row boxes per warp and plane (tma_store_rows_split): built, parity-green, MEASURED SLOWER
-// (f16x2 encoder 10.66 -> 10.92 ms, out_layer 43.3 -> 45.3 us: twice the store instructions and half-warp staging writes cost
-// more than the hidden buffer wait returns); opt-in for A/B timing with CDR_SPLIT_STORE=1
-static bool tc_use_split_store() {
-  const char* e = getenv("CDR_SPLIT_STORE");
-  return e && e[0] == '1';
-}
-// CTA pairs with a multicast A tile (kernel template parameter CL): CDR_CLUSTER=0 turns them off for A/B timing
-static bool tc_use_cluster() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("CDR_CLUSTER");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v == 1;
-}
-// cta_group::2 pairs (kernel template parameter CL = 2): CDR_CTA_PAIR=0 turns them off for A/B timing.  The pair takes
-// two consecutive 128-pixel blocks: an even number of pixel blocks, no residual, unit stride.
-// Where they pay (measured, see the kernel comment) the caller asks for them with TcLaunch::pair2; CDR_CTA_PAIR=0 turns
-// them off, CDR_CTA_PAIR=1 forces them on every eligible launch.
+// cta_group::2 pairs (kernel template parameter CL = 2).  The pair takes two consecutive 128-pixel blocks: an even number
+// of pixel blocks, no residual, unit stride.  Where they pay (measured, see the kernel comment) the caller asks for them
+// with TcLaunch::pair2.
 static bool tc_pair2_ok(const TcLaunch& l) {
-  const char* e = getenv("CDR_CTA_PAIR");
-  if (e && e[0] == '0') return false;
-  if (!(l.pair2 || (e && e[0] == '1')) || l.res || l.stride > 1) return false;
+  if (!l.pair2 || l.res || l.stride > 1) return false;
   const long long m = (long long)l.n_img * l.H * l.W;
   return m % (2 * kTcBM) == 0;
 }
-// can this launch run as CTA pairs?  the pair shares one A tile: an even number of N tiles per pixel block
+// can this launch run as multicast CTA pairs (CL = 1)?  the pair shares one A tile: an even number of N tiles per pixel
+// block.  Not for residual layers (DESIGN.md §7: measured slower, the pair runs in lock step and a residual stage is only
+// free once BOTH epilogues have read theirs).
 static bool tc_cluster_ok(const TcLaunch& l, int bn) {
-  if (!tc_use_cluster() || l.stride > 1 || (l.layer->n_pad / bn) % 2 != 0) return false;
-  if (l.res) {
-    // residual layers (the encoder's 1x1 projections) as multicast pairs: built, parity-green, and MEASURED SLOWER —
-    // ResNet-101, 128 images: f16x2 encoder 10.99 -> 11.43 ms, bf16 4.56 -> 5.10 ms (layer3 conv3 100 -> 114 us / 39 -> 51 us):
-    // the pair runs in lock step and a residual stage is only free once BOTH epilogues have read theirs.  Opt-in for A/B
-    // timing with CDR_RES_CLUSTER=1.
-    const char* e = getenv("CDR_RES_CLUSTER");
-    if (!(e && e[0] == '1')) return false;
-  }
+  if (l.res || l.stride > 1 || (l.layer->n_pad / bn) % 2 != 0) return false;
   if (l.deconv || l.conv3) {
     if (l.W > kTcBM || kTcBM % l.W != 0) return false;
     int rows = kTcBM / l.W;
@@ -1223,7 +1145,7 @@ static int launch_tc_t(const TcLaunch& l, cudaStream_t st) {
   p.wsi = l.layer->wsi; p.wsi_group_stride = l.b_group_rows;
   p.scale_in = l.in_slot.scale;
   p.scale_in_rows = l.in_row_scale;
-  p.amax_in = l.amax_in ? l.amax_in : l.in_slot.amax;
+  p.amax_in = l.in_slot.amax;
   p.norms = l.layer->norms;
   p.amax_out = l.out_slot.amax; p.scale_out = l.out_slot.scale;
   const int m_tiles = ceil_div(p.M, kTcBM);
@@ -1299,8 +1221,7 @@ static int launch_tc_t(const TcLaunch& l, cudaStream_t st) {
         CDR_CHECK_ARG(gs % 8 == 0, "tap_gemm_tc: output group stride must be a 16-byte multiple");
         const uint64_t dims[3] = {(uint64_t)l.c_fill, (uint64_t)p.M, (uint64_t)l.groups};
         const uint64_t strides[2] = {(uint64_t)l.c_pitch, gs};
-        p.split_store = OFMT == kFmtF16P && tc_use_split_store();
-        const uint32_t box[3] = {64, p.split_store ? 16u : 32u, 1};       // fp16 planes: two 16-row boxes per warp and plane
+        const uint32_t box[3] = {64, 32, 1};
         if (int rc = make_tmap(&tmap_c[pl], l.C.p[pl], OFMT, 3, dims, strides, box)) return rc;
       }
     }
@@ -1337,33 +1258,14 @@ static int launch_tc_t(const TcLaunch& l, cudaStream_t st) {
   }
   int grid = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
   if (CL == 2) grid = 2 * p.num_tiles < num_sms() ? 2 * p.num_tiles : num_sms();     // two CTAs per pair tile
-  cudaLaunchConfig_t cfg{};
-  cudaLaunchAttribute attr[2];
-  int n_attr = 0;
   if (CL) {
     // CL = 1: CTA 2i / 2i+1 take tiles t / t+1 = the two N tiles of one pixel block, for the same number of rounds
     if (CL == 1)
       CDR_CHECK_ARG(p.n_tiles % 2 == 0, "tap_gemm_tc: CTA pairs need an even number of N tiles");
     grid &= ~1;
-    attr[n_attr].id = cudaLaunchAttributeClusterDimension;
-    attr[n_attr].val.clusterDim.x = 2;
-    attr[n_attr].val.clusterDim.y = 1;
-    attr[n_attr].val.clusterDim.z = 1;
-    ++n_attr;
   }
-  if (tc_use_pdl()) {
-    attr[n_attr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n_attr].val.programmaticStreamSerializationAllowed = 1;
-    ++n_attr;
-  }
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(Cfg::kThreads);
-  cfg.dynamicSmemBytes = Cfg::kSmemBytes;
-  cfg.stream = st;
-  cfg.attrs = attr;
-  cfg.numAttrs = n_attr;
-  CDR_CUDA(cudaLaunchKernelEx(&cfg, tap_gemm_tc_kernel<BN, KIND, OFMT, CL>, tmap_a[0], tmap_a[1], tmap_b[0], tmap_b[1],
-                              tmap_c[0], tmap_c[1], tmap_r, tmap_r_lo, p));
+  CDR_CUDA(launch_pdl(tap_gemm_tc_kernel<BN, KIND, OFMT, CL>, grid, Cfg::kThreads, Cfg::kSmemBytes, CL != 0, st, tmap_a[0],
+                      tmap_a[1], tmap_b[0], tmap_b[1], tmap_c[0], tmap_c[1], tmap_r, tmap_r_lo, p));
   CDR_LAUNCH_OK("tap_gemm_tc_kernel");
   return CDR_OK;
 }
@@ -1374,17 +1276,12 @@ static int launch_tc(const TcLaunch& l, cudaStream_t st) {
   if (kind == kKindBF16 && ofmt == kFmtBF16) {
     if (bn == 256 && tc_pair2_ok(l)) return launch_tc_t<256, kKindBF16, kFmtBF16, 2>(l, st);
     if (bn == 256) return launch_tc_t<256, kKindBF16, kFmtBF16>(l, st);
-    if (bn == 128 && l.res && tc_cluster_ok(l, bn)) return launch_tc_t<128, kKindBF16, kFmtBF16, 1>(l, st);
     if (bn == 128) return launch_tc_t<128, kKindBF16, kFmtBF16>(l, st);
     if (bn == 64) return launch_tc_t<64, kKindBF16, kFmtBF16>(l, st);
     if (bn == 32) return launch_tc_t<32, kKindBF16, kFmtBF16>(l, st);
   } else if (kind == kKindTF32X3 && ofmt == kFmtTF32P) {
     if (bn == 128) return launch_tc_t<128, kKindTF32X3, kFmtTF32P>(l, st);
     if (bn == 32) return launch_tc_t<32, kKindTF32X3, kFmtTF32P>(l, st);
-  } else if (kind == kKindTF32X3 && ofmt == kFmtF16P) {
-    if (bn == 128) return launch_tc_t<128, kKindTF32X3, kFmtF16P>(l, st);
-  } else if (kind == kKindF16X2 && ofmt == kFmtTF32P) {
-    if (bn == 128) return launch_tc_t<128, kKindF16X2, kFmtTF32P>(l, st);
   } else if (kind == kKindF16X2 && ofmt == kFmtF16P) {
     if (bn == 128 && tc_pair2_ok(l)) return launch_tc_t<128, kKindF16X2, kFmtF16P, 2>(l, st);
     if (bn == 128 && tc_cluster_ok(l, bn)) return launch_tc_t<128, kKindF16X2, kFmtF16P, 1>(l, st);
@@ -1402,7 +1299,7 @@ static int launch_tc(const TcLaunch& l, cudaStream_t st) {
 #include "tail_pair_tc.cuh"
 namespace cdr {
 
-// CDR_FUSED_TAIL=0 keeps deconv3 / final 1x1 / soft-argmax as three launches (A/B timing, cross-check).  Read at
+// CDR_FUSED_TAIL=0 keeps deconv3 / final 1x1 / soft-argmax as three launches (the tests' reference for the fused tail).  Read at
 // every forward (one getenv) so a test can compare both paths inside one process.
 static bool tc_use_fused_tail() {
   const char* e = getenv("CDR_FUSED_TAIL");
@@ -1419,106 +1316,68 @@ struct TailLaunch {
   float4* part;             // optional soft-argmax partial records
 };
 
-template <int KIND>
-static int launch_tail_t(const TailLaunch& l, cudaStream_t st) {
-  using Cfg = TailCfg<KIND>;
-  constexpr int kAFmt = KindTraits<KIND>::kFmt;
+// bf16: the single-CTA kernel of tail_tc.cuh
+static int launch_tail(const TailLaunch& l, cudaStream_t st) {
+  using Cfg = TailCfg;
   static DeviceOnce attr_set;
   if (attr_set.need()) {
-    CDR_CUDA(cudaFuncSetAttribute(deconv_tail_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)TailSmem<KIND>::kBytes));
+    CDR_CUDA(cudaFuncSetAttribute(deconv_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
     attr_set.done();
   }
-  CDR_CHECK_ARG(l.A.fmt == kAFmt && l.dc3->kind == KIND && l.fin->kind == KIND && l.dc3->bn == Cfg::kBN &&
+  CDR_CHECK_ARG(l.A.fmt == kFmtBF16 && l.dc3->kind == kKindBF16 && l.fin->kind == kKindBF16 && l.dc3->bn == Cfg::kBN &&
                     l.fin->n_pad == 32 && l.joints <= 32 && (l.heat || l.part),
                 "deconv_tail: operand formats / packing do not match the kernel");
-  CUtensorMap tmap_a[2];
-  for (int pl = 0; pl < Cfg::kPlanes; ++pl) {
+  CUtensorMap tmap_a;
+  {
     const uint64_t dims[4] = {(uint64_t)kDecC, 32, 32, (uint64_t)l.n_img};
     const uint64_t strides[3] = {(uint64_t)kDecC, (uint64_t)kDecC * 32, (uint64_t)kDecC * 1024};
     const uint32_t box[4] = {64, 32, 4, 1};
-    if (int rc = make_tmap(&tmap_a[pl], l.A.p[pl], kAFmt, 4, dims, strides, box)) return rc;
+    if (int rc = make_tmap(&tmap_a, l.A.p[0], kFmtBF16, 4, dims, strides, box)) return rc;
   }
-  if (Cfg::kPlanes == 1) tmap_a[1] = tmap_a[0];
   TailParams p{};
   p.n_img = l.n_img;
   p.num_units = (l.n_img * 1024 / kTcBM) * 4;
   p.joints = l.joints;
   p.bias = l.dc3->bias;
-  p.wsi = l.dc3->wsi;
-  p.scale_in = l.in_slot.scale;
-  p.amax_in = l.in_slot.amax;
-  p.norms = l.dc3->norms;
   p.bias_fin = l.fin->bias;
-  p.wsi_fin = l.fin->wsi;
   p.heat = l.heat;
   p.part = l.part;
-  if (KIND == kKindF16X2)
-    CDR_CHECK_ARG(p.wsi && p.scale_in && p.amax_in && p.norms && p.wsi_fin, "deconv_tail: f16x2 operands need their scales");
   const int grid = p.num_units < num_sms() ? p.num_units : num_sms();
-  cudaLaunchConfig_t cfg{};
-  cudaLaunchAttribute attr[1];
-  int n_attr = 0;
-  if (tc_use_pdl()) {
-    attr[n_attr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n_attr].val.programmaticStreamSerializationAllowed = 1;
-    ++n_attr;
-  }
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(kTailThreads);
-  cfg.dynamicSmemBytes = TailSmem<KIND>::kBytes;
-  cfg.stream = st;
-  cfg.attrs = attr;
-  cfg.numAttrs = n_attr;
-  CDR_CUDA(cudaLaunchKernelEx(&cfg, deconv_tail_kernel<KIND>, tmap_a[0], tmap_a[1], l.dc3->map[0],
-                              l.dc3->map[Cfg::kPlanes - 1], l.fin->map[0], l.fin->map[Cfg::kPlanes - 1], p));
+  CDR_CUDA(launch_pdl(deconv_tail_kernel, grid, kTailThreads, Cfg::kSmemBytes, false, st, tmap_a, l.dc3->map[0],
+                      l.fin->map[0], p));
   CDR_LAUNCH_OK("deconv_tail_kernel");
   return CDR_OK;
 }
 
-// The same on cta_group::2 CTA pairs (tail_pair_tc.cuh).  Measured on B200 at B = 64: f16x2 653 -> 556 us; bf16 200 -> 203 us
-// (its tile is 256 channels wide — operand reads were never its limit), so bf16 stays on the single-CTA kernel.
-// CDR_TAIL_PAIR=0 / 1 forces the single-CTA / the pair kernel for both kinds.
-static bool tc_use_tail_pair(int kind) {
-  const char* e = getenv("CDR_TAIL_PAIR");
-  if (e && (e[0] == '0' || e[0] == '1')) return e[0] == '1';
-  return kind == kKindF16X2;
-}
-
-template <int KIND>
-static int launch_tail_pair_t(const TailLaunch& l, cudaStream_t st) {
-  using Cfg = TailPairCfg<KIND>;
-  constexpr int kAFmt = KindTraits<KIND>::kFmt;
+// f16x2: the same on cta_group::2 CTA pairs (tail_pair_tc.cuh).  Measured on B200 at B = 64: f16x2 653 -> 556 us; the bf16
+// tail on pairs went 200 -> 203 us (its tile is 256 channels wide — operand reads were never its limit).
+static int launch_tail_pair(const TailLaunch& l, cudaStream_t st) {
+  using Cfg = TailPairCfg;
   static DeviceOnce attr_set;
   if (attr_set.need()) {
-    CDR_CUDA(cudaFuncSetAttribute(deconv_tail_pair_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)TailPairSmem<KIND>::kBytes));
+    CDR_CUDA(cudaFuncSetAttribute(deconv_tail_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
     attr_set.done();
   }
-  CDR_CHECK_ARG(l.A.fmt == kAFmt && l.dc3->kind == KIND && l.fin->kind == KIND && l.dc3->bn == Cfg::kBN &&
+  CDR_CHECK_ARG(l.A.fmt == kFmtF16P && l.dc3->kind == kKindF16X2 && l.fin->kind == kKindF16X2 && l.dc3->bn == Cfg::kBN &&
                     l.fin->n_pad == 32 && l.joints <= 32 && (l.heat || l.part),
                 "deconv_tail_pair: operand formats / packing do not match the kernel");
   CUtensorMap tmap_a[2], tmap_b[2], tmap_w16;
-  for (int pl = 0; pl < Cfg::kPlanes; ++pl) {
+  for (int pl = 0; pl < 2; ++pl) {
     const uint64_t dims[4] = {(uint64_t)kDecC, 32, 32, (uint64_t)l.n_img};
     const uint64_t strides[3] = {(uint64_t)kDecC, (uint64_t)kDecC * 32, (uint64_t)kDecC * 1024};
     const uint32_t box[4] = {64, 32, 4, 1};
-    if (int rc = make_tmap(&tmap_a[pl], l.A.p[pl], kAFmt, 4, dims, strides, box)) return rc;
+    if (int rc = make_tmap(&tmap_a[pl], l.A.p[pl], kFmtF16P, 4, dims, strides, box)) return rc;
     // each CTA of the pair stages half of the weight tile: a box of BN/2 rows
     const uint64_t bdims[2] = {(uint64_t)l.dc3->k, (uint64_t)l.dc3->rows};
     const uint64_t bstr[1] = {(uint64_t)l.dc3->k_pitch};
     const uint32_t bbox[2] = {64, (uint32_t)(Cfg::kBN / 2)};
-    if (int rc = make_tmap(&tmap_b[pl], l.dc3->w[pl], kAFmt, 2, bdims, bstr, bbox)) return rc;
-  }
-  if (Cfg::kPlanes == 1) {
-    tmap_a[1] = tmap_a[0];
-    tmap_b[1] = tmap_b[0];
+    if (int rc = make_tmap(&tmap_b[pl], l.dc3->w[pl], kFmtF16P, 2, bdims, bstr, bbox)) return rc;
   }
   {   // 16-row boxes of the final layer's (hi) plane: each CTA's half of an N = 32 operand
     const uint64_t dims[2] = {(uint64_t)l.fin->k, (uint64_t)l.fin->rows};
     const uint64_t strides[1] = {(uint64_t)l.fin->k_pitch};
     const uint32_t box[2] = {64, 16};
-    if (int rc = make_tmap(&tmap_w16, l.fin->w[0], kAFmt, 2, dims, strides, box)) return rc;
+    if (int rc = make_tmap(&tmap_w16, l.fin->w[0], kFmtF16P, 2, dims, strides, box)) return rc;
   }
   TailParams p{};
   p.n_img = l.n_img;
@@ -1533,31 +1392,11 @@ static int launch_tail_pair_t(const TailLaunch& l, cudaStream_t st) {
   p.wsi_fin = l.fin->wsi;
   p.heat = l.heat;
   p.part = l.part;
-  if (KIND == kKindF16X2)
-    CDR_CHECK_ARG(p.wsi && p.scale_in && p.amax_in && p.norms && p.wsi_fin, "deconv_tail_pair: f16x2 operands need their scales");
+  CDR_CHECK_ARG(p.wsi && p.scale_in && p.amax_in && p.norms && p.wsi_fin, "deconv_tail_pair: f16x2 operands need their scales");
   int grid = p.num_units < num_sms() ? p.num_units : num_sms();
   grid &= ~1;
-  cudaLaunchConfig_t cfg{};
-  cudaLaunchAttribute attr[2];
-  int n_attr = 0;
-  attr[n_attr].id = cudaLaunchAttributeClusterDimension;
-  attr[n_attr].val.clusterDim.x = 2;
-  attr[n_attr].val.clusterDim.y = 1;
-  attr[n_attr].val.clusterDim.z = 1;
-  ++n_attr;
-  if (tc_use_pdl()) {
-    attr[n_attr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n_attr].val.programmaticStreamSerializationAllowed = 1;
-    ++n_attr;
-  }
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(kTailThreads);
-  cfg.dynamicSmemBytes = TailPairSmem<KIND>::kBytes;
-  cfg.stream = st;
-  cfg.attrs = attr;
-  cfg.numAttrs = n_attr;
-  CDR_CUDA(cudaLaunchKernelEx(&cfg, deconv_tail_pair_kernel<KIND>, tmap_a[0], tmap_a[1], tmap_b[0], tmap_b[1], l.fin->map[0],
-                              l.fin->map[Cfg::kPlanes - 1], tmap_w16, p));
+  CDR_CUDA(launch_pdl(deconv_tail_pair_kernel, grid, kTailThreads, Cfg::kSmemBytes, true, st, tmap_a[0], tmap_a[1], tmap_b[0],
+                      tmap_b[1], l.fin->map[0], l.fin->map[1], tmap_w16, p));
   CDR_LAUNCH_OK("deconv_tail_pair_kernel");
   return CDR_OK;
 }
@@ -1570,20 +1409,8 @@ static int launch_tail_merge(const float4* part, const float* P_l, const float* 
   p.kp[0] = kp_l; p.kp[1] = kp_r;
   p.xyz = xyz;
   p.batch = batch; p.joints = joints; p.scale = scale;
-  cudaLaunchConfig_t cfg{};
-  cudaLaunchAttribute attr[1];
-  int n_attr = 0;
-  if (tc_use_pdl()) {           // its launch latency hides behind the tail kernel (which lets dependents launch early)
-    attr[n_attr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n_attr].val.programmaticStreamSerializationAllowed = 1;
-    ++n_attr;
-  }
-  cfg.gridDim = dim3(batch);
-  cfg.blockDim = dim3(32 * (joints < 1 ? 1 : joints > 32 ? 32 : joints));   // a half-warp per heat-map
-  cfg.stream = st;
-  cfg.attrs = attr;
-  cfg.numAttrs = n_attr;
-  CDR_CUDA(cudaLaunchKernelEx(&cfg, tail_merge_dlt_kernel, p));
+  // PDL: its launch latency hides behind the tail kernel (which lets dependents launch early); a half-warp per heat-map
+  CDR_CUDA(launch_pdl(tail_merge_dlt_kernel, batch, 32 * (joints < 1 ? 1 : joints > 32 ? 32 : joints), 0, false, st, p));
   CDR_LAUNCH_OK("tail_merge_dlt_kernel");
   return CDR_OK;
 }
@@ -1647,9 +1474,9 @@ __global__ void pack_deconv_tc_kernel(CdrConvBn s, int cin, int cout, int n_pad,
   store_weight<kSplit>(w0, w1, idx, deconv_weight(s, cin, cout, phase, n, kk));
 }
 
-// One block per packed weight row: max |w| and ||w||_1 of the row (block reduction), then
-//   kWrite: the row scaled by 2^t (max lands in [2^13, 2^14)) as fp16 hi/lo planes, wsi[row] = 2^-t;
-//   always: atomicMax of the row's L1 norm and |bias| into norms[0..1] (the output-scale bound).
+// One block per packed weight row: max |w| and ||w||_1 of the row (block reduction), then the row scaled by 2^t (max lands
+// in [2^13, 2^14)) as fp16 hi/lo planes, wsi[row] = 2^-t, and (norms != NULL) atomicMax of the row's L1 norm and |bias|
+// into norms[0..1] (the output-scale bound).
 // folded weight of a conv (Cout,Cin,kh,kw) with `taps` = kh*kw at packed position (n, tap*Cin + ci), tap = ky*kw + kx
 __device__ __forceinline__ float conv_taps_weight(const CdrConvBn& s, int cout, int cin, int taps, int n, int kk) {
   if (n >= cout || kk >= taps * cin) return 0.f;
@@ -1664,7 +1491,7 @@ __device__ __forceinline__ float deconv_dgrad_weight(const CdrConvBn& s, int cin
 }
 // kDeconv: 0 = 1x1 conv, 1 = transposed conv (4 phases), >= 2: conv with kDeconv taps in encoder order (use 9; the 1x1
 // convs of the encoder go through mode 0), -1: deconv_dgrad_weight (`cout` = Cin rows, `cin` = Cout per tap)
-template <int kDeconv, bool kWrite>
+template <int kDeconv>
 __global__ void __launch_bounds__(256)
 pack_rows_f16_kernel(CdrConvBn s, int cout, int cin, int k_pitch, int n_pad, __half* __restrict__ w_hi,
                      __half* __restrict__ w_lo, float* __restrict__ wsi, float* __restrict__ bias_out,
@@ -1702,16 +1529,13 @@ pack_rows_f16_kernel(CdrConvBn s, int cout, int cin, int k_pitch, int n_pad, __h
   const int t = f16_pow2_exp(mx);
   if (threadIdx.x == 0) {
     const float b = n < cout ? tc_folded_bias(s, n) : 0.f;
-    if (kWrite) {
-      wsi[row] = ldexpf(1.f, -t);
-      if (phase == 0) bias_out[n] = b;
-    }
+    wsi[row] = ldexpf(1.f, -t);
+    if (phase == 0) bias_out[n] = b;
     if (norms) {
       atomicMax(reinterpret_cast<unsigned int*>(norms), __float_as_uint(l1 * 1.001f));   // non-negative floats
       atomicMax(reinterpret_cast<unsigned int*>(norms + 1), __float_as_uint(fabsf(b)));
     }
   }
-  if (!kWrite) return;
   const float up = ldexpf(1.f, t);
   for (int kk = threadIdx.x; kk < k_pitch; kk += blockDim.x) {
     const float X = val(kk) * up;
@@ -1767,27 +1591,20 @@ static void plan_layer(TcLayer& L, Bump1K& b, int kind, int rows, int k, int k_p
 
 static size_t plan_tc_weights(TcPack& pk, const TcWeights& w, void* base) {
   Bump1K b(base);
-  if (!base) pk.fusion_kind = pk.mode == kModeHybrid && tc_fusion_f16() ? kKindF16X2 : mode_fusion_kind(pk.mode);
-  const int fk = pk.fusion_kind, dk = mode_decoder_kind(pk.mode);
-  const int bn_f = fk == kKindBF16 ? 256 : 128;
-  int bn_d = dk == kKindBF16 ? 256 : 128;
-  if (const char* e = getenv("CDR_BF16_DECONV_BN"))     // experiment knob: UMMA N = 128 vs 256 at equal math
-    if (dk == kKindBF16 && atoi(e) == 128) bn_d = 128;
-  const bool scaled = dk == kKindF16X2;          // outputs feeding the decoder are stored in kFmtF16P
+  const int k = mode_kind(pk.mode);
+  const int bn = k == kKindBF16 ? 256 : 128;
+  const bool f16 = k == kKindF16X2;        // every output but the heat-maps is stored in kFmtF16P: each layer needs its norms
   if (w.has_fusion) {
-    // conv_layer1 reads the encoder's latents (post-ReLU, bounded): in hybrid mode it runs f16x2 like the
-    // decoder (half the MMA time of 3xTF32 at K = 2048); its output feeds the FTL, so it stays tf32 planes
-    const bool f16 = fk == kKindF16X2;      // every fusion output is stored in kFmtF16P: each layer needs its norms
     const FusionDims& fd = w.fd;
     const int n1 = fd.n1_pad(), n2 = fd.n2_pad();
-    plan_layer(pk.cf1, b, pk.mode == kModeHybrid ? kKindF16X2 : fk, n1, kFeatC, kFeatC, 128, n1, n1, f16);
-    plan_layer(pk.cf2a, b, fk, n2, 2 * fd.h2, 2 * fd.h2, 128, n2, n2, f16);
-    plan_layer(pk.cf2b, b, fk, n2, fd.h2, fd.h2, 128, n2, n2, f16);
-    plan_layer(pk.out, b, fk, 2 * kFeatC, fd.h1, fd.h1p, bn_f, kFeatC, 2 * kFeatC, scaled);
+    plan_layer(pk.cf1, b, k, n1, kFeatC, kFeatC, 128, n1, n1, f16);
+    plan_layer(pk.cf2a, b, k, n2, 2 * fd.h2, 2 * fd.h2, 128, n2, n2, f16);
+    plan_layer(pk.cf2b, b, k, n2, fd.h2, fd.h2, 128, n2, n2, f16);
+    plan_layer(pk.out, b, k, 2 * kFeatC, fd.h1, fd.h1p, bn, kFeatC, 2 * kFeatC, f16);
   }
   for (int i = 0; i < 3; ++i)
-    plan_layer(pk.dc[i], b, dk, 4 * kDecC, 4 * kTcDcCin[i], 4 * kTcDcCin[i], bn_d, kDecC, kDecC, scaled);
-  plan_layer(pk.fin, b, dk, w.fin_npad, kDecC, kDecC, 32, w.fin_npad, w.fin_npad, false);
+    plan_layer(pk.dc[i], b, k, 4 * kDecC, 4 * kTcDcCin[i], 4 * kTcDcCin[i], bn, kDecC, kDecC, f16);
+  plan_layer(pk.fin, b, k, w.fin_npad, kDecC, kDecC, 32, w.fin_npad, w.fin_npad, false);
   return b.off;
 }
 
@@ -1825,8 +1642,8 @@ int tc_weights_create(const CdrWeightPtrs& src, int mode, TcWeights& w, cudaStre
     void* w1 = L.w[1] ? (uint8_t*)L.w[1] + row_off * L.k_pitch * elem : nullptr;
     const unsigned grid = (unsigned)ceil_div<long long>(total, 256);
     if (L.kind == kKindF16X2) {
-      pack_rows_f16_kernel<0, true><<<rows, 256, 0, st>>>(s, cout, cin, L.k_pitch, rows, (__half*)w0, (__half*)w1,
-                                                              L.wsi + row_off, L.bias + bias_off, L.norms);
+      pack_rows_f16_kernel<0><<<rows, 256, 0, st>>>(s, cout, cin, L.k_pitch, rows, (__half*)w0, (__half*)w1, L.wsi + row_off,
+                                                    L.bias + bias_off, L.norms);
       CDR_LAUNCH_OK("pack_rows_f16_kernel");
       return CDR_OK;
     }
@@ -1835,11 +1652,6 @@ int tc_weights_create(const CdrWeightPtrs& src, int mode, TcWeights& w, cudaStre
     else
       pack_conv1x1_tc_kernel<false><<<grid, 256, 0, st>>>(s, cout, cin, L.k_pitch, rows, w0, w1, L.bias + bias_off);
     CDR_LAUNCH_OK("pack_conv1x1_tc_kernel");
-    if (L.norms) {   // only the norms (the layer itself is not fp16-scaled, its output is)
-      pack_rows_f16_kernel<0, false><<<rows, 256, 0, st>>>(s, cout, cin, L.k_pitch, rows, nullptr, nullptr, nullptr,
-                                                               nullptr, L.norms);
-      CDR_LAUNCH_OK("pack_rows_f16_kernel");
-    }
     return CDR_OK;
   };
   int rc;
@@ -1858,7 +1670,7 @@ int tc_weights_create(const CdrWeightPtrs& src, int mode, TcWeights& w, cudaStre
     TcLayer& L = pk->dc[i];
     const int K = 4 * kTcDcCin[i];
     if (L.kind == kKindF16X2) {
-      pack_rows_f16_kernel<1, true><<<4 * kDecC, 256, 0, st>>>(src.deconv[i], kDecC, kTcDcCin[i], K, kDecC,
+      pack_rows_f16_kernel<1><<<4 * kDecC, 256, 0, st>>>(src.deconv[i], kDecC, kTcDcCin[i], K, kDecC,
                                                                   (__half*)L.w[0], (__half*)L.w[1], L.wsi, L.bias, L.norms);
       CDR_LAUNCH_OK("pack_rows_f16_kernel");
     } else {
@@ -1884,12 +1696,12 @@ void tc_weights_destroy(TcWeights& w) {
 }
 
 // ------------------------------------------------------------------------------------------
-constexpr int kNumSlots = 12;      // ScaleSlot pairs: 0 g (amax only), 1 x1, 2 d1, 3 d2, 4 d3, 5 x0 (hybrid mode);
+constexpr int kNumSlots = 12;      // ScaleSlot pairs: 0 unused, 1 x1, 2 d1, 3 d2, 4 d3, 5 x0 (f16x2 mode);
                                    // fp16 fusion block: 6 y1, 7 z, 8 f1, 9 f2, 10 g, 11 {max row L1 of P+, of P}
 struct TcHeadWs {
   float* pinv;
   float* slots;
-  float* x0_rs;             // hybrid mode: one scale per x0 row (layout.cu: nchw_to_rows_f16p_rowscale_kernel)
+  float* x0_rs;             // f16x2 mode: one scale per x0 row (layout.cu: nchw_to_rows_f16p_rowscale_kernel)
   Act x0, y1, z, f1, f2, g, x1, d1, d2, d3;
   float* hm;
   float4* part;             // fused decoder tail: soft-argmax partial records (2B, J, kTailSlots)
@@ -1908,15 +1720,15 @@ static Act take_act(Bump1K& b, size_t elems, int fmt) {
   a.p[1] = fmt_planes(fmt) == 2 ? b.take(elems * fmt_elem(fmt)) : nullptr;
   return a;
 }
-static TcHeadWs plan_tc_head(void* base, int B, int J, int mode, int fusion_kind, const FusionDims& fd) {
+static TcHeadWs plan_tc_head(void* base, int B, int J, int mode, const FusionDims& fd) {
   Bump1K b(base);
   const size_t N = 2 * (size_t)B;
-  const int ff = kind_fmt(fusion_kind), df = kind_fmt(mode_decoder_kind(mode));
+  const int ff = kind_fmt(mode_kind(mode)), df = ff;
   TcHeadWs w;
   w.pinv = (float*)b.take(N * 12 * sizeof(float));
   w.slots = (float*)b.take(2 * kNumSlots * sizeof(float));
   w.x0_rs = (float*)b.take(N * kFeatHW * sizeof(float));
-  w.x0 = take_act(b, N * kFeatHW * kFeatC, mode == kModeHybrid ? kFmtF16P : ff);
+  w.x0 = take_act(b, N * kFeatHW * kFeatC, ff);
   w.y1 = take_act(b, N * kFeatHW * fd.h1p, ff);
   w.z = take_act(b, (size_t)B * kFeatHW * 2 * fd.h2, ff);
   w.f1 = take_act(b, (size_t)B * kFeatHW * fd.h2, ff);
@@ -1938,7 +1750,7 @@ struct TcDecWs {
 };
 static TcDecWs plan_tc_dec(void* base, int N, int mode) {
   Bump1K b(base);
-  const int df = kind_fmt(mode_decoder_kind(mode));
+  const int df = kind_fmt(mode_kind(mode));
   TcDecWs w;
   w.slots = (float*)b.take(2 * kNumSlots * sizeof(float));
   w.x1 = take_act(b, (size_t)N * kFeatHW * kFeatC, df);
@@ -1950,7 +1762,7 @@ static TcDecWs plan_tc_dec(void* base, int N, int mode) {
 }
 
 int tc_head_workspace_bytes(const TcWeights& w, int batch, size_t* bytes) {
-  *bytes = plan_tc_head(nullptr, batch, w.joints, w.kind, ((const TcPack*)w.impl)->fusion_kind, w.fd).bytes;
+  *bytes = plan_tc_head(nullptr, batch, w.joints, w.kind, w.fd).bytes;
   return CDR_OK;
 }
 int tc_decoder_workspace_bytes(const TcWeights& w, int n_images, size_t* bytes) {
@@ -1961,11 +1773,6 @@ int tc_decoder_workspace_bytes(const TcWeights& w, int n_images, size_t* bytes) 
 // NCHW fp32 latents (one tensor, or two whose rows are stacked: the stereo views) -> pixel-major rows
 // in the format of `out`.  kFmtF16P (single tensor only): the tensor scale comes from the exact amax
 // of the input (one extra pass over 0.5 MB / image).
-// CDR_ROW_SCALE=0: keep the two-launch {amax, transposition} form with one tensor scale (A/B timing, cross-check)
-static bool tc_use_row_scale() {
-  const char* e = getenv("CDR_ROW_SCALE");
-  return !(e && e[0] == '0');
-}
 // *row_scale (in: buffer of n rows or NULL; out: NULL when the tensor-scale form ran)
 static int to_rows(const float* feat, const float* feat2, int n_img, const Act& out, ScaleSlot sl, float** row_scale,
                    cudaStream_t st) {
@@ -1975,7 +1782,7 @@ static int to_rows(const float* feat, const float* feat2, int n_img, const Act& 
     return launch_nchw_to_rows_bf16(feat, feat2, n_img, kFeatC, kFeatHW, (__nv_bfloat16*)out.p[0], kFeatC, st);
   if (out.fmt == kFmtTF32P)
     return launch_nchw_to_rows_split(feat, feat2, n_img, kFeatC, kFeatHW, (float*)out.p[0], (float*)out.p[1], kFeatC, st);
-  if (rs && tc_use_row_scale() && nchw_rowscale_ok(feat, feat2, n_img, kFeatC, kFeatHW, kFeatC)) {
+  if (rs && nchw_rowscale_ok(feat, feat2, n_img, kFeatC, kFeatHW, kFeatC)) {
     *row_scale = rs;
     return launch_nchw_to_rows_f16p_rowscale(feat, feat2, n_img, kFeatC, kFeatHW, out.p[0], out.p[1], kFeatC, rs, sl.amax, st);
   }
@@ -1985,8 +1792,8 @@ static int to_rows(const float* feat, const float* feat2, int n_img, const Act& 
 // FTL of both views in one launch
 // kFmtF16P: in_slot = scale / amax of the input, out_slot = where the output's go, l1max = max row L1 norm of `mats`
 static int ftl_act2(const Act& in0, const Act& in1, int in_pitch, const float* const mats[2], int rows, int cols, int blk, int n,
-                    const Act& out0, const Act& out1, int out_pitch, int out_fill, float* amax_out, ScaleSlot in_slot,
-                    ScaleSlot out_slot, const float* l1max, cudaStream_t st) {
+                    const Act& out0, const Act& out1, int out_pitch, int out_fill, ScaleSlot in_slot, ScaleSlot out_slot,
+                    const float* l1max, cudaStream_t st) {
   if (in0.fmt == kFmtF16P) {
     const void* ih[2] = {in0.p[0], in1.p[0]};
     const void* il[2] = {in0.p[1], in1.p[1]};
@@ -2004,13 +1811,12 @@ static int ftl_act2(const Act& in0, const Act& in1, int in_pitch, const float* c
   const float* il[2] = {(const float*)in0.p[1], (const float*)in1.p[1]};
   float* oh[2] = {(float*)out0.p[0], (float*)out1.p[0]};
   float* ol[2] = {(float*)out0.p[1], (float*)out1.p[1]};
-  return launch_ftl_split2(ih, il, in_pitch, mats, rows, cols, blk, n, kFeatHW, oh, ol, out_pitch, out_fill, 2,
-                           amax_out, st);
+  return launch_ftl_split2(ih, il, in_pitch, mats, rows, cols, blk, n, kFeatHW, oh, ol, out_pitch, out_fill, 2, st);
 }
 
 // Can this pack run deconv3 + final 1x1 (+ soft-argmax partials) as the one kernel of tail_tc.cuh?
 static bool tail_fusable(const TcWeights& w) {
-  const int dk = mode_decoder_kind(w.kind);
+  const int dk = mode_kind(w.kind);
   const TcPack* pk = (const TcPack*)w.impl;
   return tc_use_fused_tail() && (dk == kKindBF16 || dk == kKindF16X2) && w.fin_npad == 32 &&
          pk->dc[2].bn == (dk == kKindBF16 ? 256 : 128);
@@ -2036,7 +1842,7 @@ static int tc_decoder(const TcWeights& w, const Act& x1, int N, const Act& d1, c
     l.C = outs[i]; l.c_pitch = kDecC; l.c_fill = kDecC; l.relu = 1; l.out_mode = kOutDeconv;
     l.in_slot = slot(slots, 1 + i); l.out_slot = slot(slots, 2 + i);
     // cta_group::2 pairs: measured to pay on every bf16 (BN = 256) and f16x2 transposed conv (see the kernel comment)
-    l.pair2 = mode_decoder_kind(w.kind) == kKindBF16 || mode_decoder_kind(w.kind) == kKindF16X2;
+    l.pair2 = mode_kind(w.kind) == kKindBF16 || mode_kind(w.kind) == kKindF16X2;
     if (int rc = launch_tc(l, st)) return rc;
     in = outs[i];
     side *= 2;
@@ -2048,10 +1854,9 @@ static int tc_decoder(const TcWeights& w, const Act& x1, int N, const Act& d1, c
     t.dc3 = &pk->dc[2]; t.fin = &pk->fin;
     t.in_slot = slot(slots, 3);
     t.heat = heat; t.part = part;
-    const bool bf = mode_decoder_kind(w.kind) == kKindBF16;
+    const bool bf = mode_kind(w.kind) == kKindBF16;
     // (n_img * 8 pixel blocks: always an even number, so the pair form applies to every batch)
-    const int rc = tc_use_tail_pair(mode_decoder_kind(w.kind)) ? (bf ? launch_tail_pair_t<kKindBF16>(t, st) : launch_tail_pair_t<kKindF16X2>(t, st))
-                                      : (bf ? launch_tail_t<kKindBF16>(t, st) : launch_tail_t<kKindF16X2>(t, st));
+    const int rc = bf ? launch_tail(t, st) : launch_tail_pair(t, st);
     set_stage(nullptr);
     return rc;
   }
@@ -2119,15 +1924,11 @@ __global__ void bf16_rows_to_tf32p_kernel(const __nv_bfloat16* __restrict__ in, 
 }
 
 // A side stream per (host thread, device) for work that can overlap the main chain of a forward (the pseudo-inverses).
-// CDR_SIDE_LANE=0 keeps everything on the caller's stream.
+// NULL when it cannot be created: everything then stays on the caller's stream.
 struct SideLane {
   cudaStream_t stream = nullptr;
   cudaEvent_t fork = nullptr, join = nullptr;
 };
-static bool tc_use_side_lane() {
-  const char* e = getenv("CDR_SIDE_LANE");
-  return !(e && e[0] == '0');
-}
 static SideLane* side_lane() {
   static thread_local SideLane lanes[kMaxDevices];
   SideLane& l = lanes[current_device()];
@@ -2149,10 +1950,10 @@ int tc_head_forward(const TcWeights& w, const void* feat_rows, int feat_planes, 
                     const CdrHeadTaps* taps, void* workspace, size_t workspace_bytes, cudaStream_t st) {
   const TcPack* pk = (const TcPack*)w.impl;
   const int mode = w.kind;
-  const bool scaled = mode_decoder_kind(mode) == kKindF16X2;
-  const bool fus16 = w.has_fusion && pk->fusion_kind == kKindF16X2;   // fusion activations in kFmtF16P (slots 6..11)
+  const bool scaled = mode_kind(mode) == kKindF16X2;
+  const bool fus16 = w.has_fusion && scaled;   // fusion activations in kFmtF16P (slots 6..11)
   const int B = batch, N = 2 * batch, J = w.joints;
-  TcHeadWs ws = plan_tc_head(workspace, B, J, mode, pk->fusion_kind, w.fd);
+  TcHeadWs ws = plan_tc_head(workspace, B, J, mode, w.fd);
   const FusionDims& fd = w.fd;
   if (ws.bytes > workspace_bytes) {
     set_error("cdr_head_forward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
@@ -2167,7 +1968,7 @@ int tc_head_forward(const TcWeights& w, const void* feat_rows, int feat_planes, 
     // The pseudo-inverses (2B threads of fp64 Jacobi: ~14 us of pure latency) are not needed before the inverse
     // FTL: they run on a side stream forked here and joined there, under the layout pass and conv_layer1.  The fork /
     // join are plain event record / wait pairs, which a CUDA-graph capture of `st` turns into graph edges.
-    lane = tc_use_side_lane() ? side_lane() : nullptr;
+    lane = side_lane();
     cudaStream_t ps = st;
     if (lane) {
       CDR_CUDA(cudaEventRecord(lane->fork, st));
@@ -2229,7 +2030,7 @@ int tc_head_forward(const TcWeights& w, const void* feat_rows, int feat_planes, 
   set_stage("ftl_inv");
   if (lane) CDR_CUDA(cudaStreamWaitEvent(st, lane->join, 0));      // join: the pseudo-inverses are complete
   if ((rc = ftl_act2(ws.y1, act_offset(ws.y1, (size_t)B * kFeatHW * fd.h1p), fd.h1p, pinv, 4, 3, fd.blk, B, ws.z,
-                     act_offset(ws.z, (size_t)fd.h2), 2 * fd.h2, fd.h2, nullptr, slot(ws.slots, 6), slot(ws.slots, 7),
+                     act_offset(ws.z, (size_t)fd.h2), 2 * fd.h2, fd.h2, slot(ws.slots, 6), slot(ws.slots, 7),
                      ws.slots + 2 * 11, st)))
     return rc;
   set_stage("cf_conv2");
@@ -2248,7 +2049,7 @@ int tc_head_forward(const TcWeights& w, const void* feat_rows, int feat_planes, 
   set_stage("ftl_fwd");
   const float* Pv[2] = {P_l, P_r};
   if ((rc = ftl_act2(ws.f2, ws.f2, fd.h2, Pv, 3, 4, fd.blk, B, ws.g, act_offset(ws.g, (size_t)B * kFeatHW * fd.h1p),
-                     fd.h1p, fd.h1p, scaled ? slot(ws.slots, 0).amax : nullptr, slot(ws.slots, 9), slot(ws.slots, 10),
+                     fd.h1p, fd.h1p, slot(ws.slots, 9), slot(ws.slots, 10),
                      ws.slots + 2 * 11 + 1, st)))
     return rc;
   set_stage("cf_out");
@@ -2259,8 +2060,8 @@ int tc_head_forward(const TcWeights& w, const void* feat_rows, int feat_planes, 
     l.layer = &pk->out; l.b_group_rows = kFeatC; l.n = kFeatC; l.bias_group_stride = kFeatC;
     l.C = ws.x1; l.c_group_stride = (long long)B * kFeatHW * kFeatC; l.c_pitch = kFeatC; l.c_fill = kFeatC;
     l.relu = 1; l.out_mode = kOutRows;
-    l.amax_in = slot(ws.slots, 0).amax; l.out_slot = slot(ws.slots, 1);
-    if (fus16) { l.amax_in = nullptr; l.in_slot = slot(ws.slots, 10); }
+    l.out_slot = slot(ws.slots, 1);
+    if (fus16) l.in_slot = slot(ws.slots, 10);
     if ((rc = launch_tc(l, st))) return rc;
   }
   if (tail_fusable(w)) {
@@ -2397,7 +2198,7 @@ static size_t plan_encoder(EncPack& e, const CdrEncoderSpec& spec, void* base) {
     cin = o;
   }
   if (spec.stem.weight) {
-    e.stem_w = b.take(f16 ? stem_weight_bytes_f32() : stem_weight_bytes());
+    e.stem_w = b.take(f16 ? stem_weight_bytes_f16x2() : stem_weight_bytes());
     e.stem_b = (float*)b.take(64 * sizeof(float));
   }
   return b.off;
@@ -2437,10 +2238,10 @@ int tc_encoder_create(const CdrEncoderSpec& spec, int kind, void** out, cudaStre
   auto pack = [&](const CdrConvBn& s, TcLayer& L, int cout, int cin_l, int taps) -> int {
     if (L.kind == kKindF16X2) {
       if (taps == 9)
-        pack_rows_f16_kernel<9, true><<<L.n_pad, 256, 0, st>>>(s, cout, cin_l, L.k_pitch, L.n_pad, (__half*)L.w[0],
+        pack_rows_f16_kernel<9><<<L.n_pad, 256, 0, st>>>(s, cout, cin_l, L.k_pitch, L.n_pad, (__half*)L.w[0],
                                                                 (__half*)L.w[1], L.wsi, L.bias, L.norms);
       else
-        pack_rows_f16_kernel<0, true><<<L.n_pad, 256, 0, st>>>(s, cout, cin_l, L.k_pitch, L.n_pad, (__half*)L.w[0],
+        pack_rows_f16_kernel<0><<<L.n_pad, 256, 0, st>>>(s, cout, cin_l, L.k_pitch, L.n_pad, (__half*)L.w[0],
                                                                 (__half*)L.w[1], L.wsi, L.bias, L.norms);
       CDR_LAUNCH_OK("pack_rows_f16_kernel");
       return layer_maps(L);
@@ -2453,7 +2254,7 @@ int tc_encoder_create(const CdrEncoderSpec& spec, int kind, void** out, cudaStre
   };
   if (spec.stem.weight) {
     CDR_CHECK_ARG(spec.in_channels == 64, "cdr_encoder_create: the stem produces 64 channels");
-    if (int rc = kind == kKindF16X2 ? launch_pack_stem_f32(spec.stem, (float*)e->stem_w, e->stem_b, st)
+    if (int rc = kind == kKindF16X2 ? launch_pack_stem_f16x2(spec.stem, e->stem_w, e->stem_b, st)
                                     : launch_pack_stem(spec.stem, e->stem_w, e->stem_b, st))
       return rc;
   }
@@ -2599,7 +2400,7 @@ int tc_encoder_forward_images(const void* enc, const void* images, int is_u8, co
     // slot 0 of the layer workspace = {amax, scale} of the pooled tensor; every slot is zeroed here, before the stem
     EncWs lw = plan_enc_ws(e, ws.layers, n, H / 4, W / 4);
     CDR_CUDA(cudaMemsetAsync(lw.slots, 0, lw.slot_bytes, st));
-    if (int rc = launch_stem_f32(images, is_u8, mean, std, n, H, W, (const float*)e.stem_w, e.stem_b, (float*)ws.conv_out,
+    if (int rc = launch_stem_f32(images, is_u8, mean, std, n, H, W, e.stem_w, e.stem_b, (float*)ws.conv_out,
                                  ws.pooled.p[0], ws.pooled.p[1], lw.slots, st))
       return rc;
     return enc_layers(e, ws.pooled, true, n, H / 4, W / 4, out_rows, ws.layers, ws.layer_bytes, st);
@@ -2631,9 +2432,8 @@ static int enc_conv(const TcLayer& L, const Act& in, ScaleSlot in_slot, int cin,
   }
   l.res_pitch = cout;
   // cta_group::2 pairs for the MMA-bound wide layers (conv1 / conv2 of a block: BN = 256 in bf16, every f16x2 one), as
-  // on the decoder's transposed convs (layer4 conv2 38.2 -> 35.1 us, conv1 24.6 -> 23.6 us); CDR_ENC_PAIR=0: off
-  const char* ep = getenv("CDR_ENC_PAIR");
-  l.pair2 = (L.bn == 256 || L.kind == kKindF16X2) && !res && stride <= 1 && !(ep && ep[0] == '0');
+  // on the decoder's transposed convs (layer4 conv2 38.2 -> 35.1 us, conv1 24.6 -> 23.6 us)
+  l.pair2 = (L.bn == 256 || L.kind == kKindF16X2) && !res && stride <= 1;
   return launch_tc(l, st);
 }
 
@@ -2792,7 +2592,7 @@ int tc_deconv_train_forward(const float* x, const float* weight, int n, int cin,
   CdrConvBn cb{};
   cb.weight = weight;
   TcLayer& L = ws.L;
-  pack_rows_f16_kernel<1, true><<<L.rows, 256, 0, st>>>(cb, cout, cin, L.k_pitch, L.n_pad, (__half*)L.w[0],
+  pack_rows_f16_kernel<1><<<L.rows, 256, 0, st>>>(cb, cout, cin, L.k_pitch, L.n_pad, (__half*)L.w[0],
                                                         (__half*)L.w[1], L.wsi, L.bias, nullptr);
   CDR_LAUNCH_OK("pack_rows_f16_kernel");
   if (int rc = layer_maps(L)) return rc;
@@ -2863,21 +2663,8 @@ static int launch_wgrad(const DtShape& d, const Act& xa, ScaleSlot sx, const Act
     }
   }
   const int grid = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
-  cudaLaunchConfig_t cfg{};
-  cudaLaunchAttribute attr[1];
-  int n_attr = 0;
-  if (tc_use_pdl()) {
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    n_attr = 1;
-  }
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(Cfg::kThreads);
-  cfg.dynamicSmemBytes = Cfg::kSmemBytes;
-  cfg.stream = st;
-  cfg.attrs = attr;
-  cfg.numAttrs = n_attr;
-  CDR_CUDA(cudaLaunchKernelEx(&cfg, kern, ma[0], ma[1], mb[0], mb[1], ma[0], ma[0], ma[0], ma[0], p));
+  CDR_CUDA(launch_pdl(kern, grid, Cfg::kThreads, Cfg::kSmemBytes, false, st, ma[0], ma[1], mb[0], mb[1], ma[0], ma[0], ma[0],
+                      ma[0], p));
   CDR_LAUNCH_OK("tap_gemm_tc_kernel");
   return CDR_OK;
 }
@@ -2900,7 +2687,7 @@ int tc_deconv_train_backward(const void* saved, const float* weight, const float
     CdrConvBn cb{};
     cb.weight = weight;
     TcLayer& L = ws.L;
-    pack_rows_f16_kernel<-1, true><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
+    pack_rows_f16_kernel<-1><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
                                                            (__half*)L.w[1], L.wsi, L.bias, nullptr);
     CDR_LAUNCH_OK("pack_rows_f16_kernel");
     if (int rc = layer_maps(L)) return rc;

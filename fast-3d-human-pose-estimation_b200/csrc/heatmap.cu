@@ -30,8 +30,8 @@ constexpr int kTileBytes = 16384;  // one 64x64 fp32 heat-map
 // the arg-max stress at 20 000 maps).  With stages == warps every warp owns one stage.
 // A stage is busy for (HBM latency + one warp's two passes over the tile), so bytes in flight per SM and
 // consumer parallelism both bound the stream: 8 x 16 KB reached 5.1 TB/s (78 % of the measured HBM peak)
-// with the XU pipe (EX2 + fp64 conversions) at 46 %.  CDR_HEAT_WARPS=8|10|12 overrides the default.
-constexpr int kHeatWarpsDefault = 10;   // B200, 8192-pose stream: 8 -> 5.40, 10 -> 5.91, 12 -> 5.33 TB/s (12: 14 warps cap ptxas at 128 registers, the DLT warp spills)
+// with the XU pipe (EX2 + fp64 conversions) at 46 %.
+constexpr int kHeatWarps = 10;   // B200, 8192-pose stream: 8 -> 5.40, 10 -> 5.91, 12 -> 5.33 TB/s (12: 14 warps cap ptxas at 128 registers, the DLT warp spills)
 constexpr int kHeatWarpsMin = 8;   // smallest instantiation: the fused pose hand-off needs 2J >= warps
 constexpr int kPoseBufs = 4;
 constexpr int kMaxTilesPerPose = 2 * kMaxJoints;
@@ -384,16 +384,6 @@ __global__ void __launch_bounds__(32 * (NW + 2), 1) heat_stream_kernel(const Hea
   }
 }
 
-static int heat_warps() {
-  static int nw = 0;
-  if (nw == 0) {
-    const char* e = getenv("CDR_HEAT_WARPS");
-    const int v = e ? atoi(e) : kHeatWarpsDefault;
-    nw = (v == 8 || v == 10 || v == 12) ? v : kHeatWarpsDefault;
-  }
-  return nw;
-}
-
 template <typename T, bool kArgmax, int NW>
 static int launch_heat_nw(const HeatParams& p, cudaStream_t st) {
   const size_t smem = sizeof(HeatSmem<NW>) + 128;
@@ -412,14 +402,9 @@ static int launch_heat_nw(const HeatParams& p, cudaStream_t st) {
 template <typename T, bool kArgmax>
 static int launch_heat(const HeatParams& p, cudaStream_t st) {
   // the fused pose hand-off needs every consumer warp to see every pose (2J >= warps)
-  int nw = heat_warps();
   const bool fused = !kArgmax && p.P[0] != nullptr;
-  if (fused && 2 * p.joints < nw) nw = 2 * p.joints >= 10 ? 10 : 8;
-  switch (nw) {
-    case 8: return launch_heat_nw<T, kArgmax, 8>(p, st);
-    case 10: return launch_heat_nw<T, kArgmax, 10>(p, st);
-    default: return launch_heat_nw<T, kArgmax, 12>(p, st);
-  }
+  if (fused && 2 * p.joints < kHeatWarps) return launch_heat_nw<T, kArgmax, kHeatWarpsMin>(p, st);
+  return launch_heat_nw<T, kArgmax, kHeatWarps>(p, st);
 }
 
 static int check_heat_shape(const char* who, int H, int W, int elem_bytes) {

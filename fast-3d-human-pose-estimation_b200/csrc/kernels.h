@@ -39,10 +39,10 @@ int launch_nchw_to_rows_bf16(const float* in, const float* in2, int n_img, int C
 // fp32 hi/lo planes for the 3xTF32 tensor-core path (common.cuh: split_tf32)
 int launch_nchw_to_rows_split(const float* in, const float* in2, int n_img, int C, int HW, float* out_hi, float* out_lo,
                               int out_pitch, cudaStream_t st);
-// FTL of `views` (1 or 2) tensors in one launch.  amax_out (optional): atomicMax of max |out| (pre-zeroed float)
+// FTL of `views` (1 or 2) tensors in one launch
 int launch_ftl_split2(const float* const in_hi[2], const float* const in_lo[2], int in_pitch, const float* const mats[2],
                       int rows, int cols, int blk, int n, int hw, float* const out_hi[2], float* const out_lo[2],
-                      int out_pitch, int out_fill, int views, float* amax_out, cudaStream_t st);
+                      int out_pitch, int out_fill, int views, cudaStream_t st);
 int launch_ftl_f16p2(const void* const in_hi[2], const void* const in_lo[2], int in_pitch, const float* const mats[2],
                      int rows, int cols, int blk, int n, int hw, void* const out_hi[2], void* const out_lo[2],
                      int out_pitch, int out_fill, const float* scale_in, const float* amax_in, const float* l1max,
@@ -79,11 +79,11 @@ size_t stem_weight_bytes();
 // x: fp32 NCHW (is_u8 = 0) or uint8 NHWC frames normalised on the fly with HOST arrays mean[3], std[3]
 int launch_stem(const void* x, int is_u8, const float* mean, const float* std, int n, int H, int W, const void* w,
                 const float* bias, void* conv_out, void* pooled, cudaStream_t st);
-// the same at fp32 accuracy (FFMA): fp32 weights [147][64], conv_out fp32 NHWC scratch, pooled as scaled fp16 hi/lo
-// planes; slot = {amax, scale} of the pooled tensor (amax pre-zeroed)
-int launch_pack_stem_f32(const CdrConvBn& s, float* w, float* bias, cudaStream_t st);
-size_t stem_weight_bytes_f32();
-int launch_stem_f32(const void* x, int is_u8, const float* mean, const float* std, int n, int H, int W, const float* w,
+// the same at fp32 accuracy (fp16 hi/lo operands on mma.sync): weights as fp16 hi/lo planes + per-channel scales,
+// conv_out fp32 NHWC scratch, pooled as scaled fp16 hi/lo planes; slot = {amax, scale} of the pooled tensor (amax pre-zeroed)
+int launch_pack_stem_f16x2(const CdrConvBn& s, void* w, float* bias, cudaStream_t st);
+size_t stem_weight_bytes_f16x2();
+int launch_stem_f32(const void* x, int is_u8, const float* mean, const float* std, int n, int H, int W, const void* w,
                     const float* bias, float* conv_out, void* pooled_hi, void* pooled_lo, float* slot, cudaStream_t st);
 
 // train_ops.cu: BatchNorm2d in training mode (+ optional fused ReLU) and the reference's three losses, forward / backward

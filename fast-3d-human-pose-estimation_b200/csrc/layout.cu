@@ -433,10 +433,9 @@ ftl_vec_kernel(const FtlViews<T> fv, int in_pitch, int blk, long long total4, in
 template <int ROWS, int COLS>
 __global__ void __launch_bounds__(256)
 ftl_split_vec_kernel(const FtlViews<float> fv, int in_pitch, int blk, long long total4, int hw, int out_pitch,
-                     int out_fill, float* __restrict__ amax_out) {
+                     int out_fill) {
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const bool v1 = blockIdx.y != 0;   // select, not index: a dynamically indexed __grid_constant__ struct is copied to local memory
-  float amax = 0.f;
   if (idx < total4) {
     const int blk4 = blk >> 2;
     const long long row = idx / blk4;
@@ -460,7 +459,6 @@ ftl_split_vec_kernel(const FtlViews<float> fv, int in_pitch, int blk, long long 
 #pragma unroll
         for (int k = 0; k < COLS; ++k) acc = fmaf(__ldg(m + r * COLS + k), x[k].v[e], acc);
         split_tf32(acc, hi.v[e], lo.v[e]);
-        amax = fmaxf(amax, fabsf(acc));
       }
       st4((v1 ? fv.out[1] : fv.out[0]) + o + r * blk, hi);
       st4((v1 ? fv.out_lo[1] : fv.out_lo[0]) + o + r * blk, lo);
@@ -469,11 +467,6 @@ ftl_split_vec_kernel(const FtlViews<float> fv, int in_pitch, int blk, long long 
       st4((v1 ? fv.out[1] : fv.out[0]) + o + ROWS * blk, Vec4{{0.f, 0.f, 0.f, 0.f}});
       st4((v1 ? fv.out_lo[1] : fv.out_lo[0]) + o + ROWS * blk, Vec4{{0.f, 0.f, 0.f, 0.f}});
     }
-  }
-  if (amax_out) {   // max |out| for the scale of the tensor the next conv writes (gemm_tc.cu: kFmtF16P)
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, o));
-    if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<unsigned int*>(amax_out), __float_as_uint(amax));
   }
 }
 
@@ -488,8 +481,7 @@ static bool ftl_vec_ok(int elem_bytes, int in_pitch, int blk, int out_pitch, int
 
 template <int ROWS, int COLS>
 __global__ void __launch_bounds__(256)
-ftl_split_kernel(const FtlViews<float> fv, int in_pitch, int blk, long long total, int hw, int out_pitch, int out_fill,
-                 float* __restrict__ amax_out) {
+ftl_split_kernel(const FtlViews<float> fv, int in_pitch, int blk, long long total, int hw, int out_pitch, int out_fill) {
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const int view = blockIdx.y;
   const float* __restrict__ in_hi = fv.in[view];
@@ -497,8 +489,7 @@ ftl_split_kernel(const FtlViews<float> fv, int in_pitch, int blk, long long tota
   const float* __restrict__ mats = fv.mats[view];
   float* __restrict__ out_hi = fv.out[view];
   float* __restrict__ out_lo = fv.out_lo[view];
-  float amax = 0.f;
-  if (idx < total) {
+  if (idx >= total) return;
   const long long row = idx / blk;
   const int c = (int)(idx - row * blk);
   const float* m = mats + (row / hw) * (ROWS * COLS);
@@ -518,23 +509,16 @@ ftl_split_kernel(const FtlViews<float> fv, int in_pitch, int blk, long long tota
     split_tf32(acc, hi, lo);
     out_hi[o + r * blk + c] = hi;
     out_lo[o + r * blk + c] = lo;
-    amax = fmaxf(amax, fabsf(acc));
   }
   if (c < out_fill - ROWS * blk) {
     out_hi[o + ROWS * blk + c] = 0.f;
     out_lo[o + ROWS * blk + c] = 0.f;
   }
-  }
-  if (amax_out) {   // max |out| for the scale of the tensor the next conv writes (gemm_tc.cu: kFmtF16P)
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, o));
-    if ((threadIdx.x & 31) == 0) atomicMax(reinterpret_cast<unsigned int*>(amax_out), __float_as_uint(amax));
-  }
 }
 
 int launch_ftl_split2(const float* const in_hi[2], const float* const in_lo[2], int in_pitch, const float* const mats[2],
                       int rows, int cols, int blk, int n, int hw, float* const out_hi[2], float* const out_lo[2],
-                      int out_pitch, int out_fill, int views, float* amax_out, cudaStream_t st) {
+                      int out_pitch, int out_fill, int views, cudaStream_t st) {
   CDR_CHECK_ARG(views == 1 || views == 2, "ftl_split: 1 or 2 views");
   FtlViews<float> fv{};
   for (int v = 0; v < views; ++v) {
@@ -549,17 +533,17 @@ int launch_ftl_split2(const float* const in_hi[2], const float* const in_lo[2], 
                   views > 1 ? out_hi[1] : nullptr, views > 1 ? out_lo[1] : nullptr})) {
     const dim3 grid4((unsigned)ceil_div<long long>(total / 4, 256), views);
     if (rows == 4)
-      ftl_split_vec_kernel<4, 3><<<grid4, 256, 0, st>>>(fv, in_pitch, blk, total / 4, hw, out_pitch, out_fill, amax_out);
+      ftl_split_vec_kernel<4, 3><<<grid4, 256, 0, st>>>(fv, in_pitch, blk, total / 4, hw, out_pitch, out_fill);
     else
-      ftl_split_vec_kernel<3, 4><<<grid4, 256, 0, st>>>(fv, in_pitch, blk, total / 4, hw, out_pitch, out_fill, amax_out);
+      ftl_split_vec_kernel<3, 4><<<grid4, 256, 0, st>>>(fv, in_pitch, blk, total / 4, hw, out_pitch, out_fill);
     CDR_LAUNCH_OK("ftl_split_vec_kernel");
     return CDR_OK;
   }
   const dim3 grid((unsigned)ceil_div<long long>(total, 256), views);
   if (rows == 4 && cols == 3)
-    ftl_split_kernel<4, 3><<<grid, 256, 0, st>>>(fv, in_pitch, blk, total, hw, out_pitch, out_fill, amax_out);
+    ftl_split_kernel<4, 3><<<grid, 256, 0, st>>>(fv, in_pitch, blk, total, hw, out_pitch, out_fill);
   else if (rows == 3 && cols == 4)
-    ftl_split_kernel<3, 4><<<grid, 256, 0, st>>>(fv, in_pitch, blk, total, hw, out_pitch, out_fill, amax_out);
+    ftl_split_kernel<3, 4><<<grid, 256, 0, st>>>(fv, in_pitch, blk, total, hw, out_pitch, out_fill);
   else {
     set_error("ftl_split: only (4x3) and (3x4) matrices are supported");
     return CDR_ERR_UNSUPPORTED;

@@ -211,9 +211,8 @@ __device__ __forceinline__ void tma_store_5d(const void* tmap, const void* src_s
                : "memory");
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-// all of this thread's committed bulk groups have finished READING their shared-memory source
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-// ... all but the kPending most recent ones
+// all of this thread's committed bulk groups but the kPending most recent ones have finished READING their shared-memory
+// source
 template <int kPending>
 __device__ __forceinline__ void bulk_wait_read() {
   asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(kPending) : "memory");

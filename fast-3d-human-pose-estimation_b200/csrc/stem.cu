@@ -236,132 +236,9 @@ int launch_stem(const void* x, int is_u8, const float* mean, const float* std, i
 }
 
 
-// ------------------------------------------------------------------------------------------
-// The same stem at fp32 accuracy for the f16x2 ("fp32") encoder, first version (kept as the CDR_STEM_FFMA=1 cross-check of the
-// tensor-core form further down): fp32 FFMA (the conv is 2.3 % of the encoder's
-// FLOPs), fp32 NHWC scratch, then the max-pool writes the scaled fp16 hi/lo planes the tcgen05 layers read.  The
-// pooled tensor's scale comes from the EXACT maximum (max-pool commutes with max): the conv kernel atomicMax-es its
-// post-ReLU outputs into slot[0], the pool kernel turns that into slot[1] = 2^(13 - ilogb(amax)).
-constexpr int kStemK32 = 147;                      // (ky, kx, ci) = 7 * 21
-constexpr int kPatchPitch32 = 208;                 // floats per patch row: 69 * 3 = 207 (+1)
-constexpr int kStem32SmemBytes = (kStemK32 * kStemCo + kPatchH * kPatchPitch32) * (int)sizeof(float);
-
-// conv1 (64,3,7,7) + bn1 -> fp32 [ky*21 + kx*3 + ci][64] with channels PERMUTED inside a row: position
-// 16*j + 4*cg + e holds channel 16*j + 4*cg + e (identity) — kept plain; the kernel's lanes read float4s at 4*cg + 16*j
-__global__ void pack_stem_f32_kernel(CdrConvBn s, float* __restrict__ w, float* __restrict__ bias) {
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= kStemK32 * kStemCo) return;
-  const int k = idx / kStemCo, n = idx - k * kStemCo;
-  const double sc = (double)s.bn_weight[n] / sqrt((double)s.bn_var[n] + 1e-5);
-  if (k == 0) bias[n] = (float)((double)s.bn_bias[n] - (double)s.bn_mean[n] * sc);
-  const int ky = k / 21, r = k - ky * 21, kx = r / 3, ci = r - kx * 3;
-  w[idx] = (float)((double)s.weight[((n * 3 + ci) * 7 + ky) * 7 + kx] * sc);
-}
-
-// grid (conv rows / 8, images), 256 threads: warp = one conv row of the 8 x 32 tile; lane = (pxg = lane >> 2: columns
-// pxg + 8*i, i < 4; cg = lane & 3: channels 16*j + 4*cg .. +3, j < 4) -> 4 x 16 outputs per thread.  Patch reads of a
-// warp hit 8 distinct banks (stride 6 floats), weight reads are one 64-byte segment per float4 load.
-template <bool kU8>
-__global__ void __launch_bounds__(256, 2)      // two CTAs per SM: one loads its patch while the other runs its FMAs
-stem_conv_f32_kernel(const void* __restrict__ xin, int H, int W, const StemNorm nrm, const float* __restrict__ wpk,
-                     const float* __restrict__ bias, float* __restrict__ out, float* __restrict__ amax_out) {
-  extern __shared__ __align__(16) float smem_f[];
-  float* s_w = smem_f;                               // [147][64]
-  float* s_p = smem_f + kStemK32 * kStemCo;          // [21][208]
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int cg = lane & 3, pxg = lane >> 2;
-  const int img = blockIdx.y, oy0 = blockIdx.x * kTileH;
-  const int Ho = H >> 1, Wo = W >> 1;
-  for (int i = threadIdx.x; i < kStemK32 * kStemCo / 4; i += 256)
-    reinterpret_cast<float4*>(s_w)[i] = __ldg(reinterpret_cast<const float4*>(wpk) + i);
-  float4 bv[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) bv[j] = __ldg(reinterpret_cast<const float4*>(bias + 16 * j + 4 * cg));
-  const float* xi = reinterpret_cast<const float*>(xin) + (size_t)img * 3 * H * W;
-  const uint8_t* xu = reinterpret_cast<const uint8_t*>(xin) + (size_t)img * 3 * H * W;
-  float mx = 0.f;
-  for (int ox0 = 0; ox0 < Wo; ox0 += kTileW) {
-    __syncthreads();
-    const int iy0 = 2 * oy0 - 3, ix0 = 2 * ox0 - 3;
-    if constexpr (!kU8) {
-      for (int i = threadIdx.x; i < kPatchH * 3 * kPatchW; i += 256) {
-        const int col = i % kPatchW, rc = i / kPatchW;
-        const int ci = rc % 3, row = rc / 3;
-        const int iy = iy0 + row, ix = ix0 + col;
-        float v = 0.f;
-        if (iy >= 0 && iy < H && ix >= 0 && ix < W) v = __ldg(xi + ((size_t)ci * H + iy) * W + ix);
-        s_p[row * kPatchPitch32 + col * 3 + ci] = v;
-      }
-    } else {
-      for (int i = threadIdx.x; i < kPatchH * 3 * kPatchW; i += 256) {
-        const int e = i % (3 * kPatchW), row = i / (3 * kPatchW);
-        const int col = e / 3, ci = e - col * 3;
-        const int iy = iy0 + row, ix = ix0 + col;
-        float v = 0.f;                                                 // zero padding applies AFTER normalisation
-        if (iy >= 0 && iy < H && ix >= 0 && ix < W) {
-          const float u = (float)__ldg(xu + ((size_t)iy * W + ix) * 3 + ci);
-          v = __fdiv_rn(__fsub_rn(__fdiv_rn(u, 255.f), nrm.mean[ci]), nrm.std[ci]);
-        }
-        s_p[row * kPatchPitch32 + e] = v;
-      }
-    }
-    __syncthreads();
-    float acc[4][16];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-      for (int c = 0; c < 16; ++c) acc[i][c] = 0.f;
-    // pixel (warp, pxg + 8 i): patch origin (2*warp, 2*(pxg + 8 i)) -> element offset 2*warp*pitch + 6*(pxg + 8 i)
-    const float* pr = s_p + (2 * warp) * kPatchPitch32 + 6 * pxg;
-#pragma unroll 1
-    for (int ky = 0; ky < 7; ++ky) {
-      const float* prow = pr + ky * kPatchPitch32;
-      const float* wrow = s_w + (ky * 21) * kStemCo + 4 * cg;
-#pragma unroll 7
-      for (int r = 0; r < 21; ++r) {
-        float a[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) a[i] = prow[48 * i + r];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float4 w4 = *reinterpret_cast<const float4*>(wrow + r * kStemCo + 16 * j);
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            acc[i][4 * j] = fmaf(a[i], w4.x, acc[i][4 * j]);
-            acc[i][4 * j + 1] = fmaf(a[i], w4.y, acc[i][4 * j + 1]);
-            acc[i][4 * j + 2] = fmaf(a[i], w4.z, acc[i][4 * j + 2]);
-            acc[i][4 * j + 3] = fmaf(a[i], w4.w, acc[i][4 * j + 3]);
-          }
-        }
-      }
-    }
-    const int oy = oy0 + warp;
-    if (oy < Ho) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int ox = ox0 + pxg + 8 * i;
-        if (ox < Wo) {
-          float* o = out + (((size_t)img * Ho + oy) * Wo + ox) * kStemCo + 4 * cg;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            float4 v;
-            v.x = fmaxf(acc[i][4 * j] + bv[j].x, 0.f);
-            v.y = fmaxf(acc[i][4 * j + 1] + bv[j].y, 0.f);
-            v.z = fmaxf(acc[i][4 * j + 2] + bv[j].z, 0.f);
-            v.w = fmaxf(acc[i][4 * j + 3] + bv[j].w, 0.f);
-            mx = fmaxf(mx, fmaxf(fmaxf(v.x, v.y), fmaxf(v.z, v.w)));
-            *reinterpret_cast<float4*>(o + 16 * j) = v;
-          }
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-  if (lane == 0) atomicMax(reinterpret_cast<unsigned int*>(amax_out), __float_as_uint(mx));   // mx >= 0
-}
-
-// max-pool 3x3 stride 2 pad 1 on NHWC fp32 (post-ReLU) -> scaled fp16 hi/lo planes; slot = {amax (complete), scale}
+// max-pool 3x3 stride 2 pad 1 on NHWC fp32 (post-ReLU) -> scaled fp16 hi/lo planes; slot = {amax (complete), scale}.
+// The pooled tensor's scale comes from the EXACT maximum (max-pool commutes with max): the fp32-accurate stem conv
+// atomicMax-es its post-ReLU outputs into slot[0], this kernel turns that into slot[1] = 2^(13 - ilogb(amax)).
 __global__ void __launch_bounds__(256)
 maxpool3s2_f16p_kernel(const float* __restrict__ in, int Hi, int Wi, int C8, long long total, __half* __restrict__ hi,
                        __half* __restrict__ lo, float* __restrict__ slot) {
@@ -409,8 +286,7 @@ maxpool3s2_f16p_kernel(const float* __restrict__ in, int Hi, int Wi, int C8, lon
 
 
 // ------------------------------------------------------------------------------------------
-// The fp32-accurate stem on the tensor cores (round 2, replaces the FFMA kernel above in the f16x2 encoder: 1.02 ->
-// see DESIGN.md §7): the bf16 kernel's implicit GEMM on warp-level mma.sync.m16n8k16, with BOTH operands as fp16 hi/lo
+// The stem at fp32 accuracy for the f16x2 ("fp32") encoder, on the tensor cores (DESIGN.md §7): the bf16 kernel's implicit GEMM on warp-level mma.sync.m16n8k16, with BOTH operands as fp16 hi/lo
 // pairs and three MMAs per product — x w = xh wh + 2^-11 (xh wl + xl wh) (+ 2^-22 xl wl, dropped) — exactly the f16x2
 // scheme of gemm_tc.cu.  fp16 products are exact in the fp32 accumulators; main and correction terms accumulate
 // separately (K = 147: no long same-signed chain).  Pixels need no scale (|x| < 65504; the lo plane keeps values down
@@ -585,26 +461,19 @@ stem_conv_f16x2_kernel(const void* __restrict__ xin, int H, int W, const StemNor
   if (lane == 0) atomicMax(reinterpret_cast<unsigned int*>(amax_out), __float_as_uint(mx));   // mx >= 0
 }
 
-// packed buffer of the fp32-accurate stem: [fp32 weights [147][64] (FFMA cross-check) | fp16 hi [64][168] | fp16 lo | wsi [64]]
-constexpr size_t kStem32WBytes = (size_t)kStemK32 * kStemCo * sizeof(float);                     // 37632
+// packed buffer of the fp32-accurate stem: [fp16 hi [64][168] | fp16 lo | wsi [64]]
 constexpr size_t kStem16PlaneBytes = (size_t)kStemCo * kStemWPitch * sizeof(__half);             // 21504
-static bool stem_use_ffma() {          // CDR_STEM_FFMA=1: the CUDA-core kernel (A/B timing, cross-check)
-  const char* e = getenv("CDR_STEM_FFMA");
-  return e && e[0] == '1';
-}
-int launch_pack_stem_f32(const CdrConvBn& s, float* w, float* bias, cudaStream_t st) {
+int launch_pack_stem_f16x2(const CdrConvBn& s, void* w, float* bias, cudaStream_t st) {
   CDR_CHECK_ARG(s.weight && s.bn_weight && s.bn_bias && s.bn_mean && s.bn_var && w && bias, "pack_stem: bad args");
-  pack_stem_f32_kernel<<<ceil_div(kStemK32 * kStemCo, 256), 256, 0, st>>>(s, w, bias);
-  CDR_LAUNCH_OK("pack_stem_f32_kernel");
-  uint8_t* b = reinterpret_cast<uint8_t*>(w) + kStem32WBytes;
+  uint8_t* b = reinterpret_cast<uint8_t*>(w);
   pack_stem_f16x2_kernel<<<kStemCo, 64, 0, st>>>(s, reinterpret_cast<__half*>(b), reinterpret_cast<__half*>(b + kStem16PlaneBytes),
                                                  reinterpret_cast<float*>(b + 2 * kStem16PlaneBytes), bias);
   CDR_LAUNCH_OK("pack_stem_f16x2_kernel");
   return CDR_OK;
 }
-size_t stem_weight_bytes_f32() { return kStem32WBytes + 2 * kStem16PlaneBytes + kStemCo * sizeof(float); }
+size_t stem_weight_bytes_f16x2() { return 2 * kStem16PlaneBytes + kStemCo * sizeof(float); }
 
-int launch_stem_f32(const void* x, int is_u8, const float* mean, const float* std, int n, int H, int W, const float* w,
+int launch_stem_f32(const void* x, int is_u8, const float* mean, const float* std, int n, int H, int W, const void* w,
                     const float* bias, float* conv_out, void* pooled_hi, void* pooled_lo, float* slot, cudaStream_t st) {
   CDR_CHECK_ARG(x && w && bias && conv_out && pooled_hi && pooled_lo && slot && n > 0, "stem: bad args");
   CDR_CHECK_ARG(!is_u8 || (mean && std), "stem: uint8 frames need mean / std");
@@ -616,42 +485,26 @@ int launch_stem_f32(const void* x, int is_u8, const float* mean, const float* st
   CDR_CHECK_ARG(H % 16 == 0 && W % 64 == 0, "stem: image %dx%d must have H %% 16 == 0 and W %% 64 == 0", H, W);
   CDR_CHECK_ARG(((uintptr_t)conv_out & 15) == 0 && ((uintptr_t)pooled_hi & 15) == 0 && ((uintptr_t)pooled_lo & 15) == 0 &&
                     ((uintptr_t)w & 15) == 0, "stem: alignment");
-  static DeviceOnce attr_set[2], attr16_set[2];
+  static DeviceOnce attr_set[2];
   const int Ho = H / 2, Wo = W / 2;
-  if (!stem_use_ffma()) {
-    // tensor-core form: fp16 hi/lo operands, 3 mma.sync per product
-    const uint8_t* b = reinterpret_cast<const uint8_t*>(w) + kStem32WBytes;
-    const __half* wh = reinterpret_cast<const __half*>(b);
-    const __half* wl = reinterpret_cast<const __half*>(b + kStem16PlaneBytes);
-    const float* wsi = reinterpret_cast<const float*>(b + 2 * kStem16PlaneBytes);
-    if (is_u8) {
-      if (attr16_set[1].need()) {
-        CDR_CUDA(cudaFuncSetAttribute(stem_conv_f16x2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStem16SmemBytes));
-        attr16_set[1].done();
-      }
-      stem_conv_f16x2_kernel<true><<<dim3(Ho / kTileH, n), 256, kStem16SmemBytes, st>>>(x, H, W, nrm, wh, wl, wsi, bias, conv_out, slot);
-    } else {
-      if (attr16_set[0].need()) {
-        CDR_CUDA(cudaFuncSetAttribute(stem_conv_f16x2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStem16SmemBytes));
-        attr16_set[0].done();
-      }
-      stem_conv_f16x2_kernel<false><<<dim3(Ho / kTileH, n), 256, kStem16SmemBytes, st>>>(x, H, W, nrm, wh, wl, wsi, bias, conv_out, slot);
-    }
-    CDR_LAUNCH_OK("stem_conv_f16x2_kernel");
-  } else if (is_u8) {
+  const uint8_t* b = reinterpret_cast<const uint8_t*>(w);
+  const __half* wh = reinterpret_cast<const __half*>(b);
+  const __half* wl = reinterpret_cast<const __half*>(b + kStem16PlaneBytes);
+  const float* wsi = reinterpret_cast<const float*>(b + 2 * kStem16PlaneBytes);
+  if (is_u8) {
     if (attr_set[1].need()) {
-      CDR_CUDA(cudaFuncSetAttribute(stem_conv_f32_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStem32SmemBytes));
+      CDR_CUDA(cudaFuncSetAttribute(stem_conv_f16x2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStem16SmemBytes));
       attr_set[1].done();
     }
-    stem_conv_f32_kernel<true><<<dim3(Ho / kTileH, n), 256, kStem32SmemBytes, st>>>(x, H, W, nrm, w, bias, conv_out, slot);
+    stem_conv_f16x2_kernel<true><<<dim3(Ho / kTileH, n), 256, kStem16SmemBytes, st>>>(x, H, W, nrm, wh, wl, wsi, bias, conv_out, slot);
   } else {
     if (attr_set[0].need()) {
-      CDR_CUDA(cudaFuncSetAttribute(stem_conv_f32_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStem32SmemBytes));
+      CDR_CUDA(cudaFuncSetAttribute(stem_conv_f16x2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kStem16SmemBytes));
       attr_set[0].done();
     }
-    stem_conv_f32_kernel<false><<<dim3(Ho / kTileH, n), 256, kStem32SmemBytes, st>>>(x, H, W, nrm, w, bias, conv_out, slot);
+    stem_conv_f16x2_kernel<false><<<dim3(Ho / kTileH, n), 256, kStem16SmemBytes, st>>>(x, H, W, nrm, wh, wl, wsi, bias, conv_out, slot);
   }
-  if (stem_use_ffma()) CDR_LAUNCH_OK("stem_conv_f32_kernel");
+  CDR_LAUNCH_OK("stem_conv_f16x2_kernel");
   const long long total = (long long)n * (Ho / 2) * (Wo / 2) * (kStemCo / 8);
   maxpool3s2_f16p_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(
       conv_out, Ho, Wo, kStemCo / 8, total, (__half*)pooled_hi, (__half*)pooled_lo, slot);

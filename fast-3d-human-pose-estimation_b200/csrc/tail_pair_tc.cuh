@@ -1,19 +1,22 @@
-// The fused decoder tail of tail_tc.cuh on cta_group::2 CTA pairs (included by gemm_tc.cu after tail_tc.cuh).
+// The fused decoder tail of tail_tc.cuh for the f16x2 decoder, on cta_group::2 CTA pairs (included by gemm_tc.cu after
+// tail_tc.cuh).
 //
-// Same arithmetic, same partial records, same merge kernel.  What changes is who feeds the tensor cores: a cluster of two
+// Same structure, same partial records, same merge kernel.  The operands are scaled fp16 hi/lo planes (gemm_tc.cu:
+// kKindF16X2): BN = 128 (TMEM holds 2 main-chunk + 2 correction accumulators of 128 columns), the two channel halves of a
+// pixel block run back to back and the heat partial of the first half waits in registers of the heat warps; A2 = 32 KB =
+// one 64-channel K chunk in both planes, so a tile takes two hand-offs (column group 0, then group 1).
+// What changes against tail_tc.cuh is who feeds the tensor cores: a cluster of two
 // CTAs takes two consecutive 128-pixel blocks of the same output phase, every CTA stages its own A rows and HALF of
 // each weight tile, the leader (cluster rank 0) issues every tcgen05.mma for both SMs (M = 256) — main loop AND the heat
 // MMAs — and each CTA's convert / heat warps work on the accumulator rows in their own TMEM.  Per SM and MMA the tensor
 // core then reads A + B/2 from shared memory instead of A + B, and the TMA fills shrink by the same B/2: the f16x2 main
 // loop asked 213 B/clk of a 128 B/clk shared memory (gemm_tc.cu, CL = 2 comment).
 //
-// Shared memory per CTA:  f16x2  3 stages x 48 KB [A hi | A lo | B hi (64 rows) | B lo] + A2 32 KB + final-layer tiles 24 KB
-//                         bf16   4 stages x 32 KB [A | B (128 rows)]                    + A2 64 KB + final-layer tiles  8 KB
+// Shared memory per CTA: 3 stages x 48 KB [A hi | A lo | B hi (64 rows) | B lo] + A2 32 KB + final-layer tiles 24 KB.
 // Final-layer operand of the pair (the B operand of a cta_group::2 MMA is split by rows between the two CTAs, at the SAME
 // shared-memory offset in both):
-//   f16x2, N = 64 form  hi . [Wh ; Wl]: region X holds Wh (32 rows) in CTA 0 and Wl (32 rows) in CTA 1;
-//          N = 32 form  lo . Wh       : region Y holds Wh rows 0-15 in CTA 0 and rows 16-31 in CTA 1;
-//   bf16,  N = 32       A2 . W        : rows 0-15 in CTA 0, 16-31 in CTA 1.
+//   N = 64 form  hi . [Wh ; Wl]: region X holds Wh (32 rows) in CTA 0 and Wl (32 rows) in CTA 1;
+//   N = 32 form  lo . Wh       : region Y holds Wh rows 0-15 in CTA 0 and rows 16-31 in CTA 1.
 // Barriers: the leader's instances of full[] / a2_full / chunk_empty[] / tmem_empty[] collect both CTAs (TMA bytes through
 // cp.async.bulk.tensor.cta_group::2, thread arrivals through mapa + mbarrier.arrive.shared::cluster); everything the
 // issuer publishes (stage release, chunk / tile / heat completion, A2 release) is a multicast commit to both CTAs.
@@ -21,38 +24,23 @@
 
 namespace cdr {
 
-template <int KIND> struct TailPairCfg;
-template <> struct TailPairCfg<kKindBF16> {
-  static constexpr int kBN = 256, kNH = 1, kPlanes = 1, kStages = 4;
-  static constexpr int kBHalfBytes = (kBN / 2) * 128;                       // 16 KB
-  static constexpr int kStageBytes = kABytes + kBHalfBytes;                 // 32 KB
-  static constexpr int kA2Bytes = 4 * kABytes;
-  static constexpr int kWxBytes = 0, kWyBytes = 4 * 16 * 128;               // 4 chunks x 16 rows
-  static constexpr int kRounds = 1, kRoundWarps = 8;
-};
-template <> struct TailPairCfg<kKindF16X2> {
-  static constexpr int kBN = 128, kNH = 2, kPlanes = 2, kStages = 3;
+struct TailPairCfg {
+  static constexpr int kBN = 128, kNH = 2, kStages = 3;
   static constexpr int kBHalfBytes = (kBN / 2) * 128;                       // 8 KB per plane
   static constexpr int kStageBytes = 2 * kABytes + 2 * kBHalfBytes;         // 48 KB
-  static constexpr int kA2Bytes = 2 * kABytes;
+  static constexpr int kA2Bytes = 2 * kABytes;                              // one 64-channel K chunk, hi and lo planes
   static constexpr int kWxBytes = 4 * 32 * 128, kWyBytes = 4 * 16 * 128;    // (half, chunk) x 32 rows / x 16 rows
-  static constexpr int kRounds = 2, kRoundWarps = 4;
-};
-template <int KIND> struct TailPairSmem {
-  using Cfg = TailPairCfg<KIND>;
-  static constexpr size_t kBytes = (size_t)Cfg::kStages * Cfg::kStageBytes + Cfg::kA2Bytes + Cfg::kWxBytes + Cfg::kWyBytes +
-                                   1024 + 512;
-  static_assert(kBytes <= 227 * 1024, "shared memory budget");
+  static constexpr int kRounds = 2, kRoundWarps = 4;                        // hand-offs per tile, warps per hand-off
+  static constexpr size_t kSmemBytes = (size_t)kStages * kStageBytes + kA2Bytes + kWxBytes + kWyBytes + 1024 + 512;
+  static_assert(kSmemBytes <= 227 * 1024, "shared memory budget");
 };
 
-template <int KIND>
 __global__ void __launch_bounds__(kTailThreads, 1)
 deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_a_lo,
                         const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_b_lo,
                         const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ CUtensorMap tmap_w_lo,
                         const __grid_constant__ CUtensorMap tmap_w16, const TailParams p) {
-  using Cfg = TailPairCfg<KIND>;
-  constexpr bool kSplit = KIND == kKindF16X2;
+  using Cfg = TailPairCfg;
   constexpr int BN = Cfg::kBN, NH = Cfg::kNH, S = Cfg::kStages;
   constexpr int kNumKb = 16;
   constexpr int kW = 32, kHW = 1024;
@@ -61,11 +49,11 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
   // stage s: [A (hi) | A lo | B half (hi) | B half lo]
   auto st_a = [&](int s, int plane) { return smem + (size_t)s * Cfg::kStageBytes + (size_t)plane * kABytes; };
   auto st_b = [&](int s, int plane) {
-    return smem + (size_t)s * Cfg::kStageBytes + (size_t)Cfg::kPlanes * kABytes + (size_t)plane * Cfg::kBHalfBytes;
+    return smem + (size_t)s * Cfg::kStageBytes + (size_t)2 * kABytes + (size_t)plane * Cfg::kBHalfBytes;
   };
   uint8_t* a2 = smem + (size_t)S * Cfg::kStageBytes;
-  uint8_t* wx = a2 + Cfg::kA2Bytes;              // f16x2: 4 x 4 KB, index nh * 2 + j
-  uint8_t* wy = wx + Cfg::kWxBytes;              // 4 x 2 KB, index nh * 2 + j (f16x2) / K chunk (bf16)
+  uint8_t* wx = a2 + Cfg::kA2Bytes;              // 4 x 4 KB, index nh * 2 + j
+  uint8_t* wy = wx + Cfg::kWxBytes;              // 4 x 2 KB, index nh * 2 + j
   uint64_t* bars = reinterpret_cast<uint64_t*>(wy + Cfg::kWyBytes);
   uint64_t* full = bars;                     // [S]  leader's: both CTAs' TMA bytes
   uint64_t* empty = bars + S;                // [S]  own: multicast commit
@@ -88,11 +76,9 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
     ptx::prefetch_tmap(&tmap_b);
     ptx::prefetch_tmap(&tmap_w);
     ptx::prefetch_tmap(&tmap_w16);
-    if (kSplit) {
-      ptx::prefetch_tmap(&tmap_a_lo);
-      ptx::prefetch_tmap(&tmap_b_lo);
-      ptx::prefetch_tmap(&tmap_w_lo);
-    }
+    ptx::prefetch_tmap(&tmap_a_lo);
+    ptx::prefetch_tmap(&tmap_b_lo);
+    ptx::prefetch_tmap(&tmap_w_lo);
     for (int s = 0; s < S; ++s) {
       ptx::mbar_init(&full[s], 1);
       ptx::mbar_init(&empty[s], 1);
@@ -135,13 +121,9 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
       const uint32_t wf_leader = ptx::mapa_u32(ptx::smem_u32(wf_full), 0);
       if (ptx::elect_one()) {
         if (rank == 0) ptx::mbar_arrive_expect_tx(wf_full, 2 * (Cfg::kWxBytes + Cfg::kWyBytes));
-        if constexpr (!kSplit) {
-          for (int c = 0; c < 4; ++c) ptx::tma_load_2d_2sm(wy + c * 2048, &tmap_w16, wf_leader, 64 * c, 16 * (int)rank);
-        } else {
-          for (int c = 0; c < 4; ++c) {            // c = half * 2 + chunk: channels [64c, 64c + 64)
-            ptx::tma_load_2d_2sm(wx + c * 4096, rank == 0 ? &tmap_w : &tmap_w_lo, wf_leader, 64 * c, 0);
-            ptx::tma_load_2d_2sm(wy + c * 2048, &tmap_w16, wf_leader, 64 * c, 16 * (int)rank);
-          }
+        for (int c = 0; c < 4; ++c) {              // c = half * 2 + chunk: channels [64c, 64c + 64)
+          ptx::tma_load_2d_2sm(wx + c * 4096, rank == 0 ? &tmap_w : &tmap_w_lo, wf_leader, 64 * c, 0);
+          ptx::tma_load_2d_2sm(wy + c * 2048, &tmap_w16, wf_leader, 64 * c, 16 * (int)rank);
         }
       }
       __syncwarp();
@@ -162,9 +144,9 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
             if (ptx::elect_one()) {
               if (rank == 0) ptx::mbar_arrive_expect_tx(&full[s], 2 * Cfg::kStageBytes);
               ptx::tma_load_4d_2sm(st_a(s, 0), &tmap_a, full_leader, k0, dx, ys, img0);
-              if (kSplit) ptx::tma_load_4d_2sm(st_a(s, 1), &tmap_a_lo, full_leader, k0, dx, ys, img0);
+              ptx::tma_load_4d_2sm(st_a(s, 1), &tmap_a_lo, full_leader, k0, dx, ys, img0);
               ptx::tma_load_2d_2sm(st_b(s, 0), &tmap_b, full_leader, bk, brow);
-              if (kSplit) ptx::tma_load_2d_2sm(st_b(s, 1), &tmap_b_lo, full_leader, bk, brow);
+              ptx::tma_load_2d_2sm(st_b(s, 1), &tmap_b_lo, full_leader, bk, brow);
             }
             __syncwarp();
           }
@@ -175,7 +157,7 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
     // ===================================================================== MMA issuer (leader CTA only; converged)
     if (rank == 0) {
       const uint32_t tb = __shfl_sync(0xffffffffu, tmem_base, 0);
-      constexpr uint32_t fmt = KIND == kKindBF16 ? 1u : 0u;
+      constexpr uint32_t fmt = 0u;             // kind::f16 operand format: f16
       constexpr uint32_t kM2 = (uint32_t)((2 * kTcBM) >> 4) << 24;          // M = 256 across the pair
       constexpr uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(BN >> 3) << 17) | kM2;
       constexpr uint32_t idesc_n32 = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(32 >> 3) << 17) | kM2;
@@ -194,37 +176,24 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
         ptx::tc_fence_after();
         const uint32_t t = r / Cfg::kRounds, j = r % Cfg::kRounds;
         const uint32_t acc = t & 1;
-        if constexpr (!kSplit) {
-          const uint32_t d = tb + acc * BN;
-          const uint64_t da0 = desc(a2), dw0 = desc(wy);
-          if (ptx::elect_one()) {
+        // [hi.Wh | hi.Wl] in ONE N = 64 MMA: the hi and lo planes of the 32 final-layer rows are adjacent 32-row blocks
+        // of the operand and their accumulators adjacent 32-column blocks in TMEM — the hi plane of A2 is read once
+        // instead of twice (the heat MMAs are bound by their operand reads); lo.Wh then adds into the correction columns.
+        const uint32_t nh = t % NH;            // tiles alternate between the two channel halves of a unit
+        const uint32_t d_hm = tb + (2 + acc) * BN, d_hc = d_hm + 32;
+        const uint64_t da = desc(a2), dal = desc(a2 + kABytes);
+        const uint64_t dx = desc(wx) + (uint64_t)((nh * 2 + j) * (4096 >> 4));     // [Wh ; Wl] split across the pair
+        const uint64_t dy = desc(wy) + (uint64_t)((nh * 2 + j) * (2048 >> 4));     // Wh split across the pair
+        const uint32_t first = j != 0;
+        if (ptx::elect_one()) {
 #pragma unroll
-            for (int c = 0; c < 4; ++c) {
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                ptx::umma_f16_2sm(d, da0 + (uint64_t)(c * (kABytes >> 4) + 2 * k), dw0 + (uint64_t)(c * (2048 >> 4) + 2 * k),
-                                  idesc_n32, (c | k) != 0);
-            }
-            ptx::umma_commit_2sm_mc(&a2_empty[j], 3);
-            ptx::umma_commit_2sm_mc(&heat_full[acc], 3);
+          for (int k = 0; k < 4; ++k) {
+            const uint64_t o = (uint64_t)(2 * k);
+            ptx::umma_f16_2sm(d_hm, da + o, dx + o, idesc_n64, k ? 1u : first);      // hi * [hi ; lo]
+            ptx::umma_f16_2sm(d_hc, dal + o, dy + o, idesc_n32, 1u);                 // lo * hi
           }
-        } else {
-          const uint32_t nh = t % NH;
-          const uint32_t d_hm = tb + (2 + acc) * BN, d_hc = d_hm + 32;
-          const uint64_t da = desc(a2), dal = desc(a2 + kABytes);
-          const uint64_t dx = desc(wx) + (uint64_t)((nh * 2 + j) * (4096 >> 4));     // [Wh ; Wl] split across the pair
-          const uint64_t dy = desc(wy) + (uint64_t)((nh * 2 + j) * (2048 >> 4));     // Wh split across the pair
-          const uint32_t first = j != 0;
-          if (ptx::elect_one()) {
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const uint64_t o = (uint64_t)(2 * k);
-              ptx::umma_f16_2sm(d_hm, da + o, dx + o, idesc_n64, k ? 1u : first);      // hi * [hi ; lo]
-              ptx::umma_f16_2sm(d_hc, dal + o, dy + o, idesc_n32, 1u);                 // lo * hi
-            }
-            ptx::umma_commit_2sm_mc(&a2_empty[j], 3);
-            if (j == Cfg::kRounds - 1) ptx::umma_commit_2sm_mc(&heat_full[acc], 3);
-          }
+          ptx::umma_commit_2sm_mc(&a2_empty[j], 3);
+          if (j == Cfg::kRounds - 1) ptx::umma_commit_2sm_mc(&heat_full[acc], 3);
         }
         __syncwarp();
       };
@@ -250,59 +219,43 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
           if (tl >= 2) force_rounds((tl - 1) * Cfg::kRounds);
           ptx::mbar_wait(&tmem_empty[acc], ((tl >> 1) & 1) ^ 1u);
           ptx::tc_fence_after();
-          if constexpr (!kSplit) {
-            const uint32_t d_tmem = tb + acc * BN;
-            for (int kb = 0; kb < kNumKb; ++kb, ++it) {
+          const uint32_t d_corr = tb + (2 + acc) * BN;
+          for (int kb0 = 0; kb0 < kNumKb; kb0 += kSplitChunk, ++ch) {
+            const int buf = ch & 1;
+            // The drain of this chunk buffer may sit behind a hand-off only this warp can complete (column group 1
+            // waits for group 0's heat MMAs before it writes A2, then drains): keep serving rounds while waiting.
+            {
+              const long long t0 = clock64();
+              while (!__all_sync(0xffffffffu, ptx::mbar_test_wait(&chunk_empty[buf], ((ch >> 1) & 1) ^ 1u))) {
+                poll_rounds();
+                if (clock64() - t0 > 8000000000LL) __trap();
+              }
+            }
+            ptx::tc_fence_after();
+            const uint32_t d_main = tb + (uint32_t)(buf * BN);
+            const int kb1 = kb0 + kSplitChunk < kNumKb ? kb0 + kSplitChunk : kNumKb;
+            for (int kb = kb0; kb < kb1; ++kb, ++it) {
               poll_rounds();
               const int s = it % S;
               ptx::mbar_wait(&full[s], (it / S) & 1);
               ptx::tc_fence_after();
-              const uint64_t da = desc(st_a(s, 0)), db = desc(st_b(s, 0));
+              const uint64_t da = desc(st_a(s, 0)), dal = desc(st_a(s, 1));
+              const uint64_t db = desc(st_b(s, 0)), dbl = desc(st_b(s, 1));
+              const uint32_t first = kb != 0, first_main = kb > kb0;
               if (ptx::elect_one()) {
 #pragma unroll
-                for (int k = 0; k < 4; ++k)
-                  ptx::umma_f16_2sm(d_tmem, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, (kb | k) != 0);
+                for (int k = 0; k < 4; ++k) {
+                  const uint64_t o = (uint64_t)(2 * k);
+                  ptx::umma_f16_2sm(d_corr, dal + o, db + o, idesc, k ? 1u : first);        // lo*hi
+                  ptx::umma_f16_2sm(d_corr, da + o, dbl + o, idesc, 1u);                    // hi*lo
+                  ptx::umma_f16_2sm(d_main, da + o, db + o, idesc, k ? 1u : first_main);    // hi*hi, short chain
+                }
                 ptx::umma_commit_2sm_mc(&empty[s], 3);
               }
               __syncwarp();
             }
-          } else {
-            const uint32_t d_corr = tb + (2 + acc) * BN;
-            for (int kb0 = 0; kb0 < kNumKb; kb0 += kSplitChunk, ++ch) {
-              const int buf = ch & 1;
-              {
-                const long long t0 = clock64();
-                while (!__all_sync(0xffffffffu, ptx::mbar_test_wait(&chunk_empty[buf], ((ch >> 1) & 1) ^ 1u))) {
-                  poll_rounds();
-                  if (clock64() - t0 > 8000000000LL) __trap();
-                }
-              }
-              ptx::tc_fence_after();
-              const uint32_t d_main = tb + (uint32_t)(buf * BN);
-              const int kb1 = kb0 + kSplitChunk < kNumKb ? kb0 + kSplitChunk : kNumKb;
-              for (int kb = kb0; kb < kb1; ++kb, ++it) {
-                poll_rounds();
-                const int s = it % S;
-                ptx::mbar_wait(&full[s], (it / S) & 1);
-                ptx::tc_fence_after();
-                const uint64_t da = desc(st_a(s, 0)), dal = desc(st_a(s, 1));
-                const uint64_t db = desc(st_b(s, 0)), dbl = desc(st_b(s, 1));
-                const uint32_t first = kb != 0, first_main = kb > kb0;
-                if (ptx::elect_one()) {
-#pragma unroll
-                  for (int k = 0; k < 4; ++k) {
-                    const uint64_t o = (uint64_t)(2 * k);
-                    ptx::umma_f16_2sm(d_corr, dal + o, db + o, idesc, k ? 1u : first);        // lo*hi
-                    ptx::umma_f16_2sm(d_corr, da + o, dbl + o, idesc, 1u);                    // hi*lo
-                    ptx::umma_f16_2sm(d_main, da + o, db + o, idesc, k ? 1u : first_main);    // hi*hi, short chain
-                  }
-                  ptx::umma_commit_2sm_mc(&empty[s], 3);
-                }
-                __syncwarp();
-              }
-              if (ptx::elect_one()) ptx::umma_commit_2sm_mc(&chunk_full[buf], 3);
-              __syncwarp();
-            }
+            if (ptx::elect_one()) ptx::umma_commit_2sm_mc(&chunk_full[buf], 3);
+            __syncwarp();
           }
           if (ptx::elect_one()) ptx::umma_commit_2sm_mc(&tmem_full[acc], 3);
           __syncwarp();
@@ -321,15 +274,14 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
     const int row = q * 32 + lane;
     const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16);
     uint32_t tl = 0, ch = 0;
-    float a_inv = 1.f, s_out = 1.f;
-    if constexpr (kSplit) {
-      a_inv = 1.f / __ldcg(p.scale_in);
-      const float bound = __ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1);
-      s_out = f16_pow2_scale(bound);
-    }
-    auto wait_a2_free = [&]() {              // own a2_empty[]: released for both CTAs by multicast commits (tail_tc.cuh)
-      if constexpr (!kSplit) ptx::mbar_wait(&a2_empty[0], (tl & 1) ^ 1u);
-      else if (grp == 0) ptx::mbar_wait(&a2_empty[1], (tl & 1) ^ 1u);
+    const float a_inv = 1.f / __ldcg(p.scale_in);
+    const float s_out = f16_pow2_scale(__ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1));
+    // A2 is free for this warp's hand-off of tile tl once the heat MMAs of the hand-off BEFORE it have completed:
+    //   column group 0: group 1's hand-off of tile tl-1 -> a2_empty[1], phase tl-1
+    //   column group 1: group 0's hand-off of tile tl   -> a2_empty[0], phase tl
+    // ("phase -1" of a fresh barrier reads as complete.)  Own a2_empty[]: released for both CTAs by multicast commits.
+    auto wait_a2_free = [&]() {
+      if (grp == 0) ptx::mbar_wait(&a2_empty[1], (tl & 1) ^ 1u);
       else ptx::mbar_wait(&a2_empty[0], tl & 1);
     };
     auto publish_a2 = [&]() {
@@ -344,99 +296,63 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
         const uint32_t acc = tl & 1;
         const int n_base = nh * BN + cb0;
         const float* __restrict__ bias = p.bias + n_base;
-        if constexpr (!kSplit) {
-          ptx::mbar_wait(&tmem_full[acc], (tl >> 1) & 1);
-          ptx::tc_fence_after();
-          wait_a2_free();
-#pragma unroll 1
-          for (int c = 0; c < kCols; c += 64) {
-            uint32_t r0[32], r1[32];
-            ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)(acc * BN + cb0 + c), r0);
-            ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)(acc * BN + cb0 + c + 32), r1);
-            ptx::tmem_ld_wait();
-            uint32_t w[32];
+        float sum[kCols];
 #pragma unroll
-            for (int j4 = 0; j4 < 8; ++j4) {
-              const float4 b4 = __ldg(reinterpret_cast<const float4*>(bias + c) + j4);
-              const float4 b5 = __ldg(reinterpret_cast<const float4*>(bias + c + 32) + j4);
-              const __nv_bfloat162 x0 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r0[4 * j4]) + b4.x, 0.f),
-                                                              fmaxf(__uint_as_float(r0[4 * j4 + 1]) + b4.y, 0.f));
-              const __nv_bfloat162 x1 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r0[4 * j4 + 2]) + b4.z, 0.f),
-                                                              fmaxf(__uint_as_float(r0[4 * j4 + 3]) + b4.w, 0.f));
-              const __nv_bfloat162 y0 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r1[4 * j4]) + b5.x, 0.f),
-                                                              fmaxf(__uint_as_float(r1[4 * j4 + 1]) + b5.y, 0.f));
-              const __nv_bfloat162 y1 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r1[4 * j4 + 2]) + b5.z, 0.f),
-                                                              fmaxf(__uint_as_float(r1[4 * j4 + 3]) + b5.w, 0.f));
-              w[2 * j4] = *reinterpret_cast<const uint32_t*>(&x0);
-              w[2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&x1);
-              w[16 + 2 * j4] = *reinterpret_cast<const uint32_t*>(&y0);
-              w[16 + 2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&y1);
-            }
-            const uint32_t base = ptx::smem_u32(a2) + (uint32_t)(((cb0 + c) >> 6) * kABytes) + (uint32_t)row * 128u;
-#pragma unroll
-            for (int j = 0; j < 8; ++j)
-              tail_st(base + (uint32_t)((j ^ (row & 7)) << 4), w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
-          }
-          publish_a2();
-        } else {
-          float sum[kCols];
-#pragma unroll
-          for (int j = 0; j < kCols; ++j) sum[j] = 0.f;
-          for (int kb0 = 0; kb0 < kNumKb; kb0 += kSplitChunk, ++ch) {
-            const int buf = ch & 1;
-            ptx::mbar_wait(&chunk_full[buf], (ch >> 1) & 1);
-            ptx::tc_fence_after();
-#pragma unroll
-            for (int c = 0; c < kCols; c += 32) {
-              uint32_t r[32];
-              ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)(buf * BN + cb0 + c), r);
-              ptx::tmem_ld_wait();
-#pragma unroll
-              for (int j = 0; j < 32; ++j) sum[c + j] += __uint_as_float(r[j]);
-            }
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) arrive_leader(&chunk_empty[buf]);
-          }
-          ptx::mbar_wait(&tmem_full[acc], (tl >> 1) & 1);
+        for (int j = 0; j < kCols; ++j) sum[j] = 0.f;
+        for (int kb0 = 0; kb0 < kNumKb; kb0 += kSplitChunk, ++ch) {
+          const int buf = ch & 1;
+          ptx::mbar_wait(&chunk_full[buf], (ch >> 1) & 1);
           ptx::tc_fence_after();
 #pragma unroll
           for (int c = 0; c < kCols; c += 32) {
             uint32_t r[32];
-            ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)((2 + acc) * BN + cb0 + c), r);
+            ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)(buf * BN + cb0 + c), r);
             ptx::tmem_ld_wait();
 #pragma unroll
-            for (int j = 0; j < 32; ++j) sum[c + j] = fmaf(__uint_as_float(r[j]), 1.f / kLoScale, sum[c + j]);
+            for (int j = 0; j < 32; ++j) sum[c + j] += __uint_as_float(r[j]);
           }
-          const float* __restrict__ wsi = p.wsi + (size_t)g * kDecC + n_base;
-          uint32_t wh[32], wl[32];
-#pragma unroll
-          for (int j4 = 0; j4 < kCols / 4; ++j4) {
-            const float4 w4 = __ldg(reinterpret_cast<const float4*>(wsi) + j4);
-            const float4 b4 = __ldg(reinterpret_cast<const float4*>(bias) + j4);
-            const float v0 = fmaxf(sum[4 * j4] * (a_inv * w4.x) + b4.x, 0.f) * s_out;
-            const float v1 = fmaxf(sum[4 * j4 + 1] * (a_inv * w4.y) + b4.y, 0.f) * s_out;
-            const float v2 = fmaxf(sum[4 * j4 + 2] * (a_inv * w4.z) + b4.z, 0.f) * s_out;
-            const float v3 = fmaxf(sum[4 * j4 + 3] * (a_inv * w4.w) + b4.w, 0.f) * s_out;
-            const __half2 h01 = __floats2half2_rn(v0, v1), h23 = __floats2half2_rn(v2, v3);
-            const float2 f01 = __half22float2(h01), f23 = __half22float2(h23);
-            const __half2 l01 = __floats2half2_rn((v0 - f01.x) * kLoScale, (v1 - f01.y) * kLoScale);
-            const __half2 l23 = __floats2half2_rn((v2 - f23.x) * kLoScale, (v3 - f23.y) * kLoScale);
-            wh[2 * j4] = *reinterpret_cast<const uint32_t*>(&h01);
-            wh[2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&h23);
-            wl[2 * j4] = *reinterpret_cast<const uint32_t*>(&l01);
-            wl[2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&l23);
-          }
-          wait_a2_free();
-          const uint32_t base = ptx::smem_u32(a2) + (uint32_t)row * 128u;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const uint32_t o = (uint32_t)((j ^ (row & 7)) << 4);
-            tail_st(base + o, wh[4 * j], wh[4 * j + 1], wh[4 * j + 2], wh[4 * j + 3]);
-            tail_st(base + kABytes + o, wl[4 * j], wl[4 * j + 1], wl[4 * j + 2], wl[4 * j + 3]);
-          }
-          publish_a2();
+          ptx::tc_fence_before();
+          __syncwarp();
+          if (lane == 0) arrive_leader(&chunk_empty[buf]);
         }
+        ptx::mbar_wait(&tmem_full[acc], (tl >> 1) & 1);
+        ptx::tc_fence_after();
+#pragma unroll
+        for (int c = 0; c < kCols; c += 32) {
+          uint32_t r[32];
+          ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)((2 + acc) * BN + cb0 + c), r);
+          ptx::tmem_ld_wait();
+#pragma unroll
+          for (int j = 0; j < 32; ++j) sum[c + j] = fmaf(__uint_as_float(r[j]), 1.f / kLoScale, sum[c + j]);
+        }
+        const float* __restrict__ wsi = p.wsi + (size_t)g * kDecC + n_base;
+        uint32_t wh[32], wl[32];
+#pragma unroll
+        for (int j4 = 0; j4 < kCols / 4; ++j4) {
+          const float4 w4 = __ldg(reinterpret_cast<const float4*>(wsi) + j4);
+          const float4 b4 = __ldg(reinterpret_cast<const float4*>(bias) + j4);
+          const float v0 = fmaxf(sum[4 * j4] * (a_inv * w4.x) + b4.x, 0.f) * s_out;
+          const float v1 = fmaxf(sum[4 * j4 + 1] * (a_inv * w4.y) + b4.y, 0.f) * s_out;
+          const float v2 = fmaxf(sum[4 * j4 + 2] * (a_inv * w4.z) + b4.z, 0.f) * s_out;
+          const float v3 = fmaxf(sum[4 * j4 + 3] * (a_inv * w4.w) + b4.w, 0.f) * s_out;
+          const __half2 h01 = __floats2half2_rn(v0, v1), h23 = __floats2half2_rn(v2, v3);
+          const float2 f01 = __half22float2(h01), f23 = __half22float2(h23);
+          const __half2 l01 = __floats2half2_rn((v0 - f01.x) * kLoScale, (v1 - f01.y) * kLoScale);
+          const __half2 l23 = __floats2half2_rn((v2 - f23.x) * kLoScale, (v3 - f23.y) * kLoScale);
+          wh[2 * j4] = *reinterpret_cast<const uint32_t*>(&h01);
+          wh[2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&h23);
+          wl[2 * j4] = *reinterpret_cast<const uint32_t*>(&l01);
+          wl[2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&l23);
+        }
+        wait_a2_free();
+        const uint32_t base = ptx::smem_u32(a2) + (uint32_t)row * 128u;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const uint32_t o = (uint32_t)((j ^ (row & 7)) << 4);
+          ptx::st_shared_v4(base + o, wh[4 * j], wh[4 * j + 1], wh[4 * j + 2], wh[4 * j + 3]);
+          ptx::st_shared_v4(base + kABytes + o, wl[4 * j], wl[4 * j + 1], wl[4 * j + 2], wl[4 * j + 3]);
+        }
+        publish_a2();
       }
     }
   } else {
@@ -445,11 +361,8 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
     const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16);
     const int J = p.joints;
     uint32_t tl = 0;
-    float fin_scale = 1.f;
-    if constexpr (kSplit) {
-      const float bound = __ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1);
-      fin_scale = ldexpf(1.f, -f16_pow2_exp(bound));
-    }
+    // 1 / s(deconv3 activation)
+    const float fin_scale = ldexpf(1.f, -f16_pow2_exp(__ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1)));
     const float kLog2e = 1.4426950408889634f;
     for (int pu = pu0; pu < num_pu; pu += pu_step) {
       const int g = pu & 3, m0 = unit_m0(pu);
@@ -459,22 +372,14 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
         const uint32_t acc = tl & 1;
         ptx::mbar_wait(&heat_full[acc], (tl >> 1) & 1);
         ptx::tc_fence_after();
-        uint32_t r[32];
-        if constexpr (!kSplit) {
-          ptx::tmem_ld_32x32b_x32(lane_addr + acc * BN, r);
-          ptx::tmem_ld_wait();
+        uint32_t r[32], rc[32];
+        ptx::tmem_ld_32x32b_x32(lane_addr + (2 + acc) * BN, r);
+        ptx::tmem_ld_32x32b_x32(lane_addr + (2 + acc) * BN + 32, rc);
+        ptx::tmem_ld_wait();
 #pragma unroll
-          for (int j = 0; j < 32; ++j) hv[j] = __uint_as_float(r[j]);
-        } else {
-          uint32_t rc[32];
-          ptx::tmem_ld_32x32b_x32(lane_addr + (2 + acc) * BN, r);
-          ptx::tmem_ld_32x32b_x32(lane_addr + (2 + acc) * BN + 32, rc);
-          ptx::tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const float v = fmaf(__uint_as_float(rc[j]), 1.f / kLoScale, __uint_as_float(r[j]));
-            hv[j] = nh == 0 ? v : hv[j] + v;
-          }
+        for (int j = 0; j < 32; ++j) {
+          const float v = fmaf(__uint_as_float(rc[j]), 1.f / kLoScale, __uint_as_float(r[j]));
+          hv[j] = nh == 0 ? v : hv[j] + v;       // the first half's partial waits here, in registers
         }
         ptx::tc_fence_before();
         __syncwarp();
@@ -489,7 +394,7 @@ deconv_tail_pair_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid
       for (int j = 0; j < 32; ++j) {
         if (j < J) {
           float v = hv[j];
-          if constexpr (kSplit) v *= fin_scale * __ldg(p.wsi_fin + j);
+          v *= fin_scale * __ldg(p.wsi_fin + j);
           v += __ldg(p.bias_fin + j);
           if (p.heat) p.heat[((size_t)img * J + j) * 4096 + oy * 64 + ox] = v;
           if (p.part) {

@@ -5,8 +5,8 @@
 //
 // Per (128-pixel block of the 32x32 input grid, output phase g) the main loop is the tap-GEMM of gemm_tc.cu (4 taps as
 // shifted 4-D TMA boxes, tcgen05.mma into TMEM).  Then, instead of storing the tile:
-//   convert warps (8)  TMEM -> registers, + folded-BN bias, ReLU, encode (bf16 | scaled fp16 hi/lo planes) and write the
-//                      tile into a 128B-swizzled shared-memory buffer "A2" laid out as the A operand of a second MMA;
+//   convert warps (8)  TMEM -> registers, + folded-BN bias, ReLU, encode bf16 and write the tile into a 128B-swizzled
+//                      shared-memory buffer "A2" laid out as the A operand of a second MMA;
 //   MMA issuer         polls for A2 between K blocks of the NEXT tile and issues heat[128 x 32] (+)= A2 * Wfin^T
 //                      (Wfin resident in shared memory) into TMEM columns of the accumulator the convert warps have
 //                      just finished reading — no extra TMEM;
@@ -16,12 +16,8 @@
 // A second, tiny kernel merges the 128 partials of every heat-map (online-softmax merge in fp64), scales to image
 // pixels and runs the per-joint DLT (+ MPJPE terms) — tail_merge_dlt_kernel.
 //
-// Two operand kinds:
-//   bf16  : BN = 256 (whole channel range per tile), ring of 3 x 48 KB K-blocks, A2 = 64 KB (one hand-off per tile).
-//   f16x2 : BN = 128 (TMEM holds 2 main-chunk + 2 correction accumulators of 128 columns), the two channel halves of a
-//           pixel block run back to back in the same CTA and the heat partial of the first half waits in registers of the
-//           heat warps.  Ring of 5 x 32 KB half-slots (a K-block = an A slot [hi|lo] + a B slot [hi|lo]), A2 = 32 KB =
-//           one 64-channel K chunk in both planes: two hand-offs per tile (column group 0, then group 1).
+// This kernel runs the bf16 decoder: BN = 256 (whole channel range per tile), ring of 3 x 48 KB K-blocks, A2 = 64 KB (one
+// hand-off per tile).  The f16x2 decoder runs the same tail on cta_group::2 CTA pairs (tail_pair_tc.cuh).
 #pragma once
 
 namespace cdr {
@@ -43,50 +39,27 @@ struct TailParams {
   float4* part;             // (n_img, J, kTailSlots) records {max, sum e, sum lane*e, -}
 };
 
-template <int KIND> struct TailCfg;
-template <> struct TailCfg<kKindBF16> {
-  static constexpr int kBN = 256, kNH = 1, kPlanes = 1;
-  static constexpr int kSlotsPerKb = 1, kSlots = 3, kSlotBytes = kABytes + kBN * 128;     // 48 KB
+struct TailCfg {
+  static constexpr int kBN = 256;
+  static constexpr int kSlots = 3, kSlotBytes = kABytes + kBN * 128;     // 48 KB
   static constexpr int kA2Bytes = 4 * kABytes;          // four 64-channel K chunks
   static constexpr int kWfBytes = 4 * 32 * 128;         // 32 rows x 256 channels bf16
-  static constexpr int kRounds = 1, kRoundWarps = 8;
-};
-template <> struct TailCfg<kKindF16X2> {
-  static constexpr int kBN = 128, kNH = 2, kPlanes = 2;
-  static constexpr int kSlotsPerKb = 2, kSlots = 5, kSlotBytes = 2 * kABytes;             // 32 KB: [hi | lo]
-  static constexpr int kA2Bytes = 2 * kABytes;          // one 64-channel K chunk, hi and lo planes
-  static constexpr int kWfBytes = 2 * 2 * 2 * 32 * 128; // (half, chunk, plane) x 32 rows x 64 channels fp16
-  static constexpr int kRounds = 2, kRoundWarps = 4;
-};
-template <int KIND> struct TailSmem {
-  using Cfg = TailCfg<KIND>;
-  static constexpr size_t kBytes = (size_t)Cfg::kSlots * Cfg::kSlotBytes + Cfg::kA2Bytes + Cfg::kWfBytes + 1024 + 512;
-  static_assert(kBytes <= 227 * 1024, "shared memory budget");
+  static constexpr size_t kSmemBytes = (size_t)kSlots * kSlotBytes + kA2Bytes + kWfBytes + 1024 + 512;
+  static_assert(kSmemBytes <= 227 * 1024, "shared memory budget");
 };
 constexpr int kTailThreads = 32 * 14;     // producer, MMA issuer, 8 convert warps, 4 heat warps
 
-__device__ __forceinline__ void tail_st(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
-#ifdef CDR_EXP_TAIL_NO_HANDOFF   /* timing experiment: the converted tile is computed and dropped */
-  if (a == 0x12345678u && b == 0x9abcdef0u) ptx::st_shared_v4(addr, a, b, c, d);
-#else
-  ptx::st_shared_v4(addr, a, b, c, d);
-#endif
-}
 __device__ __forceinline__ float ptx_ex2(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));   // one MUFU.EX2, rel. error 2^-22
   return y;
 }
 
-template <int KIND>
 __global__ void __launch_bounds__(kTailThreads, 1)
-deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_a_lo,
-                   const __grid_constant__ CUtensorMap tmap_b, const __grid_constant__ CUtensorMap tmap_b_lo,
-                   const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ CUtensorMap tmap_w_lo,
-                   const TailParams p) {
-  using Cfg = TailCfg<KIND>;
-  constexpr bool kSplit = KIND == kKindF16X2;
-  constexpr int BN = Cfg::kBN, NH = Cfg::kNH, S = Cfg::kSlots, SPK = Cfg::kSlotsPerKb;
+deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
+                   const __grid_constant__ CUtensorMap tmap_w, const TailParams p) {
+  using Cfg = TailCfg;
+  constexpr int BN = Cfg::kBN, S = Cfg::kSlots;
   constexpr int kNumKb = 16;                       // 4 taps x 256 input channels / 64
   constexpr int kW = 32, kHW = 1024;               // input grid of deconv3
   extern __shared__ uint8_t smem_raw[];
@@ -97,17 +70,13 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
   uint64_t* bars = reinterpret_cast<uint64_t*>(wf + Cfg::kWfBytes);
   uint64_t* full = bars;                     // [S]
   uint64_t* empty = bars + S;                // [S]
-  uint64_t* tmem_full = bars + 2 * S;        // [2] tile accumulator (bf16) / correction accumulator (f16x2) complete
+  uint64_t* tmem_full = bars + 2 * S;        // [2] tile accumulator complete
   uint64_t* tmem_empty = bars + 2 * S + 2;   // [2] heat of that accumulator read: 4 heat warps
-  uint64_t* chunk_full = bars + 2 * S + 4;   // [2] f16x2: main-term chunk
-  uint64_t* chunk_empty = bars + 2 * S + 6;  // [2]
-  uint64_t* heat_full = bars + 2 * S + 8;    // [2]
-  uint64_t* a2_full = bars + 2 * S + 10;     // one phase per hand-off round
-  uint64_t* a2_empty = bars + 2 * S + 11;    // [2] heat MMAs of column group j's round complete (bf16: [0] only).  One
-                                             // barrier per group: its waiter is the OTHER group, which cannot fall two
-                                             // phases behind (a parity wait only tells the current phase from the last)
-  uint64_t* wf_full = bars + 2 * S + 13;
-  uint32_t* tmem_base_slot = reinterpret_cast<uint32_t*>(bars + 2 * S + 14);
+  uint64_t* heat_full = bars + 2 * S + 4;    // [2]
+  uint64_t* a2_full = bars + 2 * S + 6;      // one phase per hand-off (tile)
+  uint64_t* a2_empty = bars + 2 * S + 7;     // heat MMAs of the last hand-off complete
+  uint64_t* wf_full = bars + 2 * S + 8;
+  uint32_t* tmem_base_slot = reinterpret_cast<uint32_t*>(bars + 2 * S + 9);
 
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);   // provably warp-uniform (see the issuer)
   const int lane = threadIdx.x & 31;
@@ -117,11 +86,6 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     ptx::prefetch_tmap(&tmap_a);
     ptx::prefetch_tmap(&tmap_b);
     ptx::prefetch_tmap(&tmap_w);
-    if (kSplit) {
-      ptx::prefetch_tmap(&tmap_a_lo);
-      ptx::prefetch_tmap(&tmap_b_lo);
-      ptx::prefetch_tmap(&tmap_w_lo);
-    }
     for (int s = 0; s < S; ++s) {
       ptx::mbar_init(&full[s], 1);
       ptx::mbar_init(&empty[s], 1);
@@ -129,13 +93,10 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     for (int a = 0; a < 2; ++a) {
       ptx::mbar_init(&tmem_full[a], 1);
       ptx::mbar_init(&tmem_empty[a], 4);
-      ptx::mbar_init(&chunk_full[a], 1);
-      ptx::mbar_init(&chunk_empty[a], 8);
       ptx::mbar_init(&heat_full[a], 1);
     }
-    ptx::mbar_init(a2_full, Cfg::kRoundWarps);
-    ptx::mbar_init(&a2_empty[0], 1);
-    ptx::mbar_init(&a2_empty[1], 1);
+    ptx::mbar_init(a2_full, 8);
+    ptx::mbar_init(a2_empty, 1);
     ptx::mbar_init(wf_full, 1);
     ptx::fence_mbar_init();
   }
@@ -143,12 +104,10 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
   ptx::tc_fence_before();
   __syncthreads();
   ptx::tc_fence_after();
-  ptx::grid_dep_wait();              // d2 and its scale slots are complete and visible
+  ptx::grid_dep_wait();              // d2 is complete and visible
   const uint32_t tmem_base = *tmem_base_slot;
-  // TMEM columns.  bf16 : [0,256) [256,512) two tile accumulators; heat of tile t in the first 32 columns of ITS
-  //                       accumulator (written after the convert warps have drained it).
-  //                f16x2: [0,128) [128,256) main-term chunk accumulators, [256,384) [384,512) correction accumulators;
-  //                       heat of tile t in columns [0,32) (main) and [32,64) (correction) of its correction accumulator.
+  // TMEM columns: [0,256) [256,512) two tile accumulators; heat of tile t in the first 32 columns of ITS accumulator
+  // (written after the convert warps have drained it).
 
   if (warp == 0) {
     // ===================================================================== TMA producer (converged; an elected lane issues)
@@ -156,14 +115,7 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
       // final-layer weights: resident for the whole kernel
       if (ptx::elect_one()) {
         ptx::mbar_arrive_expect_tx(wf_full, Cfg::kWfBytes);
-        if constexpr (!kSplit) {
-          for (int c = 0; c < 4; ++c) ptx::tma_load_2d(wf + c * 4096, &tmap_w, wf_full, 64 * c, 0);
-        } else {
-          for (int c = 0; c < 4; ++c) {            // c = half * 2 + chunk: channels [64c, 64c + 64)
-            ptx::tma_load_2d(wf + (c * 2 + 0) * 4096, &tmap_w, wf_full, 64 * c, 0);
-            ptx::tma_load_2d(wf + (c * 2 + 1) * 4096, &tmap_w_lo, wf_full, 64 * c, 0);
-          }
-        }
+        for (int c = 0; c < 4; ++c) ptx::tma_load_2d(wf + c * 4096, &tmap_w, wf_full, 64 * c, 0);
       }
       __syncwarp();
       uint32_t pos = 0;                          // ring position (slots)
@@ -171,43 +123,19 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
         const int g = unit & 3, m0 = (unit >> 2) * kTcBM;
         const int py = g >> 1, px = g & 1;
         const int img0 = m0 / kHW, y0 = (m0 - img0 * kHW) / kW;
-        for (int nh = 0; nh < NH; ++nh) {
-          for (int kb = 0; kb < kNumKb; ++kb) {
-            const int tap = kb >> 2, k0 = (kb & 3) * 64;
-            const int dy = py - (tap >> 1), dx = px - (tap & 1);
-            const int brow = g * kDecC + nh * BN;
-            const int bk = tap * kDecC + k0, ys = y0 + dy;
-            if constexpr (!kSplit) {
-              const int s = pos % S;
-              ptx::mbar_wait(&empty[s], ((pos / S) & 1) ^ 1u);
-              if (ptx::elect_one()) {
-                ptx::mbar_arrive_expect_tx(&full[s], Cfg::kSlotBytes);
-                ptx::tma_load_4d(slot_ptr(s), &tmap_a, &full[s], k0, dx, ys, img0);
-                ptx::tma_load_2d(slot_ptr(s) + kABytes, &tmap_b, &full[s], bk, brow);
-              }
-              __syncwarp();
-              ++pos;
-            } else {
-              int s = pos % S;
-              ptx::mbar_wait(&empty[s], ((pos / S) & 1) ^ 1u);
-              if (ptx::elect_one()) {
-                ptx::mbar_arrive_expect_tx(&full[s], Cfg::kSlotBytes);
-                ptx::tma_load_4d(slot_ptr(s), &tmap_a, &full[s], k0, dx, ys, img0);
-                ptx::tma_load_4d(slot_ptr(s) + kABytes, &tmap_a_lo, &full[s], k0, dx, ys, img0);
-              }
-              __syncwarp();
-              ++pos;
-              s = pos % S;
-              ptx::mbar_wait(&empty[s], ((pos / S) & 1) ^ 1u);
-              if (ptx::elect_one()) {
-                ptx::mbar_arrive_expect_tx(&full[s], Cfg::kSlotBytes);
-                ptx::tma_load_2d(slot_ptr(s), &tmap_b, &full[s], bk, brow);
-                ptx::tma_load_2d(slot_ptr(s) + kABytes, &tmap_b_lo, &full[s], bk, brow);
-              }
-              __syncwarp();
-              ++pos;
-            }
+        for (int kb = 0; kb < kNumKb; ++kb, ++pos) {
+          const int tap = kb >> 2, k0 = (kb & 3) * 64;
+          const int dy = py - (tap >> 1), dx = px - (tap & 1);
+          const int brow = g * kDecC;
+          const int bk = tap * kDecC + k0, ys = y0 + dy;
+          const int s = pos % S;
+          ptx::mbar_wait(&empty[s], ((pos / S) & 1) ^ 1u);
+          if (ptx::elect_one()) {
+            ptx::mbar_arrive_expect_tx(&full[s], Cfg::kSlotBytes);
+            ptx::tma_load_4d(slot_ptr(s), &tmap_a, &full[s], k0, dx, ys, img0);
+            ptx::tma_load_2d(slot_ptr(s) + kABytes, &tmap_b, &full[s], bk, brow);
           }
+          __syncwarp();
         }
       }
     }
@@ -218,7 +146,7 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     // issue-bound).  Barrier polls that steer control flow are made warp-uniform with a vote.
     {
       const uint32_t tb = __shfl_sync(0xffffffffu, tmem_base, 0);
-      constexpr uint32_t fmt = KIND == kKindBF16 ? 1u : 0u;
+      constexpr uint32_t fmt = 1u;             // kind::f16 operand format: bf16
       constexpr uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(BN >> 3) << 17) |
                                  ((uint32_t)(kTcBM >> 4) << 24);
       constexpr uint32_t idesc_heat = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(32 >> 3) << 17) |
@@ -226,68 +154,34 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
       constexpr uint64_t desc_hi = ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) |
                                    ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
       auto desc = [&](const uint8_t* ptr) { return desc_hi | (uint64_t)((ptx::smem_u32(ptr) >> 4) & 0x3FFF); };
-      uint32_t pos = 0, tl = 0, ch = 0;
-      uint32_t rounds_issued = 0;              // hand-off rounds whose heat MMAs have been issued
-      uint32_t rounds_due = 0;                 // rounds of tiles whose main loop has been issued
+      uint32_t pos = 0, tl = 0;
+      uint32_t rounds_issued = 0;              // hand-offs (tiles) whose heat MMAs have been issued
+      uint32_t rounds_due = 0;                 // tiles whose main loop has been issued
       bool wf_ready = false;
-      // heat MMAs of hand-off round r (tile r / kRounds): its A2 buffer is full -> issue, release A2, publish heat
-      auto issue_round = [&](uint32_t r) {
+      // heat MMAs of tile t: its A2 buffer is full -> issue, release A2, publish heat
+      auto issue_round = [&](uint32_t t) {
         if (!wf_ready) {
           ptx::mbar_wait(wf_full, 0);
           wf_ready = true;
         }
         ptx::tc_fence_after();
-        const uint32_t t = r / Cfg::kRounds, j = r % Cfg::kRounds;
         const uint32_t acc = t & 1;
-#if defined(CDR_EXP_TAIL_NO_HANDOFF) || defined(CDR_EXP_TAIL_NO_HEAT_MMA)   /* timing experiments: results are wrong */
-        constexpr bool kHeatMma = false;
-#else
-        constexpr bool kHeatMma = true;
-#endif
-        if constexpr (!kSplit) {
-          const uint32_t d = tb + acc * BN;
-          const uint64_t da0 = desc(a2), dw0 = desc(wf);
-          if (ptx::elect_one()) {
-            if constexpr (kHeatMma) {
+        const uint32_t d = tb + acc * BN;
+        const uint64_t da0 = desc(a2), dw0 = desc(wf);
+        if (ptx::elect_one()) {
 #pragma unroll
-              for (int c = 0; c < 4; ++c) {
+          for (int c = 0; c < 4; ++c) {
 #pragma unroll
-                for (int k = 0; k < 4; ++k)
-                  ptx::umma_f16(d, da0 + (uint64_t)(c * (kABytes >> 4) + 2 * k), dw0 + (uint64_t)(c * (4096 >> 4) + 2 * k),
-                                idesc_heat, (c | k) != 0);
-              }
-            }
-            ptx::umma_commit(&a2_empty[j]);
-            ptx::umma_commit(&heat_full[acc]);
+            for (int k = 0; k < 4; ++k)
+              ptx::umma_f16(d, da0 + (uint64_t)(c * (kABytes >> 4) + 2 * k), dw0 + (uint64_t)(c * (4096 >> 4) + 2 * k),
+                            idesc_heat, (c | k) != 0);
           }
-        } else {
-          const uint32_t nh = t % NH;           // tiles alternate between the two channel halves of a unit
-          // [hi.Wh | hi.Wl] in ONE N = 64 MMA: the hi and lo planes of the 32 final-layer rows are adjacent 32-row blocks
-          // in shared memory (one 64-row K-major tile) and their accumulators adjacent 32-column blocks in TMEM — the
-          // hi plane of A2 is read once instead of twice (the heat MMAs are bound by their operand reads: N = 32 computes
-          // in 16 cycles what takes 40 to read); lo.Wh then adds into the correction columns.
-          constexpr uint32_t idesc_heat64 = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(64 >> 3) << 17) |
-                                            ((uint32_t)(kTcBM >> 4) << 24);
-          const uint32_t d_hm = tb + (2 + acc) * BN, d_hc = d_hm + 32;
-          const uint64_t da = desc(a2), dal = desc(a2 + kABytes);
-          const uint64_t dw = desc(wf) + (uint64_t)(((nh * 2 + j) * 2) * (4096 >> 4));      // rows 0-31 hi, 32-63 lo
-          const uint32_t first = j != 0;
-          if (ptx::elect_one()) {
-            if constexpr (kHeatMma) {
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                const uint64_t o = (uint64_t)(2 * k);
-                ptx::umma_f16(d_hm, da + o, dw + o, idesc_heat64, k ? 1u : first);         // hi * [hi ; lo]
-                ptx::umma_f16(d_hc, dal + o, dw + o, idesc_heat, 1u);                      // lo * hi
-              }
-            }
-            ptx::umma_commit(&a2_empty[j]);
-            if (j == Cfg::kRounds - 1) ptx::umma_commit(&heat_full[acc]);
-          }
+          ptx::umma_commit(a2_empty);
+          ptx::umma_commit(&heat_full[acc]);
         }
         __syncwarp();
       };
-      // has the next due hand-off round been written?  (a vote makes the answer — and the branch — warp-uniform)
+      // has the next due hand-off been written?  (a vote makes the answer — and the branch — warp-uniform)
       auto round_ready = [&]() {
         return rounds_issued < rounds_due && __all_sync(0xffffffffu, ptx::mbar_test_wait(a2_full, rounds_issued & 1));
       };
@@ -304,75 +198,30 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
           ++rounds_issued;
         }
       };
-      for (int unit = blockIdx.x; unit < p.num_units; unit += gridDim.x) {
-        for (int nh = 0; nh < NH; ++nh, ++tl) {
-          const uint32_t acc = tl & 1;
-          // the heat of the tile that used this accumulator must have been issued before we can wait for its readers
-          if (tl >= 2) force_rounds((tl - 1) * Cfg::kRounds);
-          ptx::mbar_wait(&tmem_empty[acc], ((tl >> 1) & 1) ^ 1u);
+      for (int unit = blockIdx.x; unit < p.num_units; unit += gridDim.x, ++tl) {
+        const uint32_t acc = tl & 1;
+        // the heat of the tile that used this accumulator must have been issued before we can wait for its readers
+        if (tl >= 2) force_rounds(tl - 1);
+        ptx::mbar_wait(&tmem_empty[acc], ((tl >> 1) & 1) ^ 1u);
+        ptx::tc_fence_after();
+        const uint32_t d_tmem = tb + acc * BN;
+        for (int kb = 0; kb < kNumKb; ++kb, ++pos) {
+          poll_rounds();
+          const int s = pos % S;
+          ptx::mbar_wait(&full[s], (pos / S) & 1);
           ptx::tc_fence_after();
-          if constexpr (!kSplit) {
-            const uint32_t d_tmem = tb + acc * BN;
-            for (int kb = 0; kb < kNumKb; ++kb, ++pos) {
-              poll_rounds();
-              const int s = pos % S;
-              ptx::mbar_wait(&full[s], (pos / S) & 1);
-              ptx::tc_fence_after();
-              const uint64_t da = desc(slot_ptr(s)), db = desc(slot_ptr(s) + kABytes);
-              if (ptx::elect_one()) {
+          const uint64_t da = desc(slot_ptr(s)), db = desc(slot_ptr(s) + kABytes);
+          if (ptx::elect_one()) {
 #pragma unroll
-                for (int k = 0; k < 4; ++k)
-                  ptx::umma_f16(d_tmem, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, (kb | k) != 0);
-                ptx::umma_commit(&empty[s]);
-              }
-              __syncwarp();
-            }
-          } else {
-            const uint32_t d_corr = tb + (2 + acc) * BN;
-            for (int kb0 = 0; kb0 < kNumKb; kb0 += kSplitChunk, ++ch) {
-              const int buf = ch & 1;
-              // The drain of this chunk buffer may sit behind a hand-off only this warp can complete (column group 1
-              // waits for group 0's heat MMAs before it writes A2, then drains): keep serving rounds while waiting.
-              {
-                const long long t0 = clock64();
-                while (!__all_sync(0xffffffffu, ptx::mbar_test_wait(&chunk_empty[buf], ((ch >> 1) & 1) ^ 1u))) {
-                  poll_rounds();
-                  if (clock64() - t0 > 8000000000LL) __trap();     // protocol bug: fail the launch, never hang the GPU
-                }
-              }
-              ptx::tc_fence_after();
-              const uint32_t d_main = tb + (uint32_t)(buf * BN);
-              const int kb1 = kb0 + kSplitChunk < kNumKb ? kb0 + kSplitChunk : kNumKb;
-              for (int kb = kb0; kb < kb1; ++kb, pos += 2) {
-                poll_rounds();
-                const int sa = pos % S, sb = (pos + 1) % S;
-                ptx::mbar_wait(&full[sa], (pos / S) & 1);
-                ptx::mbar_wait(&full[sb], ((pos + 1) / S) & 1);
-                ptx::tc_fence_after();
-                const uint64_t da = desc(slot_ptr(sa)), dal = desc(slot_ptr(sa) + kABytes);
-                const uint64_t db = desc(slot_ptr(sb)), dbl = desc(slot_ptr(sb) + kABytes);
-                const uint32_t first = kb != 0, first_main = kb > kb0;
-                if (ptx::elect_one()) {
-#pragma unroll
-                  for (int k = 0; k < 4; ++k) {
-                    const uint64_t o = (uint64_t)(2 * k);
-                    ptx::umma_f16(d_corr, dal + o, db + o, idesc, k ? 1u : first);        // lo*hi
-                    ptx::umma_f16(d_corr, da + o, dbl + o, idesc, 1u);                    // hi*lo
-                    ptx::umma_f16(d_main, da + o, db + o, idesc, k ? 1u : first_main);    // hi*hi, short chain
-                  }
-                  ptx::umma_commit(&empty[sa]);
-                  ptx::umma_commit(&empty[sb]);
-                }
-                __syncwarp();
-              }
-              if (ptx::elect_one()) ptx::umma_commit(&chunk_full[buf]);
-              __syncwarp();
-            }
+            for (int k = 0; k < 4; ++k)
+              ptx::umma_f16(d_tmem, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, (kb | k) != 0);
+            ptx::umma_commit(&empty[s]);
           }
-          if (ptx::elect_one()) ptx::umma_commit(&tmem_full[acc]);
           __syncwarp();
-          rounds_due += Cfg::kRounds;
         }
+        if (ptx::elect_one()) ptx::umma_commit(&tmem_full[acc]);
+        __syncwarp();
+        ++rounds_due;
       }
       force_rounds(rounds_due);
     }
@@ -385,134 +234,48 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     const int cb0 = grp * kCols;
     const int row = q * 32 + lane;                 // this thread's pixel inside the tile
     const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16);
-    uint32_t tl = 0, ch = 0;
-    float a_inv = 1.f, s_out = 1.f;
-    if constexpr (kSplit) {
-      a_inv = 1.f / __ldcg(p.scale_in);
-      const float bound = __ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1);
-      s_out = f16_pow2_scale(bound);
-    }
-    // A2 is free for this warp's round of tile tl once the heat MMAs of the round BEFORE it have completed:
-    //   bf16 (one round per tile)   : round of tile tl-1                     -> a2_empty[0], phase tl-1
-    //   f16x2, column group 0       : group 1's round of tile tl-1           -> a2_empty[1], phase tl-1
-    //   f16x2, column group 1       : group 0's round of tile tl             -> a2_empty[0], phase tl
-    // ("phase -1" of a fresh barrier reads as complete.)
-    auto wait_a2_free = [&]() {
-#ifdef CDR_EXP_TAIL_NO_HANDOFF
-      return;
-#endif
-      if constexpr (!kSplit) ptx::mbar_wait(&a2_empty[0], (tl & 1) ^ 1u);
-      else if (grp == 0) ptx::mbar_wait(&a2_empty[1], (tl & 1) ^ 1u);
-      else ptx::mbar_wait(&a2_empty[0], tl & 1);
-    };
-    auto publish_a2 = [&]() {
+    const float* __restrict__ bias = p.bias + cb0;   // first output channel of this warp
+    uint32_t tl = 0;
+    for (int unit = blockIdx.x; unit < p.num_units; unit += gridDim.x, ++tl) {
+      const uint32_t acc = tl & 1;
+      ptx::mbar_wait(&tmem_full[acc], (tl >> 1) & 1);
+      ptx::tc_fence_after();
+      // A2 is free once the heat MMAs of tile tl-1 have completed ("phase -1" of a fresh barrier reads as complete)
+      ptx::mbar_wait(a2_empty, (tl & 1) ^ 1u);
+#pragma unroll 1
+      for (int c = 0; c < kCols; c += 64) {
+        uint32_t r0[32], r1[32];
+        ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)(acc * BN + cb0 + c), r0);
+        ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)(acc * BN + cb0 + c + 32), r1);
+        ptx::tmem_ld_wait();
+        uint32_t w[32];
+#pragma unroll
+        for (int j4 = 0; j4 < 8; ++j4) {
+          const float4 b4 = __ldg(reinterpret_cast<const float4*>(bias + c) + j4);
+          const float4 b5 = __ldg(reinterpret_cast<const float4*>(bias + c + 32) + j4);
+          const __nv_bfloat162 x0 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r0[4 * j4]) + b4.x, 0.f),
+                                                          fmaxf(__uint_as_float(r0[4 * j4 + 1]) + b4.y, 0.f));
+          const __nv_bfloat162 x1 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r0[4 * j4 + 2]) + b4.z, 0.f),
+                                                          fmaxf(__uint_as_float(r0[4 * j4 + 3]) + b4.w, 0.f));
+          const __nv_bfloat162 y0 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r1[4 * j4]) + b5.x, 0.f),
+                                                          fmaxf(__uint_as_float(r1[4 * j4 + 1]) + b5.y, 0.f));
+          const __nv_bfloat162 y1 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r1[4 * j4 + 2]) + b5.z, 0.f),
+                                                          fmaxf(__uint_as_float(r1[4 * j4 + 3]) + b5.w, 0.f));
+          w[2 * j4] = *reinterpret_cast<const uint32_t*>(&x0);
+          w[2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&x1);
+          w[16 + 2 * j4] = *reinterpret_cast<const uint32_t*>(&y0);
+          w[16 + 2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&y1);
+        }
+        // K chunk (cb0 + c) / 64 of A2: row `row`, 128 bytes, 16-byte pieces XOR-swizzled by the row (SWIZZLE_128B)
+        const uint32_t base = ptx::smem_u32(a2) + (uint32_t)(((cb0 + c) >> 6) * kABytes) + (uint32_t)row * 128u;
+#pragma unroll
+        for (int j = 0; j < 8; ++j)
+          ptx::st_shared_v4(base + (uint32_t)((j ^ (row & 7)) << 4), w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
+      }
       ptx::fence_proxy_async();                    // generic-proxy writes -> visible to the tensor core's smem reads
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(a2_full);
-    };
-    for (int unit = blockIdx.x; unit < p.num_units; unit += gridDim.x) {
-      const int g = unit & 3;
-      for (int nh = 0; nh < NH; ++nh, ++tl) {
-        const uint32_t acc = tl & 1;
-        const int n_base = nh * BN + cb0;          // first output channel of this warp
-        const float* __restrict__ bias = p.bias + n_base;
-        if constexpr (!kSplit) {
-          ptx::mbar_wait(&tmem_full[acc], (tl >> 1) & 1);
-          ptx::tc_fence_after();
-          wait_a2_free();
-#pragma unroll 1
-          for (int c = 0; c < kCols; c += 64) {
-            uint32_t r0[32], r1[32];
-            ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)(acc * BN + cb0 + c), r0);
-            ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)(acc * BN + cb0 + c + 32), r1);
-            ptx::tmem_ld_wait();
-            uint32_t w[32];
-#pragma unroll
-            for (int j4 = 0; j4 < 8; ++j4) {
-              const float4 b4 = __ldg(reinterpret_cast<const float4*>(bias + c) + j4);
-              const float4 b5 = __ldg(reinterpret_cast<const float4*>(bias + c + 32) + j4);
-              const __nv_bfloat162 x0 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r0[4 * j4]) + b4.x, 0.f),
-                                                              fmaxf(__uint_as_float(r0[4 * j4 + 1]) + b4.y, 0.f));
-              const __nv_bfloat162 x1 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r0[4 * j4 + 2]) + b4.z, 0.f),
-                                                              fmaxf(__uint_as_float(r0[4 * j4 + 3]) + b4.w, 0.f));
-              const __nv_bfloat162 y0 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r1[4 * j4]) + b5.x, 0.f),
-                                                              fmaxf(__uint_as_float(r1[4 * j4 + 1]) + b5.y, 0.f));
-              const __nv_bfloat162 y1 = __floats2bfloat162_rn(fmaxf(__uint_as_float(r1[4 * j4 + 2]) + b5.z, 0.f),
-                                                              fmaxf(__uint_as_float(r1[4 * j4 + 3]) + b5.w, 0.f));
-              w[2 * j4] = *reinterpret_cast<const uint32_t*>(&x0);
-              w[2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&x1);
-              w[16 + 2 * j4] = *reinterpret_cast<const uint32_t*>(&y0);
-              w[16 + 2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&y1);
-            }
-            // K chunk (cb0 + c) / 64 of A2: row `row`, 128 bytes, 16-byte pieces XOR-swizzled by the row (SWIZZLE_128B)
-            const uint32_t base = ptx::smem_u32(a2) + (uint32_t)(((cb0 + c) >> 6) * kABytes) + (uint32_t)row * 128u;
-#pragma unroll
-            for (int j = 0; j < 8; ++j)
-              tail_st(base + (uint32_t)((j ^ (row & 7)) << 4), w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
-          }
-          publish_a2();
-        } else {
-          float sum[kCols];
-#pragma unroll
-          for (int j = 0; j < kCols; ++j) sum[j] = 0.f;
-          for (int kb0 = 0; kb0 < kNumKb; kb0 += kSplitChunk, ++ch) {
-            const int buf = ch & 1;
-            ptx::mbar_wait(&chunk_full[buf], (ch >> 1) & 1);
-            ptx::tc_fence_after();
-#pragma unroll
-            for (int c = 0; c < kCols; c += 32) {
-              uint32_t r[32];
-              ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)(buf * BN + cb0 + c), r);
-              ptx::tmem_ld_wait();
-#pragma unroll
-              for (int j = 0; j < 32; ++j) sum[c + j] += __uint_as_float(r[j]);
-            }
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) ptx::mbar_arrive(&chunk_empty[buf]);
-          }
-          ptx::mbar_wait(&tmem_full[acc], (tl >> 1) & 1);
-          ptx::tc_fence_after();
-#pragma unroll
-          for (int c = 0; c < kCols; c += 32) {
-            uint32_t r[32];
-            ptx::tmem_ld_32x32b_x32(lane_addr + (uint32_t)((2 + acc) * BN + cb0 + c), r);
-            ptx::tmem_ld_wait();
-#pragma unroll
-            for (int j = 0; j < 32; ++j) sum[c + j] = fmaf(__uint_as_float(r[j]), 1.f / kLoScale, sum[c + j]);
-          }
-          // finish (undo the operand scales, + bias, ReLU) and encode the 64 channels as scaled fp16 hi / lo planes
-          const float* __restrict__ wsi = p.wsi + (size_t)g * kDecC + n_base;
-          uint32_t wh[32], wl[32];
-#pragma unroll
-          for (int j4 = 0; j4 < kCols / 4; ++j4) {
-            const float4 w4 = __ldg(reinterpret_cast<const float4*>(wsi) + j4);
-            const float4 b4 = __ldg(reinterpret_cast<const float4*>(bias) + j4);
-            const float v0 = fmaxf(sum[4 * j4] * (a_inv * w4.x) + b4.x, 0.f) * s_out;
-            const float v1 = fmaxf(sum[4 * j4 + 1] * (a_inv * w4.y) + b4.y, 0.f) * s_out;
-            const float v2 = fmaxf(sum[4 * j4 + 2] * (a_inv * w4.z) + b4.z, 0.f) * s_out;
-            const float v3 = fmaxf(sum[4 * j4 + 3] * (a_inv * w4.w) + b4.w, 0.f) * s_out;
-            const __half2 h01 = __floats2half2_rn(v0, v1), h23 = __floats2half2_rn(v2, v3);
-            const float2 f01 = __half22float2(h01), f23 = __half22float2(h23);
-            const __half2 l01 = __floats2half2_rn((v0 - f01.x) * kLoScale, (v1 - f01.y) * kLoScale);
-            const __half2 l23 = __floats2half2_rn((v2 - f23.x) * kLoScale, (v3 - f23.y) * kLoScale);
-            wh[2 * j4] = *reinterpret_cast<const uint32_t*>(&h01);
-            wh[2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&h23);
-            wl[2 * j4] = *reinterpret_cast<const uint32_t*>(&l01);
-            wl[2 * j4 + 1] = *reinterpret_cast<const uint32_t*>(&l23);
-          }
-          wait_a2_free();                          // round of this tile written by this column group
-          const uint32_t base = ptx::smem_u32(a2) + (uint32_t)row * 128u;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const uint32_t o = (uint32_t)((j ^ (row & 7)) << 4);
-            tail_st(base + o, wh[4 * j], wh[4 * j + 1], wh[4 * j + 2], wh[4 * j + 3]);
-            tail_st(base + kABytes + o, wl[4 * j], wl[4 * j + 1], wl[4 * j + 2], wl[4 * j + 3]);
-          }
-          publish_a2();
-        }
-      }
     }
   } else {
     // ===================================================================== heat warps (10..13)
@@ -520,41 +283,21 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
     const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16);
     const int J = p.joints;
     uint32_t tl = 0;
-    float fin_scale = 1.f;                         // 1 / s(deconv3 activation)
-    if constexpr (kSplit) {
-      const float bound = __ldcg(p.amax_in) * __ldg(p.norms) + __ldg(p.norms + 1);
-      fin_scale = ldexpf(1.f, -f16_pow2_exp(bound));
-    }
     const float kLog2e = 1.4426950408889634f;
-    for (int unit = blockIdx.x; unit < p.num_units; unit += gridDim.x) {
+    for (int unit = blockIdx.x; unit < p.num_units; unit += gridDim.x, ++tl) {
       const int g = unit & 3, m0 = (unit >> 2) * kTcBM;
+      const uint32_t acc = tl & 1;
+      ptx::mbar_wait(&heat_full[acc], (tl >> 1) & 1);
+      ptx::tc_fence_after();
+      uint32_t r[32];
+      ptx::tmem_ld_32x32b_x32(lane_addr + acc * BN, r);
+      ptx::tmem_ld_wait();
       float hv[32];
 #pragma unroll
-      for (int nh = 0; nh < NH; ++nh, ++tl) {
-        const uint32_t acc = tl & 1;
-        ptx::mbar_wait(&heat_full[acc], (tl >> 1) & 1);
-        ptx::tc_fence_after();
-        uint32_t r[32];
-        if constexpr (!kSplit) {
-          ptx::tmem_ld_32x32b_x32(lane_addr + acc * BN, r);
-          ptx::tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 32; ++j) hv[j] = __uint_as_float(r[j]);
-        } else {
-          uint32_t rc[32];
-          ptx::tmem_ld_32x32b_x32(lane_addr + (2 + acc) * BN, r);
-          ptx::tmem_ld_32x32b_x32(lane_addr + (2 + acc) * BN + 32, rc);
-          ptx::tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const float v = fmaf(__uint_as_float(rc[j]), 1.f / kLoScale, __uint_as_float(r[j]));
-            hv[j] = nh == 0 ? v : hv[j] + v;       // the first half's partial waits here, in registers
-          }
-        }
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(&tmem_empty[acc]);
-      }
+      for (int j = 0; j < 32; ++j) hv[j] = __uint_as_float(r[j]);
+      ptx::tc_fence_before();
+      __syncwarp();
+      if (lane == 0) ptx::mbar_arrive(&tmem_empty[acc]);
       // ---- one output pixel per thread: input pixel (y, x = lane) of image img, output (2y + py, 2x + px)
       const int img = m0 / kHW;
       const int y = (m0 - img * kHW) / kW + q;
@@ -564,9 +307,7 @@ deconv_tail_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
 #pragma unroll
       for (int j = 0; j < 32; ++j) {
         if (j < J) {                               // warp-uniform
-          float v = hv[j];
-          if constexpr (kSplit) v *= fin_scale * __ldg(p.wsi_fin + j);
-          v += __ldg(p.bias_fin + j);
+          const float v = hv[j] + __ldg(p.bias_fin + j);
           if (p.heat) p.heat[((size_t)img * J + j) * 4096 + oy * 64 + ox] = v;
           if (p.part) {                            // warp-uniform
             float m = v;

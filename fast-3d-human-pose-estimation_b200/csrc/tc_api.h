@@ -8,7 +8,7 @@ struct TcWeights {
   void* pool = nullptr;   // one cudaMalloc holding every packed layer
   void* impl = nullptr;   // TcPack (gemm_tc.cu): per-layer pointers + weight tensor maps
   int joints = 0, has_fusion = 0, fin_npad = 0;
-  int kind = 0;           // pack mode: 0 = bf16, 1 = tf32x3, 2 = hybrid (fusion tf32x3, decoder f16x2)
+  int kind = 0;           // pack mode: 0 = bf16, 1 = tf32x3, 2 = f16x2 (gemm_tc.cu: TcMode)
   FusionDims fd;          // fusion widths (common.cuh)
 };
 

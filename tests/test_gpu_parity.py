@@ -91,8 +91,8 @@ def _nhwc_to_nchw(t, c):  # (..., 64, C) -> (..., C, 8, 8)
 
 @pytest.mark.parametrize("precision", ["fp32", "tf32x3", "fp32_ffma"])
 def test_head_fp32_vs_fp64_oracle_stagewise(cuda_pkg, precision):
-    """fp32 results: 'fp32' = tcgen05 with the decoder on scaled fp16 two-term operands (f16x2) and
-    the fusion block on 3xTF32 (default); 'tf32x3' = 3xTF32 everywhere; 'fp32_ffma' = CUDA cores."""
+    """fp32 results: 'fp32' = tcgen05 with the fusion block and the decoder on scaled fp16 two-term operands (f16x2,
+    default); 'tf32x3' = 3xTF32 everywhere; 'fp32_ffma' = CUDA cores."""
     b = 4
     sd = synth.make_head_state_dict(seed=0, calibrated=True, randomize_bn=True)
     feats, cams = synth.make_features(b, seed=1), synth.make_cameras(b, seed=2)
@@ -1005,17 +1005,12 @@ def test_baseline_config3_full_size(cuda_pkg):
     assert err <= TOL_3D_MM
 
 
-@pytest.mark.parametrize("pair", ["default", "0", "1"])
 @pytest.mark.parametrize("precision,b", [("bf16", 3), ("fp32", 3), ("fp32", 64), ("bf16", 64)])
-def test_fused_decoder_tail_matches_unfused_and_oracle(cuda_pkg, precision, b, pair, monkeypatch):
-    """deconv3 -> ReLU -> final 1x1 -> soft-argmax partials as ONE kernel (tail_tc.cuh: second tcgen05.mma on the ReLU'd
-    tile, per-row online-softmax partials merged in fp64) against the three-launch path of the same library
-    (CDR_FUSED_TAIL=0) — heat-maps to accumulation-order rounding, 2D joints <= 1e-4 px — and, at B = 3, against the
-    fp64 oracle with the flat tolerance."""
-    if pair != "default":                        # single-CTA kernel / cta_group::2 pair kernel (tail_pair_tc.cuh), both kinds
-        if b == 64 and pair == "0":
-            pytest.skip("covered at B=3")
-        monkeypatch.setenv("CDR_TAIL_PAIR", pair)
+def test_fused_decoder_tail_matches_unfused_and_oracle(cuda_pkg, precision, b, monkeypatch):
+    """deconv3 -> ReLU -> final 1x1 -> soft-argmax partials as ONE kernel (bf16: tail_tc.cuh; fp32: the cta_group::2 pair
+    kernel of tail_pair_tc.cuh; a second tcgen05.mma on the ReLU'd tile, per-row online-softmax partials merged in fp64)
+    against the three-launch path of the same library (CDR_FUSED_TAIL=0) — heat-maps to accumulation-order rounding, 2D
+    joints <= 1e-4 px — and, at B = 3, against the fp64 oracle with the flat tolerance."""
     sd = synth.make_head_state_dict(seed=0, calibrated=True, randomize_bn=True)
     feats, cams = synth.make_features(b, seed=1), synth.make_cameras(b, seed=2)
     m = _model(cuda_pkg, sd, precision=precision)
