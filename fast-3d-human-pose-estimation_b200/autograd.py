@@ -16,6 +16,10 @@ The decoder's transposed convolutions have one too, forward and backward on the 
 accuracy (independent of torch's TF32 flags):
 
     y = conv_transpose2d(x, weight)                   # == F.conv_transpose2d(x, weight, stride=2, padding=1)
+
+and so do the head's 1x1 convolutions (the fusion block's and ``decoder.final_layer``), bias included:
+
+    y = conv1x1(x, weight, bias)                      # == F.conv2d(x, weight, bias) for a (Cout, Cin, 1, 1) weight
 """
 from __future__ import annotations
 
@@ -201,3 +205,83 @@ def conv_transpose2d(x, weight):
     libcdrhead at fp32 accuracy.  x (N, Cin, H, W), weight (Cin, Cout, 4, 4): CUDA float32, Cin and Cout multiples
     of 64, H == W in {8, 16, 32}; anything else raises ValueError."""
     return _ConvTranspose2d.apply(x, weight)
+
+
+def _aligned(t):
+    """t contiguous with a 16-byte-aligned address (a contiguous view may start mid-allocation)."""
+    t = t.contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
+def _conv1x1_args(x, weight, bias):
+    """Checks of conv1x1's inputs, all before any CUDA call: ValueError, there is no fallback."""
+    ts = (x, weight) if bias is None else (x, weight, bias)
+    if not all(isinstance(t, torch.Tensor) for t in ts):
+        raise ValueError("conv1x1: x, weight and bias must be tensors")
+    if x.dim() != 4 or weight.dim() != 4 or tuple(weight.shape[2:]) != (1, 1) or weight.shape[1] != x.shape[1]:
+        raise ValueError(f"conv1x1: x (N, Cin, H, W) and weight (Cout, Cin, 1, 1) expected, got {tuple(x.shape)} and "
+                         f"{tuple(weight.shape)}")
+    n, cin, h, w = x.shape
+    cout = weight.shape[0]
+    if bias is not None and tuple(bias.shape) != (cout,):
+        raise ValueError(f"conv1x1: bias of shape ({cout},) expected, got {tuple(bias.shape)}")
+    if not (n >= 1 and 1 <= cin <= 4096 and 1 <= cout <= 4096 and (h * w) % 64 == 0 and h * w > 0
+            and n * h * w <= 1 << 22):
+        raise ValueError(f"conv1x1: unsupported shape x {tuple(x.shape)}, weight {tuple(weight.shape)} "
+                         "(1 <= Cin, Cout <= 4096, H*W a multiple of 64, N*H*W <= 2^22)")
+    if any(t.dtype != torch.float32 for t in ts):
+        raise ValueError(f"conv1x1: float32 expected, got {', '.join(str(t.dtype) for t in ts)}")
+    if not all(t.is_cuda and t.device == x.device for t in ts):
+        raise ValueError("conv1x1: x, weight and bias must be CUDA tensors on one device (there is no CPU fallback)")
+    return _aligned(x), _aligned(weight), None if bias is None else _aligned(bias)
+
+
+class _Conv1x1(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, weight, bias):
+        x, weight, bias = _conv1x1_args(x, weight, bias)
+        n, cin, h, w = x.shape
+        cout = weight.shape[0]
+        L = _lib.lib()
+        saved_b, ws_b = C.c_size_t(), C.c_size_t()
+        _lib.check(L.cdr_conv1x1_train_workspace_bytes(n, cin, cout, h, w, C.byref(saved_b), C.byref(ws_b)))
+        dev = x.device
+        y = torch.empty((n, cout, h, w), dtype=torch.float32, device=dev)
+        saved = torch.empty(saved_b.value, dtype=torch.uint8, device=dev)     # x as fp16 planes, for the weight gradient
+        ws = torch.empty(ws_b.value, dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(L.cdr_conv1x1_train_forward(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(bias), n, cin, cout, h, w,
+                                                   _lib.ptr(y), _lib.ptr(saved), saved_b.value, _lib.ptr(ws), ws_b.value,
+                                                   _lib.current_stream_ptr(dev)))
+        ctx.save_for_backward(saved, weight)
+        ctx.dims = (n, cin, cout, h, w)
+        ctx.ws_bytes = ws_b.value
+        return y
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_y):
+        saved, weight = ctx.saved_tensors
+        n, cin, cout, h, w = ctx.dims
+        need_x, need_w, need_b = ctx.needs_input_grad[:3]
+        if not (need_x or need_w or need_b):
+            return None, None, None
+        dy = _aligned(_chk(grad_y, "conv1x1: grad"))
+        dev = dy.device
+        dx = torch.empty((n, cin, h, w), dtype=torch.float32, device=dev) if need_x else None
+        dw = torch.empty((cout, cin, 1, 1), dtype=torch.float32, device=dev) if need_w else None
+        db = torch.empty((cout,), dtype=torch.float32, device=dev) if need_b else None
+        ws = torch.empty(ctx.ws_bytes, dtype=torch.uint8, device=dev)
+        L = _lib.lib()
+        with torch.cuda.device(dev):
+            _lib.check(L.cdr_conv1x1_train_backward(_lib.ptr(saved), _lib.ptr(weight), _lib.ptr(dy), n, cin, cout, h, w,
+                                                    _lib.ptr(dx), _lib.ptr(dw), _lib.ptr(db), _lib.ptr(ws), ctx.ws_bytes,
+                                                    _lib.current_stream_ptr(dev)))
+        return dx, dw, db
+
+
+def conv1x1(x, weight, bias=None):
+    """F.conv2d(x, weight, bias) for a (Cout, Cin, 1, 1) weight, forward and backward on libcdrhead at fp32 accuracy.
+    x (N, Cin, H, W), bias (Cout) or None: CUDA float32, 1 <= Cin, Cout <= 4096, H*W a multiple of 64,
+    N*H*W <= 2^22; anything else raises ValueError."""
+    return _Conv1x1.apply(x, weight, bias)

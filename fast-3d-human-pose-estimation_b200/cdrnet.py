@@ -438,15 +438,16 @@ class CDRNet(nn.Module):
 
     def forward_train(self, xs, proj_list):
         """The training-mode forward of train_cdr.py:105 (models/cdrnet.py:224-268 with autograd), SURVEY §8f rank 3
-        — an explicit HYBRID, not a fallback of the inference path.  The decoder's three transposed convolutions
-        (95 % of the head's FLOPs) run forward and backward in libcdrhead.so at fp32 accuracy (autograd.py:
-        ``conv_transpose2d``, on the weights of ``decoder.deconv{1,2,3}.0``); the fusion block's 1x1 convs and
-        ``decoder.final_layer`` are still this module's own torch children (library GEMMs: cuDNN + torch autograd, like
-        the encoder).  The head's train-mode BatchNorm + ReLU (losses.py: batch statistics, running-stat update) and the
-        three operators the reference hand-rolls — ``ftl`` (:45-56), ``process_heatmap`` (:120-149) and ``dlt``
-        (:151-179) — and the pseudo-inverse run forward AND backward in libcdrhead.so (autograd.py, losses.py).  Needs
-        ``CDRNet(..., trainable=True)``; projection matrices get no gradient (data in the reference)."""
-        from .autograd import conv_transpose2d, dlt, ftl, soft_argmax_2d
+        — an explicit HYBRID, not a fallback of the inference path.  Every convolution of the head runs forward and
+        backward in libcdrhead.so at fp32 accuracy, independent of torch's TF32 flags (autograd.py): the decoder's three
+        transposed convolutions (``conv_transpose2d`` on the weights of ``decoder.deconv{1,2,3}.0``) and the 1x1 convs
+        of the fusion block and ``decoder.final_layer`` (``conv1x1``, bias included).  The head's train-mode BatchNorm +
+        ReLU (losses.py: batch statistics, running-stat update), the three operators the reference hand-rolls —
+        ``ftl`` (:45-56), ``process_heatmap`` (:120-149) and ``dlt`` (:151-179) — and the pseudo-inverse run forward
+        AND backward in libcdrhead.so too (autograd.py, losses.py).  Only the encoder (cuDNN + torch autograd) and the
+        optimizer stay with torch.  Needs ``CDRNet(..., trainable=True)``; projection matrices get no gradient (data in
+        the reference)."""
+        from .autograd import conv1x1, conv_transpose2d, dlt, ftl, soft_argmax_2d
         if not self.trainable:
             raise RuntimeError("forward_train needs CDRNet(..., trainable=True)")
         pl = _as_f32_cuda(proj_list[0], "proj_list")
@@ -461,8 +462,8 @@ class CDRNet(nn.Module):
         from .losses import batch_norm_train
 
         def cbr(seq, x, i=0):
-            """conv (a library GEMM through torch, like the encoder) -> train-mode BatchNorm + ReLU on libcdrhead"""
-            return batch_norm_train(seq[i](x), seq[i + 1], relu=True)
+            """1x1 conv -> train-mode BatchNorm + ReLU, both on libcdrhead"""
+            return batch_norm_train(conv1x1(x, seq[i].weight, seq[i].bias), seq[i + 1], relu=True)
 
         def dcbr(seq, x):
             """transposed conv on libcdrhead -> train-mode BatchNorm + ReLU"""
@@ -476,7 +477,8 @@ class CDRNet(nn.Module):
         for v in range(2):
             o = cbr(cf.out_layer[v], ftl(f, projs[v]))                        # :79-81
             d = self.decoder
-            h = d.final_layer(dcbr(d.deconv3, dcbr(d.deconv2, dcbr(d.deconv1, o))))   # models/decoder.py:39-46
+            h = conv1x1(dcbr(d.deconv3, dcbr(d.deconv2, dcbr(d.deconv1, o))), d.final_layer.weight,
+                        d.final_layer.bias)                                   # models/decoder.py:39-46
             kps.append(soft_argmax_2d(h, img_size / h.shape[2]))              # :243-250
         return kps, dlt(pl, pr, kps[0], kps[1])                               # :252-268
 

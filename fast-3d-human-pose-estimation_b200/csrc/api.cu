@@ -704,3 +704,48 @@ extern "C" int cdr_deconv_train_backward(const void* saved, const float* weight,
   return tc_deconv_train_backward(saved, weight, dy, n, cin, cout, h, w, dx, dweight, workspace, workspace_bytes,
                                   (cudaStream_t)stream);
 }
+
+// ------------------------------------------------------------------------------------------
+// Training 1x1 convolutions (gemm_tc.cu: tc_conv1x1_train_*)
+static int conv1x1_train_shape(const char* fn, int n, int cin, int cout, int h, int w) {
+  CDR_CHECK_ARG(n >= 1 && cin >= 1 && cin <= 4096 && cout >= 1 && cout <= 4096 && h >= 1 && w >= 1 &&
+                    ((long long)h * w) % 64 == 0 && (long long)n * h * w <= (1LL << 22),
+                "%s: unsupported shape n=%d cin=%d cout=%d h=%d w=%d (1 <= Cin, Cout <= 4096, h*w a multiple of 64, "
+                "n*h*w <= 2^22)", fn, n, cin, cout, h, w);
+  return CDR_OK;
+}
+extern "C" int cdr_conv1x1_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes,
+                                                 size_t* workspace_bytes) {
+  CDR_CHECK_ARG(saved_bytes && workspace_bytes, "cdr_conv1x1_train_workspace_bytes: null pointer");
+  if (int rc = conv1x1_train_shape("cdr_conv1x1_train_workspace_bytes", n, cin, cout, h, w)) return rc;
+  *saved_bytes = conv1x1_train_saved_bytes(n, cin, cout, h, w);
+  *workspace_bytes = conv1x1_train_workspace_bytes(n, cin, cout, h, w);
+  return CDR_OK;
+}
+extern "C" int cdr_conv1x1_train_forward(const float* x, const float* weight, const float* bias, int n, int cin,
+                                         int cout, int h, int w, float* y, void* saved, size_t saved_bytes,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
+  CDR_CHECK_ARG(x && weight && y && saved && workspace, "cdr_conv1x1_train_forward: null pointer");
+  if (int rc = conv1x1_train_shape("cdr_conv1x1_train_forward", n, cin, cout, h, w)) return rc;
+  CDR_CHECK_ARG(al16(x) && al16(weight) && ((uintptr_t)bias & 3) == 0 && al16(y) && ((uintptr_t)saved & 255) == 0 &&
+                    ((uintptr_t)workspace & 255) == 0,
+                "cdr_conv1x1_train_forward: tensors must be 16-byte (bias 4-byte), saved / workspace 256-byte aligned");
+  if (saved_bytes < conv1x1_train_saved_bytes(n, cin, cout, h, w)) {
+    set_error("cdr_conv1x1_train_forward: saved %zu < required %zu bytes", saved_bytes,
+              conv1x1_train_saved_bytes(n, cin, cout, h, w));
+    return CDR_ERR_WORKSPACE;
+  }
+  return tc_conv1x1_train_forward(x, weight, bias, n, cin, cout, h, w, y, saved, workspace, workspace_bytes,
+                                  (cudaStream_t)stream);
+}
+extern "C" int cdr_conv1x1_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin,
+                                          int cout, int h, int w, float* dx, float* dweight, float* dbias,
+                                          void* workspace, size_t workspace_bytes, void* stream) {
+  CDR_CHECK_ARG(saved && weight && dy && workspace, "cdr_conv1x1_train_backward: null pointer");
+  if (int rc = conv1x1_train_shape("cdr_conv1x1_train_backward", n, cin, cout, h, w)) return rc;
+  CDR_CHECK_ARG(al16(weight) && al16(dy) && al16(dx) && al16(dweight) && ((uintptr_t)dbias & 3) == 0 &&
+                    ((uintptr_t)saved & 255) == 0 && ((uintptr_t)workspace & 255) == 0,
+                "cdr_conv1x1_train_backward: tensors must be 16-byte (dbias 4-byte), saved / workspace 256-byte aligned");
+  return tc_conv1x1_train_backward(saved, weight, dy, n, cin, cout, h, w, dx, dweight, dbias, workspace,
+                                   workspace_bytes, (cudaStream_t)stream);
+}

@@ -378,11 +378,12 @@ constexpr int kSplitChunk = 8;
 // multicast commits to both CTAs' barriers; "accumulator drained" arrivals of the peer's epilogue warps go to the
 // leader's barriers through the cluster window (mapa + mbarrier.arrive.shared::cluster).
 //
-// kMN (f16x2, BN = 128, CL = 0): the weight gradient of a k4 s2 p1 transposed conv (deconv_train_backward).  One tile =
-// 128 input channels ci (M) x 128 output channels co (N) of one tap (ky, kx) and one K slice; K = the pixels of x.
-// Both operands are read straight from the pixel-major fp16 planes, so they are MN-major (channels contiguous): A = x,
-// two 64-channel x 64-pixel boxes; B = dy, the same 64 pixels in the same (img, y, x) order through the stride-2 box
-// shifted by (kx - 1, ky - 1).  The UMMA descriptors carry the MN-major SWIZZLE_128B layout (LBO = the 8 KB between
+// kMN (f16x2, BN = 128, CL = 0): weight gradients, K = pixels.  One tile = 128 channels of A (M) x 128 channels of B (N)
+// of one group g = slice * taps + tap and one K slice.  Both operands are read straight from the pixel-major fp16 planes,
+// so they are MN-major (channels contiguous): A = two 64-channel x 64-pixel boxes; B = the same 64 pixels in the same
+// (img, y, x) order.  tap_mode kTapConv4s2: a k4 s2 p1 transposed conv (deconv_train_backward; A = x, B = dy through the
+// stride-2 box shifted by (kx - 1, ky - 1), 16 taps).  kTapNone: a 1x1 conv (conv1x1_train_backward; A = dy, B = x,
+// both 2-D maps, 1 tap).  The UMMA descriptors carry the MN-major SWIZZLE_128B layout (LBO = the 8 KB between
 // the two 64-channel halves, SBO = 1024 B between 8-pixel groups) and the instruction descriptor the transpose bits.
 // The epilogue stores the raw fp32 tile (still times s_x * s_dy) into the slice's partial; wgrad_reduce_kernel sums
 // the slices in a fixed order.
@@ -518,9 +519,11 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
           const int bk = tap * p.cin + k0;
           const int brow = g * p.b_group_rows + n_tile * BN + (kPair2 ? (int)cta_rank * (BN / 2) : 0);   // CL = 2: my half of B
           if constexpr (kMN) {
-            // wgrad: g = slice * 16 + (ky * 4 + kx); 64 pixels of x from k0 of the slice (p.cin pixels per slice; a block
-            // is whole rows of one image since W | 64 | H*W) and the dy pixels (2y - 1 + ky, 2x - 1 + kx) they pair with
-            const int wt = g & 15, pix0 = (g >> 4) * p.cin + k0;
+            // wgrad: g = slice * 16 + (ky * 4 + kx) (kTapConv4s2) or slice (kTapNone); 64 pixels of A from k0 of the slice
+            // (p.cin pixels per slice; for the stride-2 box a block is whole rows of one image since W | 64 | H*W) and the
+            // B pixels they pair with: the same ones, or the dy pixels (2y - 1 + ky, 2x - 1 + kx)
+            const bool s2 = p.tap_mode == kTapConv4s2;
+            const int wt = s2 ? g & 15 : 0, pix0 = (s2 ? g >> 4 : g) * p.cin + k0;
             const int wimg = pix0 / HW, wy = (pix0 - wimg * HW) / p.W;
             const int co0 = n_tile * BN;
             if (ptx::elect_one()) {
@@ -532,8 +535,11 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
 #pragma unroll
                 for (int h = 0; h < 2; ++h) {
                   ptx::tma_load_2d(stage_a(s, pl) + h * (kABytes / 2), ma, &full[s], m0 + 64 * h, pix0);
-                  ptx::tma_load_4d(stage_b(s, pl) + h * (Cfg::kBBytes / 2), mb, &full[s], co0 + 64 * h, (wt & 3) - 1,
-                                   2 * wy + (wt >> 2) - 1, wimg);
+                  if (s2)
+                    ptx::tma_load_4d(stage_b(s, pl) + h * (Cfg::kBBytes / 2), mb, &full[s], co0 + 64 * h, (wt & 3) - 1,
+                                     2 * wy + (wt >> 2) - 1, wimg);
+                  else
+                    ptx::tma_load_2d(stage_b(s, pl) + h * (Cfg::kBBytes / 2), mb, &full[s], co0 + 64 * h, pix0);
                 }
               }
             }
@@ -1483,14 +1489,16 @@ __device__ __forceinline__ float conv_taps_weight(const CdrConvBn& s, int cout, 
   const int tap = kk / cin, ci = kk - tap * cin;
   return (float)((double)s.weight[((size_t)n * cin + ci) * taps + tap] * tc_bn_scale(s, n));
 }
-// the data-gradient operand of a transposed conv (Cin,Cout,4,4) at packed position (ci, tap*Cout + co), tap = ky*4 + kx
-__device__ __forceinline__ float deconv_dgrad_weight(const CdrConvBn& s, int cin, int cout, int ci, int kk) {
-  if (ci >= cin) return 0.f;
+// the data-gradient operand W^T at packed position (ci, tap*Cout + co): kTaps = 16, a transposed conv's weight
+// (Cin,Cout,4,4) with tap = ky*4 + kx; kTaps = 1, a 1x1 conv's weight (Cout,Cin).  Zero in the padded rows and K pitch.
+template <int kTaps>
+__device__ __forceinline__ float dgrad_weight(const CdrConvBn& s, int cin, int cout, int ci, int kk) {
+  if (ci >= cin || kk >= kTaps * cout) return 0.f;
   const int tap = kk / cout, co = kk - tap * cout;
-  return s.weight[((size_t)ci * cout + co) * 16 + tap];
+  return kTaps == 1 ? s.weight[(size_t)co * cin + ci] : s.weight[((size_t)ci * cout + co) * kTaps + tap];
 }
 // kDeconv: 0 = 1x1 conv, 1 = transposed conv (4 phases), >= 2: conv with kDeconv taps in encoder order (use 9; the 1x1
-// convs of the encoder go through mode 0), -1: deconv_dgrad_weight (`cout` = Cin rows, `cin` = Cout per tap)
+// convs of the encoder go through mode 0), < 0: dgrad_weight<-kDeconv> (`cout` = Cin rows, `cin` = Cout per tap)
 template <int kDeconv>
 __global__ void __launch_bounds__(256)
 pack_rows_f16_kernel(CdrConvBn s, int cout, int cin, int k_pitch, int n_pad, __half* __restrict__ w_hi,
@@ -1501,7 +1509,7 @@ pack_rows_f16_kernel(CdrConvBn s, int cout, int cin, int k_pitch, int n_pad, __h
   const int n = row % n_pad, phase = row / n_pad;
   auto val = [&](int kk) -> float {
     if constexpr (kDeconv >= 2) return conv_taps_weight(s, cout, cin, kDeconv, n, kk);
-    if constexpr (kDeconv < 0) return deconv_dgrad_weight(s, cout, cin, n, kk);
+    if constexpr (kDeconv < 0) return dgrad_weight<-kDeconv>(s, cout, cin, n, kk);
     return kDeconv ? deconv_weight(s, cin, cout, phase, n, kk) : conv1x1_weight(s, cout, cin, n, kk);
   };
   float mx = 0.f, l1 = 0.f;
@@ -2525,21 +2533,22 @@ int tc_set_debug(unsigned int* d) {
 //               wgrad_reduce_kernel (fixed slice order: bitwise deterministic, no atomics)
 // x and dy are encoded with ONE power-of-two scale per tensor (exact amax first): wgrad reduces over pixels, so per-pixel
 // scales would not factor out of its sums.  The x planes and their {amax, scale} slot are what the forward saves.
+
+// wgrad K slices: powers of two while the `tiles` output tiles do not fill two waves of 148 SMs and a slice keeps >= 16 of
+// the `kb` K blocks.  A function of the shape only, so the summation order (and the result, bit for bit) does not depend
+// on the device.
+static int wgrad_slices(long long kb, long long tiles) {
+  int s = 1;
+  while (tiles * s < 2 * 148 && kb % (2 * s) == 0 && kb / (2 * s) >= 16) s *= 2;
+  return s;
+}
 struct DtShape {
   int n, cin, cout, h, w;
   size_t x_rows() const { return (size_t)n * h * w; }
   size_t dy_rows() const { return (size_t)n * 4 * h * w; }
   int npo() const { return round_up(cout, 128); }     // forward: packed output channels per phase
   int npi() const { return round_up(cin, 128); }      // dgrad: packed output channels
-  // wgrad K slices: powers of two while the tiles do not fill two waves of 148 SMs and a slice keeps >= 16 K blocks.  A
-  // function of the shape only, so the summation order (and the result, bit for bit) does not depend on the device.
-  int slices() const {
-    const long long kb = (long long)n * h * w / 64;
-    const int tiles = (cin / 64 + 1) / 2 * ((cout / 64 + 1) / 2) * 16;
-    int s = 1;
-    while ((long long)tiles * s < 2 * 148 && kb % (2 * s) == 0 && kb / (2 * s) >= 16) s *= 2;
-    return s;
-  }
+  int slices() const { return wgrad_slices((long long)n * h * w / 64, (cin / 64 + 1) / 2 * ((cout / 64 + 1) / 2) * 16); }
 };
 struct DtWs {
   TcLayer L;                 // forward: [4 phases][npo][4*cin]; backward: dgrad [npi][16*cout]
@@ -2570,11 +2579,12 @@ size_t deconv_train_workspace_bytes(int n, int cin, int cout, int h, int w) {
   return f > bw ? f : bw;
 }
 
-// NCHW fp32 -> fp16 planes with one tensor scale (exact amax pass first)
-static int to_planes_tensor_scale(const float* in, int n, int c, int hw, const Act& a, ScaleSlot sl, cudaStream_t st) {
+// NCHW fp32 -> fp16 planes with one tensor scale (exact amax pass first); columns [c, pitch) are written as zeros
+static int to_planes_tensor_scale(const float* in, int n, int c, int hw, int pitch, const Act& a, ScaleSlot sl,
+                                  cudaStream_t st) {
   CDR_CUDA(cudaMemsetAsync(sl.amax, 0, sizeof(float), st));
   if (int rc = launch_amax_f32(in, nullptr, (long long)n * c * hw, sl.amax, st)) return rc;
-  return launch_nchw_to_rows_f16p(in, nullptr, n, c, hw, a.p[0], a.p[1], c, sl.amax, sl.scale, st);
+  return launch_nchw_to_rows_f16p(in, nullptr, n, c, hw, a.p[0], a.p[1], pitch, sl.amax, sl.scale, st);
 }
 
 int tc_deconv_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, float* y,
@@ -2588,7 +2598,7 @@ int tc_deconv_train_forward(const float* x, const float* weight, int n, int cin,
   set_stage("deconv_train_fwd");
   ScaleSlot sx;
   const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
-  if (int rc = to_planes_tensor_scale(x, n, cin, h * w, xa, sx, st)) return rc;
+  if (int rc = to_planes_tensor_scale(x, n, cin, h * w, cin, xa, sx, st)) return rc;
   CdrConvBn cb{};
   cb.weight = weight;
   TcLayer& L = ws.L;
@@ -2608,22 +2618,28 @@ int tc_deconv_train_forward(const float* x, const float* weight, int n, int cin,
   return rc;
 }
 
-// dW[ci][co][tap] = (sum over slices, in order, of part[slice][tap][ci][co]) / (s_x * s_dy)
+// dW[r][c][tap] = (sum over slices, in order, of part[slice][tap][r][c]) / (s_x * s_dy): a transposed conv's
+// (Cin, Cout, 4, 4) with r = ci, c = co, 16 taps; a 1x1 conv's (Cout, Cin, 1, 1) with r = co, c = ci, 1 tap
 __global__ void __launch_bounds__(256)
-wgrad_reduce_kernel(const float* __restrict__ part, int slices, int cin, int cout, int ldc, const float* __restrict__ sx,
-                    const float* __restrict__ sdy, float* __restrict__ dw) {
+wgrad_reduce_kernel(const float* __restrict__ part, int slices, int taps, int rows, int cols, int ldc,
+                    const float* __restrict__ sx, const float* __restrict__ sdy, float* __restrict__ dw) {
   const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= (long long)cin * cout * 16) return;
-  const int t = (int)(idx & 15);
-  const long long r = idx >> 4;
-  const int co = (int)(r % cout), ci = (int)(r / cout);
+  if (idx >= (long long)rows * cols * taps) return;
+  const int t = (int)(idx % taps);
+  const long long r = idx / taps;
+  const int c = (int)(r % cols), row = (int)(r / cols);
   const float ix = 1.f / __ldcg(sx), id = 1.f / __ldcg(sdy);      // powers of two: exact
   float s = 0.f;
-  for (int sl = 0; sl < slices; ++sl) s += __ldcg(part + (((size_t)sl * 16 + t) * cin + ci) * ldc + co);
+  for (int sl = 0; sl < slices; ++sl) s += __ldcg(part + (((size_t)sl * taps + t) * rows + row) * ldc + c);
   dw[idx] = s * ix * id;
 }
 
-static int launch_wgrad(const DtShape& d, const Act& xa, ScaleSlot sx, const Act& dya, float* part, cudaStream_t st) {
+// The kMN GEMM over n*h*w pixels split into `slices` K slices: part[slice * taps + tap] (m rows, pitch round_up(nb, 128))
+// = A^T B.  A: m channels of a pixel-major fp16 planes buffer (pitch a_pitch), scale slot `sa`.  B: nb channels (pitch
+// b_pitch), either the same pixels through a 2-D map (1 tap), or (b_s2) the 2h x 2w dy of a k4 s2 p1 transposed conv
+// through the stride-2 box, 16 taps.
+static int launch_wgrad(int n, int h, int w, const Act& a, int m, int a_pitch, ScaleSlot sa, const Act& b, int nb,
+                        int b_pitch, bool b_s2, int slices, float* part, cudaStream_t st) {
   using Cfg = TcCfg<128, kKindF16X2, kFmtF16P, 0>;
   auto kern = tap_gemm_tc_kernel<128, kKindF16X2, kFmtF16P, 0, true>;
   static DeviceOnce attr_set;
@@ -2631,35 +2647,39 @@ static int launch_wgrad(const DtShape& d, const Act& xa, ScaleSlot sx, const Act
     CDR_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
     attr_set.done();
   }
-  const int hw = d.h * d.w, slices = d.slices();
-  const long long kb = (long long)d.n * hw / 64;
+  const long long rows = (long long)n * h * w, kb = rows / 64;
   TcGemmParams p{};
-  p.M = d.cin;
-  p.n_img = d.n; p.H = d.h; p.W = d.w;
+  p.M = m;
+  p.n_img = n; p.H = h; p.W = w;
   p.cin = (int)(kb / slices) * 64;           // pixels per K slice
-  p.ntaps = 1; p.tap_mode = kTapNone; p.stride = 1;
-  p.groups = 16 * slices;
-  p.n_tiles = d.npo() / 128;
-  p.n = d.cout;
-  p.C = part; p.c_pitch = d.npo(); p.c_fill = d.cout;
+  p.ntaps = 1; p.tap_mode = b_s2 ? kTapConv4s2 : kTapNone; p.stride = 1;
+  p.groups = (b_s2 ? 16 : 1) * slices;
+  p.n_tiles = round_up(nb, 128) / 128;
+  p.n = nb;
+  p.C = part; p.c_pitch = round_up(nb, 128); p.c_fill = nb;
   p.out_mode = kOutPlanar;
-  p.scale_in = sx.scale;
-  p.num_tiles = (d.npi() / 128) * p.groups * p.n_tiles;
+  p.scale_in = sa.scale;
+  p.num_tiles = ceil_div(m, 128) * p.groups * p.n_tiles;
   CUtensorMap ma[2], mb[2];
   for (int pl = 0; pl < 2; ++pl) {
-    {   // x planes: (pixels, cin) rows, boxes of 64 channels x 64 pixels
-      const uint64_t dims[2] = {(uint64_t)d.cin, (uint64_t)d.x_rows()};
-      const uint64_t strides[1] = {(uint64_t)d.cin};
+    {   // A planes: (pixels, a_pitch) rows, boxes of 64 channels x 64 pixels
+      const uint64_t dims[2] = {(uint64_t)a_pitch, (uint64_t)rows};
+      const uint64_t strides[1] = {(uint64_t)a_pitch};
       const uint32_t box[2] = {64, 64};
-      if (int rc = make_tmap(&ma[pl], xa.p[pl], kFmtF16P, 2, dims, strides, box)) return rc;
+      if (int rc = make_tmap(&ma[pl], a.p[pl], kFmtF16P, 2, dims, strides, box)) return rc;
     }
-    {   // dy planes (n, 2h, 2w, cout) seen with element stride 2: 64 channels x (w x 64/w) pixels x 1 image
-      const uint64_t iw = 2 * (uint64_t)d.w, ih = 2 * (uint64_t)d.h;
-      const uint64_t dims[4] = {(uint64_t)d.cout, iw, ih, (uint64_t)d.n};
-      const uint64_t strides[3] = {(uint64_t)d.cout, (uint64_t)d.cout * iw, (uint64_t)d.cout * iw * ih};
-      const uint32_t box[4] = {64, (uint32_t)(2 * d.w), (uint32_t)(2 * (64 / d.w)), 1};
+    if (b_s2) {   // dy planes (n, 2h, 2w, b_pitch) seen with element stride 2: 64 channels x (w x 64/w) pixels x 1 image
+      const uint64_t iw = 2 * (uint64_t)w, ih = 2 * (uint64_t)h;
+      const uint64_t dims[4] = {(uint64_t)b_pitch, iw, ih, (uint64_t)n};
+      const uint64_t strides[3] = {(uint64_t)b_pitch, (uint64_t)b_pitch * iw, (uint64_t)b_pitch * iw * ih};
+      const uint32_t box[4] = {64, (uint32_t)(2 * w), (uint32_t)(2 * (64 / w)), 1};
       const uint32_t estr[4] = {1, 2, 2, 1};
-      if (int rc = make_tmap(&mb[pl], dya.p[pl], kFmtF16P, 4, dims, strides, box, estr)) return rc;
+      if (int rc = make_tmap(&mb[pl], b.p[pl], kFmtF16P, 4, dims, strides, box, estr)) return rc;
+    } else {      // B planes: (pixels, b_pitch) rows, like A
+      const uint64_t dims[2] = {(uint64_t)b_pitch, (uint64_t)rows};
+      const uint64_t strides[1] = {(uint64_t)b_pitch};
+      const uint32_t box[2] = {64, 64};
+      if (int rc = make_tmap(&mb[pl], b.p[pl], kFmtF16P, 2, dims, strides, box)) return rc;
     }
   }
   const int grid = p.num_tiles < num_sms() ? p.num_tiles : num_sms();
@@ -2682,12 +2702,12 @@ int tc_deconv_train_backward(const void* saved, const float* weight, const float
   ScaleSlot sd, sx;
   const Act dya = planes_act(ws.dy_planes, d.dy_rows(), cout, &sd);     // one copy feeds both GEMMs
   const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
-  if (int rc = to_planes_tensor_scale(dy, n, cout, 4 * h * w, dya, sd, st)) return rc;
+  if (int rc = to_planes_tensor_scale(dy, n, cout, 4 * h * w, cout, dya, sd, st)) return rc;
   if (dx) {
     CdrConvBn cb{};
     cb.weight = weight;
     TcLayer& L = ws.L;
-    pack_rows_f16_kernel<-1><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
+    pack_rows_f16_kernel<-16><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
                                                            (__half*)L.w[1], L.wsi, L.bias, nullptr);
     CDR_LAUNCH_OK("pack_rows_f16_kernel");
     if (int rc = layer_maps(L)) return rc;
@@ -2701,11 +2721,165 @@ int tc_deconv_train_backward(const void* saved, const float* weight, const float
     if (int rc = launch_tc(l, st)) return rc;
   }
   if (dw) {
-    if (int rc = launch_wgrad(d, xa, sx, dya, ws.part, st)) return rc;
+    if (int rc = launch_wgrad(n, h, w, xa, cin, cin, sx, dya, cout, cout, true, d.slices(), ws.part, st)) return rc;
     const long long total = (long long)cin * cout * 16;
-    wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, d.slices(), cin, cout, d.npo(),
-                                                                                   sx.scale, sd.scale, dw);
+    wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, d.slices(), 16, cin, cout,
+                                                                                   d.npo(), sx.scale, sd.scale, dw);
     CDR_LAUNCH_OK("wgrad_reduce_kernel");
+  }
+  set_stage(nullptr);
+  return CDR_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// Training a 1x1 Conv2d(Cin, Cout, bias optional) at fp32 accuracy on the same f16x2 tap-GEMM:
+//   forward  y  = kTapNone over the x planes, weights (+ bias) packed per call, planar epilogue straight into NCHW fp32
+//   dgrad    dx = kTapNone over the dy planes, B = W^T packed [ci][co] (dgrad_weight<1>), planar NCHW fp32 out
+//   wgrad    dW = the kMN kernel with M = Cout (A = dy) and N = Cin (B = x), both 2-D pixel-major maps, K split into
+//               slices -> wgrad_reduce_kernel with 1 tap writes (Cout, Cin, 1, 1) directly
+//   dbias    db = bias_grad_kernel: a fixed-order fp64 sum over the pixels of every channel
+// Channel counts need not be multiples of 64: the x and dy planes are stored with a pitch of round_up(C, 64) whose pad
+// columns the encoder writes as zeros, the packed weights' K pitch is zero-filled, and output channels past Cout / Cin
+// are masked by the epilogue.  x and dy carry one power-of-two tensor scale each, as in the deconv op.
+struct C1Shape {
+  int n, cin, cout, h, w;
+  size_t rows() const { return (size_t)n * h * w; }
+  int pin() const { return round_up(cin, 64); }       // x planes pitch = forward K
+  int pout() const { return round_up(cout, 64); }     // dy planes pitch = dgrad K
+  static int bn(int c) { return c <= 32 ? 32 : 128; }
+  int slices() const { return wgrad_slices((long long)rows() / 64, (long long)ceil_div(cout, 128) * ceil_div(cin, 128)); }
+};
+struct C1Ws {
+  TcLayer L;                 // forward: [round_up(Cout, bn)][pin]; backward: dgrad [round_up(Cin, bn)][pout]
+  void* dy_planes = nullptr; // backward: dy as an fp16 planes buffer [hi | lo | {amax, scale}], pitch pout
+  float* part = nullptr;     // backward: wgrad partials [slice][cout][round_up(cin, 128)]
+  size_t bytes = 0;
+};
+static C1Ws plan_conv1x1_train(void* base, const C1Shape& d, bool backward) {
+  C1Ws ws;
+  Bump1K b(base);
+  if (!backward) {
+    const int bn = C1Shape::bn(d.cout), np = round_up(d.cout, bn);
+    plan_layer(ws.L, b, kKindF16X2, np, d.pin(), d.pin(), bn, np, np, false);
+  } else {
+    const int bn = C1Shape::bn(d.cin), np = round_up(d.cin, bn);
+    plan_layer(ws.L, b, kKindF16X2, np, d.pout(), d.pout(), bn, np, np, false);
+    ws.dy_planes = b.take(2 * planes_stride_bytes(d.rows(), d.pout()) + 1024);
+    ws.part = (float*)b.take((size_t)d.slices() * d.cout * round_up(d.cin, 128) * sizeof(float));
+  }
+  ws.bytes = b.off;
+  return ws;
+}
+size_t conv1x1_train_saved_bytes(int n, int cin, int cout, int h, int w) {
+  const C1Shape d{n, cin, cout, h, w};
+  return 2 * planes_stride_bytes(d.rows(), d.pin()) + 1024;
+}
+size_t conv1x1_train_workspace_bytes(int n, int cin, int cout, int h, int w) {
+  const C1Shape d{n, cin, cout, h, w};
+  const size_t f = plan_conv1x1_train(nullptr, d, false).bytes, bw = plan_conv1x1_train(nullptr, d, true).bytes;
+  return f > bw ? f : bw;
+}
+
+// one packed 1x1 GEMM over `rows` pixels of an fp16 planes buffer, planar fp32 NCHW output of `nout` channels
+static int conv1x1_gemm(const C1Shape& d, const Act& a, int k_pitch, ScaleSlot sa, const TcLayer& L, int nout, float* out,
+                        cudaStream_t st) {
+  TcLaunch l{};
+  l.A = a; l.a_pitch = k_pitch;
+  l.n_img = d.n; l.H = d.h; l.W = d.w; l.cin = k_pitch; l.groups = 1;
+  l.a_rows_total = (long long)d.rows();
+  l.layer = &L; l.b_group_rows = 0; l.n = nout; l.bias_group_stride = 0;
+  l.C.p[0] = out; l.relu = 0; l.out_mode = kOutPlanar;
+  l.in_slot = sa;
+  return launch_tc(l, st);
+}
+
+int tc_conv1x1_train_forward(const float* x, const float* weight, const float* bias, int n, int cin, int cout, int h,
+                             int w, float* y, void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  const C1Shape d{n, cin, cout, h, w};
+  C1Ws ws = plan_conv1x1_train(workspace, d, false);
+  if (workspace_bytes < ws.bytes) {
+    set_error("cdr_conv1x1_train_forward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
+    return CDR_ERR_WORKSPACE;
+  }
+  set_stage("conv1x1_train_fwd");
+  ScaleSlot sx;
+  const Act xa = planes_act(saved, d.rows(), d.pin(), &sx);
+  if (int rc = to_planes_tensor_scale(x, n, cin, h * w, d.pin(), xa, sx, st)) return rc;
+  CdrConvBn cb{};
+  cb.weight = weight;
+  cb.bias = bias;
+  TcLayer& L = ws.L;
+  pack_rows_f16_kernel<0><<<L.rows, 256, 0, st>>>(cb, cout, cin, L.k_pitch, L.n_pad, (__half*)L.w[0], (__half*)L.w[1],
+                                                  L.wsi, L.bias, nullptr);
+  CDR_LAUNCH_OK("pack_rows_f16_kernel");
+  if (int rc = layer_maps(L)) return rc;
+  const int rc = conv1x1_gemm(d, xa, d.pin(), sx, L, cout, y, st);
+  set_stage(nullptr);
+  return rc;
+}
+
+// db[c] = sum over images and pixels of dy[img][c][pixel]: one block per channel, float4 element j*256 + thread of the
+// channel's (image, pixel) sequence to that thread, fp64 partial sums, a fixed tree: bitwise deterministic, no atomics
+__global__ void __launch_bounds__(256)
+bias_grad_kernel(const float* __restrict__ dy, int n, int c, int hw, float* __restrict__ db) {
+  __shared__ double red[256];
+  const int ch = blockIdx.x, hw4 = hw >> 2;                 // hw is a multiple of 64
+  const long long total4 = (long long)n * hw4;
+  double s = 0.0;
+  for (long long i = threadIdx.x; i < total4; i += 256) {
+    const long long img = i / hw4;
+    const float4 v = __ldg(reinterpret_cast<const float4*>(dy + (img * c + ch) * hw) + (i - img * hw4));
+    s += ((double)v.x + (double)v.y) + ((double)v.z + (double)v.w);
+  }
+  red[threadIdx.x] = s;
+  __syncthreads();
+#pragma unroll
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) db[ch] = (float)red[0];
+}
+
+int tc_conv1x1_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                              int w, float* dx, float* dw, float* db, void* workspace, size_t workspace_bytes,
+                              cudaStream_t st) {
+  const C1Shape d{n, cin, cout, h, w};
+  C1Ws ws = plan_conv1x1_train(workspace, d, true);
+  if (workspace_bytes < ws.bytes) {
+    set_error("cdr_conv1x1_train_backward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
+    return CDR_ERR_WORKSPACE;
+  }
+  if (!dx && !dw && !db) return CDR_OK;
+  set_stage("conv1x1_train_bwd");
+  if (db) {
+    bias_grad_kernel<<<cout, 256, 0, st>>>(dy, n, cout, h * w, db);
+    CDR_LAUNCH_OK("bias_grad_kernel");
+  }
+  if (dx || dw) {
+    ScaleSlot sd, sx;
+    const Act dya = planes_act(ws.dy_planes, d.rows(), d.pout(), &sd);     // one copy feeds both GEMMs
+    const Act xa = planes_act(saved, d.rows(), d.pin(), &sx);
+    if (int rc = to_planes_tensor_scale(dy, n, cout, h * w, d.pout(), dya, sd, st)) return rc;
+    if (dx) {
+      CdrConvBn cb{};
+      cb.weight = weight;
+      TcLayer& L = ws.L;
+      pack_rows_f16_kernel<-1><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
+                                                       (__half*)L.w[1], L.wsi, L.bias, nullptr);
+      CDR_LAUNCH_OK("pack_rows_f16_kernel");
+      if (int rc = layer_maps(L)) return rc;
+      if (int rc = conv1x1_gemm(d, dya, d.pout(), sd, L, cin, dx, st)) return rc;
+    }
+    if (dw) {
+      const int slices = d.slices();
+      if (int rc = launch_wgrad(n, h, w, dya, cout, d.pout(), sd, xa, cin, d.pin(), false, slices, ws.part, st)) return rc;
+      const long long total = (long long)cout * cin;
+      wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, slices, 1, cout, cin,
+                                                                                     round_up(cin, 128), sx.scale,
+                                                                                     sd.scale, dw);
+      CDR_LAUNCH_OK("wgrad_reduce_kernel");
+    }
   }
   set_stage(nullptr);
   return CDR_OK;

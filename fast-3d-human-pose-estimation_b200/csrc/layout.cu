@@ -96,7 +96,7 @@ int launch_nchw_to_rows_f32(const float* in, const float* in2, int n_img, int C,
 }
 int launch_nchw_to_rows_bf16(const float* in, const float* in2, int n_img, int C, int HW, __nv_bfloat16* out,
                              int out_pitch, cudaStream_t st) {
-  if (C % 64 == 0 && HW % 64 == 0 && out_pitch % 2 == 0 && ((uintptr_t)in & 7) == 0 && (!in2 || ((uintptr_t)in2 & 7) == 0)) {
+  if (C % 64 == 0 && HW % 64 == 0 && out_pitch == C && ((uintptr_t)in & 7) == 0 && (!in2 || ((uintptr_t)in2 & 7) == 0)) {
     CDR_CHECK_ARG(in && out && n_img > 0 && out_pitch >= C, "nchw_to_rows: bad args");
     dim3 grid(C / 64, HW / 64, in2 ? 2 * n_img : n_img);
     nchw_to_rows16_kernel<false><<<grid, 256, 0, st>>>(in, in2, n_img, C, HW, out, nullptr, out_pitch, nullptr, nullptr);
@@ -172,7 +172,8 @@ int launch_amax_f32(const float* in, const float* in2, long long n, float* amax,
 }
 
 // scaled fp16 hi/lo planes (gemm_tc.cu: kFmtF16P): X = x * s with s = 2^(13 - ilogb(amax)) (common.cuh: f16_pow2_scale),
-// hi = rn_f16(X), lo = rn_f16((X - hi) * 2^11); block (0,0,0) publishes s.
+// hi = rn_f16(X), lo = rn_f16((X - hi) * 2^11); block (0,0,0) publishes s.  Columns [C, out_pitch) of every row are
+// written as zeros: a padded K pitch reaches the GEMM, and stale bytes there could be NaN (NaN * 0 poisons the sum).
 __global__ void __launch_bounds__(256)
 nchw_to_rows_f16p_kernel(const float* __restrict__ in, const float* __restrict__ in2, int n_first, int C, int HW,
                          __half* __restrict__ out_hi, __half* __restrict__ out_lo, int out_pitch,
@@ -192,10 +193,11 @@ nchw_to_rows_f16p_kernel(const float* __restrict__ in, const float* __restrict__
     }
   }
   __syncthreads();
-  if (c0 + tx < C) {
+  if (c0 + tx < out_pitch) {
+    const bool pad = c0 + tx >= C;
     for (int pp = ty; pp < 64; pp += 8) {
       if (p0 + pp < HW) {
-        const float X = tile[tx][pp] * s;
+        const float X = pad ? 0.f : tile[tx][pp] * s;
         const __half h = __float2half_rn(X);
         const size_t o = ((size_t)img * HW + p0 + pp) * out_pitch + c0 + tx;
         out_hi[o] = h;
@@ -208,13 +210,13 @@ int launch_nchw_to_rows_f16p(const float* in, const float* in2, int n_img, int C
                              int out_pitch, const float* amax, float* scale_out, cudaStream_t st) {
   CDR_CHECK_ARG(in && out_hi && out_lo && amax && scale_out && n_img > 0 && C > 0 && HW > 0 && out_pitch >= C,
                 "nchw_to_rows_f16p: bad args");
-  if (C % 64 == 0 && HW % 64 == 0 && out_pitch % 2 == 0 && ((uintptr_t)in & 7) == 0 && (!in2 || ((uintptr_t)in2 & 7) == 0)) {
+  if (C % 64 == 0 && HW % 64 == 0 && out_pitch == C && ((uintptr_t)in & 7) == 0 && (!in2 || ((uintptr_t)in2 & 7) == 0)) {
     dim3 grid16(C / 64, HW / 64, in2 ? 2 * n_img : n_img);
     nchw_to_rows16_kernel<true><<<grid16, 256, 0, st>>>(in, in2, n_img, C, HW, out_hi, out_lo, out_pitch, amax, scale_out);
     CDR_LAUNCH_OK("nchw_to_rows16_kernel");
     return CDR_OK;
   }
-  dim3 grid(ceil_div(C, 32), ceil_div(HW, 64), in2 ? 2 * n_img : n_img);
+  dim3 grid(ceil_div(out_pitch, 32), ceil_div(HW, 64), in2 ? 2 * n_img : n_img);
   nchw_to_rows_f16p_kernel<<<grid, 256, 0, st>>>(in, in2, n_img, C, HW, (__half*)out_hi, (__half*)out_lo, out_pitch, amax,
                                                  scale_out);
   CDR_LAUNCH_OK("nchw_to_rows_f16p_kernel");

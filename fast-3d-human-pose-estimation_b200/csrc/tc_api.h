@@ -48,4 +48,13 @@ int tc_deconv_train_forward(const float* x, const float* weight, int n, int cin,
 int tc_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
                              int w, float* dx, float* dw, void* workspace, size_t workspace_bytes, cudaStream_t st);
 
+// Training a 1x1 Conv2d(Cin, Cout, bias optional) at fp32 accuracy (f16x2) — gemm_tc.cu
+size_t conv1x1_train_saved_bytes(int n, int cin, int cout, int h, int w);
+size_t conv1x1_train_workspace_bytes(int n, int cin, int cout, int h, int w);
+int tc_conv1x1_train_forward(const float* x, const float* weight, const float* bias, int n, int cin, int cout, int h,
+                             int w, float* y, void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st);
+int tc_conv1x1_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                              int w, float* dx, float* dw, float* db, void* workspace, size_t workspace_bytes,
+                              cudaStream_t st);
+
 }  // namespace cdr

@@ -347,6 +347,22 @@ int cdr_deconv_train_forward(const float* x, const float* weight, int n, int cin
 int cdr_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
                               int w, float* dx, float* dweight, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- Training 1x1 convolutions: Conv2d(Cin, Cout, 1), bias optional, at fp32 accuracy on the tensor cores (the same
+ * scaled fp16 hi/lo operands), forward and backward.  x (n, Cin, h, w), weight (Cout, Cin, 1, 1), bias (Cout) or NULL,
+ * y / dy (n, Cout, h, w), all fp32 NCHW; x, weight, y, dy, dx, dweight 16-byte aligned, bias / dbias 4-byte.
+ * Supported: n >= 1, 1 <= Cin, Cout <= 4096, h*w a multiple of 64, n*h*w <= 2^22 (CDR_ERR_INVALID otherwise).
+ * `saved` and the workspace work as for cdr_deconv_train_*.  The backward writes dx (n, Cin, h, w), dweight
+ * (Cout, Cin, 1, 1) and / or dbias (Cout); a NULL pointer skips that output.  dweight and dbias are bitwise
+ * deterministic (fixed-order reductions, no atomics). */
+int cdr_conv1x1_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes,
+                                      size_t* workspace_bytes);
+int cdr_conv1x1_train_forward(const float* x, const float* weight, const float* bias, int n, int cin, int cout, int h,
+                              int w, float* y, void* saved, size_t saved_bytes, void* workspace, size_t workspace_bytes,
+                              void* stream);
+int cdr_conv1x1_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                               int w, float* dx, float* dweight, float* dbias, void* workspace, size_t workspace_bytes,
+                               void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
