@@ -20,6 +20,10 @@ accuracy (independent of torch's TF32 flags):
 and so do the head's 1x1 convolutions (the fusion block's and ``decoder.final_layer``), bias included:
 
     y = conv1x1(x, weight, bias)                      # == F.conv2d(x, weight, bias) for a (Cout, Cin, 1, 1) weight
+
+and so do the encoder's 3x3 convolutions, at stride 1 and 2:
+
+    y = conv3x3(x, weight, stride)                    # == F.conv2d(x, weight, stride=stride, padding=1), no bias
 """
 from __future__ import annotations
 
@@ -285,3 +289,77 @@ def conv1x1(x, weight, bias=None):
     x (N, Cin, H, W), bias (Cout) or None: CUDA float32, 1 <= Cin, Cout <= 4096, H*W a multiple of 64,
     N*H*W <= 2^22; anything else raises ValueError."""
     return _Conv1x1.apply(x, weight, bias)
+
+
+def _conv3x3_args(x, weight, stride):
+    """Checks of conv3x3's inputs, all before any CUDA call: ValueError, there is no fallback."""
+    if not (isinstance(x, torch.Tensor) and isinstance(weight, torch.Tensor)):
+        raise ValueError("conv3x3: x and weight must be tensors")
+    if x.dim() != 4 or weight.dim() != 4 or tuple(weight.shape[2:]) != (3, 3) or weight.shape[1] != x.shape[1]:
+        raise ValueError(f"conv3x3: x (N, Cin, H, W) and weight (Cout, Cin, 3, 3) expected, got {tuple(x.shape)} and "
+                         f"{tuple(weight.shape)}")
+    n, cin, h, w = x.shape
+    cout = weight.shape[0]
+    ok = type(stride) is int and stride in (1, 2) and n >= 1 and all(64 <= c <= 2048 and c % 64 == 0 for c in (cin, cout))
+    ok = ok and h % stride == 0 and w % stride == 0
+    ho, wo = (h // stride, w // stride) if ok else (0, 0)
+    if not (ok and wo in (8, 16, 32, 64) and (ho * wo == 64 or (ho * wo) % 128 == 0) and n * ho * wo <= 1 << 22):
+        raise ValueError(f"conv3x3: unsupported shape x {tuple(x.shape)}, weight {tuple(weight.shape)}, stride {stride!r} "
+                         "(stride 1 or 2, Cin and Cout multiples of 64 in [64, 2048], H and W divisible by the stride; "
+                         "output W a power of two in [8, 64], output H*W = 64 or a multiple of 128, N*H*W <= 2^22)")
+    if x.dtype != torch.float32 or weight.dtype != torch.float32:
+        raise ValueError(f"conv3x3: float32 expected, got {x.dtype} and {weight.dtype}")
+    if not (x.is_cuda and weight.is_cuda) or x.device != weight.device:
+        raise ValueError("conv3x3: x and weight must be CUDA tensors on one device (there is no CPU fallback)")
+    return _aligned(x), _aligned(weight)
+
+
+class _Conv3x3(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, weight, stride):
+        x, weight = _conv3x3_args(x, weight, stride)
+        n, cin, h, w = x.shape
+        cout = weight.shape[0]
+        L = _lib.lib()
+        saved_b, ws_b = C.c_size_t(), C.c_size_t()
+        _lib.check(L.cdr_conv3x3_train_workspace_bytes(n, cin, cout, h, w, stride, C.byref(saved_b), C.byref(ws_b)))
+        dev = x.device
+        y = torch.empty((n, cout, h // stride, w // stride), dtype=torch.float32, device=dev)
+        saved = torch.empty(saved_b.value, dtype=torch.uint8, device=dev)     # x as fp16 planes, for the weight gradient
+        ws = torch.empty(ws_b.value, dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            _lib.check(L.cdr_conv3x3_train_forward(_lib.ptr(x), _lib.ptr(weight), n, cin, cout, h, w, stride,
+                                                   _lib.ptr(y), _lib.ptr(saved), saved_b.value, _lib.ptr(ws), ws_b.value,
+                                                   _lib.current_stream_ptr(dev)))
+        ctx.save_for_backward(saved, weight)
+        ctx.dims = (n, cin, cout, h, w, stride)
+        ctx.ws_bytes = ws_b.value
+        return y
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_y):
+        saved, weight = ctx.saved_tensors
+        n, cin, cout, h, w, stride = ctx.dims
+        need_x, need_w = ctx.needs_input_grad[:2]
+        if not (need_x or need_w):
+            return None, None, None
+        dy = _aligned(_chk(grad_y, "conv3x3: grad"))
+        dev = dy.device
+        dx = torch.empty((n, cin, h, w), dtype=torch.float32, device=dev) if need_x else None
+        dw = torch.empty((cout, cin, 3, 3), dtype=torch.float32, device=dev) if need_w else None
+        ws = torch.empty(ctx.ws_bytes, dtype=torch.uint8, device=dev)
+        L = _lib.lib()
+        with torch.cuda.device(dev):
+            _lib.check(L.cdr_conv3x3_train_backward(_lib.ptr(saved), _lib.ptr(weight), _lib.ptr(dy), n, cin, cout, h, w,
+                                                    stride, _lib.ptr(dx), _lib.ptr(dw), _lib.ptr(ws), ctx.ws_bytes,
+                                                    _lib.current_stream_ptr(dev)))
+        return dx, dw, None
+
+
+def conv3x3(x, weight, stride=1):
+    """F.conv2d(x, weight, stride=stride, padding=1) for a (Cout, Cin, 3, 3) weight without bias, forward and backward
+    on libcdrhead at fp32 accuracy.  x (N, Cin, H, W): CUDA float32, stride 1 or 2, Cin and Cout multiples of 64 in
+    [64, 2048], H and W divisible by the stride, the output's width a power of two in [8, 64], its H*W 64 or a multiple
+    of 128 and N*H*W <= 2^22; anything else raises ValueError."""
+    return _Conv3x3.apply(x, weight, stride)

@@ -291,13 +291,16 @@ class CDRNet(nn.Module):
     everywhere; 'fp32_ffma' = the same arithmetic on CUDA cores (cross-check); 'bf16' = bf16 operands on tcgen05."""
 
     def __init__(self, cfg, n_views=2, nj=19, fusion_in_dim=2048, fusion_hid_ch1=300,
-                 fusion_hid_ch2=400, precision="fp32", encoder_precision=None, trainable=False):
+                 fusion_hid_ch2=400, precision="fp32", encoder_precision=None, trainable=False, train_encoder_on_library=False):
         """encoder_precision: 'fp32' — this library's tcgen05 encoder at the reference's precision (scaled fp16 hi/lo
         planes, 3 MMAs per product; needs precision='fp32'); 'torch' (default — the reference's nn.Module on torch/cuDNN, fp32) or
         'bf16' (Bottleneck stages on libcdrhead's tcgen05 kernels, stem on cuDNN bf16; SURVEY §8f).
-        trainable: opt in to ``forward`` in training mode (``forward_train``, SURVEY §8f rank 3 slice)."""
+        trainable: opt in to ``forward`` in training mode (``forward_train``, SURVEY §8f rank 3 slice).
+        train_encoder_on_library: ``forward_train`` runs a Bottleneck encoder through ``ResNet.forward_train`` (its 1x1 /
+        3x3 convs and BatchNorms on libcdrhead at fp32 accuracy) instead of the torch modules (DESIGN.md §7)."""
         super().__init__()
         self.trainable = bool(trainable)
+        self.train_encoder_on_library = bool(train_encoder_on_library)
         encoder_precision = _default_encoder_precision(encoder_precision)
         if encoder_precision not in ("torch", "bf16", "fp32"):
             raise ValueError(f"encoder_precision must be 'torch', 'bf16' or 'fp32', got {encoder_precision!r}")
@@ -444,9 +447,12 @@ class CDRNet(nn.Module):
         of the fusion block and ``decoder.final_layer`` (``conv1x1``, bias included).  The head's train-mode BatchNorm +
         ReLU (losses.py: batch statistics, running-stat update), the three operators the reference hand-rolls —
         ``ftl`` (:45-56), ``process_heatmap`` (:120-149) and ``dlt`` (:151-179) — and the pseudo-inverse run forward
-        AND backward in libcdrhead.so too (autograd.py, losses.py).  Only the encoder (cuDNN + torch autograd) and the
-        optimizer stay with torch.  Needs ``CDRNet(..., trainable=True)``; projection matrices get no gradient (data in
-        the reference)."""
+        AND backward in libcdrhead.so too (autograd.py, losses.py).  With ``train_encoder_on_library=True`` a Bottleneck
+        encoder (ResNet-50/101/152) trains on the library as well (``ResNet.forward_train``): its 1x1 convs through
+        ``conv1x1``, its 3x3 convs through ``conv3x3`` and its BatchNorms through ``batch_norm_train``, one call per view
+        so that BatchNorm sees per-view batch statistics, as in the reference; otherwise the encoder runs on torch (cuDNN
+        + torch autograd).  The encoder's stem (7x7 conv, BatchNorm, ReLU, max-pool) and the optimizer always stay with
+        torch.  Needs ``CDRNet(..., trainable=True)``; projection matrices get no gradient (data in the reference)."""
         from .autograd import conv1x1, conv_transpose2d, dlt, ftl, soft_argmax_2d
         if not self.trainable:
             raise RuntimeError("forward_train needs CDRNet(..., trainable=True)")
@@ -468,7 +474,8 @@ class CDRNet(nn.Module):
         def dcbr(seq, x):
             """transposed conv on libcdrhead -> train-mode BatchNorm + ReLU"""
             return batch_norm_train(conv_transpose2d(x, seq[0].weight), seq[1], relu=True)
-        feats = [self.encoder(xs[v]) for v in range(2)]                       # :231-234
+        enc = self.encoder.forward_train if self.train_encoder_on_library else self.encoder
+        feats = [enc(xs[v]) for v in range(2)]                                # :231-234, one call per view
         cf = self.CF
         z = torch.cat([ftl(cbr(cf.conv_layer1, feats[v]), pinv[v]) for v in range(2)], dim=1)      # :62-70
         f = cbr(cf.conv_layer2, cbr(cf.conv_layer2, z), 3)                    # :74

@@ -749,3 +749,53 @@ extern "C" int cdr_conv1x1_train_backward(const void* saved, const float* weight
   return tc_conv1x1_train_backward(saved, weight, dy, n, cin, cout, h, w, dx, dweight, dbias, workspace,
                                    workspace_bytes, (cudaStream_t)stream);
 }
+
+// ------------------------------------------------------------------------------------------
+// Training 3x3 convolutions (gemm_tc.cu: tc_conv3x3_train_*).  h, w: the input map.  The output map's H*W must be 64 or
+// a multiple of 128: the tap-GEMM's 128-pixel tile is one 4-D box of whole rows (or of two whole 64-pixel images).
+static int conv3x3_train_shape(const char* fn, int n, int cin, int cout, int h, int w, int stride) {
+  const bool s_ok = stride == 1 || stride == 2;
+  const bool c_ok = cin >= 64 && cin <= 2048 && cin % 64 == 0 && cout >= 64 && cout <= 2048 && cout % 64 == 0;
+  const bool g_ok = s_ok && h >= 1 && w >= 1 && h % stride == 0 && w % stride == 0;
+  const long long ho = g_ok ? h / stride : 0, wo = g_ok ? w / stride : 0, hw = ho * wo;
+  const bool o_ok = g_ok && (wo == 8 || wo == 16 || wo == 32 || wo == 64) && (hw == 64 || hw % 128 == 0);
+  CDR_CHECK_ARG(n >= 1 && c_ok && o_ok && (long long)n * hw <= (1LL << 22),
+                "%s: unsupported shape n=%d cin=%d cout=%d h=%d w=%d stride=%d (stride 1 or 2, Cin and Cout multiples of 64 "
+                "in [64, 2048], h and w divisible by the stride; output W a power of two in [8, 64], output H*W = 64 or a "
+                "multiple of 128, n*H*W <= 2^22)", fn, n, cin, cout, h, w, stride);
+  return CDR_OK;
+}
+extern "C" int cdr_conv3x3_train_workspace_bytes(int n, int cin, int cout, int h, int w, int stride, size_t* saved_bytes,
+                                                 size_t* workspace_bytes) {
+  CDR_CHECK_ARG(saved_bytes && workspace_bytes, "cdr_conv3x3_train_workspace_bytes: null pointer");
+  if (int rc = conv3x3_train_shape("cdr_conv3x3_train_workspace_bytes", n, cin, cout, h, w, stride)) return rc;
+  *saved_bytes = conv3x3_train_saved_bytes(n, cin, cout, h, w, stride);
+  *workspace_bytes = conv3x3_train_workspace_bytes(n, cin, cout, h, w, stride);
+  return CDR_OK;
+}
+extern "C" int cdr_conv3x3_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w,
+                                         int stride, float* y, void* saved, size_t saved_bytes, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
+  CDR_CHECK_ARG(x && weight && y && saved && workspace, "cdr_conv3x3_train_forward: null pointer");
+  if (int rc = conv3x3_train_shape("cdr_conv3x3_train_forward", n, cin, cout, h, w, stride)) return rc;
+  CDR_CHECK_ARG(al16(x) && al16(weight) && al16(y) && ((uintptr_t)saved & 255) == 0 && ((uintptr_t)workspace & 255) == 0,
+                "cdr_conv3x3_train_forward: tensors must be 16-byte, saved / workspace 256-byte aligned");
+  if (saved_bytes < conv3x3_train_saved_bytes(n, cin, cout, h, w, stride)) {
+    set_error("cdr_conv3x3_train_forward: saved %zu < required %zu bytes", saved_bytes,
+              conv3x3_train_saved_bytes(n, cin, cout, h, w, stride));
+    return CDR_ERR_WORKSPACE;
+  }
+  return tc_conv3x3_train_forward(x, weight, n, cin, cout, h, w, stride, y, saved, workspace, workspace_bytes,
+                                  (cudaStream_t)stream);
+}
+extern "C" int cdr_conv3x3_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin,
+                                          int cout, int h, int w, int stride, float* dx, float* dweight, void* workspace,
+                                          size_t workspace_bytes, void* stream) {
+  CDR_CHECK_ARG(saved && weight && dy && workspace, "cdr_conv3x3_train_backward: null pointer");
+  if (int rc = conv3x3_train_shape("cdr_conv3x3_train_backward", n, cin, cout, h, w, stride)) return rc;
+  CDR_CHECK_ARG(al16(weight) && al16(dy) && al16(dx) && al16(dweight) && ((uintptr_t)saved & 255) == 0 &&
+                    ((uintptr_t)workspace & 255) == 0,
+                "cdr_conv3x3_train_backward: tensors must be 16-byte, saved / workspace 256-byte aligned");
+  return tc_conv3x3_train_backward(saved, weight, dy, n, cin, cout, h, w, stride, dx, dweight, workspace,
+                                   workspace_bytes, (cudaStream_t)stream);
+}

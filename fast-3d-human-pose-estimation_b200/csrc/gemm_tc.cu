@@ -382,8 +382,9 @@ constexpr int kSplitChunk = 8;
 // of one group g = slice * taps + tap and one K slice.  Both operands are read straight from the pixel-major fp16 planes,
 // so they are MN-major (channels contiguous): A = two 64-channel x 64-pixel boxes; B = the same 64 pixels in the same
 // (img, y, x) order.  tap_mode kTapConv4s2: a k4 s2 p1 transposed conv (deconv_train_backward; A = x, B = dy through the
-// stride-2 box shifted by (kx - 1, ky - 1), 16 taps).  kTapNone: a 1x1 conv (conv1x1_train_backward; A = dy, B = x,
-// both 2-D maps, 1 tap).  The UMMA descriptors carry the MN-major SWIZZLE_128B layout (LBO = the 8 KB between
+// stride-2 box shifted by (kx - 1, ky - 1), 16 taps).  kTapConv3: a 3x3 pad-1 conv at stride p.stride
+// (conv3x3_train_backward; A = dy, B = x through the stride-1 or stride-2 box shifted by (kx - 1, ky - 1), 9 taps).
+// kTapNone: a 1x1 conv (conv1x1_train_backward; A = dy, B = x, both 2-D maps, 1 tap).  The UMMA descriptors carry the MN-major SWIZZLE_128B layout (LBO = the 8 KB between
 // the two 64-channel halves, SBO = 1024 B between 8-pixel groups) and the instruction descriptor the transpose bits.
 // The epilogue stores the raw fp32 tile (still times s_x * s_dy) into the slice's partial; wgrad_reduce_kernel sums
 // the slices in a fixed order.
@@ -519,11 +520,12 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
           const int bk = tap * p.cin + k0;
           const int brow = g * p.b_group_rows + n_tile * BN + (kPair2 ? (int)cta_rank * (BN / 2) : 0);   // CL = 2: my half of B
           if constexpr (kMN) {
-            // wgrad: g = slice * 16 + (ky * 4 + kx) (kTapConv4s2) or slice (kTapNone); 64 pixels of A from k0 of the slice
-            // (p.cin pixels per slice; for the stride-2 box a block is whole rows of one image since W | 64 | H*W) and the
-            // B pixels they pair with: the same ones, or the dy pixels (2y - 1 + ky, 2x - 1 + kx)
-            const bool s2 = p.tap_mode == kTapConv4s2;
-            const int wt = s2 ? g & 15 : 0, pix0 = (s2 ? g >> 4 : g) * p.cin + k0;
+            // wgrad: g = slice * kw^2 + (ky * kw + kx), kw = 4 (kTapConv4s2), 3 (kTapConv3) or 1 (kTapNone); 64 pixels
+            // of A from k0 of the slice (p.cin pixels per slice; for the 4-D box a block is whole rows of one image since
+            // W | 64 | H*W) and the B pixels they pair with: the same ones, or (stride * y - 1 + ky, stride * x - 1 + kx)
+            const int kw = p.tap_mode == kTapConv4s2 ? 4 : p.tap_mode == kTapConv3 ? 3 : 1;
+            const int sl = g / (kw * kw), wt = g - sl * kw * kw, wky = wt / kw, wkx = wt - wky * kw;
+            const int pix0 = sl * p.cin + k0;
             const int wimg = pix0 / HW, wy = (pix0 - wimg * HW) / p.W;
             const int co0 = n_tile * BN;
             if (ptx::elect_one()) {
@@ -535,9 +537,9 @@ tap_gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
 #pragma unroll
                 for (int h = 0; h < 2; ++h) {
                   ptx::tma_load_2d(stage_a(s, pl) + h * (kABytes / 2), ma, &full[s], m0 + 64 * h, pix0);
-                  if (s2)
-                    ptx::tma_load_4d(stage_b(s, pl) + h * (Cfg::kBBytes / 2), mb, &full[s], co0 + 64 * h, (wt & 3) - 1,
-                                     2 * wy + (wt >> 2) - 1, wimg);
+                  if (kw > 1)
+                    ptx::tma_load_4d(stage_b(s, pl) + h * (Cfg::kBBytes / 2), mb, &full[s], co0 + 64 * h, wkx - 1,
+                                     p.stride * wy + wky - 1, wimg);
                   else
                     ptx::tma_load_2d(stage_b(s, pl) + h * (Cfg::kBBytes / 2), mb, &full[s], co0 + 64 * h, pix0);
                 }
@@ -1437,13 +1439,18 @@ __device__ __forceinline__ float conv1x1_weight(const CdrConvBn& s, int cout, in
   if (n >= cout || k >= cin) return 0.f;
   return (float)((double)s.weight[(size_t)n * cin + k] * tc_bn_scale(s, n));
 }
-// folded weight of a transposed conv (Cin,Cout,4,4) at packed position (phase, n, tap*Cin + ci)
+// folded weight of a transposed conv (Cin,Cout,4,4) at packed position (phase, n, tap*Cin + ci).  kK = 3: the weight
+// is (Cin,Cout,3,3), read as its 4x4 zero-padding at index 3 (a 3x3 stride-2 pad-1 conv's data gradient)
+template <int kK = 4>
 __device__ __forceinline__ float deconv_weight(const CdrConvBn& s, int cin, int cout, int phase, int n, int kk) {
   if (n >= cout) return 0.f;
   const int tap = kk / cin, ci = kk - tap * cin;
   const int py = phase >> 1, px = phase & 1, ty = tap >> 1, tx = tap & 1;
   const int ky = 1 - py + 2 * ty, kx = 1 - px + 2 * tx;
-  return (float)((double)s.weight[(((size_t)ci * cout + n) * 4 + ky) * 4 + kx] * tc_bn_scale(s, n));
+  if constexpr (kK == 3) {
+    if (ky == 3 || kx == 3) return 0.f;
+  }
+  return (float)((double)s.weight[(((size_t)ci * cout + n) * kK + ky) * kK + kx] * tc_bn_scale(s, n));
 }
 template <bool kSplit>
 __device__ __forceinline__ void store_weight(void* w0, void* w1, long long idx, float v) {
@@ -1490,16 +1497,21 @@ __device__ __forceinline__ float conv_taps_weight(const CdrConvBn& s, int cout, 
   return (float)((double)s.weight[((size_t)n * cin + ci) * taps + tap] * tc_bn_scale(s, n));
 }
 // the data-gradient operand W^T at packed position (ci, tap*Cout + co): kTaps = 16, a transposed conv's weight
-// (Cin,Cout,4,4) with tap = ky*4 + kx; kTaps = 1, a 1x1 conv's weight (Cout,Cin).  Zero in the padded rows and K pitch.
+// (Cin,Cout,4,4) with tap = ky*4 + kx; kTaps = 9, a 3x3 conv's weight (Cout,Cin,3,3) with the taps flipped,
+// W[co][ci][2 - ky][2 - kx] for tap = ky*3 + kx; kTaps = 1, a 1x1 conv's weight (Cout,Cin).  Zero in the padded rows
+// and K pitch.
 template <int kTaps>
 __device__ __forceinline__ float dgrad_weight(const CdrConvBn& s, int cin, int cout, int ci, int kk) {
   if (ci >= cin || kk >= kTaps * cout) return 0.f;
   const int tap = kk / cout, co = kk - tap * cout;
-  return kTaps == 1 ? s.weight[(size_t)co * cin + ci] : s.weight[((size_t)ci * cout + co) * kTaps + tap];
+  if constexpr (kTaps == 1) return s.weight[(size_t)co * cin + ci];
+  if constexpr (kTaps == 9) return s.weight[((size_t)co * cin + ci) * 9 + (8 - tap)];
+  return s.weight[((size_t)ci * cout + co) * kTaps + tap];
 }
-// kDeconv: 0 = 1x1 conv, 1 = transposed conv (4 phases), >= 2: conv with kDeconv taps in encoder order (use 9; the 1x1
-// convs of the encoder go through mode 0), < 0: dgrad_weight<-kDeconv> (`cout` = Cin rows, `cin` = Cout per tap)
-template <int kDeconv>
+// kDeconv: 0 = 1x1 conv, 1 = transposed conv (4 phases; kDeconvK = 3 reads a 3x3 weight, see deconv_weight), >= 2: conv
+// with kDeconv taps in encoder order (use 9; the 1x1 convs of the encoder go through mode 0), < 0:
+// dgrad_weight<-kDeconv> (`cout` = Cin rows, `cin` = Cout per tap)
+template <int kDeconv, int kDeconvK = 4>
 __global__ void __launch_bounds__(256)
 pack_rows_f16_kernel(CdrConvBn s, int cout, int cin, int k_pitch, int n_pad, __half* __restrict__ w_hi,
                      __half* __restrict__ w_lo, float* __restrict__ wsi, float* __restrict__ bias_out,
@@ -1510,7 +1522,7 @@ pack_rows_f16_kernel(CdrConvBn s, int cout, int cin, int k_pitch, int n_pad, __h
   auto val = [&](int kk) -> float {
     if constexpr (kDeconv >= 2) return conv_taps_weight(s, cout, cin, kDeconv, n, kk);
     if constexpr (kDeconv < 0) return dgrad_weight<-kDeconv>(s, cout, cin, n, kk);
-    return kDeconv ? deconv_weight(s, cin, cout, phase, n, kk) : conv1x1_weight(s, cout, cin, n, kk);
+    return kDeconv ? deconv_weight<kDeconvK>(s, cin, cout, phase, n, kk) : conv1x1_weight(s, cout, cin, n, kk);
   };
   float mx = 0.f, l1 = 0.f;
   for (int kk = threadIdx.x; kk < k_pitch; kk += blockDim.x) {
@@ -2636,10 +2648,11 @@ wgrad_reduce_kernel(const float* __restrict__ part, int slices, int taps, int ro
 
 // The kMN GEMM over n*h*w pixels split into `slices` K slices: part[slice * taps + tap] (m rows, pitch round_up(nb, 128))
 // = A^T B.  A: m channels of a pixel-major fp16 planes buffer (pitch a_pitch), scale slot `sa`.  B: nb channels (pitch
-// b_pitch), either the same pixels through a 2-D map (1 tap), or (b_s2) the 2h x 2w dy of a k4 s2 p1 transposed conv
-// through the stride-2 box, 16 taps.
+// b_pitch), either the same pixels through a 2-D map (b_k = 1, 1 tap), or a (b_stride*h) x (b_stride*w) map through the
+// stride-b_stride box shifted by (kx - 1, ky - 1), b_k^2 taps: b_k = 4, b_stride = 2, the dy of a k4 s2 p1 transposed
+// conv; b_k = 3, the x of a 3x3 pad-1 conv at stride 1 or 2.
 static int launch_wgrad(int n, int h, int w, const Act& a, int m, int a_pitch, ScaleSlot sa, const Act& b, int nb,
-                        int b_pitch, bool b_s2, int slices, float* part, cudaStream_t st) {
+                        int b_pitch, int b_k, int b_stride, int slices, float* part, cudaStream_t st) {
   using Cfg = TcCfg<128, kKindF16X2, kFmtF16P, 0>;
   auto kern = tap_gemm_tc_kernel<128, kKindF16X2, kFmtF16P, 0, true>;
   static DeviceOnce attr_set;
@@ -2652,8 +2665,8 @@ static int launch_wgrad(int n, int h, int w, const Act& a, int m, int a_pitch, S
   p.M = m;
   p.n_img = n; p.H = h; p.W = w;
   p.cin = (int)(kb / slices) * 64;           // pixels per K slice
-  p.ntaps = 1; p.tap_mode = b_s2 ? kTapConv4s2 : kTapNone; p.stride = 1;
-  p.groups = (b_s2 ? 16 : 1) * slices;
+  p.ntaps = 1; p.tap_mode = b_k == 4 ? kTapConv4s2 : b_k == 3 ? kTapConv3 : kTapNone; p.stride = b_stride;
+  p.groups = b_k * b_k * slices;
   p.n_tiles = round_up(nb, 128) / 128;
   p.n = nb;
   p.C = part; p.c_pitch = round_up(nb, 128); p.c_fill = nb;
@@ -2668,12 +2681,13 @@ static int launch_wgrad(int n, int h, int w, const Act& a, int m, int a_pitch, S
       const uint32_t box[2] = {64, 64};
       if (int rc = make_tmap(&ma[pl], a.p[pl], kFmtF16P, 2, dims, strides, box)) return rc;
     }
-    if (b_s2) {   // dy planes (n, 2h, 2w, b_pitch) seen with element stride 2: 64 channels x (w x 64/w) pixels x 1 image
-      const uint64_t iw = 2 * (uint64_t)w, ih = 2 * (uint64_t)h;
+    if (b_k > 1) {   // B planes (n, s*h, s*w, b_pitch) seen with element stride s: 64 channels x (w x 64/w) pixels x 1 image
+      const uint32_t s = (uint32_t)b_stride;
+      const uint64_t iw = s * (uint64_t)w, ih = s * (uint64_t)h;
       const uint64_t dims[4] = {(uint64_t)b_pitch, iw, ih, (uint64_t)n};
       const uint64_t strides[3] = {(uint64_t)b_pitch, (uint64_t)b_pitch * iw, (uint64_t)b_pitch * iw * ih};
-      const uint32_t box[4] = {64, (uint32_t)(2 * w), (uint32_t)(2 * (64 / w)), 1};
-      const uint32_t estr[4] = {1, 2, 2, 1};
+      const uint32_t box[4] = {64, s * (uint32_t)w, s * (uint32_t)(64 / w), 1};
+      const uint32_t estr[4] = {1, s, s, 1};
       if (int rc = make_tmap(&mb[pl], b.p[pl], kFmtF16P, 4, dims, strides, box, estr)) return rc;
     } else {      // B planes: (pixels, b_pitch) rows, like A
       const uint64_t dims[2] = {(uint64_t)b_pitch, (uint64_t)rows};
@@ -2721,7 +2735,7 @@ int tc_deconv_train_backward(const void* saved, const float* weight, const float
     if (int rc = launch_tc(l, st)) return rc;
   }
   if (dw) {
-    if (int rc = launch_wgrad(n, h, w, xa, cin, cin, sx, dya, cout, cout, true, d.slices(), ws.part, st)) return rc;
+    if (int rc = launch_wgrad(n, h, w, xa, cin, cin, sx, dya, cout, cout, 4, 2, d.slices(), ws.part, st)) return rc;
     const long long total = (long long)cin * cout * 16;
     wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, d.slices(), 16, cin, cout,
                                                                                    d.npo(), sx.scale, sd.scale, dw);
@@ -2873,13 +2887,148 @@ int tc_conv1x1_train_backward(const void* saved, const float* weight, const floa
     }
     if (dw) {
       const int slices = d.slices();
-      if (int rc = launch_wgrad(n, h, w, dya, cout, d.pout(), sd, xa, cin, d.pin(), false, slices, ws.part, st)) return rc;
+      if (int rc = launch_wgrad(n, h, w, dya, cout, d.pout(), sd, xa, cin, d.pin(), 1, 1, slices, ws.part, st)) return rc;
       const long long total = (long long)cout * cin;
       wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, slices, 1, cout, cin,
                                                                                      round_up(cin, 128), sx.scale,
                                                                                      sd.scale, dw);
       CDR_LAUNCH_OK("wgrad_reduce_kernel");
     }
+  }
+  set_stage(nullptr);
+  return CDR_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// Training a 3x3 pad-1 Conv2d(Cin, Cout, stride s, bias=False) at fp32 accuracy on the same f16x2 tap-GEMM.  h x w is
+// the input map, H x W = h/s x w/s the output.
+//   forward  y  = kTapConv3 over the x planes (s = 2: the element-strided box), weights packed unfolded per call
+//               (pack_rows_f16_kernel<9>), planar epilogue straight into NCHW fp32
+//   dgrad    s = 1: dx = kTapConv3 over the dy planes, B = W^T with the taps flipped (dgrad_weight<9>)
+//            s = 2: dx = conv_transpose2d(dy, W4, stride 2, pad 1) with W4 = W zero-padded to 4x4 at index 3: the
+//               transposed-conv forward (kTapDeconv, planar_deconv) over the dy planes, W4 read by deconv_weight<3>
+//   wgrad    dW = the kMN kernel with M = Cout (A = dy, a 2-D pixel map) and N = Cin (B = x through the stride-s box
+//               shifted by (kx - 1, ky - 1)), 9 taps, K split into slices -> wgrad_reduce_kernel writes (Cout, Cin, 3, 3)
+// Cin and Cout are multiples of 64, so the x and dy planes have pitch Cin and Cout.  One power-of-two tensor scale each.
+struct C3Shape {
+  int n, cin, cout, h, w, s;
+  int ho() const { return h / s; }
+  int wo() const { return w / s; }
+  size_t x_rows() const { return (size_t)n * h * w; }
+  size_t y_rows() const { return (size_t)n * ho() * wo(); }
+  int npo() const { return round_up(cout, 128); }     // forward: packed output channels
+  int npi() const { return round_up(cin, 128); }      // dgrad: packed output channels (per phase for s = 2)
+  int slices() const { return wgrad_slices((long long)y_rows() / 64, (long long)(npo() / 128) * (npi() / 128) * 9); }
+};
+struct C3Ws {
+  TcLayer L;                 // forward: [npo][9*cin]; backward: dgrad [npi][9*cout] (s = 1) or [4 phases][npi][4*cout]
+  void* dy_planes = nullptr; // backward: dy as an fp16 planes buffer [hi | lo | {amax, scale}]
+  float* part = nullptr;     // backward: wgrad partials [slice][tap][cout][npi]
+  size_t bytes = 0;
+};
+static C3Ws plan_conv3x3_train(void* base, const C3Shape& d, bool backward) {
+  C3Ws ws;
+  Bump1K b(base);
+  if (!backward) {
+    plan_layer(ws.L, b, kKindF16X2, d.npo(), 9 * d.cin, 9 * d.cin, 128, d.npo(), d.npo(), false);
+  } else {
+    if (d.s == 1) plan_layer(ws.L, b, kKindF16X2, d.npi(), 9 * d.cout, 9 * d.cout, 128, d.npi(), d.npi(), false);
+    else plan_layer(ws.L, b, kKindF16X2, 4 * d.npi(), 4 * d.cout, 4 * d.cout, 128, d.npi(), d.npi(), false);
+    ws.dy_planes = b.take(2 * planes_stride_bytes(d.y_rows(), d.cout) + 1024);
+    ws.part = (float*)b.take((size_t)d.slices() * 9 * d.cout * d.npi() * sizeof(float));
+  }
+  ws.bytes = b.off;
+  return ws;
+}
+size_t conv3x3_train_saved_bytes(int n, int cin, int cout, int h, int w, int stride) {
+  const C3Shape d{n, cin, cout, h, w, stride};
+  return 2 * planes_stride_bytes(d.x_rows(), cin) + 1024;
+}
+size_t conv3x3_train_workspace_bytes(int n, int cin, int cout, int h, int w, int stride) {
+  const C3Shape d{n, cin, cout, h, w, stride};
+  const size_t f = plan_conv3x3_train(nullptr, d, false).bytes, bw = plan_conv3x3_train(nullptr, d, true).bytes;
+  return f > bw ? f : bw;
+}
+
+int tc_conv3x3_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, int stride,
+                             float* y, void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  const C3Shape d{n, cin, cout, h, w, stride};
+  C3Ws ws = plan_conv3x3_train(workspace, d, false);
+  if (workspace_bytes < ws.bytes) {
+    set_error("cdr_conv3x3_train_forward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
+    return CDR_ERR_WORKSPACE;
+  }
+  set_stage("conv3x3_train_fwd");
+  ScaleSlot sx;
+  const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
+  if (int rc = to_planes_tensor_scale(x, n, cin, h * w, cin, xa, sx, st)) return rc;
+  CdrConvBn cb{};
+  cb.weight = weight;
+  TcLayer& L = ws.L;
+  pack_rows_f16_kernel<9><<<L.rows, 256, 0, st>>>(cb, cout, cin, L.k_pitch, L.n_pad, (__half*)L.w[0], (__half*)L.w[1],
+                                                  L.wsi, L.bias, nullptr);
+  CDR_LAUNCH_OK("pack_rows_f16_kernel");
+  if (int rc = layer_maps(L)) return rc;
+  TcLaunch l{};
+  l.A = xa; l.a_pitch = cin;
+  l.n_img = n; l.H = d.ho(); l.W = d.wo(); l.cin = cin; l.conv3 = 1; l.stride = stride; l.groups = 1;
+  l.a_rows_total = (long long)d.x_rows();
+  l.layer = &L; l.b_group_rows = 0; l.n = cout; l.bias_group_stride = 0;
+  l.C.p[0] = y; l.relu = 0; l.out_mode = kOutPlanar;
+  l.in_slot = sx;
+  const int rc = launch_tc(l, st);
+  set_stage(nullptr);
+  return rc;
+}
+
+int tc_conv3x3_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                              int w, int stride, float* dx, float* dw, void* workspace, size_t workspace_bytes,
+                              cudaStream_t st) {
+  const C3Shape d{n, cin, cout, h, w, stride};
+  C3Ws ws = plan_conv3x3_train(workspace, d, true);
+  if (workspace_bytes < ws.bytes) {
+    set_error("cdr_conv3x3_train_backward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
+    return CDR_ERR_WORKSPACE;
+  }
+  if (!dx && !dw) return CDR_OK;
+  set_stage("conv3x3_train_bwd");
+  const int ho = d.ho(), wo = d.wo();
+  ScaleSlot sd, sx;
+  const Act dya = planes_act(ws.dy_planes, d.y_rows(), cout, &sd);     // one copy feeds both GEMMs
+  const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
+  if (int rc = to_planes_tensor_scale(dy, n, cout, ho * wo, cout, dya, sd, st)) return rc;
+  if (dx) {
+    CdrConvBn cb{};
+    cb.weight = weight;
+    TcLayer& L = ws.L;
+    TcLaunch l{};
+    l.A = dya; l.a_pitch = cout;
+    l.n_img = n; l.H = ho; l.W = wo; l.cin = cout;
+    l.a_rows_total = (long long)d.y_rows();
+    l.layer = &L; l.bias_group_stride = 0;
+    l.n = cin;
+    l.C.p[0] = dx; l.relu = 0; l.out_mode = kOutPlanar;
+    l.in_slot = sd;
+    if (stride == 1) {
+      pack_rows_f16_kernel<-9><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
+                                                       (__half*)L.w[1], L.wsi, L.bias, nullptr);
+      l.conv3 = 1; l.groups = 1; l.b_group_rows = 0;
+    } else {
+      pack_rows_f16_kernel<1, 3><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
+                                                         (__half*)L.w[1], L.wsi, L.bias, nullptr);
+      l.deconv = 1; l.groups = 4; l.b_group_rows = L.n_pad; l.planar_deconv = 1;
+    }
+    CDR_LAUNCH_OK("pack_rows_f16_kernel");
+    if (int rc = layer_maps(L)) return rc;
+    if (int rc = launch_tc(l, st)) return rc;
+  }
+  if (dw) {
+    const int slices = d.slices();
+    if (int rc = launch_wgrad(n, ho, wo, dya, cout, cout, sd, xa, cin, cin, 3, stride, slices, ws.part, st)) return rc;
+    const long long total = (long long)cout * cin * 9;
+    wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, slices, 9, cout, cin, d.npi(),
+                                                                                   sx.scale, sd.scale, dw);
+    CDR_LAUNCH_OK("wgrad_reduce_kernel");
   }
   set_stage(nullptr);
   return CDR_OK;

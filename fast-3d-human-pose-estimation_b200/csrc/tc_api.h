@@ -57,4 +57,13 @@ int tc_conv1x1_train_backward(const void* saved, const float* weight, const floa
                               int w, float* dx, float* dw, float* db, void* workspace, size_t workspace_bytes,
                               cudaStream_t st);
 
+// Training a 3x3 pad-1 Conv2d(Cin, Cout, stride 1 or 2, bias=False) at fp32 accuracy (f16x2) — gemm_tc.cu
+size_t conv3x3_train_saved_bytes(int n, int cin, int cout, int h, int w, int stride);
+size_t conv3x3_train_workspace_bytes(int n, int cin, int cout, int h, int w, int stride);
+int tc_conv3x3_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, int stride,
+                             float* y, void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st);
+int tc_conv3x3_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                              int w, int stride, float* dx, float* dw, void* workspace, size_t workspace_bytes,
+                              cudaStream_t st);
+
 }  // namespace cdr

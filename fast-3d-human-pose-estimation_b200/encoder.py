@@ -13,6 +13,10 @@ import torch
 import torch.nn.functional as F
 from torch import nn
 
+# bound once, at import: the encoder's training forward does not follow a later rebinding of ``autograd.conv1x1`` (the
+# head's training-step tests swap that name for cuDNN's to compare the head's 1x1 convs alone)
+from .autograd import conv1x1 as _conv1x1, conv3x3 as _conv3x3
+
 _SPEC = {18: ("basic", (2, 2, 2, 2)), 34: ("basic", (3, 4, 6, 3)),
          50: ("bottleneck", (3, 4, 6, 3)), 101: ("bottleneck", (3, 4, 23, 3)),
          152: ("bottleneck", (3, 8, 36, 3))}
@@ -79,10 +83,41 @@ class ResNet(nn.Module):
                 cin = planes * exp
             setattr(self, f"layer{li}", nn.Sequential(*blocks))
         self.out_channels = cin
+        self.kind = kind
 
     def forward(self, x):
         x = self.maxpool(self.relu(self.bn1(self.conv1(x))))
         return self.layer4(self.layer3(self.layer2(self.layer1(x))))
+
+    def forward_train(self, x):
+        """``forward`` in training mode with every Bottleneck block on libcdrhead, forward and backward at fp32 accuracy
+        whatever torch's TF32 flags say: conv1 / conv3 and the downsample conv (on the stride-2 slice, an exact identity
+        for a 1x1 conv) through ``conv1x1``, conv2 through ``conv3x3``, every BatchNorm through ``batch_norm_train``
+        (batch statistics and the running-stat update, as nn.BatchNorm2d in training mode).  The stem (7x7 conv over 3
+        channels, BatchNorm, ReLU, max-pool) stays on torch.  The library's shape limits apply: at N images per call,
+        256 x 256 inputs are inside them for every N up to 64.  ``CDRNet(..., train_encoder_on_library=True)``
+        calls it for each view from ``forward_train``."""
+        if self.kind != "bottleneck":
+            raise ValueError("ResNet.forward_train: only Bottleneck encoders (ResNet-50/101/152) train on the library")
+        x = self.maxpool(self.relu(self.bn1(self.conv1(x))))
+        for layer in (self.layer1, self.layer2, self.layer3, self.layer4):
+            for b in layer:
+                x = _bottleneck_train(b, x)
+        return x
+
+
+def _bottleneck_train(b, x):
+    """one Bottleneck block of ResNet.forward_train: relu(bn3(conv3(relu(bn2(conv2(relu(bn1(conv1(x)))))))) + r)"""
+    from .losses import batch_norm_train
+    y = batch_norm_train(_conv1x1(x, b.conv1.weight), b.bn1, relu=True)
+    y = batch_norm_train(_conv3x3(y, b.conv2.weight, b.conv2.stride[0]), b.bn2, relu=True)
+    y = batch_norm_train(_conv1x1(y, b.conv3.weight), b.bn3)
+    r = x
+    if b.downsample is not None:
+        conv, bn = b.downsample[0], b.downsample[1]
+        s = conv.stride[0]
+        r = batch_norm_train(_conv1x1(x if s == 1 else x[:, :, ::s, ::s], conv.weight), bn)
+    return F.relu(y + r)
 
 
 IMAGENET_MEAN = (0.485, 0.456, 0.406)      # inference.py:42-43

@@ -363,6 +363,22 @@ int cdr_conv1x1_train_backward(const void* saved, const float* weight, const flo
                                int w, float* dx, float* dweight, float* dbias, void* workspace, size_t workspace_bytes,
                                void* stream);
 
+/* ---- Training 3x3 convolutions: Conv2d(Cin, Cout, 3, stride, padding 1, bias=False) with stride 1 or 2, at fp32
+ * accuracy on the tensor cores (the same scaled fp16 hi/lo operands), forward and backward.  x (n, Cin, h, w) with h x w
+ * the INPUT map, weight (Cout, Cin, 3, 3), y / dy (n, Cout, h/stride, w/stride), all fp32 NCHW, 16-byte aligned.
+ * Supported: n >= 1, Cin and Cout multiples of 64 in [64, 2048], h and w divisible by the stride, and for the output
+ * map H x W: W a power of two in [8, 64], H*W = 64 or a multiple of 128, n*H*W <= 2^22 (CDR_ERR_INVALID otherwise).
+ * `saved` and the workspace work as for cdr_deconv_train_*.  The backward writes dx (n, Cin, h, w) and / or dweight
+ * (Cout, Cin, 3, 3); a NULL pointer skips that output.  dweight is bitwise deterministic (fixed-order reduction). */
+int cdr_conv3x3_train_workspace_bytes(int n, int cin, int cout, int h, int w, int stride, size_t* saved_bytes,
+                                      size_t* workspace_bytes);
+int cdr_conv3x3_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, int stride,
+                              float* y, void* saved, size_t saved_bytes, void* workspace, size_t workspace_bytes,
+                              void* stream);
+int cdr_conv3x3_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                               int w, int stride, float* dx, float* dweight, void* workspace, size_t workspace_bytes,
+                               void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
