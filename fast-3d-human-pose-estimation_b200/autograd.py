@@ -28,6 +28,8 @@ and so do the encoder's 3x3 convolutions, at stride 1 and 2:
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
+from typing import Callable
 
 import torch
 
@@ -142,219 +144,119 @@ def ftl(x, mats):
     return _FTL.apply(x, mats)
 
 
-def _deconv_args(x, weight):
-    """Checks of conv_transpose2d's inputs, all before any CUDA call: ValueError, there is no fallback."""
-    if not (isinstance(x, torch.Tensor) and isinstance(weight, torch.Tensor)):
-        raise ValueError("conv_transpose2d: x and weight must be tensors")
-    if x.dim() != 4 or weight.dim() != 4 or tuple(weight.shape[2:]) != (4, 4) or weight.shape[0] != x.shape[1]:
-        raise ValueError(f"conv_transpose2d: x (N, Cin, H, W) and weight (Cin, Cout, 4, 4) expected, got "
-                         f"{tuple(x.shape)} and {tuple(weight.shape)}")
-    n, cin, h, w = x.shape
-    cout = weight.shape[1]
-    if n < 1 or cin % 64 or cout % 64 or h != w or h not in (8, 16, 32):
-        raise ValueError(f"conv_transpose2d: unsupported shape x {tuple(x.shape)}, weight {tuple(weight.shape)} "
-                         "(Cin and Cout multiples of 64, H == W in {8, 16, 32})")
-    if x.dtype != torch.float32 or weight.dtype != torch.float32:
-        raise ValueError(f"conv_transpose2d: float32 expected, got {x.dtype} and {weight.dtype}")
-    if not (x.is_cuda and weight.is_cuda) or x.device != weight.device:
-        raise ValueError("conv_transpose2d: x and weight must be CUDA tensors on one device (there is no CPU fallback)")
-    return x.contiguous(), weight.contiguous()
-
-
-class _ConvTranspose2d(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, x, weight):
-        x, weight = _deconv_args(x, weight)
-        n, cin, h, w = x.shape
-        cout = weight.shape[1]
-        L = _lib.lib()
-        saved_b, ws_b = C.c_size_t(), C.c_size_t()
-        _lib.check(L.cdr_deconv_train_workspace_bytes(n, cin, cout, h, w, C.byref(saved_b), C.byref(ws_b)))
-        dev = x.device
-        y = torch.empty((n, cout, 2 * h, 2 * w), dtype=torch.float32, device=dev)
-        saved = torch.empty(saved_b.value, dtype=torch.uint8, device=dev)     # x as fp16 planes, for the weight gradient
-        ws = torch.empty(ws_b.value, dtype=torch.uint8, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(L.cdr_deconv_train_forward(_lib.ptr(x), _lib.ptr(weight), n, cin, cout, h, w, _lib.ptr(y),
-                                                  _lib.ptr(saved), saved_b.value, _lib.ptr(ws), ws_b.value,
-                                                  _lib.current_stream_ptr(dev)))
-        ctx.save_for_backward(saved, weight)
-        ctx.dims = (n, cin, cout, h, w)
-        ctx.ws_bytes = ws_b.value
-        return y
-
-    @staticmethod
-    @torch.autograd.function.once_differentiable
-    def backward(ctx, grad_y):
-        saved, weight = ctx.saved_tensors
-        n, cin, cout, h, w = ctx.dims
-        need_x, need_w = ctx.needs_input_grad[:2]
-        if not (need_x or need_w):
-            return None, None
-        dy = _chk(grad_y, "conv_transpose2d: grad")
-        dev = dy.device
-        dx = torch.empty((n, cin, h, w), dtype=torch.float32, device=dev) if need_x else None
-        dw = torch.empty((cin, cout, 4, 4), dtype=torch.float32, device=dev) if need_w else None
-        ws = torch.empty(ctx.ws_bytes, dtype=torch.uint8, device=dev)
-        L = _lib.lib()
-        with torch.cuda.device(dev):
-            _lib.check(L.cdr_deconv_train_backward(_lib.ptr(saved), _lib.ptr(weight), _lib.ptr(dy), n, cin, cout, h, w,
-                                                   _lib.ptr(dx), _lib.ptr(dw), _lib.ptr(ws), ctx.ws_bytes,
-                                                   _lib.current_stream_ptr(dev)))
-        return dx, dw
-
-
-def conv_transpose2d(x, weight):
-    """F.conv_transpose2d(x, weight, stride=2, padding=1) for 4x4 kernels without bias, forward and backward on
-    libcdrhead at fp32 accuracy.  x (N, Cin, H, W), weight (Cin, Cout, 4, 4): CUDA float32, Cin and Cout multiples
-    of 64, H == W in {8, 16, 32}; anything else raises ValueError."""
-    return _ConvTranspose2d.apply(x, weight)
-
-
 def _aligned(t):
     """t contiguous with a 16-byte-aligned address (a contiguous view may start mid-allocation)."""
     t = t.contiguous()
     return t if t.data_ptr() % 16 == 0 else t.clone()
 
 
-def _conv1x1_args(x, weight, bias):
-    """Checks of conv1x1's inputs, all before any CUDA call: ValueError, there is no fallback."""
+@dataclasses.dataclass(frozen=True)
+class _TrainConvOp:
+    """One training convolution of libcdrhead: what the shared Function needs to know about it."""
+    name: str            # the public function, for messages
+    lib: str             # its C entry points cdr_<lib>_train_{workspace_bytes,forward,backward}
+    k: int               # kernel size
+    cin_dim: int         # the weight's Cin dimension: 0 for a transposed conv's (Cin, Cout, k, k), 1 for a conv's
+    has_bias: bool
+    out_hw: Callable     # (h, w, *extra int args) -> the output's (H, W)
+
+
+_DECONV = _TrainConvOp("conv_transpose2d", "deconv", 4, 0, False, lambda h, w: (2 * h, 2 * w))
+_CONV1X1 = _TrainConvOp("conv1x1", "conv1x1", 1, 1, True, lambda h, w: (h, w))
+_CONV3X3 = _TrainConvOp("conv3x3", "conv3x3", 3, 1, False, lambda h, w, s: (h // s, w // s))
+
+
+def _train_conv_args(op, x, weight, bias, extra):
+    """Checks of a training conv's inputs, all before any CUDA call: ValueError, there is no fallback.  The shape's
+    domain is the library's: cdr_<lib>_train_workspace_bytes decides it without a device, and its byte counts are the
+    ones the forward uses.  -> x, weight, bias, the C shape arguments, saved bytes, workspace bytes."""
     ts = (x, weight) if bias is None else (x, weight, bias)
     if not all(isinstance(t, torch.Tensor) for t in ts):
-        raise ValueError("conv1x1: x, weight and bias must be tensors")
-    if x.dim() != 4 or weight.dim() != 4 or tuple(weight.shape[2:]) != (1, 1) or weight.shape[1] != x.shape[1]:
-        raise ValueError(f"conv1x1: x (N, Cin, H, W) and weight (Cout, Cin, 1, 1) expected, got {tuple(x.shape)} and "
-                         f"{tuple(weight.shape)}")
+        raise ValueError(f"{op.name}: x, weight and bias must be tensors")
+    if x.dim() != 4 or weight.dim() != 4 or tuple(weight.shape[2:]) != (op.k, op.k) or \
+            weight.shape[op.cin_dim] != x.shape[1]:
+        layout = "Cin, Cout" if op.cin_dim == 0 else "Cout, Cin"
+        raise ValueError(f"{op.name}: x (N, Cin, H, W) and weight ({layout}, {op.k}, {op.k}) expected, got "
+                         f"{tuple(x.shape)} and {tuple(weight.shape)}")
     n, cin, h, w = x.shape
-    cout = weight.shape[0]
+    cout = weight.shape[1 - op.cin_dim]
     if bias is not None and tuple(bias.shape) != (cout,):
-        raise ValueError(f"conv1x1: bias of shape ({cout},) expected, got {tuple(bias.shape)}")
-    if not (n >= 1 and 1 <= cin <= 4096 and 1 <= cout <= 4096 and (h * w) % 64 == 0 and h * w > 0
-            and n * h * w <= 1 << 22):
-        raise ValueError(f"conv1x1: unsupported shape x {tuple(x.shape)}, weight {tuple(weight.shape)} "
-                         "(1 <= Cin, Cout <= 4096, H*W a multiple of 64, N*H*W <= 2^22)")
+        raise ValueError(f"{op.name}: bias of shape ({cout},) expected, got {tuple(bias.shape)}")
+    if not all(type(e) is int for e in extra):
+        raise ValueError(f"{op.name}: an int stride expected, got {extra[0]!r}")
+    L = _lib.lib()
+    dims = (n, cin, cout, h, w, *extra)
+    saved_b, ws_b = C.c_size_t(), C.c_size_t()
+    if getattr(L, f"cdr_{op.lib}_train_workspace_bytes")(*dims, C.byref(saved_b), C.byref(ws_b)):
+        raise ValueError(f"{op.name}: unsupported shape x {tuple(x.shape)}, weight {tuple(weight.shape)}"
+                         f"{''.join(f', stride {e!r}' for e in extra)} ({L.cdr_last_error().decode(errors='replace')})")
     if any(t.dtype != torch.float32 for t in ts):
-        raise ValueError(f"conv1x1: float32 expected, got {', '.join(str(t.dtype) for t in ts)}")
+        raise ValueError(f"{op.name}: float32 expected, got {', '.join(str(t.dtype) for t in ts)}")
     if not all(t.is_cuda and t.device == x.device for t in ts):
-        raise ValueError("conv1x1: x, weight and bias must be CUDA tensors on one device (there is no CPU fallback)")
-    return _aligned(x), _aligned(weight), None if bias is None else _aligned(bias)
+        raise ValueError(f"{op.name}: x, weight and bias must be CUDA tensors on one device (there is no CPU fallback)")
+    return (_aligned(x), _aligned(weight), None if bias is None else _aligned(bias), dims, saved_b.value,
+            ws_b.value)
 
 
-class _Conv1x1(torch.autograd.Function):
+class _TrainConv(torch.autograd.Function):
+    """conv_transpose2d, conv1x1 and conv3x3: forward and backward through the op's cdr_<lib>_train_* entry points.
+    extra: the int arguments that follow (n, cin, cout, h, w) in them (conv3x3's stride)."""
+
     @staticmethod
-    def forward(ctx, x, weight, bias):
-        x, weight, bias = _conv1x1_args(x, weight, bias)
-        n, cin, h, w = x.shape
-        cout = weight.shape[0]
+    def forward(ctx, op, x, weight, bias, *extra):
+        x, weight, bias, dims, saved_b, ws_b = _train_conv_args(op, x, weight, bias, extra)
+        n, _, cout, h, w = dims[:5]
         L = _lib.lib()
-        saved_b, ws_b = C.c_size_t(), C.c_size_t()
-        _lib.check(L.cdr_conv1x1_train_workspace_bytes(n, cin, cout, h, w, C.byref(saved_b), C.byref(ws_b)))
         dev = x.device
-        y = torch.empty((n, cout, h, w), dtype=torch.float32, device=dev)
-        saved = torch.empty(saved_b.value, dtype=torch.uint8, device=dev)     # x as fp16 planes, for the weight gradient
-        ws = torch.empty(ws_b.value, dtype=torch.uint8, device=dev)
+        y = torch.empty((n, cout, *op.out_hw(h, w, *extra)), dtype=torch.float32, device=dev)
+        saved = torch.empty(saved_b, dtype=torch.uint8, device=dev)     # x as fp16 planes, for the weight gradient
+        ws = torch.empty(ws_b, dtype=torch.uint8, device=dev)
+        b = (_lib.ptr(bias),) if op.has_bias else ()
         with torch.cuda.device(dev):
-            _lib.check(L.cdr_conv1x1_train_forward(_lib.ptr(x), _lib.ptr(weight), _lib.ptr(bias), n, cin, cout, h, w,
-                                                   _lib.ptr(y), _lib.ptr(saved), saved_b.value, _lib.ptr(ws), ws_b.value,
-                                                   _lib.current_stream_ptr(dev)))
+            _lib.check(getattr(L, f"cdr_{op.lib}_train_forward")(_lib.ptr(x), _lib.ptr(weight), *b, *dims, _lib.ptr(y),
+                                                                  _lib.ptr(saved), saved_b, _lib.ptr(ws), ws_b,
+                                                                  _lib.current_stream_ptr(dev)))
         ctx.save_for_backward(saved, weight)
-        ctx.dims = (n, cin, cout, h, w)
-        ctx.ws_bytes = ws_b.value
+        ctx.op, ctx.dims, ctx.ws_bytes = op, dims, ws_b
         return y
 
     @staticmethod
     @torch.autograd.function.once_differentiable
     def backward(ctx, grad_y):
         saved, weight = ctx.saved_tensors
-        n, cin, cout, h, w = ctx.dims
-        need_x, need_w, need_b = ctx.needs_input_grad[:3]
+        op, dims = ctx.op, ctx.dims
+        n, cin, cout, h, w = dims[:5]
+        need_x, need_w, need_b = ctx.needs_input_grad[1:4]
+        no_extra = (None,) * (len(dims) - 5)
         if not (need_x or need_w or need_b):
-            return None, None, None
-        dy = _aligned(_chk(grad_y, "conv1x1: grad"))
+            return (None, None, None, None, *no_extra)
+        dy = _aligned(_chk(grad_y, f"{op.name}: grad"))
         dev = dy.device
         dx = torch.empty((n, cin, h, w), dtype=torch.float32, device=dev) if need_x else None
-        dw = torch.empty((cout, cin, 1, 1), dtype=torch.float32, device=dev) if need_w else None
+        dw = torch.empty(weight.shape, dtype=torch.float32, device=dev) if need_w else None
         db = torch.empty((cout,), dtype=torch.float32, device=dev) if need_b else None
         ws = torch.empty(ctx.ws_bytes, dtype=torch.uint8, device=dev)
+        b = (_lib.ptr(db),) if op.has_bias else ()
         L = _lib.lib()
         with torch.cuda.device(dev):
-            _lib.check(L.cdr_conv1x1_train_backward(_lib.ptr(saved), _lib.ptr(weight), _lib.ptr(dy), n, cin, cout, h, w,
-                                                    _lib.ptr(dx), _lib.ptr(dw), _lib.ptr(db), _lib.ptr(ws), ctx.ws_bytes,
-                                                    _lib.current_stream_ptr(dev)))
-        return dx, dw, db
+            _lib.check(getattr(L, f"cdr_{op.lib}_train_backward")(_lib.ptr(saved), _lib.ptr(weight), _lib.ptr(dy), *dims,
+                                                                   _lib.ptr(dx), _lib.ptr(dw), *b, _lib.ptr(ws),
+                                                                   ctx.ws_bytes, _lib.current_stream_ptr(dev)))
+        return (None, dx, dw, db, *no_extra)
+
+
+def conv_transpose2d(x, weight):
+    """F.conv_transpose2d(x, weight, stride=2, padding=1) for 4x4 kernels without bias, forward and backward on
+    libcdrhead at fp32 accuracy.  x (N, Cin, H, W), weight (Cin, Cout, 4, 4): CUDA float32, Cin and Cout multiples
+    of 64, H == W in {8, 16, 32}; anything else raises ValueError."""
+    return _TrainConv.apply(_DECONV, x, weight, None)
 
 
 def conv1x1(x, weight, bias=None):
     """F.conv2d(x, weight, bias) for a (Cout, Cin, 1, 1) weight, forward and backward on libcdrhead at fp32 accuracy.
     x (N, Cin, H, W), bias (Cout) or None: CUDA float32, 1 <= Cin, Cout <= 4096, H*W a multiple of 64,
     N*H*W <= 2^22; anything else raises ValueError."""
-    return _Conv1x1.apply(x, weight, bias)
-
-
-def _conv3x3_args(x, weight, stride):
-    """Checks of conv3x3's inputs, all before any CUDA call: ValueError, there is no fallback."""
-    if not (isinstance(x, torch.Tensor) and isinstance(weight, torch.Tensor)):
-        raise ValueError("conv3x3: x and weight must be tensors")
-    if x.dim() != 4 or weight.dim() != 4 or tuple(weight.shape[2:]) != (3, 3) or weight.shape[1] != x.shape[1]:
-        raise ValueError(f"conv3x3: x (N, Cin, H, W) and weight (Cout, Cin, 3, 3) expected, got {tuple(x.shape)} and "
-                         f"{tuple(weight.shape)}")
-    n, cin, h, w = x.shape
-    cout = weight.shape[0]
-    ok = type(stride) is int and stride in (1, 2) and n >= 1 and all(64 <= c <= 2048 and c % 64 == 0 for c in (cin, cout))
-    ok = ok and h % stride == 0 and w % stride == 0
-    ho, wo = (h // stride, w // stride) if ok else (0, 0)
-    if not (ok and wo in (8, 16, 32, 64) and (ho * wo == 64 or (ho * wo) % 128 == 0) and n * ho * wo <= 1 << 22):
-        raise ValueError(f"conv3x3: unsupported shape x {tuple(x.shape)}, weight {tuple(weight.shape)}, stride {stride!r} "
-                         "(stride 1 or 2, Cin and Cout multiples of 64 in [64, 2048], H and W divisible by the stride; "
-                         "output W a power of two in [8, 64], output H*W = 64 or a multiple of 128, N*H*W <= 2^22)")
-    if x.dtype != torch.float32 or weight.dtype != torch.float32:
-        raise ValueError(f"conv3x3: float32 expected, got {x.dtype} and {weight.dtype}")
-    if not (x.is_cuda and weight.is_cuda) or x.device != weight.device:
-        raise ValueError("conv3x3: x and weight must be CUDA tensors on one device (there is no CPU fallback)")
-    return _aligned(x), _aligned(weight)
-
-
-class _Conv3x3(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, x, weight, stride):
-        x, weight = _conv3x3_args(x, weight, stride)
-        n, cin, h, w = x.shape
-        cout = weight.shape[0]
-        L = _lib.lib()
-        saved_b, ws_b = C.c_size_t(), C.c_size_t()
-        _lib.check(L.cdr_conv3x3_train_workspace_bytes(n, cin, cout, h, w, stride, C.byref(saved_b), C.byref(ws_b)))
-        dev = x.device
-        y = torch.empty((n, cout, h // stride, w // stride), dtype=torch.float32, device=dev)
-        saved = torch.empty(saved_b.value, dtype=torch.uint8, device=dev)     # x as fp16 planes, for the weight gradient
-        ws = torch.empty(ws_b.value, dtype=torch.uint8, device=dev)
-        with torch.cuda.device(dev):
-            _lib.check(L.cdr_conv3x3_train_forward(_lib.ptr(x), _lib.ptr(weight), n, cin, cout, h, w, stride,
-                                                   _lib.ptr(y), _lib.ptr(saved), saved_b.value, _lib.ptr(ws), ws_b.value,
-                                                   _lib.current_stream_ptr(dev)))
-        ctx.save_for_backward(saved, weight)
-        ctx.dims = (n, cin, cout, h, w, stride)
-        ctx.ws_bytes = ws_b.value
-        return y
-
-    @staticmethod
-    @torch.autograd.function.once_differentiable
-    def backward(ctx, grad_y):
-        saved, weight = ctx.saved_tensors
-        n, cin, cout, h, w, stride = ctx.dims
-        need_x, need_w = ctx.needs_input_grad[:2]
-        if not (need_x or need_w):
-            return None, None, None
-        dy = _aligned(_chk(grad_y, "conv3x3: grad"))
-        dev = dy.device
-        dx = torch.empty((n, cin, h, w), dtype=torch.float32, device=dev) if need_x else None
-        dw = torch.empty((cout, cin, 3, 3), dtype=torch.float32, device=dev) if need_w else None
-        ws = torch.empty(ctx.ws_bytes, dtype=torch.uint8, device=dev)
-        L = _lib.lib()
-        with torch.cuda.device(dev):
-            _lib.check(L.cdr_conv3x3_train_backward(_lib.ptr(saved), _lib.ptr(weight), _lib.ptr(dy), n, cin, cout, h, w,
-                                                    stride, _lib.ptr(dx), _lib.ptr(dw), _lib.ptr(ws), ctx.ws_bytes,
-                                                    _lib.current_stream_ptr(dev)))
-        return dx, dw, None
+    return _TrainConv.apply(_CONV1X1, x, weight, bias)
 
 
 def conv3x3(x, weight, stride=1):
@@ -362,4 +264,4 @@ def conv3x3(x, weight, stride=1):
     on libcdrhead at fp32 accuracy.  x (N, Cin, H, W): CUDA float32, stride 1 or 2, Cin and Cout multiples of 64 in
     [64, 2048], H and W divisible by the stride, the output's width a power of two in [8, 64], its H*W 64 or a multiple
     of 128 and N*H*W <= 2^22; anything else raises ValueError."""
-    return _Conv3x3.apply(x, weight, stride)
+    return _TrainConv.apply(_CONV3X3, x, weight, None, stride)

@@ -1,5 +1,6 @@
 // C ABI of libcdrhead.so: error state, packed-weight handles, workspace planning and the
 // orchestration of the head / decoder forward passes (include/cdrhead.h).
+#include <initializer_list>
 #include <new>
 #include <string.h>
 
@@ -658,7 +659,8 @@ extern "C" int cdr_joint_loss_backward(int kind, const float* pred, const float*
 }
 
 // ------------------------------------------------------------------------------------------
-// Training the decoder's transposed convolutions (gemm_tc.cu: tc_deconv_train_*)
+// Training convolutions (gemm_tc.cu: make_train_conv, tc_train_conv_*).  Each op keeps its own domain check and codes.
+// The decoder's transposed convolutions:
 static int deconv_train_shape(const char* fn, int n, int cin, int cout, int h, int w) {
   CDR_CHECK_ARG(n > 0 && cin > 0 && cout > 0 && h > 0 && w > 0, "%s: bad shape n=%d cin=%d cout=%d h=%d w=%d", fn, n, cin,
                 cout, h, w);
@@ -669,44 +671,7 @@ static int deconv_train_shape(const char* fn, int n, int cin, int cout, int h, i
   }
   return CDR_OK;
 }
-static bool al16(const void* p) { return ((uintptr_t)p & 15) == 0; }
-extern "C" int cdr_deconv_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes,
-                                                size_t* workspace_bytes) {
-  CDR_CHECK_ARG(saved_bytes && workspace_bytes, "cdr_deconv_train_workspace_bytes: null pointer");
-  if (int rc = deconv_train_shape("cdr_deconv_train_workspace_bytes", n, cin, cout, h, w)) return rc;
-  *saved_bytes = deconv_train_saved_bytes(n, cin, cout, h, w);
-  *workspace_bytes = deconv_train_workspace_bytes(n, cin, cout, h, w);
-  return CDR_OK;
-}
-extern "C" int cdr_deconv_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w,
-                                        float* y, void* saved, size_t saved_bytes, void* workspace,
-                                        size_t workspace_bytes, void* stream) {
-  CDR_CHECK_ARG(x && weight && y && saved && workspace, "cdr_deconv_train_forward: null pointer");
-  if (int rc = deconv_train_shape("cdr_deconv_train_forward", n, cin, cout, h, w)) return rc;
-  CDR_CHECK_ARG(al16(x) && al16(weight) && al16(y) && ((uintptr_t)saved & 255) == 0 && ((uintptr_t)workspace & 255) == 0,
-                "cdr_deconv_train_forward: tensors must be 16-byte, saved / workspace 256-byte aligned");
-  if (saved_bytes < deconv_train_saved_bytes(n, cin, cout, h, w)) {
-    set_error("cdr_deconv_train_forward: saved %zu < required %zu bytes", saved_bytes,
-              deconv_train_saved_bytes(n, cin, cout, h, w));
-    return CDR_ERR_WORKSPACE;
-  }
-  return tc_deconv_train_forward(x, weight, n, cin, cout, h, w, y, saved, workspace, workspace_bytes,
-                                 (cudaStream_t)stream);
-}
-extern "C" int cdr_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin,
-                                         int cout, int h, int w, float* dx, float* dweight, void* workspace,
-                                         size_t workspace_bytes, void* stream) {
-  CDR_CHECK_ARG(saved && weight && dy && workspace, "cdr_deconv_train_backward: null pointer");
-  if (int rc = deconv_train_shape("cdr_deconv_train_backward", n, cin, cout, h, w)) return rc;
-  CDR_CHECK_ARG(al16(weight) && al16(dy) && al16(dx) && al16(dweight) && ((uintptr_t)saved & 255) == 0 &&
-                    ((uintptr_t)workspace & 255) == 0,
-                "cdr_deconv_train_backward: tensors must be 16-byte, saved / workspace 256-byte aligned");
-  return tc_deconv_train_backward(saved, weight, dy, n, cin, cout, h, w, dx, dweight, workspace, workspace_bytes,
-                                  (cudaStream_t)stream);
-}
-
-// ------------------------------------------------------------------------------------------
-// Training 1x1 convolutions (gemm_tc.cu: tc_conv1x1_train_*)
+// 1x1 convolutions:
 static int conv1x1_train_shape(const char* fn, int n, int cin, int cout, int h, int w) {
   CDR_CHECK_ARG(n >= 1 && cin >= 1 && cin <= 4096 && cout >= 1 && cout <= 4096 && h >= 1 && w >= 1 &&
                     ((long long)h * w) % 64 == 0 && (long long)n * h * w <= (1LL << 22),
@@ -714,45 +679,8 @@ static int conv1x1_train_shape(const char* fn, int n, int cin, int cout, int h, 
                 "n*h*w <= 2^22)", fn, n, cin, cout, h, w);
   return CDR_OK;
 }
-extern "C" int cdr_conv1x1_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes,
-                                                 size_t* workspace_bytes) {
-  CDR_CHECK_ARG(saved_bytes && workspace_bytes, "cdr_conv1x1_train_workspace_bytes: null pointer");
-  if (int rc = conv1x1_train_shape("cdr_conv1x1_train_workspace_bytes", n, cin, cout, h, w)) return rc;
-  *saved_bytes = conv1x1_train_saved_bytes(n, cin, cout, h, w);
-  *workspace_bytes = conv1x1_train_workspace_bytes(n, cin, cout, h, w);
-  return CDR_OK;
-}
-extern "C" int cdr_conv1x1_train_forward(const float* x, const float* weight, const float* bias, int n, int cin,
-                                         int cout, int h, int w, float* y, void* saved, size_t saved_bytes,
-                                         void* workspace, size_t workspace_bytes, void* stream) {
-  CDR_CHECK_ARG(x && weight && y && saved && workspace, "cdr_conv1x1_train_forward: null pointer");
-  if (int rc = conv1x1_train_shape("cdr_conv1x1_train_forward", n, cin, cout, h, w)) return rc;
-  CDR_CHECK_ARG(al16(x) && al16(weight) && ((uintptr_t)bias & 3) == 0 && al16(y) && ((uintptr_t)saved & 255) == 0 &&
-                    ((uintptr_t)workspace & 255) == 0,
-                "cdr_conv1x1_train_forward: tensors must be 16-byte (bias 4-byte), saved / workspace 256-byte aligned");
-  if (saved_bytes < conv1x1_train_saved_bytes(n, cin, cout, h, w)) {
-    set_error("cdr_conv1x1_train_forward: saved %zu < required %zu bytes", saved_bytes,
-              conv1x1_train_saved_bytes(n, cin, cout, h, w));
-    return CDR_ERR_WORKSPACE;
-  }
-  return tc_conv1x1_train_forward(x, weight, bias, n, cin, cout, h, w, y, saved, workspace, workspace_bytes,
-                                  (cudaStream_t)stream);
-}
-extern "C" int cdr_conv1x1_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin,
-                                          int cout, int h, int w, float* dx, float* dweight, float* dbias,
-                                          void* workspace, size_t workspace_bytes, void* stream) {
-  CDR_CHECK_ARG(saved && weight && dy && workspace, "cdr_conv1x1_train_backward: null pointer");
-  if (int rc = conv1x1_train_shape("cdr_conv1x1_train_backward", n, cin, cout, h, w)) return rc;
-  CDR_CHECK_ARG(al16(weight) && al16(dy) && al16(dx) && al16(dweight) && ((uintptr_t)dbias & 3) == 0 &&
-                    ((uintptr_t)saved & 255) == 0 && ((uintptr_t)workspace & 255) == 0,
-                "cdr_conv1x1_train_backward: tensors must be 16-byte (dbias 4-byte), saved / workspace 256-byte aligned");
-  return tc_conv1x1_train_backward(saved, weight, dy, n, cin, cout, h, w, dx, dweight, dbias, workspace,
-                                   workspace_bytes, (cudaStream_t)stream);
-}
-
-// ------------------------------------------------------------------------------------------
-// Training 3x3 convolutions (gemm_tc.cu: tc_conv3x3_train_*).  h, w: the input map.  The output map's H*W must be 64 or
-// a multiple of 128: the tap-GEMM's 128-pixel tile is one 4-D box of whole rows (or of two whole 64-pixel images).
+// 3x3 convolutions.  h, w: the input map.  The output map's H*W must be 64 or a multiple of 128: the tap-GEMM's
+// 128-pixel tile is one 4-D box of whole rows (or of two whole 64-pixel images).
 static int conv3x3_train_shape(const char* fn, int n, int cin, int cout, int h, int w, int stride) {
   const bool s_ok = stride == 1 || stride == 2;
   const bool c_ok = cin >= 64 && cin <= 2048 && cin % 64 == 0 && cout >= 64 && cout <= 2048 && cout % 64 == 0;
@@ -765,37 +693,110 @@ static int conv3x3_train_shape(const char* fn, int n, int cin, int cout, int h, 
                 "multiple of 128, n*H*W <= 2^22)", fn, n, cin, cout, h, w, stride);
   return CDR_OK;
 }
+
+// What every cdr_<op>_train_* entry point checks, in this order: the pointers in `need` are not null, the shape is in
+// the op's domain, the tensors are 16-byte aligned (null allowed: an output not wanted), the bias 4-byte, saved and the
+// workspace 256-byte, and saved holds the forward's x planes (saved_bytes = SIZE_MAX: the backward, which has no size
+// to check).  On success *d describes the op.
+static int train_conv_args(const char* fn, int kind, int n, int cin, int cout, int h, int w, int stride,
+                           std::initializer_list<const void*> need, std::initializer_list<const void*> tensors,
+                           const void* bias, const void* saved, size_t saved_bytes, const void* workspace, TrainConv* d) {
+  for (const void* p : need) CDR_CHECK_ARG(p, "%s: null pointer", fn);
+  const int rc = kind == kTrainDeconv    ? deconv_train_shape(fn, n, cin, cout, h, w)
+                 : kind == kTrainConv1x1 ? conv1x1_train_shape(fn, n, cin, cout, h, w)
+                                         : conv3x3_train_shape(fn, n, cin, cout, h, w, stride);
+  if (rc) return rc;
+  bool aligned = ((uintptr_t)bias & 3) == 0 && ((uintptr_t)saved & 255) == 0 && ((uintptr_t)workspace & 255) == 0;
+  for (const void* p : tensors) aligned = aligned && ((uintptr_t)p & 15) == 0;
+  CDR_CHECK_ARG(aligned, "%s: tensors must be 16-byte%s, saved / workspace 256-byte aligned", fn,
+                kind == kTrainConv1x1 ? " (bias 4-byte)" : "");
+  *d = make_train_conv(kind, n, cin, cout, h, w, stride);
+  if (saved_bytes != SIZE_MAX && saved_bytes < train_conv_saved_bytes(*d)) {
+    set_error("%s: saved %zu < required %zu bytes", fn, saved_bytes, train_conv_saved_bytes(*d));
+    return CDR_ERR_WORKSPACE;
+  }
+  return CDR_OK;
+}
+static int train_conv_sizes(const char* fn, int kind, int n, int cin, int cout, int h, int w, int stride,
+                            size_t* saved_bytes, size_t* workspace_bytes) {
+  TrainConv d;
+  if (int rc = train_conv_args(fn, kind, n, cin, cout, h, w, stride, {saved_bytes, workspace_bytes}, {}, nullptr, nullptr,
+                               SIZE_MAX, nullptr, &d))
+    return rc;
+  *saved_bytes = train_conv_saved_bytes(d);
+  *workspace_bytes = train_conv_workspace_bytes(d);
+  return CDR_OK;
+}
+static int train_conv_forward(const char* fn, int kind, const float* x, const float* weight, const float* bias, int n,
+                              int cin, int cout, int h, int w, int stride, float* y, void* saved, size_t saved_bytes,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+  TrainConv d;
+  if (int rc = train_conv_args(fn, kind, n, cin, cout, h, w, stride, {x, weight, y, saved, workspace}, {x, weight, y},
+                               bias, saved, saved_bytes, workspace, &d))
+    return rc;
+  return tc_train_conv_forward(d, x, weight, bias, y, saved, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+static int train_conv_backward(const char* fn, int kind, const void* saved, const float* weight, const float* dy, int n,
+                               int cin, int cout, int h, int w, int stride, float* dx, float* dweight, float* dbias,
+                               void* workspace, size_t workspace_bytes, void* stream) {
+  TrainConv d;
+  if (int rc = train_conv_args(fn, kind, n, cin, cout, h, w, stride, {saved, weight, dy, workspace},
+                               {weight, dy, dx, dweight}, dbias, saved, SIZE_MAX, workspace, &d))
+    return rc;
+  return tc_train_conv_backward(d, saved, weight, dy, dx, dweight, dbias, workspace, workspace_bytes,
+                                (cudaStream_t)stream);
+}
+
+extern "C" int cdr_deconv_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes,
+                                                size_t* workspace_bytes) {
+  return train_conv_sizes("cdr_deconv_train_workspace_bytes", kTrainDeconv, n, cin, cout, h, w, 1, saved_bytes,
+                          workspace_bytes);
+}
+extern "C" int cdr_deconv_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w,
+                                        float* y, void* saved, size_t saved_bytes, void* workspace,
+                                        size_t workspace_bytes, void* stream) {
+  return train_conv_forward("cdr_deconv_train_forward", kTrainDeconv, x, weight, nullptr, n, cin, cout, h, w, 1, y, saved,
+                            saved_bytes, workspace, workspace_bytes, stream);
+}
+extern "C" int cdr_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin,
+                                         int cout, int h, int w, float* dx, float* dweight, void* workspace,
+                                         size_t workspace_bytes, void* stream) {
+  return train_conv_backward("cdr_deconv_train_backward", kTrainDeconv, saved, weight, dy, n, cin, cout, h, w, 1, dx,
+                             dweight, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int cdr_conv1x1_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes,
+                                                 size_t* workspace_bytes) {
+  return train_conv_sizes("cdr_conv1x1_train_workspace_bytes", kTrainConv1x1, n, cin, cout, h, w, 1, saved_bytes,
+                          workspace_bytes);
+}
+extern "C" int cdr_conv1x1_train_forward(const float* x, const float* weight, const float* bias, int n, int cin,
+                                         int cout, int h, int w, float* y, void* saved, size_t saved_bytes,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
+  return train_conv_forward("cdr_conv1x1_train_forward", kTrainConv1x1, x, weight, bias, n, cin, cout, h, w, 1, y, saved,
+                            saved_bytes, workspace, workspace_bytes, stream);
+}
+extern "C" int cdr_conv1x1_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin,
+                                          int cout, int h, int w, float* dx, float* dweight, float* dbias,
+                                          void* workspace, size_t workspace_bytes, void* stream) {
+  return train_conv_backward("cdr_conv1x1_train_backward", kTrainConv1x1, saved, weight, dy, n, cin, cout, h, w, 1, dx,
+                             dweight, dbias, workspace, workspace_bytes, stream);
+}
+
 extern "C" int cdr_conv3x3_train_workspace_bytes(int n, int cin, int cout, int h, int w, int stride, size_t* saved_bytes,
                                                  size_t* workspace_bytes) {
-  CDR_CHECK_ARG(saved_bytes && workspace_bytes, "cdr_conv3x3_train_workspace_bytes: null pointer");
-  if (int rc = conv3x3_train_shape("cdr_conv3x3_train_workspace_bytes", n, cin, cout, h, w, stride)) return rc;
-  *saved_bytes = conv3x3_train_saved_bytes(n, cin, cout, h, w, stride);
-  *workspace_bytes = conv3x3_train_workspace_bytes(n, cin, cout, h, w, stride);
-  return CDR_OK;
+  return train_conv_sizes("cdr_conv3x3_train_workspace_bytes", kTrainConv3x3, n, cin, cout, h, w, stride, saved_bytes,
+                          workspace_bytes);
 }
 extern "C" int cdr_conv3x3_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w,
                                          int stride, float* y, void* saved, size_t saved_bytes, void* workspace,
                                          size_t workspace_bytes, void* stream) {
-  CDR_CHECK_ARG(x && weight && y && saved && workspace, "cdr_conv3x3_train_forward: null pointer");
-  if (int rc = conv3x3_train_shape("cdr_conv3x3_train_forward", n, cin, cout, h, w, stride)) return rc;
-  CDR_CHECK_ARG(al16(x) && al16(weight) && al16(y) && ((uintptr_t)saved & 255) == 0 && ((uintptr_t)workspace & 255) == 0,
-                "cdr_conv3x3_train_forward: tensors must be 16-byte, saved / workspace 256-byte aligned");
-  if (saved_bytes < conv3x3_train_saved_bytes(n, cin, cout, h, w, stride)) {
-    set_error("cdr_conv3x3_train_forward: saved %zu < required %zu bytes", saved_bytes,
-              conv3x3_train_saved_bytes(n, cin, cout, h, w, stride));
-    return CDR_ERR_WORKSPACE;
-  }
-  return tc_conv3x3_train_forward(x, weight, n, cin, cout, h, w, stride, y, saved, workspace, workspace_bytes,
-                                  (cudaStream_t)stream);
+  return train_conv_forward("cdr_conv3x3_train_forward", kTrainConv3x3, x, weight, nullptr, n, cin, cout, h, w, stride, y,
+                            saved, saved_bytes, workspace, workspace_bytes, stream);
 }
 extern "C" int cdr_conv3x3_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin,
                                           int cout, int h, int w, int stride, float* dx, float* dweight, void* workspace,
                                           size_t workspace_bytes, void* stream) {
-  CDR_CHECK_ARG(saved && weight && dy && workspace, "cdr_conv3x3_train_backward: null pointer");
-  if (int rc = conv3x3_train_shape("cdr_conv3x3_train_backward", n, cin, cout, h, w, stride)) return rc;
-  CDR_CHECK_ARG(al16(weight) && al16(dy) && al16(dx) && al16(dweight) && ((uintptr_t)saved & 255) == 0 &&
-                    ((uintptr_t)workspace & 255) == 0,
-                "cdr_conv3x3_train_backward: tensors must be 16-byte, saved / workspace 256-byte aligned");
-  return tc_conv3x3_train_backward(saved, weight, dy, n, cin, cout, h, w, stride, dx, dweight, workspace,
-                                   workspace_bytes, (cudaStream_t)stream);
+  return train_conv_backward("cdr_conv3x3_train_backward", kTrainConv3x3, saved, weight, dy, n, cin, cout, h, w, stride,
+                             dx, dweight, nullptr, workspace, workspace_bytes, stream);
 }

@@ -2536,15 +2536,17 @@ int tc_set_debug(unsigned int* d) {
 }
 
 // ------------------------------------------------------------------------------------------
-// Training a ConvTranspose2d(k4, s2, p1, bias=False) at fp32 accuracy: forward, data and weight gradient on the f16x2
-// tap-GEMM (scaled fp16 hi/lo operands, 3 kind::f16 MMAs per product, main term drained every kSplitChunk K blocks).
-//   forward  y  = kTapDeconv (4 phases x 4 taps) over the x planes, weights packed unfolded per call, phase-scattered
-//               straight into NCHW fp32 (kOutPlanar + planar_deconv)
-//   dgrad    dx = kTapConv4s2 (16 taps, stride-2 box over the dy planes), B = [ci][tap*Cout + co], NCHW fp32 out
+// Training convolutions at fp32 accuracy: forward, data and weight gradient on the f16x2 tap-GEMM (scaled fp16 hi/lo
+// operands, 3 kind::f16 MMAs per product, main term drained every kSplitChunk K blocks).  Every op runs the same
+// steps; make_train_conv says how one maps onto them:
+//   forward  y  = one tap-GEMM over the x planes, the weight packed per call, planar epilogue straight into NCHW fp32
+//   dgrad    dx = one tap-GEMM over the dy planes, the weight packed per call as the data-gradient operand, NCHW fp32
 //   wgrad    dW = the kMN kernel: per tap a GEMM over the pixels, K split into slices -> fp32 partials ->
 //               wgrad_reduce_kernel (fixed slice order: bitwise deterministic, no atomics)
-// x and dy are encoded with ONE power-of-two scale per tensor (exact amax first): wgrad reduces over pixels, so per-pixel
-// scales would not factor out of its sums.  The x planes and their {amax, scale} slot are what the forward saves.
+//   dbias    db = bias_grad_kernel: a fixed-order fp64 sum over the pixels of every channel
+// x and dy are encoded with ONE power-of-two scale per tensor (exact amax first): wgrad reduces over pixels, so
+// per-pixel scales would not factor out of its sums.  The x planes and their {amax, scale} slot are what the forward
+// saves; the backward encodes dy once for both of its GEMMs.
 
 // wgrad K slices: powers of two while the `tiles` output tiles do not fill two waves of 148 SMs and a slice keeps >= 16 of
 // the `kb` K blocks.  A function of the shape only, so the summation order (and the result, bit for bit) does not depend
@@ -2554,40 +2556,106 @@ static int wgrad_slices(long long kb, long long tiles) {
   while (tiles * s < 2 * 148 && kb % (2 * s) == 0 && kb / (2 * s) >= 16) s *= 2;
   return s;
 }
-struct DtShape {
-  int n, cin, cout, h, w;
-  size_t x_rows() const { return (size_t)n * h * w; }
-  size_t dy_rows() const { return (size_t)n * 4 * h * w; }
-  int npo() const { return round_up(cout, 128); }     // forward: packed output channels per phase
-  int npi() const { return round_up(cin, 128); }      // dgrad: packed output channels
-  int slices() const { return wgrad_slices((long long)n * h * w / 64, (cin / 64 + 1) / 2 * ((cout / 64 + 1) / 2) * 16); }
-};
-struct DtWs {
-  TcLayer L;                 // forward: [4 phases][npo][4*cin]; backward: dgrad [npi][16*cout]
+
+template <int kDeconv, int kDeconvK = 4>
+static void pack_rows_f16(const CdrConvBn& cb, int nout, int cin, const TcLayer& L, cudaStream_t st) {
+  pack_rows_f16_kernel<kDeconv, kDeconvK><<<L.rows, 256, 0, st>>>(cb, nout, cin, L.k_pitch, L.n_pad, (__half*)L.w[0],
+                                                                  (__half*)L.w[1], L.wsi, L.bias, nullptr);
+}
+
+// per TrainConvKind: the entry points' op (cdr_<op>_train_*) and the forward / backward stage labels
+static const char* const kTrainConvNames[3][3] = {{"deconv", "deconv_train_fwd", "deconv_train_bwd"},
+                                                  {"conv1x1", "conv1x1_train_fwd", "conv1x1_train_bwd"},
+                                                  {"conv3x3", "conv3x3_train_fwd", "conv3x3_train_bwd"}};
+static size_t train_rows(const TrainConv& d, const TrainPlanes& p) { return (size_t)d.n * p.h * p.w; }
+static const TrainPlanes& wgrad_a(const TrainConv& d) { return d.wgrad_a_is_x ? d.x : d.dy; }
+static const TrainPlanes& wgrad_b(const TrainConv& d) { return d.wgrad_a_is_x ? d.dy : d.x; }
+
+// TrainGemm: {pack, k, bn, n_pad, groups, tap, stride, H, W, n}
+TrainConv make_train_conv(int kind, int n, int cin, int cout, int h, int w, int stride) {
+  TrainConv d{};
+  d.kind = kind;
+  d.n = n;
+  const int npi = round_up(cin, 128), npo = round_up(cout, 128);
+  switch (kind) {
+    case kTrainDeconv:
+      // ConvTranspose2d(k4, s2, p1, bias=False), x h x w -> y 2h x 2w
+      //   forward  kTapDeconv (4 phases x 4 taps), weights packed unfolded, phase-scattered (planar_deconv)
+      //   dgrad    kTapConv4s2 (16 taps, stride-2 box over the dy planes), B = [ci][tap*Cout + co]
+      //   wgrad    M = Cin (A = x), N = Cout (B = dy through the stride-2 box), 16 taps
+      d.x = {cin, h, w, cin};
+      d.dy = {cout, 2 * h, 2 * w, cout};
+      d.fwd = {pack_rows_f16<1>, 4 * cin, 128, npo, 4, kTapDeconv, 1, h, w, cout};
+      d.dgrad = {pack_rows_f16<-16>, 16 * cout, 128, npi, 1, kTapConv4s2, 2, h, w, cin};
+      d.wgrad_a_is_x = true; d.b_k = 4; d.b_stride = 2;
+      break;
+    case kTrainConv1x1: {
+      // 1x1 Conv2d(Cin, Cout, bias optional)
+      //   forward  kTapNone, weights (+ bias) packed per call
+      //   dgrad    kTapNone, B = W^T packed [ci][co] (dgrad_weight<1>)
+      //   wgrad    M = Cout (A = dy), N = Cin (B = x), both 2-D pixel-major maps, 1 tap
+      // Channel counts need not be multiples of 64: the x and dy planes are stored with a pitch of round_up(C, 64)
+      // whose pad columns the encoder writes as zeros, the packed weights' K pitch is zero-filled, and output channels
+      // past Cout / Cin are masked by the epilogue.  BN = 32 for at most 32 output channels.
+      const int pin = round_up(cin, 64), pout = round_up(cout, 64);
+      const int bn_o = cout <= 32 ? 32 : 128, bn_i = cin <= 32 ? 32 : 128;
+      d.x = {cin, h, w, pin};
+      d.dy = {cout, h, w, pout};
+      d.fwd = {pack_rows_f16<0>, pin, bn_o, round_up(cout, bn_o), 1, kTapNone, 1, h, w, cout};
+      d.dgrad = {pack_rows_f16<-1>, pout, bn_i, round_up(cin, bn_i), 1, kTapNone, 1, h, w, cin};
+      d.b_k = 1; d.b_stride = 1;
+      break;
+    }
+    default: {   // kTrainConv3x3
+      // 3x3 pad-1 Conv2d(Cin, Cout, stride s, bias=False), x h x w -> y h/s x w/s
+      //   forward  kTapConv3 (s = 2: the element-strided box), weights packed unfolded (pack_rows_f16_kernel<9>)
+      //   dgrad    s = 1: kTapConv3 over the dy planes, B = W^T with the taps flipped (dgrad_weight<9>)
+      //            s = 2: dx = conv_transpose2d(dy, W4, stride 2, pad 1) with W4 = W zero-padded to 4x4 at index 3:
+      //               the transposed-conv forward (kTapDeconv, planar_deconv) over the dy planes, W4 read by
+      //               deconv_weight<3>
+      //   wgrad    M = Cout (A = dy, a 2-D pixel map), N = Cin (B = x through the stride-s box shifted by
+      //               (kx - 1, ky - 1)), 9 taps
+      const int ho = h / stride, wo = w / stride;
+      d.x = {cin, h, w, cin};
+      d.dy = {cout, ho, wo, cout};
+      d.fwd = {pack_rows_f16<9>, 9 * cin, 128, npo, 1, kTapConv3, stride, ho, wo, cout};
+      d.dgrad = stride == 1 ? TrainGemm{pack_rows_f16<-9>, 9 * cout, 128, npi, 1, kTapConv3, 1, ho, wo, cin}
+                            : TrainGemm{pack_rows_f16<1, 3>, 4 * cout, 128, npi, 4, kTapDeconv, 1, ho, wo, cin};
+      d.b_k = 3; d.b_stride = stride;
+      break;
+    }
+  }
+  const TrainPlanes &a = wgrad_a(d), &b = wgrad_b(d);
+  const long long tiles = (long long)ceil_div(a.c, 128) * ceil_div(b.c, 128) * d.b_k * d.b_k;
+  d.slices = wgrad_slices((long long)train_rows(d, a) / 64, tiles);
+  return d;
+}
+
+struct TrainConvWs {
+  TcLayer L;                 // forward: the forward GEMM's packed weight; backward: the data gradient's
   void* dy_planes = nullptr; // backward: dy as an fp16 planes buffer [hi | lo | {amax, scale}]
-  float* part = nullptr;     // backward: wgrad partials [slice][tap][cin][npo]
+  float* part = nullptr;     // backward: wgrad partials [slice][tap][M][round_up(N, 128)]
   size_t bytes = 0;
 };
-static DtWs plan_deconv_train(void* base, const DtShape& d, bool backward) {
-  DtWs ws;
+static size_t train_planes_bytes(const TrainConv& d, const TrainPlanes& p) {
+  return 2 * planes_stride_bytes(train_rows(d, p), p.pitch) + 1024;
+}
+static TrainConvWs plan_train_conv(void* base, const TrainConv& d, bool backward) {
+  TrainConvWs ws;
   Bump1K b(base);
-  if (!backward) {
-    plan_layer(ws.L, b, kKindF16X2, 4 * d.npo(), 4 * d.cin, 4 * d.cin, 128, d.npo(), d.npo(), false);
-  } else {
-    plan_layer(ws.L, b, kKindF16X2, d.npi(), 16 * d.cout, 16 * d.cout, 128, d.npi(), d.npi(), false);
-    ws.dy_planes = b.take(2 * planes_stride_bytes(d.dy_rows(), d.cout) + 1024);
-    ws.part = (float*)b.take((size_t)d.slices() * 16 * d.cin * d.npo() * sizeof(float));
+  const TrainGemm& g = backward ? d.dgrad : d.fwd;
+  plan_layer(ws.L, b, kKindF16X2, g.groups * g.n_pad, g.k, g.k, g.bn, g.n_pad, g.n_pad, false);
+  if (backward) {
+    ws.dy_planes = b.take(train_planes_bytes(d, d.dy));
+    const size_t taps = (size_t)d.b_k * d.b_k;
+    ws.part = (float*)b.take(d.slices * taps * wgrad_a(d).c * round_up(wgrad_b(d).c, 128) * sizeof(float));
   }
   ws.bytes = b.off;
   return ws;
 }
-size_t deconv_train_saved_bytes(int n, int cin, int cout, int h, int w) {
-  const DtShape d{n, cin, cout, h, w};
-  return 2 * planes_stride_bytes(d.x_rows(), cin) + 1024;
-}
-size_t deconv_train_workspace_bytes(int n, int cin, int cout, int h, int w) {
-  const DtShape d{n, cin, cout, h, w};
-  const size_t f = plan_deconv_train(nullptr, d, false).bytes, bw = plan_deconv_train(nullptr, d, true).bytes;
+size_t train_conv_saved_bytes(const TrainConv& d) { return train_planes_bytes(d, d.x); }
+size_t train_conv_workspace_bytes(const TrainConv& d) {
+  const size_t f = plan_train_conv(nullptr, d, false).bytes, bw = plan_train_conv(nullptr, d, true).bytes;
   return f > bw ? f : bw;
 }
 
@@ -2599,33 +2667,40 @@ static int to_planes_tensor_scale(const float* in, int n, int c, int hw, int pit
   return launch_nchw_to_rows_f16p(in, nullptr, n, c, hw, a.p[0], a.p[1], pitch, sl.amax, sl.scale, st);
 }
 
-int tc_deconv_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, float* y,
-                            void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  const DtShape d{n, cin, cout, h, w};
-  DtWs ws = plan_deconv_train(workspace, d, false);
-  if (workspace_bytes < ws.bytes) {
-    set_error("cdr_deconv_train_forward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
-    return CDR_ERR_WORKSPACE;
-  }
-  set_stage("deconv_train_fwd");
-  ScaleSlot sx;
-  const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
-  if (int rc = to_planes_tensor_scale(x, n, cin, h * w, cin, xa, sx, st)) return rc;
+// One forward or data-gradient GEMM: pack the weight (and bias) into L, then the tap-GEMM over the planes `a` of `in`
+// into `out`, planar NCHW fp32
+static int train_gemm(const TrainConv& d, const TrainGemm& g, const TrainPlanes& in, const Act& a, ScaleSlot sa,
+                      const float* weight, const float* bias, TcLayer& L, float* out, cudaStream_t st) {
   CdrConvBn cb{};
   cb.weight = weight;
-  TcLayer& L = ws.L;
-  pack_rows_f16_kernel<1><<<L.rows, 256, 0, st>>>(cb, cout, cin, L.k_pitch, L.n_pad, (__half*)L.w[0],
-                                                        (__half*)L.w[1], L.wsi, L.bias, nullptr);
+  cb.bias = bias;
+  g.pack(cb, g.n, in.c, L, st);
   CDR_LAUNCH_OK("pack_rows_f16_kernel");
   if (int rc = layer_maps(L)) return rc;
   TcLaunch l{};
-  l.A = xa; l.a_pitch = cin;
-  l.n_img = n; l.H = h; l.W = w; l.cin = cin; l.deconv = 1; l.groups = 4;
-  l.a_rows_total = (long long)d.x_rows();
-  l.layer = &L; l.b_group_rows = L.n_pad; l.n = cout; l.bias_group_stride = 0;
-  l.C.p[0] = y; l.relu = 0; l.out_mode = kOutPlanar; l.planar_deconv = 1;
-  l.in_slot = sx;
-  const int rc = launch_tc(l, st);
+  l.A = a; l.a_pitch = in.pitch;
+  l.n_img = d.n; l.H = g.H; l.W = g.W; l.cin = in.pitch; l.stride = g.stride; l.groups = g.groups;
+  l.deconv = g.tap == kTapDeconv; l.conv3 = g.tap == kTapConv3; l.conv4s2 = g.tap == kTapConv4s2;
+  l.a_rows_total = (long long)train_rows(d, in);
+  l.layer = &L; l.b_group_rows = g.groups > 1 ? L.n_pad : 0; l.n = g.n; l.bias_group_stride = 0;
+  l.C.p[0] = out; l.relu = 0; l.out_mode = kOutPlanar; l.planar_deconv = g.tap == kTapDeconv;
+  l.in_slot = sa;
+  return launch_tc(l, st);
+}
+
+int tc_train_conv_forward(const TrainConv& d, const float* x, const float* weight, const float* bias, float* y,
+                          void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  TrainConvWs ws = plan_train_conv(workspace, d, false);
+  if (workspace_bytes < ws.bytes) {
+    set_error("cdr_%s_train_forward: workspace %zu < required %zu bytes", kTrainConvNames[d.kind][0], workspace_bytes,
+              ws.bytes);
+    return CDR_ERR_WORKSPACE;
+  }
+  set_stage(kTrainConvNames[d.kind][1]);
+  ScaleSlot sx;
+  const Act xa = planes_act(saved, train_rows(d, d.x), d.x.pitch, &sx);
+  if (int rc = to_planes_tensor_scale(x, d.n, d.x.c, d.x.h * d.x.w, d.x.pitch, xa, sx, st)) return rc;
+  const int rc = train_gemm(d, d.fwd, d.x, xa, sx, weight, bias, ws.L, y, st);
   set_stage(nullptr);
   return rc;
 }
@@ -2703,135 +2778,6 @@ static int launch_wgrad(int n, int h, int w, const Act& a, int m, int a_pitch, S
   return CDR_OK;
 }
 
-int tc_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
-                             int w, float* dx, float* dw, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  const DtShape d{n, cin, cout, h, w};
-  DtWs ws = plan_deconv_train(workspace, d, true);
-  if (workspace_bytes < ws.bytes) {
-    set_error("cdr_deconv_train_backward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
-    return CDR_ERR_WORKSPACE;
-  }
-  if (!dx && !dw) return CDR_OK;
-  set_stage("deconv_train_bwd");
-  ScaleSlot sd, sx;
-  const Act dya = planes_act(ws.dy_planes, d.dy_rows(), cout, &sd);     // one copy feeds both GEMMs
-  const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
-  if (int rc = to_planes_tensor_scale(dy, n, cout, 4 * h * w, cout, dya, sd, st)) return rc;
-  if (dx) {
-    CdrConvBn cb{};
-    cb.weight = weight;
-    TcLayer& L = ws.L;
-    pack_rows_f16_kernel<-16><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
-                                                           (__half*)L.w[1], L.wsi, L.bias, nullptr);
-    CDR_LAUNCH_OK("pack_rows_f16_kernel");
-    if (int rc = layer_maps(L)) return rc;
-    TcLaunch l{};
-    l.A = dya; l.a_pitch = cout;
-    l.n_img = n; l.H = h; l.W = w; l.cin = cout; l.conv4s2 = 1; l.stride = 2; l.groups = 1;
-    l.a_rows_total = (long long)d.dy_rows();
-    l.layer = &L; l.b_group_rows = 0; l.n = cin; l.bias_group_stride = 0;
-    l.C.p[0] = dx; l.relu = 0; l.out_mode = kOutPlanar;
-    l.in_slot = sd;
-    if (int rc = launch_tc(l, st)) return rc;
-  }
-  if (dw) {
-    if (int rc = launch_wgrad(n, h, w, xa, cin, cin, sx, dya, cout, cout, 4, 2, d.slices(), ws.part, st)) return rc;
-    const long long total = (long long)cin * cout * 16;
-    wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, d.slices(), 16, cin, cout,
-                                                                                   d.npo(), sx.scale, sd.scale, dw);
-    CDR_LAUNCH_OK("wgrad_reduce_kernel");
-  }
-  set_stage(nullptr);
-  return CDR_OK;
-}
-
-// ------------------------------------------------------------------------------------------
-// Training a 1x1 Conv2d(Cin, Cout, bias optional) at fp32 accuracy on the same f16x2 tap-GEMM:
-//   forward  y  = kTapNone over the x planes, weights (+ bias) packed per call, planar epilogue straight into NCHW fp32
-//   dgrad    dx = kTapNone over the dy planes, B = W^T packed [ci][co] (dgrad_weight<1>), planar NCHW fp32 out
-//   wgrad    dW = the kMN kernel with M = Cout (A = dy) and N = Cin (B = x), both 2-D pixel-major maps, K split into
-//               slices -> wgrad_reduce_kernel with 1 tap writes (Cout, Cin, 1, 1) directly
-//   dbias    db = bias_grad_kernel: a fixed-order fp64 sum over the pixels of every channel
-// Channel counts need not be multiples of 64: the x and dy planes are stored with a pitch of round_up(C, 64) whose pad
-// columns the encoder writes as zeros, the packed weights' K pitch is zero-filled, and output channels past Cout / Cin
-// are masked by the epilogue.  x and dy carry one power-of-two tensor scale each, as in the deconv op.
-struct C1Shape {
-  int n, cin, cout, h, w;
-  size_t rows() const { return (size_t)n * h * w; }
-  int pin() const { return round_up(cin, 64); }       // x planes pitch = forward K
-  int pout() const { return round_up(cout, 64); }     // dy planes pitch = dgrad K
-  static int bn(int c) { return c <= 32 ? 32 : 128; }
-  int slices() const { return wgrad_slices((long long)rows() / 64, (long long)ceil_div(cout, 128) * ceil_div(cin, 128)); }
-};
-struct C1Ws {
-  TcLayer L;                 // forward: [round_up(Cout, bn)][pin]; backward: dgrad [round_up(Cin, bn)][pout]
-  void* dy_planes = nullptr; // backward: dy as an fp16 planes buffer [hi | lo | {amax, scale}], pitch pout
-  float* part = nullptr;     // backward: wgrad partials [slice][cout][round_up(cin, 128)]
-  size_t bytes = 0;
-};
-static C1Ws plan_conv1x1_train(void* base, const C1Shape& d, bool backward) {
-  C1Ws ws;
-  Bump1K b(base);
-  if (!backward) {
-    const int bn = C1Shape::bn(d.cout), np = round_up(d.cout, bn);
-    plan_layer(ws.L, b, kKindF16X2, np, d.pin(), d.pin(), bn, np, np, false);
-  } else {
-    const int bn = C1Shape::bn(d.cin), np = round_up(d.cin, bn);
-    plan_layer(ws.L, b, kKindF16X2, np, d.pout(), d.pout(), bn, np, np, false);
-    ws.dy_planes = b.take(2 * planes_stride_bytes(d.rows(), d.pout()) + 1024);
-    ws.part = (float*)b.take((size_t)d.slices() * d.cout * round_up(d.cin, 128) * sizeof(float));
-  }
-  ws.bytes = b.off;
-  return ws;
-}
-size_t conv1x1_train_saved_bytes(int n, int cin, int cout, int h, int w) {
-  const C1Shape d{n, cin, cout, h, w};
-  return 2 * planes_stride_bytes(d.rows(), d.pin()) + 1024;
-}
-size_t conv1x1_train_workspace_bytes(int n, int cin, int cout, int h, int w) {
-  const C1Shape d{n, cin, cout, h, w};
-  const size_t f = plan_conv1x1_train(nullptr, d, false).bytes, bw = plan_conv1x1_train(nullptr, d, true).bytes;
-  return f > bw ? f : bw;
-}
-
-// one packed 1x1 GEMM over `rows` pixels of an fp16 planes buffer, planar fp32 NCHW output of `nout` channels
-static int conv1x1_gemm(const C1Shape& d, const Act& a, int k_pitch, ScaleSlot sa, const TcLayer& L, int nout, float* out,
-                        cudaStream_t st) {
-  TcLaunch l{};
-  l.A = a; l.a_pitch = k_pitch;
-  l.n_img = d.n; l.H = d.h; l.W = d.w; l.cin = k_pitch; l.groups = 1;
-  l.a_rows_total = (long long)d.rows();
-  l.layer = &L; l.b_group_rows = 0; l.n = nout; l.bias_group_stride = 0;
-  l.C.p[0] = out; l.relu = 0; l.out_mode = kOutPlanar;
-  l.in_slot = sa;
-  return launch_tc(l, st);
-}
-
-int tc_conv1x1_train_forward(const float* x, const float* weight, const float* bias, int n, int cin, int cout, int h,
-                             int w, float* y, void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  const C1Shape d{n, cin, cout, h, w};
-  C1Ws ws = plan_conv1x1_train(workspace, d, false);
-  if (workspace_bytes < ws.bytes) {
-    set_error("cdr_conv1x1_train_forward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
-    return CDR_ERR_WORKSPACE;
-  }
-  set_stage("conv1x1_train_fwd");
-  ScaleSlot sx;
-  const Act xa = planes_act(saved, d.rows(), d.pin(), &sx);
-  if (int rc = to_planes_tensor_scale(x, n, cin, h * w, d.pin(), xa, sx, st)) return rc;
-  CdrConvBn cb{};
-  cb.weight = weight;
-  cb.bias = bias;
-  TcLayer& L = ws.L;
-  pack_rows_f16_kernel<0><<<L.rows, 256, 0, st>>>(cb, cout, cin, L.k_pitch, L.n_pad, (__half*)L.w[0], (__half*)L.w[1],
-                                                  L.wsi, L.bias, nullptr);
-  CDR_LAUNCH_OK("pack_rows_f16_kernel");
-  if (int rc = layer_maps(L)) return rc;
-  const int rc = conv1x1_gemm(d, xa, d.pin(), sx, L, cout, y, st);
-  set_stage(nullptr);
-  return rc;
-}
-
 // db[c] = sum over images and pixels of dy[img][c][pixel]: one block per channel, float4 element j*256 + thread of the
 // channel's (image, pixel) sequence to that thread, fp64 partial sums, a fixed tree: bitwise deterministic, no atomics
 __global__ void __launch_bounds__(256)
@@ -2855,180 +2801,38 @@ bias_grad_kernel(const float* __restrict__ dy, int n, int c, int hw, float* __re
   if (threadIdx.x == 0) db[ch] = (float)red[0];
 }
 
-int tc_conv1x1_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
-                              int w, float* dx, float* dw, float* db, void* workspace, size_t workspace_bytes,
-                              cudaStream_t st) {
-  const C1Shape d{n, cin, cout, h, w};
-  C1Ws ws = plan_conv1x1_train(workspace, d, true);
+int tc_train_conv_backward(const TrainConv& d, const void* saved, const float* weight, const float* dy, float* dx,
+                           float* dw, float* db, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  TrainConvWs ws = plan_train_conv(workspace, d, true);
   if (workspace_bytes < ws.bytes) {
-    set_error("cdr_conv1x1_train_backward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
+    set_error("cdr_%s_train_backward: workspace %zu < required %zu bytes", kTrainConvNames[d.kind][0], workspace_bytes,
+              ws.bytes);
     return CDR_ERR_WORKSPACE;
   }
   if (!dx && !dw && !db) return CDR_OK;
-  set_stage("conv1x1_train_bwd");
+  set_stage(kTrainConvNames[d.kind][2]);
   if (db) {
-    bias_grad_kernel<<<cout, 256, 0, st>>>(dy, n, cout, h * w, db);
+    bias_grad_kernel<<<d.dy.c, 256, 0, st>>>(dy, d.n, d.dy.c, d.dy.h * d.dy.w, db);
     CDR_LAUNCH_OK("bias_grad_kernel");
   }
   if (dx || dw) {
     ScaleSlot sd, sx;
-    const Act dya = planes_act(ws.dy_planes, d.rows(), d.pout(), &sd);     // one copy feeds both GEMMs
-    const Act xa = planes_act(saved, d.rows(), d.pin(), &sx);
-    if (int rc = to_planes_tensor_scale(dy, n, cout, h * w, d.pout(), dya, sd, st)) return rc;
-    if (dx) {
-      CdrConvBn cb{};
-      cb.weight = weight;
-      TcLayer& L = ws.L;
-      pack_rows_f16_kernel<-1><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
-                                                       (__half*)L.w[1], L.wsi, L.bias, nullptr);
-      CDR_LAUNCH_OK("pack_rows_f16_kernel");
-      if (int rc = layer_maps(L)) return rc;
-      if (int rc = conv1x1_gemm(d, dya, d.pout(), sd, L, cin, dx, st)) return rc;
-    }
+    const Act dya = planes_act(ws.dy_planes, train_rows(d, d.dy), d.dy.pitch, &sd);     // one copy feeds both GEMMs
+    const Act xa = planes_act(saved, train_rows(d, d.x), d.x.pitch, &sx);
+    if (int rc = to_planes_tensor_scale(dy, d.n, d.dy.c, d.dy.h * d.dy.w, d.dy.pitch, dya, sd, st)) return rc;
+    if (dx)
+      if (int rc = train_gemm(d, d.dgrad, d.dy, dya, sd, weight, nullptr, ws.L, dx, st)) return rc;
     if (dw) {
-      const int slices = d.slices();
-      if (int rc = launch_wgrad(n, h, w, dya, cout, d.pout(), sd, xa, cin, d.pin(), 1, 1, slices, ws.part, st)) return rc;
-      const long long total = (long long)cout * cin;
-      wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, slices, 1, cout, cin,
-                                                                                     round_up(cin, 128), sx.scale,
-                                                                                     sd.scale, dw);
+      const bool ax = d.wgrad_a_is_x;
+      const TrainPlanes &a = wgrad_a(d), &b = wgrad_b(d);
+      if (int rc = launch_wgrad(d.n, a.h, a.w, ax ? xa : dya, a.c, a.pitch, ax ? sx : sd, ax ? dya : xa, b.c, b.pitch,
+                                d.b_k, d.b_stride, d.slices, ws.part, st))
+        return rc;
+      const long long total = (long long)a.c * b.c * d.b_k * d.b_k;
+      wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(
+          ws.part, d.slices, d.b_k * d.b_k, a.c, b.c, round_up(b.c, 128), sx.scale, sd.scale, dw);
       CDR_LAUNCH_OK("wgrad_reduce_kernel");
     }
-  }
-  set_stage(nullptr);
-  return CDR_OK;
-}
-
-// ------------------------------------------------------------------------------------------
-// Training a 3x3 pad-1 Conv2d(Cin, Cout, stride s, bias=False) at fp32 accuracy on the same f16x2 tap-GEMM.  h x w is
-// the input map, H x W = h/s x w/s the output.
-//   forward  y  = kTapConv3 over the x planes (s = 2: the element-strided box), weights packed unfolded per call
-//               (pack_rows_f16_kernel<9>), planar epilogue straight into NCHW fp32
-//   dgrad    s = 1: dx = kTapConv3 over the dy planes, B = W^T with the taps flipped (dgrad_weight<9>)
-//            s = 2: dx = conv_transpose2d(dy, W4, stride 2, pad 1) with W4 = W zero-padded to 4x4 at index 3: the
-//               transposed-conv forward (kTapDeconv, planar_deconv) over the dy planes, W4 read by deconv_weight<3>
-//   wgrad    dW = the kMN kernel with M = Cout (A = dy, a 2-D pixel map) and N = Cin (B = x through the stride-s box
-//               shifted by (kx - 1, ky - 1)), 9 taps, K split into slices -> wgrad_reduce_kernel writes (Cout, Cin, 3, 3)
-// Cin and Cout are multiples of 64, so the x and dy planes have pitch Cin and Cout.  One power-of-two tensor scale each.
-struct C3Shape {
-  int n, cin, cout, h, w, s;
-  int ho() const { return h / s; }
-  int wo() const { return w / s; }
-  size_t x_rows() const { return (size_t)n * h * w; }
-  size_t y_rows() const { return (size_t)n * ho() * wo(); }
-  int npo() const { return round_up(cout, 128); }     // forward: packed output channels
-  int npi() const { return round_up(cin, 128); }      // dgrad: packed output channels (per phase for s = 2)
-  int slices() const { return wgrad_slices((long long)y_rows() / 64, (long long)(npo() / 128) * (npi() / 128) * 9); }
-};
-struct C3Ws {
-  TcLayer L;                 // forward: [npo][9*cin]; backward: dgrad [npi][9*cout] (s = 1) or [4 phases][npi][4*cout]
-  void* dy_planes = nullptr; // backward: dy as an fp16 planes buffer [hi | lo | {amax, scale}]
-  float* part = nullptr;     // backward: wgrad partials [slice][tap][cout][npi]
-  size_t bytes = 0;
-};
-static C3Ws plan_conv3x3_train(void* base, const C3Shape& d, bool backward) {
-  C3Ws ws;
-  Bump1K b(base);
-  if (!backward) {
-    plan_layer(ws.L, b, kKindF16X2, d.npo(), 9 * d.cin, 9 * d.cin, 128, d.npo(), d.npo(), false);
-  } else {
-    if (d.s == 1) plan_layer(ws.L, b, kKindF16X2, d.npi(), 9 * d.cout, 9 * d.cout, 128, d.npi(), d.npi(), false);
-    else plan_layer(ws.L, b, kKindF16X2, 4 * d.npi(), 4 * d.cout, 4 * d.cout, 128, d.npi(), d.npi(), false);
-    ws.dy_planes = b.take(2 * planes_stride_bytes(d.y_rows(), d.cout) + 1024);
-    ws.part = (float*)b.take((size_t)d.slices() * 9 * d.cout * d.npi() * sizeof(float));
-  }
-  ws.bytes = b.off;
-  return ws;
-}
-size_t conv3x3_train_saved_bytes(int n, int cin, int cout, int h, int w, int stride) {
-  const C3Shape d{n, cin, cout, h, w, stride};
-  return 2 * planes_stride_bytes(d.x_rows(), cin) + 1024;
-}
-size_t conv3x3_train_workspace_bytes(int n, int cin, int cout, int h, int w, int stride) {
-  const C3Shape d{n, cin, cout, h, w, stride};
-  const size_t f = plan_conv3x3_train(nullptr, d, false).bytes, bw = plan_conv3x3_train(nullptr, d, true).bytes;
-  return f > bw ? f : bw;
-}
-
-int tc_conv3x3_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, int stride,
-                             float* y, void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  const C3Shape d{n, cin, cout, h, w, stride};
-  C3Ws ws = plan_conv3x3_train(workspace, d, false);
-  if (workspace_bytes < ws.bytes) {
-    set_error("cdr_conv3x3_train_forward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
-    return CDR_ERR_WORKSPACE;
-  }
-  set_stage("conv3x3_train_fwd");
-  ScaleSlot sx;
-  const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
-  if (int rc = to_planes_tensor_scale(x, n, cin, h * w, cin, xa, sx, st)) return rc;
-  CdrConvBn cb{};
-  cb.weight = weight;
-  TcLayer& L = ws.L;
-  pack_rows_f16_kernel<9><<<L.rows, 256, 0, st>>>(cb, cout, cin, L.k_pitch, L.n_pad, (__half*)L.w[0], (__half*)L.w[1],
-                                                  L.wsi, L.bias, nullptr);
-  CDR_LAUNCH_OK("pack_rows_f16_kernel");
-  if (int rc = layer_maps(L)) return rc;
-  TcLaunch l{};
-  l.A = xa; l.a_pitch = cin;
-  l.n_img = n; l.H = d.ho(); l.W = d.wo(); l.cin = cin; l.conv3 = 1; l.stride = stride; l.groups = 1;
-  l.a_rows_total = (long long)d.x_rows();
-  l.layer = &L; l.b_group_rows = 0; l.n = cout; l.bias_group_stride = 0;
-  l.C.p[0] = y; l.relu = 0; l.out_mode = kOutPlanar;
-  l.in_slot = sx;
-  const int rc = launch_tc(l, st);
-  set_stage(nullptr);
-  return rc;
-}
-
-int tc_conv3x3_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
-                              int w, int stride, float* dx, float* dw, void* workspace, size_t workspace_bytes,
-                              cudaStream_t st) {
-  const C3Shape d{n, cin, cout, h, w, stride};
-  C3Ws ws = plan_conv3x3_train(workspace, d, true);
-  if (workspace_bytes < ws.bytes) {
-    set_error("cdr_conv3x3_train_backward: workspace %zu < required %zu bytes", workspace_bytes, ws.bytes);
-    return CDR_ERR_WORKSPACE;
-  }
-  if (!dx && !dw) return CDR_OK;
-  set_stage("conv3x3_train_bwd");
-  const int ho = d.ho(), wo = d.wo();
-  ScaleSlot sd, sx;
-  const Act dya = planes_act(ws.dy_planes, d.y_rows(), cout, &sd);     // one copy feeds both GEMMs
-  const Act xa = planes_act(saved, d.x_rows(), cin, &sx);
-  if (int rc = to_planes_tensor_scale(dy, n, cout, ho * wo, cout, dya, sd, st)) return rc;
-  if (dx) {
-    CdrConvBn cb{};
-    cb.weight = weight;
-    TcLayer& L = ws.L;
-    TcLaunch l{};
-    l.A = dya; l.a_pitch = cout;
-    l.n_img = n; l.H = ho; l.W = wo; l.cin = cout;
-    l.a_rows_total = (long long)d.y_rows();
-    l.layer = &L; l.bias_group_stride = 0;
-    l.n = cin;
-    l.C.p[0] = dx; l.relu = 0; l.out_mode = kOutPlanar;
-    l.in_slot = sd;
-    if (stride == 1) {
-      pack_rows_f16_kernel<-9><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
-                                                       (__half*)L.w[1], L.wsi, L.bias, nullptr);
-      l.conv3 = 1; l.groups = 1; l.b_group_rows = 0;
-    } else {
-      pack_rows_f16_kernel<1, 3><<<L.rows, 256, 0, st>>>(cb, cin, cout, L.k_pitch, L.n_pad, (__half*)L.w[0],
-                                                         (__half*)L.w[1], L.wsi, L.bias, nullptr);
-      l.deconv = 1; l.groups = 4; l.b_group_rows = L.n_pad; l.planar_deconv = 1;
-    }
-    CDR_LAUNCH_OK("pack_rows_f16_kernel");
-    if (int rc = layer_maps(L)) return rc;
-    if (int rc = launch_tc(l, st)) return rc;
-  }
-  if (dw) {
-    const int slices = d.slices();
-    if (int rc = launch_wgrad(n, ho, wo, dya, cout, cout, sd, xa, cin, cin, 3, stride, slices, ws.part, st)) return rc;
-    const long long total = (long long)cout * cin * 9;
-    wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(ws.part, slices, 9, cout, cin, d.npi(),
-                                                                                   sx.scale, sd.scale, dw);
-    CDR_LAUNCH_OK("wgrad_reduce_kernel");
   }
   set_stage(nullptr);
   return CDR_OK;

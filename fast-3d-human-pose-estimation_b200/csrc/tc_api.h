@@ -40,30 +40,32 @@ int tc_encoder_out_shape(const void* enc, int h, int w, int* oh, int* ow, int* o
 int tc_encoder_forward(const void* enc, const void* x, int n, int h, int w, void* out_rows, void* workspace,
                        size_t workspace_bytes, cudaStream_t st);
 
-// Training a ConvTranspose2d(k4, s2, p1, bias=False) at fp32 accuracy (f16x2) — gemm_tc.cu
-size_t deconv_train_saved_bytes(int n, int cin, int cout, int h, int w);
-size_t deconv_train_workspace_bytes(int n, int cin, int cout, int h, int w);
-int tc_deconv_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, float* y,
-                            void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st);
-int tc_deconv_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
-                             int w, float* dx, float* dw, void* workspace, size_t workspace_bytes, cudaStream_t st);
-
-// Training a 1x1 Conv2d(Cin, Cout, bias optional) at fp32 accuracy (f16x2) — gemm_tc.cu
-size_t conv1x1_train_saved_bytes(int n, int cin, int cout, int h, int w);
-size_t conv1x1_train_workspace_bytes(int n, int cin, int cout, int h, int w);
-int tc_conv1x1_train_forward(const float* x, const float* weight, const float* bias, int n, int cin, int cout, int h,
-                             int w, float* y, void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st);
-int tc_conv1x1_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
-                              int w, float* dx, float* dw, float* db, void* workspace, size_t workspace_bytes,
-                              cudaStream_t st);
-
-// Training a 3x3 pad-1 Conv2d(Cin, Cout, stride 1 or 2, bias=False) at fp32 accuracy (f16x2) — gemm_tc.cu
-size_t conv3x3_train_saved_bytes(int n, int cin, int cout, int h, int w, int stride);
-size_t conv3x3_train_workspace_bytes(int n, int cin, int cout, int h, int w, int stride);
-int tc_conv3x3_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, int stride,
-                             float* y, void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st);
-int tc_conv3x3_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
-                              int w, int stride, float* dx, float* dw, void* workspace, size_t workspace_bytes,
-                              cudaStream_t st);
+// Training convolutions at fp32 accuracy (f16x2) — gemm_tc.cu.  make_train_conv is the only code that maps an op onto
+// the tap-GEMM; the planner, the size functions, the forward and the backward read the descriptor alone.
+enum TrainConvKind { kTrainDeconv, kTrainConv1x1, kTrainConv3x3 };
+struct TcLayer;
+struct TrainPlanes { int c, h, w, pitch; };   // x or dy as fp16 planes: c channels of an n x h x w map, rows `pitch` apart
+// the forward (A = the x planes) or data-gradient (A = the dy planes) GEMM; B = the weight packed per call by `pack`
+struct TrainGemm {
+  void (*pack)(const CdrConvBn& s, int nout, int cin, const TcLayer& L, cudaStream_t st);
+  int k, bn, n_pad, groups;  // packed layer: groups * n_pad rows of k (groups = 4: one per output phase of kTapDeconv)
+  int tap, stride, H, W, n;  // TapMode (gemm_tc.cu), A box stride, pixel grid (TcLaunch::H, W), output channels
+};
+struct TrainConv {
+  int kind, n;
+  TrainPlanes x, dy;
+  TrainGemm fwd, dgrad;
+  bool wgrad_a_is_x;         // wgrad A = x, B = dy (transposed conv) or A = dy, B = x (convs): the summation order
+  int b_k, b_stride;         // wgrad B through the stride-b_stride box, b_k x b_k taps (b_k = 1: a plain 2-D map)
+  int slices;                // wgrad K slices
+};
+// h, w: the input map; stride: the 3x3 conv's (1 or 2).  The shape must be in the op's domain.
+TrainConv make_train_conv(int kind, int n, int cin, int cout, int h, int w, int stride);
+size_t train_conv_saved_bytes(const TrainConv& d);
+size_t train_conv_workspace_bytes(const TrainConv& d);
+int tc_train_conv_forward(const TrainConv& d, const float* x, const float* weight, const float* bias, float* y,
+                          void* saved, void* workspace, size_t workspace_bytes, cudaStream_t st);
+int tc_train_conv_backward(const TrainConv& d, const void* saved, const float* weight, const float* dy, float* dx,
+                           float* dw, float* db, void* workspace, size_t workspace_bytes, cudaStream_t st);
 
 }  // namespace cdr

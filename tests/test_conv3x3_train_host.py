@@ -1,6 +1,7 @@
 """CPU: the argument checks of conv3x3 and of the cdr_conv3x3_train_* entry points, none of which may touch CUDA, the
 identities the library's stride-2 and dgrad paths rest on, and the pieces of test_gpu_conv3x3_train.py that need no GPU:
-its shape table against the wgrad slice plan, and the strictness of its per-element gate."""
+its shape table against the wgrad slice plan, and the strictness of the
+per-element gate it shares with the other training convolutions (train_conv_checks.py)."""
 import ctypes as C
 import importlib.util
 import os
@@ -9,9 +10,11 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from train_conv_checks import GATE_C, f16_planes, gate
+
 
 def _domain():
-    """tests/test_gpu_conv3x3_train.py (its shape table, slice mirror and gate), imported without a GPU."""
+    """tests/test_gpu_conv3x3_train.py (its shape table and slice mirror), imported without a GPU."""
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "test_gpu_conv3x3_train.py")
     spec = importlib.util.spec_from_file_location("_conv3x3_train_domain", path)
     mod = importlib.util.module_from_spec(spec)
@@ -81,32 +84,19 @@ def test_stride2_and_dgrad_identities_in_fp64():
                                atol=0)
 
 
-def _f16_planes(t, keep_lo):
-    """fp64 emulation of the scaled fp16 planes of a tensor (layout.cu: nchw_to_rows_f16p): s = 2^min(13 - ilogb(amax),
-    127), hi = rn_f16(x s), lo = rn_f16((x s - hi) 2^11); decoded as (hi + lo 2^-11) / s, or hi / s alone."""
-    _, e = torch.frexp(t.abs().max())
-    s = 2.0 ** min(13 - (int(e) - 1), 127)
-    X = t * s
-    hi = X.half().double()
-    if not keep_lo:
-        return hi / s
-    return (hi + ((X - hi) * 2048).half().double() / 2048) / s
-
-
 @pytest.mark.parametrize("s", [1, 2])
 def test_per_element_gate_catches_a_lost_lo_plane(s):
     """With x through both planes the forward passes the per-element gate; with the hi plane alone (~2^-12 m) it
     fails.  So the gate's constant is tight enough to see the lo plane."""
-    D = _domain()
-    assert D.GATE_C <= 2.0 ** -14
+    assert GATE_C <= 2.0 ** -14
     g = torch.Generator().manual_seed(0)
     x = torch.randn((2, 64, 16, 16), generator=g).double()        # fp32 values, held in fp64
     w = torch.randn((64, 64, 3, 3), generator=g).float().double()
     ref = F.conv2d(x, w, stride=s, padding=1)
     mag = F.conv2d(x.abs(), w.abs(), stride=s, padding=1)
-    D.gate("y", F.conv2d(_f16_planes(x, True), _f16_planes(w, True), stride=s, padding=1), ref, mag)
+    gate("y", F.conv2d(f16_planes(x, True), f16_planes(w, True), stride=s, padding=1), ref, mag)
     with pytest.raises(AssertionError, match="per-element gate"):
-        D.gate("y", F.conv2d(_f16_planes(x, False), _f16_planes(w, True), stride=s, padding=1), ref, mag,
+        gate("y", F.conv2d(f16_planes(x, False), f16_planes(w, True), stride=s, padding=1), ref, mag,
                max_gate=False)
 
 

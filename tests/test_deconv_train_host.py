@@ -1,7 +1,8 @@
 """CPU: the index algebra the transposed-convolution training kernels implement (gemm_tc.cu: kTapConv4s2 and the
 MN-major weight-gradient tiles), in fp64 against torch autograd, and the argument checks of conv_transpose2d and of
 the cdr_deconv_train_* entry points, none of which may touch CUDA.  Also the pieces of test_gpu_deconv_train_domain.py
-that need no GPU: its shape table against the wgrad slice plan, and the strictness of its per-element gate."""
+that need no GPU: its shape table against the wgrad slice plan, and the strictness of the
+per-element gate it shares with the other training convolutions (train_conv_checks.py)."""
 import ctypes as C
 import importlib.util
 import os
@@ -9,6 +10,8 @@ import os
 import pytest
 import torch
 import torch.nn.functional as F
+
+from train_conv_checks import GATE_C, f16_planes, gate
 
 
 def _shifted(t, dy, dx, h, w):
@@ -65,7 +68,7 @@ def test_wgrad_is_16_per_tap_pixel_reductions(problem):
 
 
 def _domain():
-    """tests/test_gpu_deconv_train_domain.py (its shape table, slice mirror and gate), imported without a GPU."""
+    """tests/test_gpu_deconv_train_domain.py (its shape table and slice mirror), imported without a GPU."""
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "test_gpu_deconv_train_domain.py")
     spec = importlib.util.spec_from_file_location("_deconv_train_domain", path)
     mod = importlib.util.module_from_spec(spec)
@@ -98,31 +101,18 @@ def test_slice_mirror_fits_the_reported_workspace(pkg):
         assert w.value >= sl * 16 * cin * (cout + 127) // 128 * 128 * 4
 
 
-def _f16_planes(t, keep_lo):
-    """fp64 emulation of the scaled fp16 planes of a tensor (layout.cu: nchw_to_rows_f16p): s = 2^min(13 - ilogb(amax),
-    127), hi = rn_f16(x s), lo = rn_f16((x s - hi) 2^11); decoded as (hi + lo 2^-11) / s, or hi / s alone."""
-    _, e = torch.frexp(t.abs().max())
-    s = 2.0 ** min(13 - (int(e) - 1), 127)
-    X = t * s
-    hi = X.half().double()
-    if not keep_lo:
-        return hi / s
-    return (hi + ((X - hi) * 2048).half().double() / 2048) / s
-
-
 def test_per_element_gate_catches_a_lost_lo_plane():
     """With x through both planes the forward passes the per-element gate; with the hi plane alone (~2^-12 m) it
     fails.  So the gate's constant is tight enough to see the lo plane, and c <= 2^-14."""
-    D = _domain()
-    assert D.GATE_C <= 2.0 ** -14
+    assert GATE_C <= 2.0 ** -14
     g = torch.Generator().manual_seed(0)
     x = torch.randn((1, 4, 8, 8), generator=g).double()          # fp32 values, held in fp64
     w = torch.randn((4, 3, 4, 4), generator=g).float().double()
     ref = F.conv_transpose2d(x, w, stride=2, padding=1)
     mag = F.conv_transpose2d(x.abs(), w.abs(), stride=2, padding=1)
-    D.gate("y", F.conv_transpose2d(_f16_planes(x, True), w, stride=2, padding=1), ref, mag)
+    gate("y", F.conv_transpose2d(f16_planes(x, True), w, stride=2, padding=1), ref, mag)
     with pytest.raises(AssertionError, match="per-element gate"):
-        D.gate("y", F.conv_transpose2d(_f16_planes(x, False), w, stride=2, padding=1), ref, mag, max_gate=False)
+        gate("y", F.conv_transpose2d(f16_planes(x, False), w, stride=2, padding=1), ref, mag, max_gate=False)
 
 
 def test_conv_transpose2d_rejects_without_cuda(pkg, monkeypatch):

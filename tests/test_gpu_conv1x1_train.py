@@ -5,31 +5,21 @@ outside O(1), the memory contract of the cdr_conv1x1_train_* entry points, layou
 inputs, and forward_train on it."""
 import copy
 import ctypes as C
+import functools
 
 import pytest
 import torch
 import torch.nn.functional as F
 
+import train_conv_checks as checks
 from fast_3d_human_pose_estimation_b200 import synth
+from train_conv_checks import GATE_C, SENTINEL, TINY, Region, bits_equal, f32_region, graph_replay, on_side_stream
 
 pytestmark = pytest.mark.gpu
 
-GATE_MAX = 2e-5          # max error / max |reference|, as for conv_transpose2d
-# Per element: |got - ref| <= GATE_C * m + 2^-126, m = the same sum over |operands|: sum |x||w| + |b| for y, |dy||w|
-# for dx, |x||dy| for dW, |dy| for db (test_gpu_deconv_train_domain.py uses the same gate).  Losing the lo plane of an
-# fp16 hi/lo operand costs ~2^-12 (test_conv1x1_train_host.py shows this gate catches it).
-GATE_C = 2.0 ** -18
-TINY = 2.0 ** -126
-
-
 def slices(n, cin, cout, h, w):
-    """Python mirror of C1Shape::slices() in csrc/gemm_tc.cu (wgrad_slices over Cout x Cin tiles of 128)."""
-    kb = n * h * w // 64
-    tiles = -(-cout // 128) * -(-cin // 128)
-    s = 1
-    while tiles * s < 2 * 148 and kb % (2 * s) == 0 and kb // (2 * s) >= 16:
-        s *= 2
-    return s
+    """The number of K slices of the weight gradient: M = Cout over the pixels, N = Cin, 1 tap."""
+    return checks.wgrad_slices(n * h * w, cout, cin, 1)
 
 
 # (N, Cin, Cout, H, W, bias): the head's layers at the default widths (fusion_hid_ch1 = 300)
@@ -60,12 +50,8 @@ TABLE = [
 ]
 
 WORST = {"y": 0.0, "dx": 0.0, "dw": 0.0, "db": 0.0}
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _report_worst():
-    yield
-    print(f"\nworst per-element error / m over {__name__}: " + ", ".join(f"{k} {v:.3e}" for k, v in WORST.items()))
+_report_worst = checks.report_worst(WORST, __name__)
+gate = functools.partial(checks.gate, worst=WORST)
 
 
 def inputs(n, cin, cout, h, w, seed=0, ex=0, ew=0, edy=0, bias=True):
@@ -98,27 +84,6 @@ def reference(x, w, b, dy):
         dx64, dw64 = torch.autograd.grad(y64, (x64, w64), dy64)
         out.append((y64.detach(), dx64, dw64, dy64.sum((0, 2, 3))))
     return out
-
-
-def gate(name, got, ref, mag, max_gate=True):
-    """Per-element gate on every element finite in ref; every non-finite element of ref non-finite in got."""
-    got = got.detach().double()
-    assert got.shape == ref.shape, name
-    fin = torch.isfinite(ref)
-    assert not bool(torch.isfinite(got[~fin]).any()), f"{name}: finite where the reference is not"
-    got, ref, mag = got[fin], ref[fin], mag[fin]
-    err = (got - ref).abs()
-    ok = err <= GATE_C * mag + TINY                        # NaN fails
-    if not bool(ok.all()):
-        i = int((~ok).nonzero()[0])
-        raise AssertionError(f"{name}: {int((~ok).sum())} of {ok.numel()} elements outside the per-element gate, "
-                             f"first: got {float(got[i])!r} ref {float(ref[i])!r} m {float(mag[i])!r}")
-    ratio = float(((err - TINY).clamp_min(0) / mag.clamp_min(1e-300)).max()) if err.numel() else 0.0
-    WORST[name] = max(WORST[name], ratio)
-    rel = float(err.max() / ref.abs().max().clamp_min(1e-300)) if err.numel() else 0.0
-    if max_gate:
-        assert rel <= GATE_MAX, (name, rel)
-    return ratio, rel
 
 
 def check_all(pkg, x, w, b, dy, label, max_gate=True):
@@ -178,42 +143,6 @@ def test_subnormal_input(cuda_pkg, n, cin, cout, h, w):
 
 
 # ---- memory contract of the C ABI: exact byte counts, guard bytes around every buffer, stale workspace contents ----
-GUARD = 4096
-SENTINEL = 0x5A
-
-
-class Region:
-    """`nbytes` inside a larger uint8 buffer: GUARD sentinel bytes on each side, the interior filled with `fill`
-    (a byte value, "random", or None for the sentinel)."""
-
-    def __init__(self, nbytes, fill=None, gen=None):
-        self.nbytes = nbytes
-        self.buf = torch.full((GUARD + nbytes + GUARD,), SENTINEL, dtype=torch.uint8, device="cuda")
-        if fill == "random":
-            self.inner.copy_(torch.randint(0, 256, (nbytes,), dtype=torch.uint8, device="cuda", generator=gen))
-        elif fill is not None:
-            self.inner.fill_(fill)
-        assert self.buf.data_ptr() % 256 == 0
-
-    @property
-    def inner(self):
-        return self.buf[GUARD:GUARD + self.nbytes]
-
-    def f32(self, shape):
-        return self.inner.view(torch.float32).view(shape)
-
-    def guards_intact(self):
-        return bool((self.buf[:GUARD] == SENTINEL).all()) and bool((self.buf[GUARD + self.nbytes:] == SENTINEL).all())
-
-
-def _f32_region(shape):
-    n = 1
-    for d in shape:
-        n *= d
-    r = Region(4 * n)
-    return r, r.f32(shape)
-
-
 def _abi_run(pkg, x, w, b, dy, fill, gen):
     """forward, then full, dx-only, dW-only and db-only backward through the C ABI, every buffer guarded."""
     L = pkg._lib.lib()
@@ -224,15 +153,15 @@ def _abi_run(pkg, x, w, b, dy, fill, gen):
     st = pkg._lib.current_stream_ptr()
     ptr = pkg._lib.ptr
     saved, ws = Region(sb.value, fill, gen), Region(wb.value, fill, gen)
-    ry, y = _f32_region((n, cout, h, wd))
+    ry, y = f32_region((n, cout, h, wd))
     pkg._lib.check(L.cdr_conv1x1_train_forward(ptr(x), ptr(w), ptr(b), n, cin, cout, h, wd, ptr(y), ptr(saved.inner),
                                                sb.value, ptr(ws.inner), wb.value, st))
     regions, outs = [saved, ws, ry], {"y": y}
     for tag, want in (("", "xwb"), ("_xonly", "x"), ("_wonly", "w"), ("_bonly", "b")):
         ws_b = Region(wb.value, fill, gen)
-        rdx, dx = _f32_region((n, cin, h, wd)) if "x" in want else (None, None)
-        rdw, dw = _f32_region((cout, cin, 1, 1)) if "w" in want else (None, None)
-        rdb, db = _f32_region((cout,)) if "b" in want else (None, None)
+        rdx, dx = f32_region((n, cin, h, wd)) if "x" in want else (None, None)
+        rdw, dw = f32_region((cout, cin, 1, 1)) if "w" in want else (None, None)
+        rdb, db = f32_region((cout,)) if "b" in want else (None, None)
         pkg._lib.check(L.cdr_conv1x1_train_backward(ptr(saved.inner), ptr(w), ptr(dy), n, cin, cout, h, wd, ptr(dx),
                                                     ptr(dw), ptr(db), ptr(ws_b.inner), wb.value, st))
         regions += [r for r in (ws_b, rdx, rdw, rdb) if r is not None]
@@ -245,10 +174,6 @@ def _abi_run(pkg, x, w, b, dy, fill, gen):
     return {k: t.clone() for k, t in outs.items()}
 
 
-def _bits_equal(a, b):
-    return a.shape == b.shape and torch.equal(a.view(torch.int32), b.view(torch.int32))
-
-
 @pytest.mark.parametrize("n,cin,cout,h,w", [(1, 1, 1, 8, 8), (3, 65, 127, 8, 8), (2, 300, 19, 16, 16),
                                             (4, 127, 300, 8, 8)])
 def test_memory_contract(cuda_pkg, n, cin, cout, h, w):
@@ -256,12 +181,12 @@ def test_memory_contract(cuda_pkg, n, cin, cout, h, w):
     gen = torch.Generator(device="cuda").manual_seed(12)
     runs = [_abi_run(cuda_pkg, x, wt, b, dy, fill, gen) for fill in (0x00, 0xFF, "random")]
     for k in runs[0]:
-        assert all(_bits_equal(runs[0][k], r[k]) for r in runs[1:]), f"{k} depends on stale workspace contents"
+        assert all(bits_equal(runs[0][k], r[k]) for r in runs[1:]), f"{k} depends on stale workspace contents"
     a = runs[0]
-    assert _bits_equal(a["dx_xonly"], a["dx"]) and _bits_equal(a["dw_wonly"], a["dw"])
-    assert _bits_equal(a["db_bonly"], a["db"])
+    assert bits_equal(a["dx_xonly"], a["dx"]) and bits_equal(a["dw_wonly"], a["dw"])
+    assert bits_equal(a["db_bonly"], a["db"])
     got = ours(cuda_pkg, x, wt, b, dy)                   # the autograd op is the same computation
-    assert all(_bits_equal(g, a[k]) for g, k in zip(got, ("y", "dx", "dw", "db")))
+    assert all(bits_equal(g, a[k]) for g, k in zip(got, ("y", "dx", "dw", "db")))
     ref, mag = reference(x, wt, b, dy)
     for i, k in enumerate(("y", "dx", "dw", "db")):
         gate(k, a[k], ref[i], mag[i])
@@ -272,7 +197,7 @@ def test_needs_input_grad_each_alone(cuda_pkg):
     full = ours(cuda_pkg, x, w, b, dy)
     for i, need in enumerate(((True, False, False), (False, True, False), (False, False, True))):
         (g,) = ours(cuda_pkg, x, w, b, dy, need)[1:]
-        assert _bits_equal(g, full[1 + i])
+        assert bits_equal(g, full[1 + i])
 
 
 # ---- layouts, streams, CUDA graphs, repeated backward ----
@@ -290,18 +215,14 @@ def test_layouts_give_the_same_bits(cuda_pkg):
     assert not x_nc.is_contiguous()
     for xs, ws, bs, dys in ((x_cl, w_cl, b_nc, dy_cl), (x_nc, w, b, dy)):
         got = ours(cuda_pkg, xs, ws, bs, dys)
-        assert all(_bits_equal(a.contiguous(), g.contiguous()) for a, g in zip(base, got))
+        assert all(bits_equal(a.contiguous(), g.contiguous()) for a, g in zip(base, got))
 
 
 def test_side_stream_gives_the_same_bits(cuda_pkg):
     x, w, b, dy = inputs(*LAYOUT_SHAPE, seed=22)
     base = ours(cuda_pkg, x, w, b, dy)
-    s = torch.cuda.Stream()
-    s.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(s):
-        got = ours(cuda_pkg, x, w, b, dy)
-    torch.cuda.current_stream().wait_stream(s)
-    assert all(_bits_equal(a, g) for a, g in zip(base, got))
+    got = on_side_stream(ours, cuda_pkg, x, w, b, dy)
+    assert all(bits_equal(a, g) for a, g in zip(base, got))
 
 
 def test_cuda_graph_replay_equals_eager(cuda_pkg):
@@ -312,21 +233,10 @@ def test_cuda_graph_replay_equals_eager(cuda_pkg):
     def step():
         y = cuda_pkg.conv1x1(sx, sw, sb)
         return (y.detach(), *torch.autograd.grad(y, (sx, sw, sb), sdy))
-    s = torch.cuda.Stream()
-    s.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(s):
-        step()                                         # warm-up outside the capture
-    torch.cuda.current_stream().wait_stream(s)
-    g = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(g):
-        static_out = step()
     x2, w2, b2, dy2 = inputs(*LAYOUT_SHAPE, seed=24)
-    with torch.no_grad():
-        sx.copy_(x2), sw.copy_(w2), sb.copy_(b2), sdy.copy_(dy2)
-    g.replay()
-    torch.cuda.synchronize()
+    static_out = graph_replay(step, (sx, sw, sb, sdy), (x2, w2, b2, dy2))
     eager = ours(cuda_pkg, x2, w2, b2, dy2)
-    assert all(_bits_equal(a, e) for a, e in zip(static_out, eager))
+    assert all(bits_equal(a, e) for a, e in zip(static_out, eager))
 
 
 def test_two_backward_calls_and_zero_dy(cuda_pkg):
@@ -338,7 +248,7 @@ def test_two_backward_calls_and_zero_dy(cuda_pkg):
     dy = torch.randn_like(y)
     first = torch.autograd.grad(y, (x, w, b), dy, retain_graph=True)
     second = torch.autograd.grad(y, (x, w, b), dy)
-    assert all(_bits_equal(a, c) for a, c in zip(first, second))
+    assert all(bits_equal(a, c) for a, c in zip(first, second))
 
 
 # ---- non-finite inputs: a diverging run is never reported finite ----

@@ -5,32 +5,22 @@ cdr_conv3x3_train_* entry points, layouts, streams, CUDA graphs, non-finite inpu
 encoder's Bottleneck blocks on it."""
 import copy
 import ctypes as C
+import functools
 
 import pytest
 import torch
 import torch.nn.functional as F
 
+import train_conv_checks as checks
 from fast_3d_human_pose_estimation_b200 import synth
+from train_conv_checks import SENTINEL, Region, bits_equal, f32_region, graph_replay, on_side_stream
 
 pytestmark = pytest.mark.gpu
 
-GATE_MAX = 2e-5          # max error / max |reference|, as for conv_transpose2d and conv1x1
-# Per element: |got - ref| <= GATE_C * m + 2^-126, m = the same sum over |operands|: sum |x||w| for y, |dy||w| for dx,
-# |x||dy| for dW.  Losing the lo plane of an fp16 hi/lo operand costs ~2^-12 (test_conv3x3_train_host.py shows this
-# gate catches it).
-GATE_C = 2.0 ** -18
-TINY = 2.0 ** -126
-
-
 def slices(n, cin, cout, h, w, s):
-    """Python mirror of C3Shape::slices() in csrc/gemm_tc.cu (wgrad_slices over the output pixels and Cout x Cin tiles
-    of 128, 9 taps); h x w is the input map."""
-    kb = n * (h // s) * (w // s) // 64
-    tiles = -(-cout // 128) * -(-cin // 128) * 9
-    sl = 1
-    while tiles * sl < 2 * 148 and kb % (2 * sl) == 0 and kb // (2 * sl) >= 16:
-        sl *= 2
-    return sl
+    """The number of K slices of the weight gradient: M = Cout over the output pixels, N = Cin, 9 taps; h x w is the
+    input map."""
+    return checks.wgrad_slices(n * (h // s) * (w // s), cout, cin, 9)
 
 
 # (C, input H = W, stride): every distinct 3x3 conv of ResNet-50/101/152 at 256 x 256 images (conv2 of each block;
@@ -56,12 +46,8 @@ TABLE = [
 ]
 
 WORST = {"y": 0.0, "dx": 0.0, "dw": 0.0}
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _report_worst():
-    yield
-    print(f"\nworst per-element error / m over {__name__}: " + ", ".join(f"{k} {v:.3e}" for k, v in WORST.items()))
+_report_worst = checks.report_worst(WORST, __name__)
+gate = functools.partial(checks.gate, worst=WORST)
 
 
 def inputs(n, cin, cout, h, w, s, seed=0, ex=0, ew=0, edy=0):
@@ -91,30 +77,6 @@ def reference(x, w, dy, s):
         dx64, dw64 = torch.autograd.grad(y64, (x64, w64), dy64)
         out.append((y64.detach(), dx64, dw64))
     return out
-
-
-def gate(name, got, ref, mag, max_gate=True, nonfinite=None):
-    """Per-element gate on every element finite in ref; every non-finite element of ref non-finite in got.
-    `nonfinite` (optional): where got may be non-finite although ref is not."""
-    got = got.detach().double()
-    assert got.shape == ref.shape, name
-    fin = torch.isfinite(ref)
-    assert not bool(torch.isfinite(got[~fin]).any()), f"{name}: finite where the reference is not"
-    if nonfinite is not None:
-        fin = fin & ~nonfinite
-    got, ref, mag = got[fin], ref[fin], mag[fin]
-    err = (got - ref).abs()
-    ok = err <= GATE_C * mag + TINY                        # NaN fails
-    if not bool(ok.all()):
-        i = int((~ok).nonzero()[0])
-        raise AssertionError(f"{name}: {int((~ok).sum())} of {ok.numel()} elements outside the per-element gate, "
-                             f"first: got {float(got[i])!r} ref {float(ref[i])!r} m {float(mag[i])!r}")
-    ratio = float(((err - TINY).clamp_min(0) / mag.clamp_min(1e-300)).max()) if err.numel() else 0.0
-    WORST[name] = max(WORST[name], ratio)
-    rel = float(err.max() / ref.abs().max().clamp_min(1e-300)) if err.numel() else 0.0
-    if max_gate:
-        assert rel <= GATE_MAX, (name, rel)
-    return ratio, rel
 
 
 def check_all(pkg, x, w, dy, s, label, max_gate=True):
@@ -162,42 +124,6 @@ def test_subnormal_input(cuda_pkg, n, cin, cout, h, w, s):
 
 
 # ---- memory contract of the C ABI: exact byte counts, guard bytes around every buffer, stale workspace contents ----
-GUARD = 4096
-SENTINEL = 0x5A
-
-
-class Region:
-    """`nbytes` inside a larger uint8 buffer: GUARD sentinel bytes on each side, the interior filled with `fill`
-    (a byte value, "random", or None for the sentinel)."""
-
-    def __init__(self, nbytes, fill=None, gen=None):
-        self.nbytes = nbytes
-        self.buf = torch.full((GUARD + nbytes + GUARD,), SENTINEL, dtype=torch.uint8, device="cuda")
-        if fill == "random":
-            self.inner.copy_(torch.randint(0, 256, (nbytes,), dtype=torch.uint8, device="cuda", generator=gen))
-        elif fill is not None:
-            self.inner.fill_(fill)
-        assert self.buf.data_ptr() % 256 == 0
-
-    @property
-    def inner(self):
-        return self.buf[GUARD:GUARD + self.nbytes]
-
-    def f32(self, shape):
-        return self.inner.view(torch.float32).view(shape)
-
-    def guards_intact(self):
-        return bool((self.buf[:GUARD] == SENTINEL).all()) and bool((self.buf[GUARD + self.nbytes:] == SENTINEL).all())
-
-
-def _f32_region(shape):
-    n = 1
-    for d in shape:
-        n *= d
-    r = Region(4 * n)
-    return r, r.f32(shape)
-
-
 def _abi_run(pkg, x, w, dy, s, fill, gen):
     """forward, then full, dx-only and dW-only backward through the C ABI, every buffer guarded."""
     L = pkg._lib.lib()
@@ -208,14 +134,14 @@ def _abi_run(pkg, x, w, dy, s, fill, gen):
     st = pkg._lib.current_stream_ptr()
     ptr = pkg._lib.ptr
     saved, ws = Region(sb.value, fill, gen), Region(wb.value, fill, gen)
-    ry, y = _f32_region((n, cout, h // s, wd // s))
+    ry, y = f32_region((n, cout, h // s, wd // s))
     pkg._lib.check(L.cdr_conv3x3_train_forward(ptr(x), ptr(w), n, cin, cout, h, wd, s, ptr(y), ptr(saved.inner),
                                                sb.value, ptr(ws.inner), wb.value, st))
     regions, outs = [saved, ws, ry], {"y": y}
     for tag, want in (("", "xw"), ("_xonly", "x"), ("_wonly", "w")):
         ws_b = Region(wb.value, fill, gen)
-        rdx, dx = _f32_region((n, cin, h, wd)) if "x" in want else (None, None)
-        rdw, dw = _f32_region((cout, cin, 3, 3)) if "w" in want else (None, None)
+        rdx, dx = f32_region((n, cin, h, wd)) if "x" in want else (None, None)
+        rdw, dw = f32_region((cout, cin, 3, 3)) if "w" in want else (None, None)
         pkg._lib.check(L.cdr_conv3x3_train_backward(ptr(saved.inner), ptr(w), ptr(dy), n, cin, cout, h, wd, s, ptr(dx),
                                                     ptr(dw), ptr(ws_b.inner), wb.value, st))
         regions += [r for r in (ws_b, rdx, rdw) if r is not None]
@@ -228,10 +154,6 @@ def _abi_run(pkg, x, w, dy, s, fill, gen):
     return {k: t.clone() for k, t in outs.items()}
 
 
-def _bits_equal(a, b):
-    return a.shape == b.shape and torch.equal(a.view(torch.int32), b.view(torch.int32))
-
-
 @pytest.mark.parametrize("n,cin,cout,h,w,s", [(1, 64, 64, 8, 8, 1), (3, 192, 64, 4, 16, 1), (2, 128, 192, 16, 16, 2),
                                               (3, 64, 128, 32, 32, 1)])
 def test_memory_contract(cuda_pkg, n, cin, cout, h, w, s):
@@ -239,11 +161,11 @@ def test_memory_contract(cuda_pkg, n, cin, cout, h, w, s):
     gen = torch.Generator(device="cuda").manual_seed(12)
     runs = [_abi_run(cuda_pkg, x, wt, dy, s, fill, gen) for fill in (0x00, 0xFF, "random")]
     for k in runs[0]:
-        assert all(_bits_equal(runs[0][k], r[k]) for r in runs[1:]), f"{k} depends on stale workspace contents"
+        assert all(bits_equal(runs[0][k], r[k]) for r in runs[1:]), f"{k} depends on stale workspace contents"
     a = runs[0]
-    assert _bits_equal(a["dx_xonly"], a["dx"]) and _bits_equal(a["dw_wonly"], a["dw"])
+    assert bits_equal(a["dx_xonly"], a["dx"]) and bits_equal(a["dw_wonly"], a["dw"])
     got = ours(cuda_pkg, x, wt, dy, s)                   # the autograd op is the same computation
-    assert all(_bits_equal(g, a[k]) for g, k in zip(got, ("y", "dx", "dw")))
+    assert all(bits_equal(g, a[k]) for g, k in zip(got, ("y", "dx", "dw")))
     ref, mag = reference(x, wt, dy, s)
     for i, k in enumerate(("y", "dx", "dw")):
         gate(k, a[k], ref[i], mag[i])
@@ -255,7 +177,7 @@ def test_needs_input_grad_each_alone(cuda_pkg, s):
     full = ours(cuda_pkg, x, w, dy, s)
     for i, need in enumerate(((True, False), (False, True))):
         (g,) = ours(cuda_pkg, x, w, dy, s, need)[1:]
-        assert _bits_equal(g, full[1 + i])
+        assert bits_equal(g, full[1 + i])
 
 
 # ---- layouts, streams, CUDA graphs, repeated backward ----
@@ -273,19 +195,15 @@ def test_layouts_give_the_same_bits(cuda_pkg, shape):
     assert not x_nc.is_contiguous()
     for xs, ws, dys in ((x_cl, w_cl, dy_cl), (x_nc, w, dy)):
         got = ours(cuda_pkg, xs, ws, dys, s)
-        assert all(_bits_equal(a.contiguous(), g.contiguous()) for a, g in zip(base, got))
+        assert all(bits_equal(a.contiguous(), g.contiguous()) for a, g in zip(base, got))
 
 
 @pytest.mark.parametrize("shape", LAYOUT_SHAPES)
 def test_side_stream_gives_the_same_bits(cuda_pkg, shape):
     x, w, dy, s = inputs(*shape, seed=22)
     base = ours(cuda_pkg, x, w, dy, s)
-    st = torch.cuda.Stream()
-    st.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(st):
-        got = ours(cuda_pkg, x, w, dy, s)
-    torch.cuda.current_stream().wait_stream(st)
-    assert all(_bits_equal(a, g) for a, g in zip(base, got))
+    got = on_side_stream(ours, cuda_pkg, x, w, dy, s)
+    assert all(bits_equal(a, g) for a, g in zip(base, got))
 
 
 @pytest.mark.parametrize("shape", LAYOUT_SHAPES)
@@ -296,21 +214,10 @@ def test_cuda_graph_replay_equals_eager(cuda_pkg, shape):
     def step():
         y = cuda_pkg.conv3x3(sx, sw, s)
         return (y.detach(), *torch.autograd.grad(y, (sx, sw), sdy))
-    st = torch.cuda.Stream()
-    st.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(st):
-        step()                                         # warm-up outside the capture
-    torch.cuda.current_stream().wait_stream(st)
-    g = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(g):
-        static_out = step()
     x2, w2, dy2, _ = inputs(*shape, seed=24)
-    with torch.no_grad():
-        sx.copy_(x2), sw.copy_(w2), sdy.copy_(dy2)
-    g.replay()
-    torch.cuda.synchronize()
+    static_out = graph_replay(step, (sx, sw, sdy), (x2, w2, dy2))
     eager = ours(cuda_pkg, x2, w2, dy2, s)
-    assert all(_bits_equal(a, e) for a, e in zip(static_out, eager))
+    assert all(bits_equal(a, e) for a, e in zip(static_out, eager))
 
 
 @pytest.mark.parametrize("shape", LAYOUT_SHAPES)
@@ -323,7 +230,7 @@ def test_two_backward_calls_and_zero_dy(cuda_pkg, shape):
     dy = torch.randn_like(y)
     first = torch.autograd.grad(y, (x, w), dy, retain_graph=True)
     second = torch.autograd.grad(y, (x, w), dy)
-    assert all(_bits_equal(a, c) for a, c in zip(first, second))
+    assert all(bits_equal(a, c) for a, c in zip(first, second))
 
 
 # ---- non-finite inputs: a diverging run is never reported finite ----

@@ -3,30 +3,21 @@ autograd with a per-element gate: padded M / N tiles, partial main-term chunks, 
 produces, exponents far outside O(1), the memory contract of the cdr_deconv_train_* entry points, layouts, streams,
 CUDA graphs and non-finite inputs.  test_gpu_deconv_train.py covers the three CDRNet decoder layers."""
 import ctypes as C
+import functools
 
 import pytest
 import torch
 import torch.nn.functional as F
 
-pytestmark = pytest.mark.gpu
+import train_conv_checks as checks
+from train_conv_checks import SENTINEL, Region, bits_equal, f32_region, graph_replay, on_side_stream
 
-GATE_MAX = 2e-5          # max error / max |reference| (test_gpu_deconv_train.py)
-# Per element: |got - ref| <= GATE_C * m + 2^-126, m = the same sum over |operands| (sum |x||w| for y, |dy||w| for dx,
-# |x||dy| for dW).  Measured on an NVIDIA B200 (1000 W power limit) over every case of this file: worst
-# (|err| - 2^-126) / m = 3.5e-7 for y, 2.2e-7 for dx, 3.3e-7 for dW, so 2^-18 = 3.8e-6 leaves a 10.9x margin.  Losing
-# the lo plane of an fp16 hi/lo operand costs ~2^-12 (test_deconv_train_host.py shows this gate catches it).
-GATE_C = 2.0 ** -18
-TINY = 2.0 ** -126       # the fp32 subnormal range: nothing below the smallest normal is resolved by an fp32 output
+pytestmark = pytest.mark.gpu
 
 
 def slices(n, cin, cout, h):
-    """Python mirror of DtShape::slices() in csrc/gemm_tc.cu: the number of K slices of the weight gradient."""
-    kb = n * h * h // 64
-    tiles = (cin // 64 + 1) // 2 * ((cout // 64 + 1) // 2) * 16
-    s = 1
-    while tiles * s < 2 * 148 and kb % (2 * s) == 0 and kb // (2 * s) >= 16:
-        s *= 2
-    return s
+    """The number of K slices of the weight gradient: M = Cin over the x pixels, N = Cout, 16 taps."""
+    return checks.wgrad_slices(n * h * h, cin, cout, 16)
 
 
 # (N, Cin, Cout, H, wgrad slices): padded N and M tiles (Cin or Cout % 128 == 64), partial kSplitChunk chunks (K-block
@@ -45,12 +36,8 @@ TABLE = [
 ]
 
 WORST = {"y": 0.0, "dx": 0.0, "dw": 0.0}     # largest (|got - ref| - 2^-126) / m seen by the gated tests, per pass
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _report_worst():
-    yield
-    print(f"\nworst per-element error / m over {__name__}: " + ", ".join(f"{k} {v:.3e}" for k, v in WORST.items()))
+_report_worst = checks.report_worst(WORST, __name__)
+gate = functools.partial(checks.gate, worst=WORST)
 
 
 def inputs(n, cin, cout, h, seed=0, ex=0, ew=0, edy=0):
@@ -79,28 +66,6 @@ def reference(x, w, dy):
         dx64, dw64 = torch.autograd.grad(y64, (x64, w64), f(dy.detach().double()))
         out.append((y64.detach(), dx64, dw64))
     return out
-
-
-def gate(name, got, ref, mag, max_gate=True):
-    """Assert the per-element gate on every element finite in ref, and that every non-finite element of ref is
-    non-finite in got.  Returns max (|err| - 2^-126) / m and max |err| / max |ref| over the finite elements."""
-    got = got.detach().double()
-    assert got.shape == ref.shape, name
-    fin = torch.isfinite(ref)
-    assert not bool(torch.isfinite(got[~fin]).any()), f"{name}: finite where the reference is not"
-    got, ref, mag = got[fin], ref[fin], mag[fin]
-    err = (got - ref).abs()
-    ok = err <= GATE_C * mag + TINY                        # NaN fails
-    if not bool(ok.all()):
-        i = int((~ok).nonzero()[0])
-        raise AssertionError(f"{name}: {int((~ok).sum())} of {ok.numel()} elements outside the per-element gate, "
-                             f"first: got {float(got[i])!r} ref {float(ref[i])!r} m {float(mag[i])!r}")
-    ratio = float(((err - TINY).clamp_min(0) / mag.clamp_min(1e-300)).max()) if err.numel() else 0.0
-    WORST[name] = max(WORST[name], ratio)
-    rel = float(err.max() / ref.abs().max().clamp_min(1e-300)) if err.numel() else 0.0
-    if max_gate:
-        assert rel <= GATE_MAX, (name, rel)
-    return ratio, rel
 
 
 def check_all(pkg, x, w, dy, label, max_gate=True):
@@ -141,42 +106,6 @@ def test_subnormal_input(cuda_pkg, n, cin, cout, h):
 
 
 # ---- memory contract of the C ABI: exact byte counts, guard bytes around every buffer, stale workspace contents ----
-GUARD = 4096             # bytes before and after every buffer; a multiple of 256 keeps the interior 256-byte aligned
-SENTINEL = 0x5A
-
-
-class Region:
-    """`nbytes` inside a larger uint8 buffer: GUARD sentinel bytes on each side, the interior filled with `fill`
-    (a byte value, "random", or None for the sentinel)."""
-
-    def __init__(self, nbytes, fill=None, gen=None):
-        self.nbytes = nbytes
-        self.buf = torch.full((GUARD + nbytes + GUARD,), SENTINEL, dtype=torch.uint8, device="cuda")
-        if fill == "random":
-            self.inner.copy_(torch.randint(0, 256, (nbytes,), dtype=torch.uint8, device="cuda", generator=gen))
-        elif fill is not None:
-            self.inner.fill_(fill)
-        assert self.buf.data_ptr() % 256 == 0
-
-    @property
-    def inner(self):
-        return self.buf[GUARD:GUARD + self.nbytes]
-
-    def f32(self, shape):
-        return self.inner.view(torch.float32).view(shape)
-
-    def guards_intact(self):
-        return bool((self.buf[:GUARD] == SENTINEL).all()) and bool((self.buf[GUARD + self.nbytes:] == SENTINEL).all())
-
-
-def _f32_region(shape):
-    n = 1
-    for d in shape:
-        n *= d
-    r = Region(4 * n)
-    return r, r.f32(shape)
-
-
 def _abi_run(pkg, x, w, dy, fill, gen):
     """forward, full backward, dx-only and dW-only backward through the C ABI, every buffer guarded."""
     L = pkg._lib.lib()
@@ -187,14 +116,14 @@ def _abi_run(pkg, x, w, dy, fill, gen):
     st = pkg._lib.current_stream_ptr()
     ptr = pkg._lib.ptr
     saved, ws = Region(sb.value, fill, gen), Region(wb.value, fill, gen)
-    ry, y = _f32_region((n, cout, 2 * h, 2 * h))
+    ry, y = f32_region((n, cout, 2 * h, 2 * h))
     pkg._lib.check(L.cdr_deconv_train_forward(ptr(x), ptr(w), n, cin, cout, h, h, ptr(y), ptr(saved.inner), sb.value,
                                               ptr(ws.inner), wb.value, st))
     regions, outs = [saved, ws, ry], {"y": y}
     for tag, want_dx, want_dw in (("", True, True), ("_xonly", True, False), ("_wonly", False, True)):
         ws_b = Region(wb.value, fill, gen)
-        rdx, dx = _f32_region((n, cin, h, h)) if want_dx else (None, None)
-        rdw, dw = _f32_region((cin, cout, 4, 4)) if want_dw else (None, None)
+        rdx, dx = f32_region((n, cin, h, h)) if want_dx else (None, None)
+        rdw, dw = f32_region((cin, cout, 4, 4)) if want_dw else (None, None)
         pkg._lib.check(L.cdr_deconv_train_backward(ptr(saved.inner), ptr(w), ptr(dy), n, cin, cout, h, h, ptr(dx),
                                                    ptr(dw), ptr(ws_b.inner), wb.value, st))
         regions += [r for r in (ws_b, rdx, rdw) if r is not None]
@@ -208,21 +137,17 @@ def _abi_run(pkg, x, w, dy, fill, gen):
     return {k: t.clone() for k, t in outs.items()}
 
 
-def _bits_equal(a, b):
-    return a.shape == b.shape and torch.equal(a.view(torch.int32), b.view(torch.int32))
-
-
 @pytest.mark.parametrize("n,cin,cout,h", [(1, 64, 64, 8), (5, 128, 192, 32), (3, 192, 320, 16)])
 def test_memory_contract(cuda_pkg, n, cin, cout, h):
     x, w, dy = inputs(n, cin, cout, h, seed=11)
     gen = torch.Generator(device="cuda").manual_seed(12)
     runs = [_abi_run(cuda_pkg, x, w, dy, fill, gen) for fill in (0x00, 0xFF, "random")]
     for k in runs[0]:
-        assert all(_bits_equal(runs[0][k], r[k]) for r in runs[1:]), f"{k} depends on stale workspace contents"
+        assert all(bits_equal(runs[0][k], r[k]) for r in runs[1:]), f"{k} depends on stale workspace contents"
     a = runs[0]
-    assert _bits_equal(a["dx_xonly"], a["dx"]) and _bits_equal(a["dw_wonly"], a["dw"])
+    assert bits_equal(a["dx_xonly"], a["dx"]) and bits_equal(a["dw_wonly"], a["dw"])
     y, dx, dw = ours(cuda_pkg, x, w, dy)                 # the autograd op is the same computation
-    assert _bits_equal(y, a["y"]) and _bits_equal(dx, a["dx"]) and _bits_equal(dw, a["dw"])
+    assert bits_equal(y, a["y"]) and bits_equal(dx, a["dx"]) and bits_equal(dw, a["dw"])
     (ry, rdx, rdw), (my, mdx, mdw) = reference(x, w, dy)
     gate("y", a["y"], ry, my), gate("dx", a["dx"], rdx, mdx), gate("dw", a["dw"], rdw, mdw)
 
@@ -238,20 +163,20 @@ def test_layouts_give_the_same_bits(cuda_pkg):
     x_cl, dy_cl = x.to(memory_format=torch.channels_last), dy.to(memory_format=torch.channels_last)
     w_nc = w.transpose(0, 1).contiguous().transpose(0, 1)          # (Cin, Cout, 4, 4) view with Cout outermost
     assert not x_cl.is_contiguous() and not dy_cl.is_contiguous() and not w_nc.is_contiguous()
-    got = ours(cuda_pkg, x_cl, w_nc, dy_cl)
-    assert all(_bits_equal(a.contiguous(), b.contiguous()) for a, b in zip(base, got))
+    # contiguous views 4 bytes past an aligned address, as x[1:] of a larger buffer gives
+    x_off, dy_off = (torch.empty(t.numel() + 1, device="cuda")[1:].view(t.shape).copy_(t) for t in (x, dy))
+    assert x_off.is_contiguous() and x_off.data_ptr() % 16 == 4 and dy_off.data_ptr() % 16 == 4
+    for xs, ws, dys in ((x_cl, w_nc, dy_cl), (x_off, w, dy_off)):
+        got = ours(cuda_pkg, xs, ws, dys)
+        assert all(bits_equal(a.contiguous(), b.contiguous()) for a, b in zip(base, got))
 
 
 def test_side_stream_gives_the_same_bits(cuda_pkg):
     n, cin, cout, h = LAYOUT_SHAPE
     x, w, dy = inputs(n, cin, cout, h, seed=22)
     base = ours(cuda_pkg, x, w, dy)
-    s = torch.cuda.Stream()
-    s.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(s):
-        got = ours(cuda_pkg, x, w, dy)
-    torch.cuda.current_stream().wait_stream(s)
-    assert all(_bits_equal(a, b) for a, b in zip(base, got))
+    got = on_side_stream(ours, cuda_pkg, x, w, dy)
+    assert all(bits_equal(a, b) for a, b in zip(base, got))
 
 
 def test_cuda_graph_replay_equals_eager(cuda_pkg):
@@ -262,21 +187,10 @@ def test_cuda_graph_replay_equals_eager(cuda_pkg):
     def step():
         y = cuda_pkg.conv_transpose2d(sx, sw)
         return (y.detach(), *torch.autograd.grad(y, (sx, sw), sdy))
-    s = torch.cuda.Stream()
-    s.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(s):
-        step()                                         # warm-up outside the capture
-    torch.cuda.current_stream().wait_stream(s)
-    g = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(g):
-        static_out = step()
     x2, w2, dy2 = inputs(n, cin, cout, h, seed=24)
-    with torch.no_grad():
-        sx.copy_(x2), sw.copy_(w2), sdy.copy_(dy2)
-    g.replay()
-    torch.cuda.synchronize()
+    static_out = graph_replay(step, (sx, sw, sdy), (x2, w2, dy2))
     eager = ours(cuda_pkg, x2, w2, dy2)
-    assert all(_bits_equal(a, b) for a, b in zip(static_out, eager))
+    assert all(bits_equal(a, b) for a, b in zip(static_out, eager))
 
 
 # ---- non-finite inputs: a diverging run is never reported finite ----
