@@ -15,9 +15,9 @@ from .encoder import ResNet
 from .graph import HeadGraph, HeadPipeline, FramePipeline
 from .geometry import baseline_keypoints, get_max_preds, projection_matrices, triangulation
 from .metrics import calc_mpjpe, mpjpe_sums
-from .autograd import soft_argmax_2d, dlt, ftl, conv_transpose2d, conv1x1, conv3x3
+from .autograd import soft_argmax_2d, dlt, ftl, conv_transpose2d, conv1x1, conv3x3, stem_conv, max_pool3x3
 from .losses import JointsMSELoss, JointsMSESmoothLoss, MPJPELoss, batch_norm_train
 
 __all__ = ["CDRNet", "CanonicalFusion", "PoseDecoder", "PoseResNet", "ResNet", "calc_mpjpe",
-           "mpjpe_sums", "HeadGraph", "HeadPipeline", "FramePipeline", "get_max_preds", "baseline_keypoints", "triangulation", "soft_argmax_2d", "dlt", "ftl", "conv_transpose2d", "conv1x1", "conv3x3", "JointsMSELoss", "JointsMSESmoothLoss", "MPJPELoss", "batch_norm_train", "build",
+           "mpjpe_sums", "HeadGraph", "HeadPipeline", "FramePipeline", "get_max_preds", "baseline_keypoints", "triangulation", "soft_argmax_2d", "dlt", "ftl", "conv_transpose2d", "conv1x1", "conv3x3", "stem_conv", "max_pool3x3", "JointsMSELoss", "JointsMSESmoothLoss", "MPJPELoss", "batch_norm_train", "build",
            "CdrError"]

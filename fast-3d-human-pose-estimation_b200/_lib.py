@@ -128,6 +128,11 @@ _SIGNATURES = {
     "cdr_conv3x3_train_workspace_bytes": (C.c_int, [C.c_int] * 6 + [C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
     "cdr_conv3x3_train_forward": (C.c_int, [_vp, _vp] + [C.c_int] * 6 + [_vp, _vp, C.c_size_t, _vp, C.c_size_t, _vp]),
     "cdr_conv3x3_train_backward": (C.c_int, [_vp, _vp, _vp] + [C.c_int] * 6 + [_vp, _vp, _vp, C.c_size_t, _vp]),
+    "cdr_stem_train_workspace_bytes": (C.c_int, [C.c_int] * 5 + [C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
+    "cdr_stem_train_forward": (C.c_int, [_vp, _vp] + [C.c_int] * 5 + [_vp, _vp, C.c_size_t, _vp, C.c_size_t, _vp]),
+    "cdr_stem_train_backward": (C.c_int, [_vp, _vp, _vp] + [C.c_int] * 5 + [_vp, _vp, _vp, C.c_size_t, _vp]),
+    "cdr_maxpool3x3_train_forward": (C.c_int, [_vp] + [C.c_int] * 4 + [_vp, _vp, _vp]),
+    "cdr_maxpool3x3_train_backward": (C.c_int, [_vp, _vp] + [C.c_int] * 4 + [_vp, _vp]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

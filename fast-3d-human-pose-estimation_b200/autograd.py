@@ -24,6 +24,12 @@ and so do the head's 1x1 convolutions (the fusion block's and ``decoder.final_la
 and so do the encoder's 3x3 convolutions, at stride 1 and 2:
 
     y = conv3x3(x, weight, stride)                    # == F.conv2d(x, weight, stride=stride, padding=1), no bias
+
+and the encoder's stem: its 7x7 convolution (forward and weight gradient; its input, the image batch, gets no gradient)
+and its max-pool (bit for bit torch's):
+
+    y = stem_conv(x, weight)                          # == F.conv2d(x, weight, stride=2, padding=3), no bias
+    p = max_pool3x3(y)                                # == F.max_pool2d(y, 3, stride=2, padding=1)
 """
 from __future__ import annotations
 
@@ -159,11 +165,13 @@ class _TrainConvOp:
     cin_dim: int         # the weight's Cin dimension: 0 for a transposed conv's (Cin, Cout, k, k), 1 for a conv's
     has_bias: bool
     out_hw: Callable     # (h, w, *extra int args) -> the output's (H, W)
+    data_grad: bool = True   # False: the op has no input gradient, and x must not require one
 
 
 _DECONV = _TrainConvOp("conv_transpose2d", "deconv", 4, 0, False, lambda h, w: (2 * h, 2 * w))
 _CONV1X1 = _TrainConvOp("conv1x1", "conv1x1", 1, 1, True, lambda h, w: (h, w))
 _CONV3X3 = _TrainConvOp("conv3x3", "conv3x3", 3, 1, False, lambda h, w, s: (h // s, w // s))
+_STEM = _TrainConvOp("stem_conv", "stem", 7, 1, False, lambda h, w: (h // 2, w // 2), data_grad=False)
 
 
 def _train_conv_args(op, x, weight, bias, extra):
@@ -173,6 +181,8 @@ def _train_conv_args(op, x, weight, bias, extra):
     ts = (x, weight) if bias is None else (x, weight, bias)
     if not all(isinstance(t, torch.Tensor) for t in ts):
         raise ValueError(f"{op.name}: x, weight and bias must be tensors")
+    if not op.data_grad and x.requires_grad:
+        raise ValueError(f"{op.name}: x requires grad, but the op has no input gradient (its input is the image batch)")
     if x.dim() != 4 or weight.dim() != 4 or tuple(weight.shape[2:]) != (op.k, op.k) or \
             weight.shape[op.cin_dim] != x.shape[1]:
         layout = "Cin, Cout" if op.cin_dim == 0 else "Cout, Cin"
@@ -199,7 +209,8 @@ def _train_conv_args(op, x, weight, bias, extra):
 
 
 class _TrainConv(torch.autograd.Function):
-    """conv_transpose2d, conv1x1 and conv3x3: forward and backward through the op's cdr_<lib>_train_* entry points.
+    """conv_transpose2d, conv1x1, conv3x3 and stem_conv: forward and backward through the op's cdr_<lib>_train_* entry
+    points.
     extra: the int arguments that follow (n, cin, cout, h, w) in them (conv3x3's stride)."""
 
     @staticmethod
@@ -265,3 +276,55 @@ def conv3x3(x, weight, stride=1):
     [64, 2048], H and W divisible by the stride, the output's width a power of two in [8, 64], its H*W 64 or a multiple
     of 128 and N*H*W <= 2^22; anything else raises ValueError."""
     return _TrainConv.apply(_CONV3X3, x, weight, None, stride)
+
+
+def stem_conv(x, weight):
+    """F.conv2d(x, weight, stride=2, padding=3) for the ResNet stem's (64, 3, 7, 7) weight without bias, forward and
+    weight gradient on libcdrhead at fp32 accuracy.  There is no input gradient: x is the image batch, and an x that
+    requires grad raises ValueError.  x (N, 3, H, W): CUDA float32, H % 16 == 0, W % 64 == 0, N*(H/2)*(W/2) <= 2^22;
+    anything else raises ValueError."""
+    return _TrainConv.apply(_STEM, x, weight, None)
+
+
+class _MaxPool3x3(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x):
+        if not isinstance(x, torch.Tensor) or x.dim() != 4:
+            raise ValueError("max_pool3x3: x (N, C, H, W) expected")
+        n, c, h, w = x.shape
+        if min(n, c, h, w) < 1 or n * c * h * w >= 1 << 31:
+            raise ValueError(f"max_pool3x3: unsupported shape {tuple(x.shape)} (every size >= 1, N*C*H*W < 2^31)")
+        if x.dtype != torch.float32:
+            raise ValueError(f"max_pool3x3: float32 expected, got {x.dtype}")
+        if not x.is_cuda:
+            raise ValueError("max_pool3x3: a CUDA tensor expected (there is no CPU fallback)")
+        x = x.contiguous()
+        ho, wo = (h - 1) // 2 + 1, (w - 1) // 2 + 1
+        y = torch.empty((n, c, ho, wo), dtype=torch.float32, device=x.device)
+        argmax = torch.empty((n, c, ho, wo), dtype=torch.uint8, device=x.device)    # window position ky * 3 + kx
+        with torch.cuda.device(x.device):
+            _lib.check(_lib.lib().cdr_maxpool3x3_train_forward(_lib.ptr(x), n, c, h, w, _lib.ptr(y), _lib.ptr(argmax),
+                                                               _lib.current_stream_ptr(x.device)))
+        ctx.save_for_backward(argmax)
+        ctx.in_shape = (n, c, h, w)
+        return y
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_y):
+        (argmax,) = ctx.saved_tensors
+        n, c, h, w = ctx.in_shape
+        dy = _chk(grad_y, "max_pool3x3: grad")
+        dx = torch.empty((n, c, h, w), dtype=torch.float32, device=dy.device)
+        with torch.cuda.device(dy.device):
+            _lib.check(_lib.lib().cdr_maxpool3x3_train_backward(_lib.ptr(argmax), _lib.ptr(dy), n, c, h, w, _lib.ptr(dx),
+                                                                _lib.current_stream_ptr(dy.device)))
+        return dx
+
+
+def max_pool3x3(x):
+    """F.max_pool2d(x, 3, stride=2, padding=1) on NCHW float32 CUDA tensors, forward and backward on libcdrhead, equal
+    to torch's CUDA kernels bit for bit (ties go to the first maximum in row-major order, a NaN wins).  Keeps one byte
+    per output for the backward instead of torch's int64 index.  Any N, C, H, W >= 1 with N*C*H*W < 2^31; anything else
+    raises ValueError."""
+    return _MaxPool3x3.apply(x)

@@ -25,6 +25,7 @@ training mode raises.  There is no CPU / PyTorch fallback.
 from __future__ import annotations
 
 import ctypes as C
+import functools
 import os
 
 import torch
@@ -291,16 +292,22 @@ class CDRNet(nn.Module):
     everywhere; 'fp32_ffma' = the same arithmetic on CUDA cores (cross-check); 'bf16' = bf16 operands on tcgen05."""
 
     def __init__(self, cfg, n_views=2, nj=19, fusion_in_dim=2048, fusion_hid_ch1=300,
-                 fusion_hid_ch2=400, precision="fp32", encoder_precision=None, trainable=False, train_encoder_on_library=False):
+                 fusion_hid_ch2=400, precision="fp32", encoder_precision=None, trainable=False, train_encoder_on_library=False,
+                 train_stem_on_library=False):
         """encoder_precision: 'fp32' — this library's tcgen05 encoder at the reference's precision (scaled fp16 hi/lo
         planes, 3 MMAs per product; needs precision='fp32'); 'torch' (default — the reference's nn.Module on torch/cuDNN, fp32) or
         'bf16' (Bottleneck stages on libcdrhead's tcgen05 kernels, stem on cuDNN bf16; SURVEY §8f).
         trainable: opt in to ``forward`` in training mode (``forward_train``, SURVEY §8f rank 3 slice).
         train_encoder_on_library: ``forward_train`` runs a Bottleneck encoder through ``ResNet.forward_train`` (its 1x1 /
-        3x3 convs and BatchNorms on libcdrhead at fp32 accuracy) instead of the torch modules (DESIGN.md §7)."""
+        3x3 convs and BatchNorms on libcdrhead at fp32 accuracy) instead of the torch modules (DESIGN.md §7).
+        train_stem_on_library: with ``train_encoder_on_library``, the encoder's stem (7x7 conv, BatchNorm + ReLU,
+        max-pool) trains on libcdrhead as well (``ResNet.forward_train(x, stem_on_library=True)``)."""
         super().__init__()
+        if train_stem_on_library and not train_encoder_on_library:
+            raise ValueError("train_stem_on_library=True needs train_encoder_on_library=True")
         self.trainable = bool(trainable)
         self.train_encoder_on_library = bool(train_encoder_on_library)
+        self.train_stem_on_library = bool(train_stem_on_library)
         encoder_precision = _default_encoder_precision(encoder_precision)
         if encoder_precision not in ("torch", "bf16", "fp32"):
             raise ValueError(f"encoder_precision must be 'torch', 'bf16' or 'fp32', got {encoder_precision!r}")
@@ -451,8 +458,10 @@ class CDRNet(nn.Module):
         encoder (ResNet-50/101/152) trains on the library as well (``ResNet.forward_train``): its 1x1 convs through
         ``conv1x1``, its 3x3 convs through ``conv3x3`` and its BatchNorms through ``batch_norm_train``, one call per view
         so that BatchNorm sees per-view batch statistics, as in the reference; otherwise the encoder runs on torch (cuDNN
-        + torch autograd).  The encoder's stem (7x7 conv, BatchNorm, ReLU, max-pool) and the optimizer always stay with
-        torch.  Needs ``CDRNet(..., trainable=True)``; projection matrices get no gradient (data in the reference)."""
+        + torch autograd).  The encoder's stem (7x7 conv, BatchNorm, ReLU, max-pool) stays with torch unless
+        ``train_stem_on_library=True``, which puts it on the library too (``stem_conv``, ``batch_norm_train``,
+        ``max_pool3x3``).  The optimizer always stays with torch.  Needs ``CDRNet(..., trainable=True)``; projection
+        matrices get no gradient (data in the reference)."""
         from .autograd import conv1x1, conv_transpose2d, dlt, ftl, soft_argmax_2d
         if not self.trainable:
             raise RuntimeError("forward_train needs CDRNet(..., trainable=True)")
@@ -475,6 +484,8 @@ class CDRNet(nn.Module):
             """transposed conv on libcdrhead -> train-mode BatchNorm + ReLU"""
             return batch_norm_train(conv_transpose2d(x, seq[0].weight), seq[1], relu=True)
         enc = self.encoder.forward_train if self.train_encoder_on_library else self.encoder
+        if self.train_stem_on_library:
+            enc = functools.partial(enc, stem_on_library=True)
         feats = [enc(xs[v]) for v in range(2)]                                # :231-234, one call per view
         cf = self.CF
         z = torch.cat([ftl(cbr(cf.conv_layer1, feats[v]), pinv[v]) for v in range(2)], dim=1)      # :62-70

@@ -694,28 +694,54 @@ static int conv3x3_train_shape(const char* fn, int n, int cin, int cout, int h, 
   return CDR_OK;
 }
 
+// The stem's 7x7 stride-2 pad-3 convolution (stem.cu).  h, w: the input images.
+static int stem_train_shape(const char* fn, int n, int cin, int cout, int h, int w) {
+  CDR_CHECK_ARG(n >= 1 && cin == 3 && cout == 64 && h >= 16 && w >= 64 && h % 16 == 0 && w % 64 == 0 &&
+                    (long long)n * (h / 2) * (w / 2) <= (1LL << 22),
+                "%s: unsupported shape n=%d cin=%d cout=%d h=%d w=%d (Cin = 3, Cout = 64, h %% 16 == 0, w %% 64 == 0, "
+                "n*(h/2)*(w/2) <= 2^22)", fn, n, cin, cout, h, w);
+  return CDR_OK;
+}
+
+static int train_null_args(const char* fn, std::initializer_list<const void*> need) {
+  for (const void* p : need) CDR_CHECK_ARG(p, "%s: null pointer", fn);
+  return CDR_OK;
+}
+// The tensors are 16-byte aligned (null allowed: an output not wanted), the bias 4-byte, saved and the workspace
+// 256-byte, and saved holds the forward's x planes (saved_bytes = SIZE_MAX: the backward, which has no size to check).
+static int train_buffer_args(const char* fn, std::initializer_list<const void*> tensors, const void* bias, bool bias_note,
+                             const void* saved, size_t saved_bytes, size_t saved_need, const void* workspace) {
+  bool aligned = ((uintptr_t)bias & 3) == 0 && ((uintptr_t)saved & 255) == 0 && ((uintptr_t)workspace & 255) == 0;
+  for (const void* p : tensors) aligned = aligned && ((uintptr_t)p & 15) == 0;
+  CDR_CHECK_ARG(aligned, "%s: tensors must be 16-byte%s, saved / workspace 256-byte aligned", fn,
+                bias_note ? " (bias 4-byte)" : "");
+  if (saved_bytes != SIZE_MAX && saved_bytes < saved_need) {
+    set_error("%s: saved %zu < required %zu bytes", fn, saved_bytes, saved_need);
+    return CDR_ERR_WORKSPACE;
+  }
+  return CDR_OK;
+}
+
 // What every cdr_<op>_train_* entry point checks, in this order: the pointers in `need` are not null, the shape is in
-// the op's domain, the tensors are 16-byte aligned (null allowed: an output not wanted), the bias 4-byte, saved and the
-// workspace 256-byte, and saved holds the forward's x planes (saved_bytes = SIZE_MAX: the backward, which has no size
-// to check).  On success *d describes the op.
+// the op's domain, then train_buffer_args.  On success *d describes the op.
 static int train_conv_args(const char* fn, int kind, int n, int cin, int cout, int h, int w, int stride,
                            std::initializer_list<const void*> need, std::initializer_list<const void*> tensors,
                            const void* bias, const void* saved, size_t saved_bytes, const void* workspace, TrainConv* d) {
-  for (const void* p : need) CDR_CHECK_ARG(p, "%s: null pointer", fn);
+  if (int rc = train_null_args(fn, need)) return rc;
   const int rc = kind == kTrainDeconv    ? deconv_train_shape(fn, n, cin, cout, h, w)
                  : kind == kTrainConv1x1 ? conv1x1_train_shape(fn, n, cin, cout, h, w)
                                          : conv3x3_train_shape(fn, n, cin, cout, h, w, stride);
   if (rc) return rc;
-  bool aligned = ((uintptr_t)bias & 3) == 0 && ((uintptr_t)saved & 255) == 0 && ((uintptr_t)workspace & 255) == 0;
-  for (const void* p : tensors) aligned = aligned && ((uintptr_t)p & 15) == 0;
-  CDR_CHECK_ARG(aligned, "%s: tensors must be 16-byte%s, saved / workspace 256-byte aligned", fn,
-                kind == kTrainConv1x1 ? " (bias 4-byte)" : "");
   *d = make_train_conv(kind, n, cin, cout, h, w, stride);
-  if (saved_bytes != SIZE_MAX && saved_bytes < train_conv_saved_bytes(*d)) {
-    set_error("%s: saved %zu < required %zu bytes", fn, saved_bytes, train_conv_saved_bytes(*d));
-    return CDR_ERR_WORKSPACE;
-  }
-  return CDR_OK;
+  return train_buffer_args(fn, tensors, bias, kind == kTrainConv1x1, saved, saved_bytes, train_conv_saved_bytes(*d),
+                           workspace);
+}
+static int stem_train_args(const char* fn, int n, int cin, int cout, int h, int w, std::initializer_list<const void*> need,
+                           std::initializer_list<const void*> tensors, const void* saved, size_t saved_bytes,
+                           const void* workspace) {
+  if (int rc = train_null_args(fn, need)) return rc;
+  if (int rc = stem_train_shape(fn, n, cin, cout, h, w)) return rc;
+  return train_buffer_args(fn, tensors, nullptr, false, saved, saved_bytes, stem_train_saved_bytes(n, h, w), workspace);
 }
 static int train_conv_sizes(const char* fn, int kind, int n, int cin, int cout, int h, int w, int stride,
                             size_t* saved_bytes, size_t* workspace_bytes) {
@@ -799,4 +825,54 @@ extern "C" int cdr_conv3x3_train_backward(const void* saved, const float* weight
                                           size_t workspace_bytes, void* stream) {
   return train_conv_backward("cdr_conv3x3_train_backward", kTrainConv3x3, saved, weight, dy, n, cin, cout, h, w, stride,
                              dx, dweight, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int cdr_stem_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes,
+                                              size_t* workspace_bytes) {
+  const char* fn = "cdr_stem_train_workspace_bytes";
+  if (int rc = stem_train_args(fn, n, cin, cout, h, w, {saved_bytes, workspace_bytes}, {}, nullptr, SIZE_MAX, nullptr))
+    return rc;
+  *saved_bytes = stem_train_saved_bytes(n, h, w);
+  *workspace_bytes = stem_train_workspace_bytes(n, h, w);
+  return CDR_OK;
+}
+extern "C" int cdr_stem_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, float* y,
+                                      void* saved, size_t saved_bytes, void* workspace, size_t workspace_bytes,
+                                      void* stream) {
+  const char* fn = "cdr_stem_train_forward";
+  if (int rc = stem_train_args(fn, n, cin, cout, h, w, {x, weight, y, saved, workspace}, {x, weight, y}, saved, saved_bytes,
+                               workspace))
+    return rc;
+  return launch_stem_train_forward(x, weight, n, h, w, y, saved, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+extern "C" int cdr_stem_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout,
+                                       int h, int w, float* dx, float* dweight, void* workspace, size_t workspace_bytes,
+                                       void* stream) {
+  const char* fn = "cdr_stem_train_backward";
+  CDR_CHECK_ARG(!dx, "%s: the stem has no input gradient (its input is the image batch): dx must be NULL", fn);
+  if (int rc = stem_train_args(fn, n, cin, cout, h, w, {saved, weight, dy, workspace}, {weight, dy, dweight}, saved,
+                               SIZE_MAX, workspace))
+    return rc;
+  return launch_stem_train_backward(saved, dy, n, h, w, dweight, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+// ------------------------------------------------------------------------------------------
+// The stem's 3x3 stride-2 pad-1 max-pool in training (stem.cu)
+static int maxpool3x3_train_args(const char* fn, const void* argmax, const float* a, const float* b, int n, int c, int h,
+                                 int w) {
+  if (int rc = train_null_args(fn, {argmax, a, b})) return rc;
+  CDR_CHECK_ARG(n >= 1 && c >= 1 && h >= 1 && w >= 1 && (long long)n * c * h * w < (1LL << 31),
+                "%s: unsupported shape n=%d c=%d h=%d w=%d (every size >= 1, n*c*h*w < 2^31)", fn, n, c, h, w);
+  CDR_CHECK_ARG(((uintptr_t)a & 3) == 0 && ((uintptr_t)b & 3) == 0, "%s: fp32 tensors must be 4-byte aligned", fn);
+  return CDR_OK;
+}
+extern "C" int cdr_maxpool3x3_train_forward(const float* x, int n, int c, int h, int w, float* y, uint8_t* argmax,
+                                            void* stream) {
+  if (int rc = maxpool3x3_train_args("cdr_maxpool3x3_train_forward", argmax, x, y, n, c, h, w)) return rc;
+  return launch_maxpool3x3_train_forward(x, n, c, h, w, y, argmax, (cudaStream_t)stream);
+}
+extern "C" int cdr_maxpool3x3_train_backward(const uint8_t* argmax, const float* dy, int n, int c, int h, int w, float* dx,
+                                             void* stream) {
+  if (int rc = maxpool3x3_train_args("cdr_maxpool3x3_train_backward", argmax, dy, dx, n, c, h, w)) return rc;
+  return launch_maxpool3x3_train_backward(argmax, dy, n, c, h, w, dx, (cudaStream_t)stream);
 }

@@ -2720,6 +2720,14 @@ wgrad_reduce_kernel(const float* __restrict__ part, int slices, int taps, int ro
   for (int sl = 0; sl < slices; ++sl) s += __ldcg(part + (((size_t)sl * taps + t) * rows + row) * ldc + c);
   dw[idx] = s * ix * id;
 }
+int launch_wgrad_reduce(const float* part, int slices, int taps, int rows, int cols, int ldc, const float* sx,
+                        const float* sdy, float* dw, cudaStream_t st) {
+  const long long total = (long long)rows * cols * taps;
+  wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(part, slices, taps, rows, cols, ldc, sx,
+                                                                                 sdy, dw);
+  CDR_LAUNCH_OK("wgrad_reduce_kernel");
+  return CDR_OK;
+}
 
 // The kMN GEMM over n*h*w pixels split into `slices` K slices: part[slice * taps + tap] (m rows, pitch round_up(nb, 128))
 // = A^T B.  A: m channels of a pixel-major fp16 planes buffer (pitch a_pitch), scale slot `sa`.  B: nb channels (pitch
@@ -2828,10 +2836,9 @@ int tc_train_conv_backward(const TrainConv& d, const void* saved, const float* w
       if (int rc = launch_wgrad(d.n, a.h, a.w, ax ? xa : dya, a.c, a.pitch, ax ? sx : sd, ax ? dya : xa, b.c, b.pitch,
                                 d.b_k, d.b_stride, d.slices, ws.part, st))
         return rc;
-      const long long total = (long long)a.c * b.c * d.b_k * d.b_k;
-      wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(
-          ws.part, d.slices, d.b_k * d.b_k, a.c, b.c, round_up(b.c, 128), sx.scale, sd.scale, dw);
-      CDR_LAUNCH_OK("wgrad_reduce_kernel");
+      if (int rc = launch_wgrad_reduce(ws.part, d.slices, d.b_k * d.b_k, a.c, b.c, round_up(b.c, 128), sx.scale, sd.scale,
+                                       dw, st))
+        return rc;
     }
   }
   set_stage(nullptr);

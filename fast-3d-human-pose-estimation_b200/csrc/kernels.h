@@ -85,6 +85,21 @@ int launch_pack_stem_f16x2(const CdrConvBn& s, void* w, float* bias, cudaStream_
 size_t stem_weight_bytes_f16x2();
 int launch_stem_f32(const void* x, int is_u8, const float* mean, const float* std, int n, int H, int W, const void* w,
                     const float* bias, float* conv_out, void* pooled_hi, void* pooled_lo, float* slot, cudaStream_t st);
+// training (include/cdrhead.h: cdr_stem_train_*, cdr_maxpool3x3_train_*); the shape must be in the op's domain
+size_t stem_train_saved_bytes(int n, int H, int W);
+size_t stem_train_workspace_bytes(int n, int H, int W);
+int stem_train_slices(int n, int H, int W);
+int launch_stem_train_forward(const float* x, const float* weight, int n, int H, int W, float* y, void* saved,
+                              void* workspace, size_t workspace_bytes, cudaStream_t st);
+int launch_stem_train_backward(const void* saved, const float* dy, int n, int H, int W, float* dweight, void* workspace,
+                               size_t workspace_bytes, cudaStream_t st);
+int launch_maxpool3x3_train_forward(const float* x, int n, int c, int H, int W, float* y, uint8_t* argmax, cudaStream_t st);
+int launch_maxpool3x3_train_backward(const uint8_t* argmax, const float* dy, int n, int c, int H, int W, float* dx,
+                                     cudaStream_t st);
+
+// gemm_tc.cu: dw[r][c][tap] = (sum over slices, in order, of part[slice][tap][r][c]) / (*sx * *sdy), part rows ldc apart
+int launch_wgrad_reduce(const float* part, int slices, int taps, int rows, int cols, int ldc, const float* sx,
+                        const float* sdy, float* dw, cudaStream_t st);
 
 // train_ops.cu: BatchNorm2d in training mode (+ optional fused ReLU) and the reference's three losses, forward / backward
 int launch_bn_train_forward(const float* x, int n, int c, int hw, const float* gamma, const float* beta, double eps,

@@ -15,7 +15,7 @@ from torch import nn
 
 # bound once, at import: the encoder's training forward does not follow a later rebinding of ``autograd.conv1x1`` (the
 # head's training-step tests swap that name for cuDNN's to compare the head's 1x1 convs alone)
-from .autograd import conv1x1 as _conv1x1, conv3x3 as _conv3x3
+from .autograd import conv1x1 as _conv1x1, conv3x3 as _conv3x3, max_pool3x3 as _max_pool3x3, stem_conv as _stem_conv
 
 _SPEC = {18: ("basic", (2, 2, 2, 2)), 34: ("basic", (3, 4, 6, 3)),
          50: ("bottleneck", (3, 4, 6, 3)), 101: ("bottleneck", (3, 4, 23, 3)),
@@ -89,17 +89,23 @@ class ResNet(nn.Module):
         x = self.maxpool(self.relu(self.bn1(self.conv1(x))))
         return self.layer4(self.layer3(self.layer2(self.layer1(x))))
 
-    def forward_train(self, x):
+    def forward_train(self, x, stem_on_library=False):
         """``forward`` in training mode with every Bottleneck block on libcdrhead, forward and backward at fp32 accuracy
         whatever torch's TF32 flags say: conv1 / conv3 and the downsample conv (on the stride-2 slice, an exact identity
         for a 1x1 conv) through ``conv1x1``, conv2 through ``conv3x3``, every BatchNorm through ``batch_norm_train``
         (batch statistics and the running-stat update, as nn.BatchNorm2d in training mode).  The stem (7x7 conv over 3
-        channels, BatchNorm, ReLU, max-pool) stays on torch.  The library's shape limits apply: at N images per call,
-        256 x 256 inputs are inside them for every N up to 64.  ``CDRNet(..., train_encoder_on_library=True)``
-        calls it for each view from ``forward_train``."""
+        channels, BatchNorm, ReLU, max-pool) stays on torch unless ``stem_on_library=True``: then its conv runs through
+        ``stem_conv`` (fp32 accuracy, forward and weight gradient; x, the image batch, gets no gradient), its BatchNorm
+        + ReLU through ``batch_norm_train`` and its max-pool through ``max_pool3x3`` (torch's bits).  The library's shape
+        limits apply: at N images per call, 256 x 256 inputs are inside them for every N up to 64.
+        ``CDRNet(..., train_encoder_on_library=True)`` calls it for each view from ``forward_train``."""
         if self.kind != "bottleneck":
             raise ValueError("ResNet.forward_train: only Bottleneck encoders (ResNet-50/101/152) train on the library")
-        x = self.maxpool(self.relu(self.bn1(self.conv1(x))))
+        from .losses import batch_norm_train
+        if stem_on_library:
+            x = _max_pool3x3(batch_norm_train(_stem_conv(x, self.conv1.weight), self.bn1, relu=True))
+        else:
+            x = self.maxpool(self.relu(self.bn1(self.conv1(x))))
         for layer in (self.layer1, self.layer2, self.layer3, self.layer4):
             for b in layer:
                 x = _bottleneck_train(b, x)

@@ -379,6 +379,29 @@ int cdr_conv3x3_train_backward(const void* saved, const float* weight, const flo
                                int w, int stride, float* dx, float* dweight, void* workspace, size_t workspace_bytes,
                                void* stream);
 
+/* ---- Training the encoder's stem convolution: Conv2d(3, 64, 7, stride 2, padding 3, bias=False) at fp32 accuracy on
+ * warp-level tensor-core MMAs (scaled fp16 hi/lo operands, 3 MMAs per product), forward and weight gradient.
+ * x (n, 3, h, w), weight (64, 3, 7, 7), y / dy (n, 64, h/2, w/2), all fp32 NCHW, 16-byte aligned.
+ * Supported: cin = 3, cout = 64, h % 16 == 0, w % 64 == 0, n*(h/2)*(w/2) <= 2^22 (CDR_ERR_INVALID otherwise).
+ * There is NO input gradient: the stem's input is the image batch.  The backward returns CDR_ERR_INVALID unless dx is
+ * NULL; a NULL dweight makes it a no-op.  `saved` and the workspace work as for cdr_deconv_train_*.  dweight is bitwise
+ * deterministic (fixed-order reduction of its K slices, no atomics). */
+int cdr_stem_train_workspace_bytes(int n, int cin, int cout, int h, int w, size_t* saved_bytes, size_t* workspace_bytes);
+int cdr_stem_train_forward(const float* x, const float* weight, int n, int cin, int cout, int h, int w, float* y,
+                           void* saved, size_t saved_bytes, void* workspace, size_t workspace_bytes, void* stream);
+int cdr_stem_train_backward(const void* saved, const float* weight, const float* dy, int n, int cin, int cout, int h,
+                            int w, float* dx, float* dweight, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- The stem's max-pool in training: MaxPool2d(3, stride 2, padding 1) on x (n, c, h, w) fp32 NCHW -> y (n, c, ho, wo),
+ * ho = (h - 1) / 2 + 1, wo = (w - 1) / 2 + 1, equal to torch's CUDA kernel bit for bit, forward and backward.  The window
+ * is scanned in row-major order from its first in-image element; an element replaces the maximum when it is larger or
+ * NaN.  The forward writes y and `argmax`, n*c*ho*wo bytes: per output its window position ky*3 + kx.  The backward
+ * writes dx (n, c, h, w): per input element the sum, from +0.0 in (oy, ox) order, of the dy of the windows whose argmax
+ * it is.  Supported: every size >= 1, n*c*h*w < 2^31; fp32 tensors 4-byte aligned (CDR_ERR_INVALID otherwise). */
+int cdr_maxpool3x3_train_forward(const float* x, int n, int c, int h, int w, float* y, uint8_t* argmax, void* stream);
+int cdr_maxpool3x3_train_backward(const uint8_t* argmax, const float* dy, int n, int c, int h, int w, float* dx,
+                                  void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
